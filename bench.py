@@ -34,6 +34,12 @@ synth_encoder.cpp); the reference's own encoder is non-functional.
 With torchrun (N > 1) every rank drives its own GPU on its own images (weak scaling, no collective in
 the data path; torch.distributed is used only for the barrier, the max-over-ranks of the times and -- untimed
 set-up of the tiles leg -- handing the encoded 16k image from rank 0 to the others).
+
+  --dump-outputs DIR : after the timed steps, the RGB pixels the last timed step wrote, as float32: DIR/pixels.npy
+           [rows, width, 3] holds a fixed, seeded sample of whole image rows (all of them when they fit in 56 MB) and
+           DIR/pixels_rows.npy [rows, 2] float64 the (image, row) of each; with N > 1 every rank writes its own pair
+           (pixels_rank<r>.npy, pixels_rank<r>_rows.npy).  The inputs depend on the arguments only, so two builds run
+           with the same arguments can be compared file for file.
 """
 from __future__ import annotations
 
@@ -61,6 +67,7 @@ W4K, H4K, Q4K = 3840, 2160, 95
 WORKLOAD = "synthetic 3840x2160 RGB 4:4:4 baseline q=95, no restart markers (BASELINE.json configs[2])"
 SEED0 = 0x6B706567
 REF_SAMPLE_WH = 512
+DUMP_PIXEL_BYTES = 56 << 20  # the pixel sample of --dump-outputs; with its row index and headers it stays under 64 MB
 
 
 def env_int(name, default):
@@ -501,6 +508,20 @@ def leg_tiles(dec, K, rank, world, dist, device, torch, quick):
 
 
 # ---- CUDA arm -----------------------------------------------------------------------------------------
+def dump_pixels(out_dir, name, pixels):
+    """pixels [N, H, W, C] uint8 -> out_dir/<name>.npy [R, W, C] float32, R whole rows drawn with a fixed seed (every row
+    when all fit in DUMP_PIXEL_BYTES, in order), and out_dir/<name>_rows.npy [R, 2] float64: (image, row) of each."""
+    n, h, w, c = pixels.shape
+    # a JPEG is at most 65535 samples wide, so one float32 RGB row stays under 1 MB and at least one row fits
+    assert w * c * 4 <= DUMP_PIXEL_BYTES, f"a {w}-pixel row does not fit the dump budget"
+    rows_all = pixels.reshape(n * h, w, c)
+    r = min(n * h, DUMP_PIXEL_BYTES // (w * c * 4))
+    pick = np.arange(n * h) if r == n * h else np.sort(np.random.default_rng(SEED0).choice(n * h, size=r, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, f"{name}.npy"), rows_all[pick].astype(np.float32))
+    np.save(os.path.join(out_dir, f"{name}_rows.npy"), np.stack([pick // h, pick % h], axis=1).astype(np.float64))
+
+
 def run_cuda_arm(args):
     import torch
 
@@ -612,6 +633,12 @@ def run_cuda_arm(args):
     # take the larger of the event time and the host wall clock around the same region
     dev_ms = max(ev0.elapsed_time(ev1), t_wall * 1e3)
     clocks = sampler.stop()
+    if args.dump_outputs:
+        # read back now: the legs below write into the same output buffers
+        last = np.empty((NB, Hh, W, 3), dtype=np.uint8)
+        dec.d2h(last, d_out if args.sync_steps else d_outs[(args.steps - 1) & 1])
+        dump_pixels(args.dump_outputs, "pixels" if world == 1 else f"pixels_rank{rank}", last)
+        del last
 
     # ---- sustained: the same steps until at least 2 s have passed (chunks of 256 steps, one wait per chunk) ----
     sustained = None
@@ -851,7 +878,13 @@ def main():
     ap.add_argument("--quick", action="store_true", help="development runs: parity gate on one image, no sustained leg, small extra legs")
     ap.add_argument("--no-extras", action="store_true", help="skip the gray-batch and 16k-tiles legs")
     ap.add_argument("--sustain-s", type=float, default=2.0)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write a seeded sample of the pixels of the last timed step to "
+                                                          "DIR/*.npy (float32, under 64 MB; CUDA arm only)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "cuda":
+        ap.error("--dump-outputs applies to the CUDA arm")
     # stdout carries exactly ONE JSON line: whatever libraries write to file descriptor 1 (NCCL's version
     # banner, for one) is sent to stderr, and Python's own stdout keeps the original descriptor
     sys.stdout.flush()

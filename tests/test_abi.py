@@ -34,10 +34,10 @@ def test_synth_library_exports():
         assert hasattr(lib, n)
 
 
-def test_struct_layouts_match_the_header():
+def test_struct_layouts_match_the_header(tmp_path):
     """sizeof(kpeg_plan) / sizeof(kpeg_stats) as the C compiler sees them == the ctypes mirrors."""
     src = '#include <stdio.h>\n#include "kpeg_cuda.h"\nint main(){printf("%zu %zu %d\\n", sizeof(kpeg_plan), sizeof(kpeg_stats), KPEG_T_COUNT);return 0;}\n'
-    exe = Path("/tmp/kpeg_sizeof")
+    exe = tmp_path / "kpeg_sizeof"
     subprocess.run(["gcc", "-x", "c", "-", f"-I{ROOT / 'include'}", "-o", str(exe)], input=src.encode(), check=True)
     a, b, c = map(int, subprocess.run([str(exe)], capture_output=True, text=True, check=True).stdout.split())
     assert a == C.sizeof(api.Plan) and b == C.sizeof(api.Stats) and c == len(api.Stats.STAGES)

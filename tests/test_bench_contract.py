@@ -28,6 +28,32 @@ def test_reference_arm_prints_one_contract_line():
     assert d["gpu_launches"] == 0 and "workload" in d["config"]
 
 
+def test_dump_pixels_rows_and_budget(tmp_path, monkeypatch):
+    """--dump-outputs: whole rows as float32 with their (image, row); all rows when they fit, else the same seeded sample
+    on every call, within the byte budget."""
+    import numpy as np
+    import bench
+    px = np.random.default_rng(1).integers(0, 256, size=(3, 10, 7, 3), dtype=np.uint8)
+    bench.dump_pixels(str(tmp_path / "all"), "pixels", px)
+    got, idx = np.load(tmp_path / "all" / "pixels.npy"), np.load(tmp_path / "all" / "pixels_rows.npy")
+    assert got.dtype == np.float32 and idx.dtype == np.float64
+    assert np.array_equal(got, px.reshape(30, 7, 3)) and np.array_equal(idx[:, 0] * 10 + idx[:, 1], np.arange(30))
+    monkeypatch.setattr(bench, "DUMP_PIXEL_BYTES", 8 * 7 * 3 * 4)
+    for d in ("a", "b"):
+        bench.dump_pixels(str(tmp_path / d), "pixels", px)
+    got, idx = np.load(tmp_path / "a" / "pixels.npy"), np.load(tmp_path / "a" / "pixels_rows.npy").astype(int)
+    assert got.shape == (8, 7, 3) and got.nbytes <= bench.DUMP_PIXEL_BYTES
+    assert np.array_equal(got, px[idx[:, 0], idx[:, 1]]) and (np.diff(idx[:, 0] * 10 + idx[:, 1]) > 0).all()
+    assert np.array_equal(got, np.load(tmp_path / "b" / "pixels.npy"))
+
+
+def test_dump_outputs_and_steps_are_checked():
+    r = _run(["--impl", "reference", "--steps", "1", "--dump-outputs", "x"], timeout=120)
+    assert r.returncode != 0 and "--dump-outputs" in r.stderr
+    r = _run(["--steps", "0"], timeout=120)
+    assert r.returncode != 0 and "--steps" in r.stderr
+
+
 def test_cuda_arm_fails_loudly_without_a_device():
     import torch
     if torch.cuda.is_available():
