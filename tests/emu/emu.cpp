@@ -423,6 +423,38 @@ float emu_idct_fast(const int16_t zzc[64], const uint16_t qt[64], float out[64])
     return tie_band((float)A);
 }
 
+// Fast-path IDCT of one block as K3 sets it up (k3_fused.cu dequant_dezigzag): the prescaled quantisers of
+// host_tables.h, and A accumulated in fp32 the way the kernel does it -- |prescaled coefficient| * aan_unscale, pair
+// order, four partial sums for the AC terms, the DC term apart.  out[64] = fast samples (unshifted, natural order),
+// *a_out = that A; returns the tie band the kernel derives from it.
+float emu_idct_fast_k3(const int16_t zzc[64], const uint16_t qt[64], float out[64], float *a_out)
+{
+    static const ZigZagTables zz = make_zigzag_tables();
+    float qscale[64], fb[64];
+    for (int i = 0; i < 64; ++i) {
+        const int nat = zz.zz2nat[i];
+        const double s = aan_scale(nat >> 3) * aan_scale(nat & 7) / 8.0;
+        qscale[i] = (float)((double)qt[i] * s);
+        fb[nat] = (float)zzc[i] * qscale[i];
+    }
+    float A[4] = {0.0f, 0.0f, 0.0f, 0.0f}, dcterm = 0.0f;
+    for (int p = 0; p < 32; ++p)
+        for (int h = 0; h < 2; ++h) {
+            const int n = pair_nat(p, h);
+            const float f = fb[n]; // (float)c * qpair: the same product as the kernel's packed multiply
+            if (n == 0)
+                dcterm = fabsf(f) * aan_unscale(n);
+            else
+                A[2 * h + (p & 1)] = fmaf(fabsf(f), aan_unscale(n), A[2 * h + (p & 1)]);
+        }
+    const float a = ((A[0] + A[1]) + (A[2] + A[3])) + dcterm;
+    idct8x8_fast(fb);
+    for (int s = 0; s < 64; ++s)
+        out[s] = fb[s];
+    *a_out = a;
+    return tie_band(a);
+}
+
 // Huffman LUT lookup of a left-aligned 32-bit window: returns the packed entry.
 // mode 0: as the kernels do it (fast / long table / canonical); mode 1: canonical search only.
 uint32_t emu_huff_lookup(const uint8_t counts[16], const uint8_t *symbols, int is_ac, uint32_t win, int mode)
