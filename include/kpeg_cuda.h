@@ -1,5 +1,5 @@
 /*
- * kpeg_cuda.h -- C ABI of the B200 (sm_100a) baseline-JPEG decode hot path.
+ * kpeg_cuda.h -- C ABI of the B200 (sm_100a) baseline-JPEG decode hot path, and of the GPU encoder (at the end).
  *
  * libKPEG has no plugin / FFI interface of its own: its hot path is reachable only through the
  * C++ class kpeg::JPEGDecoder (reference include/Decoder.hpp:26-128) and the `kpeg` CLI
@@ -295,6 +295,52 @@ int kpeg_cuda_interleaved_to_planar(kpeg_ctx *ctx, const uint8_t *d_rgb, uint8_t
 
 /* Exact bytes of the PPM header Image::dumpRawData writes (Image.cpp:124-127); returns length. */
 int kpeg_ppm_header(int width, int height, char *buf, size_t cap);
+
+/* ---- encode: pixels -> baseline JPEG on the GPU (csrc/encode.cu) ----------------------------------------------
+ * Baseline sequential, 8-bit, one component or three (4:4:4, JFIF YCbCr), ITU-T T.81 Annex K quantisation tables
+ * scaled by the IJG quality rule, Annex K Huffman tables, optional restart interval (DRI + RSTn).  The file is byte
+ * for byte what the synthetic reference encoder writes for the same pixels (kpeg_synth_encode_pixels,
+ * include/kpeg_synth.h, with KPEG_SYNTH_QUIRK_FREE when flags has KPEG_FLAG_REF_PARITY, and KPEG_SYNTH_EMIT_RESTART
+ * when restart_interval > 0): segments in lena's order, double-precision colour transform and FDCT, lround(s / q)
+ * clamped to +-2047 (DC) / +-1023 (AC), edges replicated to whole blocks, 1-bit padding before every marker.
+ * KPEG_FLAG_REF_PARITY nudges DC values (by at most 2) so that no block has a DC difference of 0 and AC terms: the
+ * reference decoder drops the AC terms of such blocks (SURVEY F1), so only such a stream decodes to the same pixels
+ * in both decode modes and in the reference.  Without it the quantisation is plain T.81. */
+typedef struct kpeg_encode_params {
+    uint16_t width, height;     /* 1..65535 */
+    uint8_t ncomp;              /* 1 (gray) or 3 (interleaved R,G,B in; Y,Cb,Cr coded) */
+    uint8_t quality;            /* IJG 1..100, Annex K tables */
+    uint16_t restart_interval;  /* MCUs, 0 = none (no DRI) */
+    uint32_t flags;             /* KPEG_FLAG_REF_PARITY: stream safe for the reference's DC rule (SURVEY F1) */
+} kpeg_encode_params;
+
+/* Host only: the largest file kpeg_cuda_encode can write for these parameters (0 for bad parameters).
+ * Per block at most 22 DC bits + 63 x 26 AC bits = 1660 bits:
+ *  - DC: an 8-bit block's DC coefficient is (1/8) * the sum of its 64 level-shifted samples, in [-1024, 1016] for Y and
+ *    [-1020, 1020] for Cb / Cr even with quantiser 1, and the nudge moves it by 1 at most when only the previous
+ *    value is excluded (0 is excluded only at a segment's first MCU, where the prediction is 0 and |diff| <= 1025):
+ *    |difference| <= 1017 + 1025 = 2042 < 2048, category <= 11; the longest Annex K DC code of category 11 is the
+ *    chroma one, 11 bits: 11 + 11 = 22 bits.
+ *  - AC: every coefficient is clamped to +-1023, category <= 10, and the longest Annex K AC code is 16 bits: a non-zero
+ *    coefficient costs <= 26 bits; a ZRL (<= 11 bits) stands for 16 positions and EOB (<= 4 bits) for at least one, so
+ *    no position costs more than 26 bits: 63 x 26.
+ * Segments are padded to whole bytes (one byte each at most), every byte may be FF and be followed by a stuffed 00
+ * (x 2), and there is one 2-byte RSTn between segments and the 2-byte EOI: bound = header + 2 * (ceil(blocks * 1660 / 8)
+ * + segments) + 2 * segments. */
+size_t kpeg_encode_bound(const kpeg_encode_params *p);
+/* Encode host pixels ([height][width][ncomp], top-down) into the host buffer jpeg_out.  Synchronous.  When the file
+ * is larger than cap: KPEG_ERR_NOMEM, *jpeg_len = the size it needs, nothing written to jpeg_out.  Bad parameters or
+ * NULL pointers: KPEG_ERR_ARG (checked before the context is used).  stats: width/height/ncomp, scan_bytes (stuffed
+ * scan bytes written), unstuffed_bytes, segments, kernel_launches; with profiling on, ms_total and the stage times:
+ * ms[KPEG_T_H2D] / ms[KPEG_T_D2H] the copies, ms[KPEG_T_IDCT] the FDCT + quantisation, ms[KPEG_T_DC_SCAN] the DC nudge,
+ * ms[KPEG_T_ENTROPY_WRITE] bit lengths, offsets and code emission, ms[KPEG_T_UNSTUFF] byte stuffing and markers. */
+int kpeg_cuda_encode(kpeg_ctx *ctx, const kpeg_encode_params *p, const uint8_t *pixels, uint8_t *jpeg_out, size_t cap,
+                     size_t *jpeg_len, kpeg_stats *stats);
+/* Same with DEVICE buffers on the context's device: the file is assembled in d_out (header copied in, the scan written
+ * right after it by the kernels).  When it is larger than cap: KPEG_ERR_NOMEM, *jpeg_len = the size it needs, and no
+ * byte at or past d_out + cap has been written. */
+int kpeg_cuda_encode_device(kpeg_ctx *ctx, const kpeg_encode_params *p, const uint8_t *d_pixels, uint8_t *d_out, size_t cap,
+                            size_t *jpeg_len, kpeg_stats *stats);
 
 #ifdef __cplusplus
 }

@@ -49,6 +49,13 @@ typedef struct kpeg_synth_params {
 int kpeg_synth_encode(const kpeg_synth_params *p, uint8_t **out, size_t *out_len);
 void kpeg_synth_free(uint8_t *buf);
 
+/* The same encoder over caller-supplied pixels: [height][width][file_components==1 or GRAY_CONTENT ? 1 : 3]
+ * (interleaved R,G,B).  Uses width, height, file_components, quality, restart_interval, flags and threads; ignores
+ * seed and noise_amp.  kpeg_synth_encode(p) == kpeg_synth_encode_pixels(p, kpeg_synth_pixels(p)) byte for byte.
+ * With flags KPEG_SYNTH_QUIRK_FREE (or 0), plus KPEG_SYNTH_EMIT_RESTART when restart_interval > 0, this is the exact
+ * file the GPU encoder (kpeg_cuda_encode, include/kpeg_cuda.h) writes with KPEG_FLAG_REF_PARITY (or 0). */
+int kpeg_synth_encode_pixels(const kpeg_synth_params *p, const uint8_t *pixels, uint8_t **out, size_t *out_len);
+
 /* The source pixels the encoder compressed (before the lossy steps), for PSNR reporting.
  * dst is [height][width][file_components==1 or GRAY_CONTENT ? 1 : 3]. */
 int kpeg_synth_pixels(const kpeg_synth_params *p, uint8_t *dst);

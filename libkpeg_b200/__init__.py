@@ -9,10 +9,12 @@ raises when that library or a GPU is missing.
 from .api import (  # noqa: F401
     KPEG_FLAG_REF_PARITY,
     Decoder,
+    EncodeParams,
     KpegError,
     Plan,
     Stats,
     load_cuda_library,
+    encode_bound,
     parse_jfif,
     ppm_header,
 )

@@ -44,6 +44,18 @@ def build_emu() -> None:
           "-Wno-unknown-pragmas", f"-I{ROOT / 'include'}", f"-I{PKG / 'csrc'}", "-o", str(out), str(src)], cwd=emu)
 
 
+def build_emu_encode() -> None:
+    """tests/emu/emu_encode.cpp: CPU single-stepper of the encoder's kernel logic (test infrastructure)."""
+    emu = ROOT / "tests" / "emu"
+    out = emu / "libkpeg_emu_encode.so"
+    src = emu / "emu_encode.cpp"
+    deps = [src, *sorted((PKG / "csrc").glob("*.h")), ROOT / "include" / "kpeg_cuda.h"]
+    if out.exists() and all(out.stat().st_mtime >= d.stat().st_mtime for d in deps):
+        return
+    _run(["g++", "-std=c++17", "-O2", "-fPIC", "-shared", "-ffp-contract=off", "-fno-fast-math",
+          "-Wno-unknown-pragmas", f"-I{ROOT / 'include'}", f"-I{PKG / 'csrc'}", "-o", str(out), str(src)], cwd=emu)
+
+
 def have_nvcc() -> bool:
     from shutil import which
     return which(os.environ.get("NVCC", "nvcc")) is not None

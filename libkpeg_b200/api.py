@@ -77,6 +77,12 @@ class Stats(C.Structure):
         return d
 
 
+class EncodeParams(C.Structure):
+    """struct kpeg_encode_params"""
+    _fields_ = [("width", C.c_uint16), ("height", C.c_uint16), ("ncomp", C.c_uint8), ("quality", C.c_uint8),
+                ("restart_interval", C.c_uint16), ("flags", C.c_uint32)]
+
+
 # every symbol include/kpeg_cuda.h declares: (restype, argtypes)
 _u8p = C.POINTER(C.c_uint8)
 _vp = C.c_void_p
@@ -138,6 +144,10 @@ SYMBOLS = {
     "kpeg_cuda_decode_ppm_device": (C.c_int, [_vp, C.POINTER(Plan), _vp, C.c_size_t, _vp, C.c_size_t, C.POINTER(C.c_size_t),
                                              C.POINTER(C.c_size_t), C.POINTER(Stats)]),
     "kpeg_cuda_interleaved_to_planar": (C.c_int, [_vp, _vp, _vp, C.c_size_t]),
+    "kpeg_encode_bound": (C.c_size_t, [C.POINTER(EncodeParams)]),
+    "kpeg_cuda_encode": (C.c_int, [_vp, C.POINTER(EncodeParams), _vp, _vp, C.c_size_t, C.POINTER(C.c_size_t), C.POINTER(Stats)]),
+    "kpeg_cuda_encode_device": (C.c_int, [_vp, C.POINTER(EncodeParams), _vp, _vp, C.c_size_t, C.POINTER(C.c_size_t),
+                                         C.POINTER(Stats)]),
 }
 
 _lib = None
@@ -196,6 +206,29 @@ def ppm_header(width: int, height: int) -> bytes:
     buf = C.create_string_buffer(256)
     n = lib.kpeg_ppm_header(width, height, buf, 256)
     return buf.raw[:n]
+
+
+def encode_params(width: int, height: int, ncomp: int, quality: int = 90, restart_interval: int = 0,
+                  flags: int = KPEG_FLAG_REF_PARITY) -> EncodeParams:
+    """kpeg_encode_params, range-checked (ValueError) before the fields are narrowed to their C types."""
+    if not (1 <= width <= 65535 and 1 <= height <= 65535 and ncomp in (1, 3) and 1 <= quality <= 100
+            and 0 <= restart_interval <= 65535):
+        raise ValueError(f"encode parameters out of range: {width}x{height}x{ncomp} q{quality} ri{restart_interval}")
+    return EncodeParams(width, height, ncomp, quality, restart_interval, flags)
+
+
+def encode_bound(width: int, height: int, ncomp: int, quality: int = 90, restart_interval: int = 0,
+                 flags: int = KPEG_FLAG_REF_PARITY) -> int:
+    """kpeg_encode_bound: the largest file the GPU encoder can write for these parameters (host only)."""
+    p = encode_params(width, height, ncomp, quality, restart_interval, flags)
+    return int(load_cuda_library().kpeg_encode_bound(C.byref(p)))
+
+
+def _image_shape(pixels: np.ndarray):
+    """(H, W, 3) or (H, W) / (H, W, 1) uint8 -> (height, width, ncomp)"""
+    if pixels.dtype != np.uint8 or pixels.ndim not in (2, 3) or (pixels.ndim == 3 and pixels.shape[2] not in (1, 3)):
+        raise ValueError("encode takes (H, W, 3) or (H, W) uint8 pixels")
+    return pixels.shape[0], pixels.shape[1], 1 if pixels.ndim == 2 else pixels.shape[2]
 
 
 class PinnedArray:
@@ -423,6 +456,35 @@ class Decoder:
 
     def interleaved_to_planar(self, d_rgb: int, d_planes: int, npixels: int):
         self._check(self._lib.kpeg_cuda_interleaved_to_planar(self._h, d_rgb, d_planes, npixels), "interleaved_to_planar")
+
+    # -- encode ------------------------------------------------------------------------------------
+    def encode(self, pixels: np.ndarray, quality: int = 90, restart_interval: int = 0,
+               flags: int = KPEG_FLAG_REF_PARITY) -> np.ndarray:
+        """Baseline JPEG of `pixels` ((H, W, 3) RGB or (H, W) gray uint8), encoded on the GPU (kpeg_cuda_encode)."""
+        h, w, nc = _image_shape(pixels)
+        p = encode_params(w, h, nc, quality, restart_interval, flags)
+        src = np.ascontiguousarray(pixels)
+        out = np.empty(self._lib.kpeg_encode_bound(C.byref(p)), dtype=np.uint8)
+        n = C.c_size_t(0)
+        rc = self._lib.kpeg_cuda_encode(self._h, C.byref(p), _ptr(src), _ptr(out), out.size, C.byref(n),
+                                        C.byref(self.last_stats))
+        self._check(rc, "kpeg_cuda_encode")
+        return out[:n.value].copy()
+
+    def encode_device(self, d_pixels: int, width: int, height: int, ncomp: int, d_out: int, cap: int, quality: int = 90,
+                      restart_interval: int = 0, flags: int = KPEG_FLAG_REF_PARITY) -> int:
+        """kpeg_cuda_encode_device: device pixels in, the file assembled at d_out; returns its length.  A cap below it
+        raises KpegError(KPEG_ERR_NOMEM) with the size needed in `.needed`."""
+        p = encode_params(width, height, ncomp, quality, restart_interval, flags)
+        n = C.c_size_t(0)
+        rc = self._lib.kpeg_cuda_encode_device(self._h, C.byref(p), d_pixels, d_out, cap, C.byref(n),
+                                               C.byref(self.last_stats))
+        if rc == KPEG_ERR_NOMEM:
+            err = KpegError(rc, f"kpeg_cuda_encode_device: {n.value} bytes needed, {cap} given")
+            err.needed = n.value
+            raise err
+        self._check(rc, "kpeg_cuda_encode_device")
+        return n.value
 
     def decode_batch_packed_device(self, plan: Plan, n: int, d_packed: int, packed_len: int, d_out: int):
         rc = self._lib.kpeg_cuda_decode_batch_packed_device(self._h, C.byref(plan), n, d_packed, packed_len, d_out,

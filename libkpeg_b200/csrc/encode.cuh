@@ -1,0 +1,50 @@
+// encode.cuh -- launch interface of the GPU baseline-JPEG encoder (csrc/encode.cu), used by the C-ABI host code.
+#ifndef KPEG_ENCODE_CUH
+#define KPEG_ENCODE_CUH
+
+#include <cuda_runtime.h>
+#include <stddef.h>
+#include <stdint.h>
+
+#include "encode_core.h"
+
+namespace kpeg {
+namespace enc {
+
+struct EncMeta {
+    uint64_t unstuffed; // bytes of the unstuffed stream (segments padded to bytes)
+    uint64_t scan_len;  // bytes written after the header: stuffed scan + RSTn markers + EOI
+};
+
+// Device buffers of one encode (sizes: scratch_sizes).
+struct EncBufs {
+    const uint8_t *pixels;  // [height][width][ncomp]
+    const EncTables *tables;
+    int16_t *coef;          // [nblk][64] zig-zag
+    int16_t *raw;           // [nblk] DC before the nudge
+    int16_t *dc;            // [nblk] final DC (== raw without KPEG_FLAG_REF_PARITY)
+    uint8_t *has_ac;        // [nblk]
+    uint32_t *bits;         // [nblk]
+    uint64_t *off;          // [nblk + 1] exclusive scan of bits
+    uint64_t *seg_byte;     // [nseg + 1] byte offset of every segment in the unstuffed stream
+    uint32_t *words;        // unstuffed stream, big-endian words
+    void *agg;              // tile aggregates of the scans
+    uint64_t *tile_ff;      // FF bytes per stuffing tile, then their exclusive scan
+    EncMeta *meta;
+    uint8_t *out;           // where the stuffed scan goes (right after the header)
+    uint64_t out_cap;       // bytes writable at out
+};
+
+enum { BUF_COEF, BUF_RAW, BUF_DC, BUF_HAS_AC, BUF_BITS, BUF_OFF, BUF_SEG, BUF_WORDS, BUF_AGG, BUF_TILE_FF, BUF_COUNT };
+// bytes each scratch buffer needs for an image of geometry g (words and tile_ff sized for the worst-case stream)
+void scratch_sizes(const EncGeom &g, size_t sizes[BUF_COUNT]);
+
+// Stage hooks for the caller's profiling events: called after each stage with a KPEG_T_* index.
+typedef void (*StageMark)(void *user, int stage);
+
+// Enqueues E1..E5 on `s`.  Returns cudaSuccess or the first launch error.
+cudaError_t launch_encode(const EncGeom &g, const EncBufs &b, cudaStream_t s, uint32_t *launches, StageMark mark, void *user);
+
+} // namespace enc
+} // namespace kpeg
+#endif

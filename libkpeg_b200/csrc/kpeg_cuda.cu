@@ -20,6 +20,8 @@
 #include <string>
 #include <vector>
 
+#include "encode.cuh"
+#include "encode_host.h"
 #include "host_tables.h"
 #include "kernels.cuh"
 #include "kpeg_common.h"
@@ -86,6 +88,14 @@ struct Lane {
     Job job;
 };
 
+// Grow-only device scratch of the encoder (on lane 0's stream), and its tables, rebuilt when the quality changes.
+struct EncScratch {
+    DevBuf buf[enc::BUF_COUNT];
+    DevBuf tables, meta, pixels, out;
+    PinBuf h_tables, h_meta;
+    int quality = -1;
+};
+
 } // namespace
 
 struct kpeg_ctx {
@@ -139,6 +149,8 @@ struct kpeg_ctx {
     int deferred_rc = KPEG_OK;
     std::string deferred_err;
     kpeg_stats deferred_stats = {};
+
+    EncScratch enc; // kpeg_cuda_encode*
 };
 
 namespace {
@@ -578,7 +590,14 @@ int check_guards(kpeg_ctx *ctx, Lane &L)
                        {"pixels", &L.pixels},     {"meta", &L.meta},
                        {"rec", &L.rec},           {"nrec", &L.nrec},         {"rec_alt", &L.rec_alt},   {"tables", &ctx->tables},
                        {"d_stage", &L.d_stage},   {"scan_tiles[0]", &ctx->scan_tiles[0]}, {"scan_tiles[1]", &ctx->scan_tiles[1]},
-                       {"scan_tiles[2]", &ctx->scan_tiles[2]}, {"band_counts", &ctx->band_counts}, {"merged", &ctx->merged}};
+                       {"scan_tiles[2]", &ctx->scan_tiles[2]}, {"band_counts", &ctx->band_counts}, {"merged", &ctx->merged},
+                       {"enc.coef", &ctx->enc.buf[enc::BUF_COEF]}, {"enc.raw", &ctx->enc.buf[enc::BUF_RAW]},
+                       {"enc.dc", &ctx->enc.buf[enc::BUF_DC]}, {"enc.has_ac", &ctx->enc.buf[enc::BUF_HAS_AC]},
+                       {"enc.bits", &ctx->enc.buf[enc::BUF_BITS]}, {"enc.off", &ctx->enc.buf[enc::BUF_OFF]},
+                       {"enc.seg_byte", &ctx->enc.buf[enc::BUF_SEG]}, {"enc.words", &ctx->enc.buf[enc::BUF_WORDS]},
+                       {"enc.agg", &ctx->enc.buf[enc::BUF_AGG]}, {"enc.tile_ff", &ctx->enc.buf[enc::BUF_TILE_FF]},
+                       {"enc.tables", &ctx->enc.tables}, {"enc.meta", &ctx->enc.meta}, {"enc.pixels", &ctx->enc.pixels},
+                       {"enc.out", &ctx->enc.out}};
     uint8_t host[2 * GUARD_BYTES];
     for (const NamedBuf &nb : bufs) {
         const DevBuf &b = *nb.buf;
@@ -927,6 +946,13 @@ extern "C" void kpeg_cuda_destroy(kpeg_ctx *ctx)
     dev_free(ctx->band_counts);
     if (ctx->h_band_counts.p)
         cudaFreeHost(ctx->h_band_counts.p);
+    for (DevBuf &b : ctx->enc.buf)
+        dev_free(b);
+    for (DevBuf *b : {&ctx->enc.tables, &ctx->enc.meta, &ctx->enc.pixels, &ctx->enc.out})
+        dev_free(*b);
+    for (PinBuf *b : {&ctx->enc.h_tables, &ctx->enc.h_meta})
+        if (b->p)
+            cudaFreeHost(b->p);
     delete ctx;
 }
 
@@ -1766,5 +1792,165 @@ extern "C" int kpeg_cuda_read_coefficients(kpeg_ctx *ctx, int16_t *out, size_t c
     CK(cudaMemcpyAsync(out, ctx->merged.p, n * 2u, cudaMemcpyDeviceToHost, L.stream));
     CK(cudaStreamSynchronize(L.stream));
     CK(cudaGetLastError());
+    return KPEG_OK;
+}
+
+// ==================================================================================================
+// Encode (csrc/encode.cu)
+// ==================================================================================================
+
+namespace {
+
+bool encode_params_ok(const kpeg_encode_params *p)
+{
+    return p && p->width >= 1 && p->height >= 1 && (p->ncomp == 1 || p->ncomp == 3) && p->quality >= 1 && p->quality <= 100 &&
+           (p->flags & ~KPEG_FLAG_REF_PARITY) == 0u;
+}
+
+void enc_mark(void *user, int stage)
+{
+    kpeg_ctx *ctx = (kpeg_ctx *)user;
+    mark(ctx, ctx->lane[0], stage);
+}
+
+// Tables (per quality) and scratch, then E1..E5 on lane 0 and the read-back of the length word into h_meta.
+// d_out / out_cap: where the stuffed scan goes and how many bytes may be written there.
+int encode_enqueue(kpeg_ctx *ctx, const kpeg_encode_params *p, const uint8_t *d_pixels, uint8_t *d_out, uint64_t out_cap,
+                   uint32_t *launches)
+{
+    EncScratch &E = ctx->enc;
+    cudaStream_t s = ctx->lane[0].stream;
+    if (E.quality != p->quality) {
+        CK(cudaStreamSynchronize(s)); // nothing may still read the old tables or their staging copy
+        TRY(ensure_pinned(ctx, s, E.h_tables, sizeof(enc::EncTables)));
+        TRY(ensure(ctx, s, E.tables, sizeof(enc::EncTables)));
+        enc::build_tables(p->quality, (enc::EncTables *)E.h_tables.p);
+        CK(cudaMemcpyAsync(E.tables.p, E.h_tables.p, sizeof(enc::EncTables), cudaMemcpyHostToDevice, s));
+        E.quality = p->quality;
+    }
+    const enc::EncGeom g = enc::geometry(p->width, p->height, p->ncomp, p->restart_interval, p->flags);
+    size_t sz[enc::BUF_COUNT];
+    enc::scratch_sizes(g, sz);
+    for (int i = 0; i < enc::BUF_COUNT; ++i)
+        TRY(ensure(ctx, s, E.buf[i], sz[i] + 16));
+    TRY(ensure(ctx, s, E.meta, sizeof(enc::EncMeta)));
+    TRY(ensure_pinned(ctx, s, E.h_meta, sizeof(enc::EncMeta)));
+    enc::EncBufs b;
+    b.pixels = d_pixels;
+    b.tables = (const enc::EncTables *)E.tables.p;
+    b.coef = (int16_t *)E.buf[enc::BUF_COEF].p;
+    b.raw = (int16_t *)E.buf[enc::BUF_RAW].p;
+    b.dc = (int16_t *)E.buf[enc::BUF_DC].p;
+    b.has_ac = (uint8_t *)E.buf[enc::BUF_HAS_AC].p;
+    b.bits = (uint32_t *)E.buf[enc::BUF_BITS].p;
+    b.off = (uint64_t *)E.buf[enc::BUF_OFF].p;
+    b.seg_byte = (uint64_t *)E.buf[enc::BUF_SEG].p;
+    b.words = (uint32_t *)E.buf[enc::BUF_WORDS].p;
+    b.agg = E.buf[enc::BUF_AGG].p;
+    b.tile_ff = (uint64_t *)E.buf[enc::BUF_TILE_FF].p;
+    b.meta = (enc::EncMeta *)E.meta.p;
+    b.out = d_out;
+    b.out_cap = out_cap;
+    CK(enc::launch_encode(g, b, s, launches, enc_mark, ctx));
+    CK(cudaMemcpyAsync(E.h_meta.p, E.meta.p, sizeof(enc::EncMeta), cudaMemcpyDeviceToHost, s));
+    return KPEG_OK;
+}
+
+void encode_stats(kpeg_ctx *ctx, const kpeg_encode_params *p, uint32_t launches, kpeg_stats *stats)
+{
+    if (!stats)
+        return;
+    const enc::EncMeta *m = (const enc::EncMeta *)ctx->enc.h_meta.p;
+    const enc::EncGeom g = enc::geometry(p->width, p->height, p->ncomp, p->restart_interval, p->flags);
+    stats->width = p->width;
+    stats->height = p->height;
+    stats->ncomp = p->ncomp;
+    stats->scan_bytes = m->scan_len;
+    stats->unstuffed_bytes = m->unstuffed;
+    stats->segments = (uint32_t)g.nseg;
+    stats->kernel_launches = launches;
+    add_times(ctx, ctx->lane[0], stats);
+}
+
+// every pending deferred submission is completed first (its outcome is reported by kpeg_cuda_wait)
+void finish_all_deferred(kpeg_ctx *ctx)
+{
+    for (int i = 0; i < NLANES; ++i)
+        if (ctx->lane[i].job.active)
+            finish_deferred(ctx, i);
+}
+
+} // namespace
+
+extern "C" size_t kpeg_encode_bound(const kpeg_encode_params *p)
+{
+    if (!encode_params_ok(p))
+        return 0;
+    return (size_t)enc::encode_bound(p->width, p->height, p->ncomp, p->quality, p->restart_interval);
+}
+
+extern "C" int kpeg_cuda_encode(kpeg_ctx *ctx, const kpeg_encode_params *p, const uint8_t *pixels, uint8_t *jpeg_out, size_t cap,
+                                size_t *jpeg_len, kpeg_stats *stats)
+{
+    if (!ctx || !encode_params_ok(p) || !pixels || !jpeg_out || !jpeg_len)
+        return KPEG_ERR_ARG;
+    CK(cudaSetDevice(ctx->device));
+    zero_stats(stats);
+    finish_all_deferred(ctx);
+    Lane &L = ctx->lane[0];
+    EncScratch &E = ctx->enc;
+    const size_t npix = (size_t)p->width * p->height * p->ncomp;
+    const std::vector<uint8_t> hdr = enc::file_header(p->width, p->height, p->ncomp, p->quality, p->restart_interval);
+    const size_t bound = (size_t)enc::encode_bound(p->width, p->height, p->ncomp, p->quality, p->restart_interval);
+    const size_t scan_cap = std::min(cap, bound) > hdr.size() ? std::min(cap, bound) - hdr.size() : 0;
+    TRY(ensure(ctx, L.stream, E.pixels, npix + 64));
+    TRY(ensure(ctx, L.stream, E.out, scan_cap + 64));
+    mark(ctx, L, -1);
+    CK(cudaMemcpyAsync(E.pixels.p, pixels, npix, cudaMemcpyHostToDevice, L.stream));
+    mark(ctx, L, KPEG_T_H2D);
+    uint32_t launches = 0;
+    TRY(encode_enqueue(ctx, p, (const uint8_t *)E.pixels.p, (uint8_t *)E.out.p, scan_cap, &launches));
+    CK(cudaStreamSynchronize(L.stream));
+    CK(cudaGetLastError());
+    const enc::EncMeta *m = (const enc::EncMeta *)E.h_meta.p;
+    *jpeg_len = hdr.size() + m->scan_len;
+    if (*jpeg_len > cap) {
+        encode_stats(ctx, p, launches, stats);
+        return fail(ctx, KPEG_ERR_NOMEM, "output buffer smaller than the encoded file (*jpeg_len = the size needed)");
+    }
+    memcpy(jpeg_out, hdr.data(), hdr.size());
+    CK(cudaMemcpyAsync(jpeg_out + hdr.size(), E.out.p, m->scan_len, cudaMemcpyDeviceToHost, L.stream));
+    mark(ctx, L, KPEG_T_D2H);
+    CK(cudaStreamSynchronize(L.stream));
+    if (ctx->guard)
+        TRY(check_guards(ctx, L));
+    encode_stats(ctx, p, launches, stats);
+    return KPEG_OK;
+}
+
+extern "C" int kpeg_cuda_encode_device(kpeg_ctx *ctx, const kpeg_encode_params *p, const uint8_t *d_pixels, uint8_t *d_out, size_t cap,
+                                       size_t *jpeg_len, kpeg_stats *stats)
+{
+    if (!ctx || !encode_params_ok(p) || !d_pixels || !d_out || !jpeg_len)
+        return KPEG_ERR_ARG;
+    CK(cudaSetDevice(ctx->device));
+    zero_stats(stats);
+    finish_all_deferred(ctx);
+    Lane &L = ctx->lane[0];
+    const std::vector<uint8_t> hdr = enc::file_header(p->width, p->height, p->ncomp, p->quality, p->restart_interval);
+    mark(ctx, L, -1);
+    if (cap)
+        CK(cudaMemcpyAsync(d_out, hdr.data(), std::min(cap, hdr.size()), cudaMemcpyHostToDevice, L.stream));
+    const size_t scan_cap = cap > hdr.size() ? cap - hdr.size() : 0;
+    uint32_t launches = 0;
+    TRY(encode_enqueue(ctx, p, d_pixels, d_out + hdr.size(), scan_cap, &launches));
+    CK(cudaStreamSynchronize(L.stream));
+    CK(cudaGetLastError());
+    if (ctx->guard)
+        TRY(check_guards(ctx, L));
+    encode_stats(ctx, p, launches, stats);
+    *jpeg_len = hdr.size() + ((const enc::EncMeta *)ctx->enc.h_meta.p)->scan_len;
+    if (*jpeg_len > cap)
+        return fail(ctx, KPEG_ERR_NOMEM, "output buffer smaller than the encoded file (*jpeg_len = the size needed)");
     return KPEG_OK;
 }

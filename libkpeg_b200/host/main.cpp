@@ -2,21 +2,30 @@
 //
 //   kpeg -h              help text
 //   kpeg <file.jpg>      decode on the GPU, write <file>.ppm next to the input, log to kpeg.log + stdout
-//   kpeg <in.ppm> <out.jpg>   the reference's encoder entry; its encoder is non-functional
-//                        (reference README.md:23) and is out of scope here -- reported as such.
+//   kpeg <in.ppm> <out.jpg>   encode on the GPU (kpeg_cuda_encode): binary PPM (P6, maxval 255) as R,G,B or PGM (P5)
+//                        as one gray component -> baseline JPEG, Annex K tables, 4:4:4.  The reference's own
+//                        encoder is non-functional (reference README.md:23); this one writes byte for byte what
+//                        the synthetic reference encoder (host/synth_encoder.cpp) writes for the same pixels.
 // Exit status follows the reference: EXIT_SUCCESS for any 2- or 3-argument run, EXIT_FAILURE for
 // none or too many (main.cpp:54-79).  Extra, non-reference switches come before the file name:
-//   --t81        ITU-T T.81 behaviour instead of bit-exact reference parity (SURVEY F1)
+//   --t81        ITU-T T.81 behaviour instead of bit-exact reference parity (SURVEY F1); when encoding: no DC nudge
 //   --device N   CUDA device index
+//   --quality N  encoder: IJG quality 1..100 (default 90)
+//   --restart N  encoder: restart interval in MCUs (default 0: none)
 //   --devices L  several devices, e.g. 0-7 or 0,2,3: the restart-interval tiles of the image are spread over them
 //   --quiet      log only to kpeg.log
+#include <cctype>
+#include <cstdio>
 #include <cstdlib>
+#include <fstream>
 #include <iostream>
+#include <iterator>
 #include <string>
 #include <vector>
 
 #include "Decoder.hpp"
 #include "Logger.hpp"
+#include "kpeg_cuda.h"
 
 namespace
 {
@@ -27,7 +36,9 @@ namespace
         std::cout << "===========================================" << std::endl;
         std::cout << "Help\n" << std::endl;
         std::cout << "<filename.jpg>                  : Decompress a JPEG image to a PPM image" << std::endl;
-        std::cout << "<filename.ppm> <filename.jpg>   : Convert input PNG file to JPEG" << std::endl;
+        std::cout << "<filename.ppm> <filename.jpg>   : Encode a PPM (P6) or PGM (P5) image to JPEG on the GPU" << std::endl;
+        std::cout << "--quality N                     : Encoder quality 1..100 (default 90)" << std::endl;
+        std::cout << "--restart N                     : Encoder restart interval in MCUs (default 0: none)" << std::endl;
         std::cout << "-h                              : Print this help message and exit" << std::endl;
     }
 
@@ -43,6 +54,8 @@ namespace
         bool parity = true;
         int device = 0;
         std::vector<int> devices;
+        int quality = 90;
+        int restart = 0;
     };
 
     // "0-3", "0,2,5", "1": device list of --devices
@@ -64,6 +77,101 @@ namespace
             i = j + 1;
         }
         return out;
+    }
+
+    // Binary PPM (P6) or PGM (P5), maxval 255; '#' comments and any whitespace between the header fields.
+    bool readPNM( const std::string& filename, int& width, int& height, int& ncomp, std::vector<uint8_t>& pixels, std::string& why )
+    {
+        std::ifstream in( filename, std::ios::binary );
+        if ( !in ) { why = "cannot open " + filename; return false; }
+        const std::vector<uint8_t> f( ( std::istreambuf_iterator<char>( in ) ), std::istreambuf_iterator<char>() );
+        std::size_t pos = 0;
+        auto skip = [&]() {
+            while ( pos < f.size() )
+            {
+                if ( f[pos] == '#' ) { while ( pos < f.size() && f[pos] != '\n' ) ++pos; }
+                else if ( std::isspace( f[pos] ) ) ++pos;
+                else break;
+            }
+        };
+        auto number = [&]( long& v ) {
+            skip();
+            if ( pos >= f.size() || !std::isdigit( f[pos] ) ) return false;
+            v = 0;
+            while ( pos < f.size() && std::isdigit( f[pos] ) && v < 1000000 ) v = v * 10 + ( f[pos++] - '0' );
+            return v < 1000000;
+        };
+        if ( f.size() < 2 || f[0] != 'P' || ( f[1] != '6' && f[1] != '5' ) ) { why = "not a binary PPM (P6) or PGM (P5) file"; return false; }
+        ncomp = f[1] == '6' ? 3 : 1;
+        pos = 2;
+        long w = 0, h = 0, maxval = 0;
+        if ( !number( w ) || !number( h ) || !number( maxval ) ) { why = "malformed header"; return false; }
+        if ( w < 1 || h < 1 || w > 65535 || h > 65535 ) { why = "image size out of range (1..65535)"; return false; }
+        if ( maxval != 255 ) { why = "only maxval 255 is supported"; return false; }
+        if ( pos >= f.size() || !std::isspace( f[pos] ) ) { why = "malformed header"; return false; }
+        ++pos; // exactly one whitespace byte before the samples
+        const std::size_t n = (std::size_t)w * h * ncomp;
+        if ( f.size() - pos < n ) { why = "truncated pixel data"; return false; }
+        pixels.assign( f.begin() + pos, f.begin() + pos + n );
+        width = (int)w;
+        height = (int)h;
+        return true;
+    }
+
+    void encodeJPEG( const std::string& in, const std::string& out, const Options& opt )
+    {
+        if ( !isValidFilename( out ) )
+        {
+            LOG(kpeg::Logger::Level::ERROR) << "Invalid output file name passed.";
+            return;
+        }
+        int width = 0, height = 0, ncomp = 0;
+        std::vector<uint8_t> pixels;
+        std::string why;
+        if ( !readPNM( in, width, height, ncomp, pixels, why ) )
+        {
+            LOG(kpeg::Logger::Level::ERROR) << "An error ocurred while encoding: " << in << ": " << why;
+            return;
+        }
+        if ( opt.quality < 1 || opt.quality > 100 || opt.restart < 0 || opt.restart > 65535 )
+        {
+            LOG(kpeg::Logger::Level::ERROR) << "An error ocurred while encoding: --quality must be 1..100, --restart 0..65535";
+            return;
+        }
+        kpeg_encode_params p = {};
+        p.width = (uint16_t)width;
+        p.height = (uint16_t)height;
+        p.ncomp = (uint8_t)ncomp;
+        p.quality = (uint8_t)opt.quality;
+        p.restart_interval = (uint16_t)opt.restart;
+        p.flags = opt.parity ? KPEG_FLAG_REF_PARITY : 0u;
+        kpeg_ctx* ctx = nullptr;
+        if ( kpeg_cuda_acquire( opt.device, &ctx ) != KPEG_OK )
+        {
+            LOG(kpeg::Logger::Level::ERROR) << "An error ocurred while encoding: no usable CUDA device (there is no CPU encode path)";
+            return;
+        }
+        std::vector<uint8_t> jpeg( kpeg_encode_bound( &p ) );
+        std::size_t len = 0;
+        const int rc = kpeg_cuda_encode( ctx, &p, pixels.data(), jpeg.data(), jpeg.size(), &len, nullptr );
+        const std::string err = rc == KPEG_OK ? "" : kpeg_cuda_last_error( ctx );
+        kpeg_cuda_release( opt.device, ctx );
+        if ( rc != KPEG_OK )
+        {
+            LOG(kpeg::Logger::Level::ERROR) << "An error ocurred while encoding: " << err;
+            return;
+        }
+        std::ofstream o( out, std::ios::binary );
+        o.write( (const char*)jpeg.data(), (std::streamsize)len );
+        o.close();
+        if ( !o )
+        {
+            std::remove( out.c_str() );
+            LOG(kpeg::Logger::Level::ERROR) << "An error ocurred while encoding: cannot write " << out;
+            return;
+        }
+        LOG(kpeg::Logger::Level::INFO) << "Encoded " << in << " (" << width << "x" << height << ", " << ncomp
+                                       << ( ncomp == 3 ? " components" : " component" ) << ") to " << out << ": " << len << " bytes";
     }
 
     void decodeJPEG( const std::string& filename, const Options& opt )
@@ -100,6 +208,8 @@ int main( int argc, char** argv )
             else if ( a == "--quiet" ) kpeg::Logger::get().setQuiet( true );
             else if ( a == "--device" && i + 1 < argc ) opt.device = std::atoi( argv[++i] );
             else if ( a == "--devices" && i + 1 < argc ) opt.devices = parseDevices( argv[++i] );
+            else if ( a == "--quality" && i + 1 < argc ) opt.quality = std::atoi( argv[++i] );
+            else if ( a == "--restart" && i + 1 < argc ) opt.restart = std::atoi( argv[++i] );
             else args.push_back( a );
         }
 
@@ -122,8 +232,7 @@ int main( int argc, char** argv )
         }
         if ( args.size() == 2 )
         {
-            LOG(kpeg::Logger::Level::ERROR) << "An error ocurred while encoding. (the encoder is outside this build: "
-                                               "the reference's own is non-functional)";
+            encodeJPEG( args[0], args[1], opt );
             return EXIT_SUCCESS;
         }
         return EXIT_FAILURE;

@@ -5,9 +5,14 @@
 //
 // Pipeline: integer pseudo-random pixel field -> JFIF RGB->YCbCr -> 8x8 FDCT (double) ->
 // quantise (Annex K tables, IJG quality scaling) -> optional quirk-free DC nudge -> Huffman
-// entropy coding (Annex K tables) with byte stuffing and optional DRI/RSTn.
+// entropy coding (Annex K tables) with byte stuffing and optional DRI/RSTn.  Everything after the
+// pixel field is kpeg_synth_encode_pixels, which takes any pixels: it is the byte-exact reference
+// the GPU encoder (csrc/encode.cu) is tested against, so its arithmetic order is part of the
+// contract (built with -ffp-contract=off; the tables come from csrc/jfif_write.h).
 
 #include "kpeg_synth.h"
+
+#include "jfif_write.h"
 
 #include <algorithm>
 #include <cmath>
@@ -18,59 +23,7 @@
 
 namespace {
 
-// ---- ITU-T T.81 Annex K tables (public standard constants) -------------------------------------
-
-const uint8_t kLumaQ[64] = {16, 11, 10, 16, 24,  40,  51,  61,  12, 12, 14, 19, 26,  58,  60,  55,
-                            14, 13, 16, 24, 40,  57,  69,  56,  14, 17, 22, 29, 51,  87,  80,  62,
-                            18, 22, 37, 56, 68,  109, 103, 77,  24, 35, 55, 64, 81,  104, 113, 92,
-                            49, 64, 78, 87, 103, 121, 120, 101, 72, 92, 95, 98, 112, 100, 103, 99};
-const uint8_t kChromaQ[64] = {17, 18, 24, 47, 99, 99, 99, 99, 18, 21, 26, 66, 99, 99, 99, 99,
-                              24, 26, 56, 99, 99, 99, 99, 99, 47, 66, 99, 99, 99, 99, 99, 99,
-                              99, 99, 99, 99, 99, 99, 99, 99, 99, 99, 99, 99, 99, 99, 99, 99,
-                              99, 99, 99, 99, 99, 99, 99, 99, 99, 99, 99, 99, 99, 99, 99, 99};
-
-const uint8_t kDcLumaBits[16] = {0, 1, 5, 1, 1, 1, 1, 1, 1, 0, 0, 0, 0, 0, 0, 0};
-const uint8_t kDcChromaBits[16] = {0, 3, 1, 1, 1, 1, 1, 1, 1, 1, 1, 0, 0, 0, 0, 0};
-const uint8_t kDcVals[12] = {0, 1, 2, 3, 4, 5, 6, 7, 8, 9, 10, 11};
-const uint8_t kAcLumaBits[16] = {0, 2, 1, 3, 3, 2, 4, 3, 5, 5, 4, 4, 0, 0, 1, 0x7d};
-const uint8_t kAcLumaVals[162] = {
-    0x01, 0x02, 0x03, 0x00, 0x04, 0x11, 0x05, 0x12, 0x21, 0x31, 0x41, 0x06, 0x13, 0x51, 0x61, 0x07, 0x22, 0x71,
-    0x14, 0x32, 0x81, 0x91, 0xa1, 0x08, 0x23, 0x42, 0xb1, 0xc1, 0x15, 0x52, 0xd1, 0xf0, 0x24, 0x33, 0x62, 0x72,
-    0x82, 0x09, 0x0a, 0x16, 0x17, 0x18, 0x19, 0x1a, 0x25, 0x26, 0x27, 0x28, 0x29, 0x2a, 0x34, 0x35, 0x36, 0x37,
-    0x38, 0x39, 0x3a, 0x43, 0x44, 0x45, 0x46, 0x47, 0x48, 0x49, 0x4a, 0x53, 0x54, 0x55, 0x56, 0x57, 0x58, 0x59,
-    0x5a, 0x63, 0x64, 0x65, 0x66, 0x67, 0x68, 0x69, 0x6a, 0x73, 0x74, 0x75, 0x76, 0x77, 0x78, 0x79, 0x7a, 0x83,
-    0x84, 0x85, 0x86, 0x87, 0x88, 0x89, 0x8a, 0x92, 0x93, 0x94, 0x95, 0x96, 0x97, 0x98, 0x99, 0x9a, 0xa2, 0xa3,
-    0xa4, 0xa5, 0xa6, 0xa7, 0xa8, 0xa9, 0xaa, 0xb2, 0xb3, 0xb4, 0xb5, 0xb6, 0xb7, 0xb8, 0xb9, 0xba, 0xc2, 0xc3,
-    0xc4, 0xc5, 0xc6, 0xc7, 0xc8, 0xc9, 0xca, 0xd2, 0xd3, 0xd4, 0xd5, 0xd6, 0xd7, 0xd8, 0xd9, 0xda, 0xe1, 0xe2,
-    0xe3, 0xe4, 0xe5, 0xe6, 0xe7, 0xe8, 0xe9, 0xea, 0xf1, 0xf2, 0xf3, 0xf4, 0xf5, 0xf6, 0xf7, 0xf8, 0xf9, 0xfa};
-const uint8_t kAcChromaBits[16] = {0, 2, 1, 2, 4, 4, 3, 4, 7, 5, 4, 4, 0, 1, 2, 0x77};
-const uint8_t kAcChromaVals[162] = {
-    0x00, 0x01, 0x02, 0x03, 0x11, 0x04, 0x05, 0x21, 0x31, 0x06, 0x12, 0x41, 0x51, 0x07, 0x61, 0x71, 0x13, 0x22,
-    0x32, 0x81, 0x08, 0x14, 0x42, 0x91, 0xa1, 0xb1, 0xc1, 0x09, 0x23, 0x33, 0x52, 0xf0, 0x15, 0x62, 0x72, 0xd1,
-    0x0a, 0x16, 0x24, 0x34, 0xe1, 0x25, 0xf1, 0x17, 0x18, 0x19, 0x1a, 0x26, 0x27, 0x28, 0x29, 0x2a, 0x35, 0x36,
-    0x37, 0x38, 0x39, 0x3a, 0x43, 0x44, 0x45, 0x46, 0x47, 0x48, 0x49, 0x4a, 0x53, 0x54, 0x55, 0x56, 0x57, 0x58,
-    0x59, 0x5a, 0x63, 0x64, 0x65, 0x66, 0x67, 0x68, 0x69, 0x6a, 0x73, 0x74, 0x75, 0x76, 0x77, 0x78, 0x79, 0x7a,
-    0x82, 0x83, 0x84, 0x85, 0x86, 0x87, 0x88, 0x89, 0x8a, 0x92, 0x93, 0x94, 0x95, 0x96, 0x97, 0x98, 0x99, 0x9a,
-    0xa2, 0xa3, 0xa4, 0xa5, 0xa6, 0xa7, 0xa8, 0xa9, 0xaa, 0xb2, 0xb3, 0xb4, 0xb5, 0xb6, 0xb7, 0xb8, 0xb9, 0xba,
-    0xc2, 0xc3, 0xc4, 0xc5, 0xc6, 0xc7, 0xc8, 0xc9, 0xca, 0xd2, 0xd3, 0xd4, 0xd5, 0xd6, 0xd7, 0xd8, 0xd9, 0xda,
-    0xe2, 0xe3, 0xe4, 0xe5, 0xe6, 0xe7, 0xe8, 0xe9, 0xea, 0xf2, 0xf3, 0xf4, 0xf5, 0xf6, 0xf7, 0xf8, 0xf9, 0xfa};
-
-// zig-zag index -> natural (row*8+col) index
-struct ZigZag {
-    int nat[64];
-    ZigZag()
-    {
-        int i = 0;
-        for (int d = 0; d < 15; ++d) {
-            int lo = d < 8 ? 0 : d - 7, hi = d < 8 ? d : 7;
-            for (int k = lo; k <= hi; ++k) {
-                int r = (d & 1) ? k : (hi + lo - k);
-                nat[i++] = r * 8 + (d - r);
-            }
-        }
-    }
-};
-const ZigZag kZZ;
+using namespace kpeg::jfif;
 
 // ---- content ------------------------------------------------------------------------------------
 
@@ -116,25 +69,6 @@ struct Content {
 
 // ---- entropy coder ------------------------------------------------------------------------------
 
-struct HuffEnc {
-    uint16_t code[256];
-    uint8_t len[256];
-    HuffEnc(const uint8_t bits[16], const uint8_t *vals)
-    {
-        std::memset(len, 0, sizeof len);
-        std::memset(code, 0, sizeof code);
-        int c = 0, k = 0;
-        for (int L = 1; L <= 16; ++L) {
-            for (int i = 0; i < bits[L - 1]; ++i) {
-                code[vals[k]] = (uint16_t)c++;
-                len[vals[k]] = (uint8_t)L;
-                ++k;
-            }
-            c <<= 1;
-        }
-    }
-};
-
 struct BitWriter {
     std::vector<uint8_t> &out;
     uint64_t acc = 0;
@@ -175,25 +109,6 @@ inline void put_value(BitWriter &bw, int v, int cat)
         bw.put((uint32_t)(v < 0 ? v + (1 << cat) - 1 : v), cat);
 }
 
-void put16(std::vector<uint8_t> &o, int v)
-{
-    o.push_back((uint8_t)(v >> 8));
-    o.push_back((uint8_t)v);
-}
-
-void put_dht(std::vector<uint8_t> &o, int tc_th, const uint8_t bits[16], const uint8_t *vals)
-{
-    int n = 0;
-    for (int i = 0; i < 16; ++i)
-        n += bits[i];
-    o.push_back(0xFF);
-    o.push_back(0xC4);
-    put16(o, 2 + 1 + 16 + n);
-    o.push_back((uint8_t)tc_th);
-    o.insert(o.end(), bits, bits + 16);
-    o.insert(o.end(), vals, vals + n);
-}
-
 struct Geometry {
     int W, H, nc_file, nc_content, mx, my;
     long nmcu;
@@ -219,36 +134,10 @@ Geometry geometry(const kpeg_synth_params *p)
     return g;
 }
 
-void scaled_qt(const uint8_t base[64], int quality, uint8_t out_nat[64])
+// The coding path over a pixel buffer [H][W][nc_content].
+int encode_pixels(const kpeg_synth_params *p, const uint8_t *px, uint8_t **out, size_t *out_len)
 {
-    int scale = quality < 50 ? 5000 / quality : 200 - 2 * quality;
-    for (int i = 0; i < 64; ++i) {
-        int t = (base[i] * scale + 50) / 100;
-        out_nat[i] = (uint8_t)(t < 1 ? 1 : (t > 255 ? 255 : t));
-    }
-}
-
-} // namespace
-
-extern "C" int kpeg_synth_pixels(const kpeg_synth_params *p, uint8_t *dst)
-{
-    if (!check(p) || !dst)
-        return -1;
-    Geometry g = geometry(p);
-    Content ct(p->seed, p->noise_amp > 0 ? p->noise_amp : 10);
-    for (int y = 0; y < g.H; ++y)
-        for (int x = 0; x < g.W; ++x)
-            for (int c = 0; c < g.nc_content; ++c)
-                dst[((size_t)y * g.W + x) * g.nc_content + c] = (uint8_t)ct.at(x, y, c);
-    return 0;
-}
-
-extern "C" int kpeg_synth_encode(const kpeg_synth_params *p, uint8_t **out, size_t *out_len)
-{
-    if (!check(p) || !out || !out_len)
-        return -1;
     const Geometry g = geometry(p);
-    const Content ct(p->seed, p->noise_amp > 0 ? p->noise_amp : 10);
     const int nc = g.nc_file;
 
     uint8_t qnat[2][64];
@@ -256,9 +145,7 @@ extern "C" int kpeg_synth_encode(const kpeg_synth_params *p, uint8_t **out, size
     scaled_qt(kChromaQ, p->quality, qnat[1]);
 
     double cs[8][8]; // cs[x][u] = C(u)/2 * cos((2x+1) u pi / 16)
-    for (int x = 0; x < 8; ++x)
-        for (int u = 0; u < 8; ++u)
-            cs[x][u] = (u == 0 ? std::sqrt(0.125) : 0.5) * std::cos((2 * x + 1) * u * M_PI / 16.0);
+    fdct_cosines(cs);
 
     // quantised coefficients, [mcu][comp][zig-zag]
     std::vector<int16_t> coef;
@@ -276,10 +163,11 @@ extern "C" int kpeg_synth_encode(const kpeg_synth_params *p, uint8_t **out, size
                     int y = std::min(by * 8 + r, g.H - 1);
                     for (int q = 0; q < 8; ++q) {
                         int x = std::min(bx * 8 + q, g.W - 1);
+                        const uint8_t *s = px + ((size_t)y * g.W + x) * g.nc_content;
                         if (g.nc_content == 1) {
-                            blk[0][r * 8 + q] = ct.at(x, y, 0) - 128.0;
+                            blk[0][r * 8 + q] = s[0] - 128.0;
                         } else {
-                            double R = ct.at(x, y, 0), G = ct.at(x, y, 1), B = ct.at(x, y, 2);
+                            double R = s[0], G = s[1], B = s[2];
                             blk[0][r * 8 + q] = 0.299 * R + 0.587 * G + 0.114 * B - 128.0;
                             blk[1][r * 8 + q] = -0.168736 * R - 0.331264 * G + 0.5 * B;
                             blk[2][r * 8 + q] = 0.5 * R - 0.418688 * G - 0.081312 * B;
@@ -351,42 +239,8 @@ extern "C" int kpeg_synth_encode(const kpeg_synth_params *p, uint8_t **out, size
 
     std::vector<uint8_t> o;
     o.reserve((size_t)g.nmcu * nc * 24 + 1024);
-    const uint8_t soi_app0[] = {0xFF, 0xD8, 0xFF, 0xE0, 0x00, 0x10, 'J',  'F',  'I',  'F',
-                                0x00, 0x01, 0x01, 0x01, 0x00, 0x48, 0x00, 0x48, 0x00, 0x00};
-    o.insert(o.end(), soi_app0, soi_app0 + sizeof soi_app0);
-    for (int t = 0; t < (nc == 3 ? 2 : 1); ++t) {
-        o.push_back(0xFF);
-        o.push_back(0xDB);
-        put16(o, 67);
-        o.push_back((uint8_t)t);
-        for (int i = 0; i < 64; ++i)
-            o.push_back(qnat[t][kZZ.nat[i]]);
-    }
-    o.push_back(0xFF);
-    o.push_back(0xC0);
-    put16(o, 8 + 3 * nc);
-    o.push_back(8);
-    put16(o, g.H);
-    put16(o, g.W);
-    o.push_back((uint8_t)nc);
-    for (int c = 0; c < nc; ++c) {
-        o.push_back((uint8_t)(c + 1));
-        o.push_back(0x11);
-        o.push_back((uint8_t)(c ? 1 : 0));
-    }
-    put_dht(o, 0x00, kDcLumaBits, kDcVals);
-    put_dht(o, 0x10, kAcLumaBits, kAcLumaVals);
-    if (nc == 3) {
-        put_dht(o, 0x01, kDcChromaBits, kDcVals);
-        put_dht(o, 0x11, kAcChromaBits, kAcChromaVals);
-    }
     const bool emit_rst = ri > 0 && (p->flags & KPEG_SYNTH_EMIT_RESTART);
-    if (emit_rst) {
-        o.push_back(0xFF);
-        o.push_back(0xDD);
-        put16(o, 4);
-        put16(o, ri);
-    }
+    write_frame_header(o, g.W, g.H, nc, qnat, emit_rst ? ri : 0);
     const HuffEnc dcL(kDcLumaBits, kDcVals), dcC(kDcChromaBits, kDcVals);
     const HuffEnc acL(kAcLumaBits, kAcLumaVals), acC(kAcChromaBits, kAcChromaVals);
     BitWriter bw(o);
@@ -395,17 +249,7 @@ extern "C" int kpeg_synth_encode(const kpeg_synth_params *p, uint8_t **out, size
     const bool split = nc == 3 && (p->flags & KPEG_SYNTH_NON_INTERLEAVED);
     for (int scan = 0; scan < (split ? nc : 1); ++scan) {
         const int c0 = split ? scan : 0, c1 = split ? scan + 1 : nc;
-        o.push_back(0xFF);
-        o.push_back(0xDA);
-        put16(o, 6 + 2 * (c1 - c0));
-        o.push_back((uint8_t)(c1 - c0));
-        for (int c = c0; c < c1; ++c) {
-            o.push_back((uint8_t)(c + 1));
-            o.push_back((uint8_t)(c ? 0x11 : 0x00));
-        }
-        o.push_back(0x00);
-        o.push_back(0x3F);
-        o.push_back(0x00);
+        write_sos(o, c0, c1);
         int pred[3] = {0, 0, 0};
         for (long m = 0; m < g.nmcu; ++m) {
             if (emit_rst && m && (m % ri) == 0) {
@@ -456,6 +300,57 @@ extern "C" int kpeg_synth_encode(const kpeg_synth_params *p, uint8_t **out, size
     *out = buf;
     *out_len = o.size();
     return 0;
+}
+
+} // namespace
+
+extern "C" int kpeg_synth_pixels(const kpeg_synth_params *p, uint8_t *dst)
+{
+    if (!check(p) || !dst)
+        return -1;
+    Geometry g = geometry(p);
+    Content ct(p->seed, p->noise_amp > 0 ? p->noise_amp : 10);
+    for (int y = 0; y < g.H; ++y)
+        for (int x = 0; x < g.W; ++x)
+            for (int c = 0; c < g.nc_content; ++c)
+                dst[((size_t)y * g.W + x) * g.nc_content + c] = (uint8_t)ct.at(x, y, c);
+    return 0;
+}
+
+extern "C" int kpeg_synth_encode_pixels(const kpeg_synth_params *p, const uint8_t *pixels, uint8_t **out, size_t *out_len)
+{
+    if (!check(p) || !pixels || !out || !out_len)
+        return -1;
+    return encode_pixels(p, pixels, out, out_len);
+}
+
+// generate the content (in parallel, rows split as the coding pass splits them), then encode it
+extern "C" int kpeg_synth_encode(const kpeg_synth_params *p, uint8_t **out, size_t *out_len)
+{
+    if (!check(p) || !out || !out_len)
+        return -1;
+    const Geometry g = geometry(p);
+    const Content ct(p->seed, p->noise_amp > 0 ? p->noise_amp : 10);
+    std::vector<uint8_t> px;
+    try {
+        px.resize((size_t)g.W * g.H * g.nc_content);
+    } catch (...) {
+        return -2;
+    }
+    auto work = [&](int y0, int y1) {
+        for (int y = y0; y < y1; ++y)
+            for (int x = 0; x < g.W; ++x)
+                for (int c = 0; c < g.nc_content; ++c)
+                    px[((size_t)y * g.W + x) * g.nc_content + c] = (uint8_t)ct.at(x, y, c);
+    };
+    int nt = p->threads > 0 ? p->threads : (int)std::thread::hardware_concurrency();
+    nt = std::max(1, std::min(nt, std::min(g.H, 64)));
+    std::vector<std::thread> th;
+    for (int t = 0; t < nt; ++t)
+        th.emplace_back(work, (int)((long)g.H * t / nt), (int)((long)g.H * (t + 1) / nt));
+    for (auto &t : th)
+        t.join();
+    return encode_pixels(p, px.data(), out, out_len);
 }
 
 extern "C" void kpeg_synth_free(uint8_t *buf) { std::free(buf); }

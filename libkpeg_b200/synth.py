@@ -55,6 +55,9 @@ def _load():
         lib.kpeg_synth_encode.argtypes = [C.POINTER(_Params), C.POINTER(C.POINTER(C.c_uint8)), C.POINTER(C.c_size_t)]
         lib.kpeg_synth_free.restype = None
         lib.kpeg_synth_free.argtypes = [C.POINTER(C.c_uint8)]
+        lib.kpeg_synth_encode_pixels.restype = C.c_int
+        lib.kpeg_synth_encode_pixels.argtypes = [C.POINTER(_Params), C.c_void_p, C.POINTER(C.POINTER(C.c_uint8)),
+                                                 C.POINTER(C.c_size_t)]
         lib.kpeg_synth_pixels.restype = C.c_int
         lib.kpeg_synth_pixels.argtypes = [C.POINTER(_Params), C.c_void_p]
         _lib = lib
@@ -69,6 +72,26 @@ def synth_encode(p: SynthParams) -> np.ndarray:
     rc = lib.kpeg_synth_encode(C.byref(cp), C.byref(out), C.byref(n))
     if rc != 0:
         raise RuntimeError(f"kpeg_synth_encode failed: {rc}")
+    try:
+        return np.ctypeslib.as_array(out, shape=(n.value,)).copy()
+    finally:
+        lib.kpeg_synth_free(out)
+
+
+def synth_encode_pixels(p: SynthParams, pixels: np.ndarray) -> np.ndarray:
+    """The synth's coding path over given pixels ([H][W][nc] uint8, nc = 1 or 3 as synth_pixels lays them out):
+    the byte-exact reference of the GPU encoder.  seed and noise_amp are ignored."""
+    lib = _load()
+    nc = 1 if (p.file_components == 1 or (p.flags & GRAY_CONTENT)) else 3
+    px = np.ascontiguousarray(pixels, dtype=np.uint8)
+    if px.size != p.width * p.height * nc:
+        raise ValueError(f"expected {p.height}x{p.width}x{nc} pixels, got shape {pixels.shape}")
+    cp = p._c()
+    out = C.POINTER(C.c_uint8)()
+    n = C.c_size_t(0)
+    rc = lib.kpeg_synth_encode_pixels(C.byref(cp), px.ctypes.data, C.byref(out), C.byref(n))
+    if rc != 0:
+        raise RuntimeError(f"kpeg_synth_encode_pixels failed: {rc}")
     try:
         return np.ctypeslib.as_array(out, shape=(n.value,)).copy()
     finally:
