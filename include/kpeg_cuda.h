@@ -35,6 +35,9 @@ extern "C" {
 /* Reproduce MCU.cpp:97-104: a block whose DC *difference* is 0 loses its AC coefficients
  * (SURVEY F1).  ON for bit-exact parity with the reference; OFF for ITU-T T.81 behaviour. */
 #define KPEG_FLAG_REF_PARITY 1u
+/* Encode only (kpeg_encode_params.flags): code with Huffman tables optimised for the image (T.81 K.2) instead of the
+ * Annex K ones.  The decode entry points ignore it. */
+#define KPEG_FLAG_OPTIMIZE_HUFFMAN 2u
 
 /* One Huffman table as it appears in a DHT segment (Types.hpp:116, Decoder.cpp:366-459). */
 typedef struct kpeg_huff_spec {
@@ -311,21 +314,34 @@ typedef struct kpeg_encode_params {
     uint8_t ncomp;              /* 1 (gray) or 3 (interleaved R,G,B in; Y,Cb,Cr coded) */
     uint8_t quality;            /* IJG 1..100, Annex K tables */
     uint16_t restart_interval;  /* MCUs, 0 = none (no DRI) */
-    uint32_t flags;             /* KPEG_FLAG_REF_PARITY: stream safe for the reference's DC rule (SURVEY F1) */
+    uint32_t flags;             /* KPEG_FLAG_REF_PARITY: stream safe for the reference's DC rule (SURVEY F1);
+                                   KPEG_FLAG_OPTIMIZE_HUFFMAN: optimised Huffman tables (below) */
 } kpeg_encode_params;
 
+/* KPEG_FLAG_OPTIMIZE_HUFFMAN: the same quantised coefficients, coded with the optimal tables for this image's symbol
+ * counts (DC and AC luma: component 0; DC and AC chroma: components 1 and 2; counted after the DC nudge and with the DC
+ * prediction reset at restart boundaries, as the symbols are coded).  The tables follow T.81 K.2 and the K.3 length
+ * limit with libjpeg's jpeg_gen_optimal_table rule (reserved symbol 256 of frequency 1; merge the two smallest non-zero
+ * frequencies, on a tie the larger symbol; fold lengths over 16; HUFFVAL by (length, symbol)), with 64-bit frequencies
+ * and no depth limit before the fold.  Same segment order; the file is byte for byte what kpeg_synth_encode_pixels
+ * writes with KPEG_SYNTH_OPTIMIZE_HUFFMAN added.  The histogram and the tables are built on the GPU, and the DHT, DRI
+ * and SOS segments are written there too, so the call still needs no host round trip before the copy-out. */
+
 /* Host only: the largest file kpeg_cuda_encode can write for these parameters (0 for bad parameters).
- * Per block at most 22 DC bits + 63 x 26 AC bits = 1660 bits:
+ * Per block at most 22 DC bits + 63 x 26 AC bits = 1660 bits with the Annex K tables, 27 + 63 x 26 = 1665 bits with
+ * KPEG_FLAG_OPTIMIZE_HUFFMAN:
  *  - DC: an 8-bit block's DC coefficient is (1/8) * the sum of its 64 level-shifted samples, in [-1024, 1016] for Y and
  *    [-1020, 1020] for Cb / Cr even with quantiser 1, and the nudge moves it by 1 at most when only the previous
  *    value is excluded (0 is excluded only at a segment's first MCU, where the prediction is 0 and |diff| <= 1025):
  *    |difference| <= 1017 + 1025 = 2042 < 2048, category <= 11; the longest Annex K DC code of category 11 is the
- *    chroma one, 11 bits: 11 + 11 = 22 bits.
- *  - AC: every coefficient is clamped to +-1023, category <= 10, and the longest Annex K AC code is 16 bits: a non-zero
- *    coefficient costs <= 26 bits; a ZRL (<= 11 bits) stands for 16 positions and EOB (<= 4 bits) for at least one, so
- *    no position costs more than 26 bits: 63 x 26.
+ *    chroma one, 11 bits: 11 + 11 = 22 bits.  An optimised code is at most 16 bits: 16 + 11 = 27 bits.
+ *  - AC: every coefficient is clamped to +-1023, category <= 10, and the longest code is 16 bits (Annex K and
+ *    optimised alike): a non-zero coefficient costs <= 26 bits; a ZRL (<= 16 bits) stands for 16 positions and EOB
+ *    (<= 16 bits) for at least one, so no position costs more than 26 bits: 63 x 26.
+ *  - Header: an optimised DHT never holds more symbols than the Annex K one (12 DC, 162 AC), so the Annex K header
+ *    bounds both.
  * Segments are padded to whole bytes (one byte each at most), every byte may be FF and be followed by a stuffed 00
- * (x 2), and there is one 2-byte RSTn between segments and the 2-byte EOI: bound = header + 2 * (ceil(blocks * 1660 / 8)
+ * (x 2), and there is one 2-byte RSTn between segments and the 2-byte EOI: bound = header + 2 * (ceil(blocks * bits / 8)
  * + segments) + 2 * segments. */
 size_t kpeg_encode_bound(const kpeg_encode_params *p);
 /* Encode host pixels ([height][width][ncomp], top-down) into the host buffer jpeg_out.  Synchronous.  When the file
@@ -333,11 +349,13 @@ size_t kpeg_encode_bound(const kpeg_encode_params *p);
  * NULL pointers: KPEG_ERR_ARG (checked before the context is used).  stats: width/height/ncomp, scan_bytes (stuffed
  * scan bytes written), unstuffed_bytes, segments, kernel_launches; with profiling on, ms_total and the stage times:
  * ms[KPEG_T_H2D] / ms[KPEG_T_D2H] the copies, ms[KPEG_T_IDCT] the FDCT + quantisation, ms[KPEG_T_DC_SCAN] the DC nudge,
+ * ms[KPEG_T_ENTROPY_SCAN] the symbol histogram and table build (KPEG_FLAG_OPTIMIZE_HUFFMAN only),
  * ms[KPEG_T_ENTROPY_WRITE] bit lengths, offsets and code emission, ms[KPEG_T_UNSTUFF] byte stuffing and markers. */
 int kpeg_cuda_encode(kpeg_ctx *ctx, const kpeg_encode_params *p, const uint8_t *pixels, uint8_t *jpeg_out, size_t cap,
                      size_t *jpeg_len, kpeg_stats *stats);
 /* Same with DEVICE buffers on the context's device: the file is assembled in d_out (header copied in, the scan written
- * right after it by the kernels).  When it is larger than cap: KPEG_ERR_NOMEM, *jpeg_len = the size it needs, and no
+ * right after it by the kernels; with KPEG_FLAG_OPTIMIZE_HUFFMAN only the part up to SOF0 is copied in and the rest of
+ * the header is written by the kernels too).  When it is larger than cap: KPEG_ERR_NOMEM, *jpeg_len = the size it needs, and no
  * byte at or past d_out + cap has been written. */
 int kpeg_cuda_encode_device(kpeg_ctx *ctx, const kpeg_encode_params *p, const uint8_t *d_pixels, uint8_t *d_out, size_t cap,
                             size_t *jpeg_len, kpeg_stats *stats);

@@ -32,6 +32,9 @@ extern "C" {
 #define KPEG_SYNTH_GRAY_CONTENT 2u /* luminance-only content; chroma blocks (if any) are all zero */
 #define KPEG_SYNTH_QUIRK_FREE 4u   /* see above */
 #define KPEG_SYNTH_NON_INTERLEAVED 8u /* three-component files: one scan per component (T.81 A.2.3) instead of one interleaved scan */
+/* Huffman tables optimised for the image's symbol counts (T.81 K.2 / K.3, the rule of KPEG_FLAG_OPTIMIZE_HUFFMAN in
+ * include/kpeg_cuda.h) instead of the Annex K ones; the quantised coefficients do not change */
+#define KPEG_SYNTH_OPTIMIZE_HUFFMAN 16u
 
 typedef struct kpeg_synth_params {
     int32_t width, height;       /* pixels; any size >= 1 (edges are replicated to whole blocks) */
@@ -53,7 +56,8 @@ void kpeg_synth_free(uint8_t *buf);
  * (interleaved R,G,B).  Uses width, height, file_components, quality, restart_interval, flags and threads; ignores
  * seed and noise_amp.  kpeg_synth_encode(p) == kpeg_synth_encode_pixels(p, kpeg_synth_pixels(p)) byte for byte.
  * With flags KPEG_SYNTH_QUIRK_FREE (or 0), plus KPEG_SYNTH_EMIT_RESTART when restart_interval > 0, this is the exact
- * file the GPU encoder (kpeg_cuda_encode, include/kpeg_cuda.h) writes with KPEG_FLAG_REF_PARITY (or 0). */
+ * file the GPU encoder (kpeg_cuda_encode, include/kpeg_cuda.h) writes with KPEG_FLAG_REF_PARITY (or 0); adding
+ * KPEG_SYNTH_OPTIMIZE_HUFFMAN gives the file it writes with KPEG_FLAG_OPTIMIZE_HUFFMAN added. */
 int kpeg_synth_encode_pixels(const kpeg_synth_params *p, const uint8_t *pixels, uint8_t **out, size_t *out_len);
 
 /* The source pixels the encoder compressed (before the lossy steps), for PSNR reporting.

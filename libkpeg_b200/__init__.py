@@ -7,6 +7,7 @@ contains no decode logic and no CPU fallback -- every decode call goes to the CU
 raises when that library or a GPU is missing.
 """
 from .api import (  # noqa: F401
+    KPEG_FLAG_OPTIMIZE_HUFFMAN,
     KPEG_FLAG_REF_PARITY,
     Decoder,
     EncodeParams,

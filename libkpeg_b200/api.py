@@ -18,6 +18,7 @@ KPEG_OK = 0
 KPEG_ERR_FORMAT, KPEG_ERR_UNSUPPORTED, KPEG_ERR_STREAM = -1, -2, -3
 KPEG_ERR_NOMEM, KPEG_ERR_CUDA, KPEG_ERR_ARG, KPEG_ERR_NOT_CONVERGED = -4, -5, -6, -7
 KPEG_FLAG_REF_PARITY = 1
+KPEG_FLAG_OPTIMIZE_HUFFMAN = 2  # encode only: Huffman tables optimised for the image (T.81 K.2) instead of Annex K
 
 _ERR_NAMES = {
     -1: "KPEG_ERR_FORMAT", -2: "KPEG_ERR_UNSUPPORTED", -3: "KPEG_ERR_STREAM", -4: "KPEG_ERR_NOMEM",
@@ -460,7 +461,8 @@ class Decoder:
     # -- encode ------------------------------------------------------------------------------------
     def encode(self, pixels: np.ndarray, quality: int = 90, restart_interval: int = 0,
                flags: int = KPEG_FLAG_REF_PARITY) -> np.ndarray:
-        """Baseline JPEG of `pixels` ((H, W, 3) RGB or (H, W) gray uint8), encoded on the GPU (kpeg_cuda_encode)."""
+        """Baseline JPEG of `pixels` ((H, W, 3) RGB or (H, W) gray uint8), encoded on the GPU (kpeg_cuda_encode).
+        flags: KPEG_FLAG_REF_PARITY and / or KPEG_FLAG_OPTIMIZE_HUFFMAN (per-image Huffman tables: smaller files)."""
         h, w, nc = _image_shape(pixels)
         p = encode_params(w, h, nc, quality, restart_interval, flags)
         src = np.ascontiguousarray(pixels)

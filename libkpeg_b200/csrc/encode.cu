@@ -2,19 +2,24 @@
 //
 //   E1 enc_fdct_kernel     pixels -> level shift / colour transform -> 8x8 FDCT (FP64) -> quantised zig-zag int16
 //   E2 DC nudge            KPEG_FLAG_REF_PARITY only: the synth's DC chain as a scan of 5-state maps (encode_core.h)
+//   EH enc_hist_kernel     KPEG_FLAG_OPTIMIZE_HUFFMAN only: symbol counts per table (the walk E3 and E4 code)
+//   EB enc_huff_build_kernel  KPEG_FLAG_OPTIMIZE_HUFFMAN only: one warp per table turns the counts into BITS / HUFFVAL
+//                          (huff_opt.h), codes into this encode's copy of the tables, and DHT [DRI] SOS into the file
 //   E3 bit lengths         per block, then a 64-bit exclusive scan (bit offsets) and a scan of the segments'
 //                          byte-padded lengths
 //   E4 enc_emit_kernel     every block writes its codes at its bit offset into a zeroed big-endian word stream
 //   E5 stuffing            FF counts per tile, their scan, then the stream with 00 after every FF, RSTn between
 //                          segments and EOI at the end, straight into the caller's buffer after the header
 //
-// Everything after E3's scans sizes itself from device memory (the stream length is not known on the host), with
-// grid-stride loops over a grid sized for the worst-case stream, so one encode needs no host round trip.
+// Everything after E3's scans sizes itself from device memory (the stream length is not known on the host, nor, in
+// optimised mode, the header length), with grid-stride loops over a grid sized for the worst-case stream, so one
+// encode needs no host round trip.
 #include <cuda_runtime.h>
 
 #include <algorithm>
 
 #include "encode.cuh"
+#include "huff_opt.h"
 #include "kpeg_cuda.h"
 
 namespace kpeg {
@@ -308,6 +313,212 @@ __global__ void __launch_bounds__(THREADS) enc_bits_kernel(EncGeom g, const EncT
     bits[b] = bc.n;
 }
 
+// ---- EH: symbol histogram ------------------------------------------------------------------------------------
+constexpr uint32_t HIST_GRID = 148u * 4u; // CTAs (grid-stride): fewer global atomics when the per-CTA counts are flushed
+
+// Counts into the CTA's [4][256] shared histogram.  EOB and the small categories are very hot bins, so the lanes of a
+// warp that hit the same bin at the same time are folded into one shared atomic.
+struct HistVisitor {
+    uint32_t *h;
+    int t; // DC table of the block's component (0 luma, 2 chroma); t + 1 is its AC table
+    __device__ __forceinline__ void add(uint32_t bin)
+    {
+        const uint32_t m = __match_any_sync(__activemask(), bin);
+        if ((threadIdx.x & 31u) == (uint32_t)(__ffs(m) - 1))
+            atomicAdd(&h[bin], (uint32_t)__popc(m));
+    }
+    __device__ __forceinline__ void dc(int cat, int) { add((uint32_t)t * 256u + (uint32_t)cat); }
+    __device__ __forceinline__ void ac(int sym, int, int) { add((uint32_t)(t + 1) * 256u + (uint32_t)sym); }
+    __device__ __forceinline__ void zrl() { add((uint32_t)(t + 1) * 256u + 0xF0u); }
+    __device__ __forceinline__ void eob() { add((uint32_t)(t + 1) * 256u); }
+};
+
+// hist: [4][257] uint64, zeroed on the stream before
+__global__ void __launch_bounds__(THREADS) enc_hist_kernel(EncGeom g, const int16_t *__restrict__ coef, const int16_t *__restrict__ dc,
+                                                           unsigned long long *__restrict__ hist)
+{
+    __shared__ uint32_t h[4 * 256];
+    for (int i = threadIdx.x; i < 4 * 256; i += THREADS)
+        h[i] = 0;
+    __syncthreads();
+    for (uint64_t b = (uint64_t)blockIdx.x * THREADS + threadIdx.x; b < g.nblk; b += (uint64_t)gridDim.x * THREADS) {
+        int16_t zz[64];
+        load_block(coef + b * 64, zz);
+        HistVisitor v{h, b % g.ncomp ? 2 : 0};
+        walk_block(dc_diff(g, dc, b), zz, v);
+    }
+    __syncthreads();
+    for (int i = threadIdx.x; i < (g.ncomp == 3 ? 4 : 2) * 256; i += THREADS)
+        if (h[i])
+            atomicAdd(&hist[(i >> 8) * huff::NSYM + (i & 255)], (unsigned long long)h[i]);
+}
+
+// ---- EB: optimal tables, one warp per table ------------------------------------------------------------------------
+constexpr int EB_PER_LANE = (huff::NSYM + 31) / 32; // slots lane + 32 j, j < 9
+
+// Appends at out[pos], nothing at or past cap.
+struct DevSeqOut {
+    uint8_t *p;
+    uint64_t pos, cap;
+    __device__ void put(uint32_t b)
+    {
+        if (pos < cap)
+            p[pos] = (uint8_t)b;
+        ++pos;
+    }
+};
+
+// The lane's first slot in merge order, skipping `skip`: (frequency, slot), slot -1 when it holds none.
+__device__ __forceinline__ void lane_first(const uint64_t (&f)[EB_PER_LANE], int skip, uint64_t &bf, int &bs)
+{
+    const int lane = threadIdx.x & 31;
+    bf = 0;
+    bs = -1;
+#pragma unroll
+    for (int j = 0; j < EB_PER_LANE; ++j) {
+        const int s = lane + 32 * j;
+        if (f[j] && s != skip && (bs < 0 || huff::merges_first(f[j], s, bf, bs))) {
+            bf = f[j];
+            bs = s;
+        }
+    }
+}
+
+// The warp's first slot in merge order (lexicographic on (frequency, -slot)), -1 when no lane holds one.  Frequencies
+// stay below 2^64 - 2^32 (they sum to the symbol count + 1), so ~0 in the high word means "none".
+__device__ __forceinline__ int warp_first(uint64_t bf, int bs, uint64_t &f)
+{
+    const uint32_t hi = bs < 0 ? ~0u : (uint32_t)(bf >> 32);
+    const uint32_t mh = __reduce_min_sync(0xFFFFFFFFu, hi);
+    const uint32_t lo = bs >= 0 && hi == mh ? (uint32_t)bf : ~0u;
+    const uint32_t ml = __reduce_min_sync(0xFFFFFFFFu, lo);
+    f = ((uint64_t)mh << 32) | ml;
+    return __reduce_max_sync(0xFFFFFFFFu, bs >= 0 && hi == mh && lo == ml ? bs : -1);
+}
+
+// One CTA of 32 * (2 or 4) threads.  Warp t builds table t (0 DC luma, 1 AC luma, 2 DC chroma, 3 AC chroma) from
+// hist[t] with huff::optimal_table's rule: the merge loop keeps each lane's nine slots in registers and finds the two
+// slots to merge with two warp-wide argmin reductions; code lengths are leaf depths of the parent array, lane-parallel;
+// the K.3 fold runs on one lane; HUFFVAL is a counting sort by (length, symbol).  The codes go into Topt, a copy of the
+// cached tables T_ (which stay untouched); then DHT [DRI] SOS are written at out[prefix_len..) and their end is the
+// header length in meta.
+__global__ void __launch_bounds__(128) enc_huff_build_kernel(EncGeom g, const unsigned long long *__restrict__ hist,
+                                                             const EncTables *__restrict__ T_, EncTables *__restrict__ Topt,
+                                                             uint8_t *__restrict__ out, uint64_t cap, uint64_t prefix_len,
+                                                             EncMeta *__restrict__ meta)
+{
+    using namespace huff;
+    __shared__ int16_t parent[4][NNODE];
+    __shared__ int16_t node[4][NSYM];
+    __shared__ uint32_t cnt[4][MAX_DEPTH + 1];   // codes by length, the reserved one included (then folded)
+    __shared__ uint32_t start[4][MAX_DEPTH + 2]; // HUFFVAL position of the next symbol of each length
+    __shared__ uint8_t bits[4][16];
+    __shared__ uint8_t vals[4][256];
+    __shared__ uint16_t code[4][256];
+    __shared__ uint8_t len[4][256];
+    {
+        const uint64_t *src = (const uint64_t *)T_;
+        uint64_t *dst = (uint64_t *)Topt;
+        for (int i = threadIdx.x; i < (int)(sizeof(EncTables) / 8); i += blockDim.x)
+            dst[i] = src[i];
+    }
+    const int t = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    for (int n = lane; n < NNODE; n += 32)
+        parent[t][n] = -1;
+    for (int s = lane; s < NSYM; s += 32)
+        node[t][s] = (int16_t)s;
+    for (int d = lane; d < MAX_DEPTH + 2; d += 32) {
+        if (d <= MAX_DEPTH)
+            cnt[t][d] = 0;
+        start[t][d] = 0;
+    }
+    uint64_t f[EB_PER_LANE];
+    uint32_t present = 0;
+#pragma unroll
+    for (int j = 0; j < EB_PER_LANE; ++j) {
+        const int s = lane + 32 * j;
+        f[j] = s < RESERVED ? hist[t * NSYM + s] : (s == RESERVED ? 1u : 0u);
+        present |= (f[j] != 0 ? 1u : 0u) << j;
+    }
+    __syncthreads(); // Topt holds the copy before any warp writes its codes
+    for (int next = NSYM;; ++next) {
+        uint64_t bf, f1, f2;
+        int bs;
+        lane_first(f, -1, bf, bs);
+        const int c1 = warp_first(bf, bs, f1);
+        lane_first(f, c1, bf, bs);
+        const int c2 = warp_first(bf, bs, f2);
+        if (c2 < 0)
+            break;
+#pragma unroll
+        for (int j = 0; j < EB_PER_LANE; ++j) {
+            const int s = lane + 32 * j;
+            if (s == c1)
+                f[j] += f2;
+            if (s == c2)
+                f[j] = 0;
+        }
+        if (lane == 0) {
+            parent[t][node[t][c1]] = parent[t][node[t][c2]] = (int16_t)next;
+            node[t][c1] = (int16_t)next;
+        }
+    }
+    __syncwarp();
+    int dep[EB_PER_LANE];
+    int dmax = 0;
+#pragma unroll
+    for (int j = 0; j < EB_PER_LANE; ++j) {
+        const int s = lane + 32 * j;
+        dep[j] = (present >> j) & 1u ? leaf_depth(parent[t], s) : 0;
+        dmax = max(dmax, dep[j]);
+        if (dep[j]) {
+            atomicAdd(&cnt[t][dep[j]], 1u);
+            if (s != RESERVED)
+                atomicAdd(&start[t][dep[j] + 1], 1u);
+        }
+    }
+    dmax = __reduce_max_sync(0xFFFFFFFFu, dmax);
+    __syncwarp();
+    if (lane == 0)
+        for (int d = 1; d <= dmax; ++d)
+            start[t][d + 1] += start[t][d];
+    __syncwarp();
+    // HUFFVAL: symbols 32 j .. 32 j + 31 in turn; lanes of equal length take consecutive places in lane order
+#pragma unroll
+    for (int j = 0; j < RESERVED / 32; ++j) {
+        const int d = dep[j];
+        const uint32_t m = __match_any_sync(0xFFFFFFFFu, d);
+        if (d)
+            vals[t][start[t][d] + __popc(m & ((1u << lane) - 1u))] = (uint8_t)(lane + 32 * j);
+        __syncwarp();
+        if (d && lane == __ffs(m) - 1)
+            start[t][d] += __popc(m);
+        __syncwarp();
+    }
+    if (lane == 0) {
+        fold_lengths(cnt[t], dmax, bits[t]);
+        canonical_codes(bits[t], vals[t], code[t], len[t]);
+    }
+    __syncwarp();
+    if (t & 1) {
+        for (int s = lane; s < 256; s += 32) {
+            Topt->ac_code[t >> 1][s] = code[t][s];
+            Topt->ac_len[t >> 1][s] = len[t][s];
+        }
+    } else if (lane < 16) {
+        Topt->dc_code[t >> 1][lane] = code[t][lane];
+        Topt->dc_len[t >> 1][lane] = len[t][lane];
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        DevSeqOut o{out, prefix_len, cap};
+        const uint8_t *const bp[4] = {bits[0], bits[1], bits[2], bits[3]};
+        const uint8_t *const vp[4] = {vals[0], vals[1], vals[2], vals[3]};
+        put_header_tail(o, (int)g.ncomp, bp, vp, (int)g.ri);
+        meta->hdr_len = o.pos;
+    }
+}
+
 struct DevWords {
     uint32_t *w;
     __device__ void store(uint64_t i, uint32_t v) { w[i] = v; }
@@ -370,8 +581,10 @@ __global__ void __launch_bounds__(STUFF_THREADS) enc_stuff_count_kernel(const ui
 }
 
 // one CTA: exclusive scan of the tiles' FF counts, and the length of what E5 writes
+// host_hdr: the length of the header the host wrote (Annex K mode), 0 when EB wrote the header and its length
 __global__ void __launch_bounds__(STUFF_THREADS) enc_stuff_spine_kernel(const uint64_t *__restrict__ seg_byte, uint64_t nseg,
-                                                                       uint64_t *__restrict__ tile_ff, EncMeta *__restrict__ meta)
+                                                                       uint64_t *__restrict__ tile_ff, uint64_t host_hdr,
+                                                                       EncMeta *__restrict__ meta)
 {
     __shared__ unsigned long long smem[32];
     const uint64_t N = seg_byte[nseg], ntiles = (N + STUFF_TILE - 1) / STUFF_TILE;
@@ -390,6 +603,8 @@ __global__ void __launch_bounds__(STUFF_THREADS) enc_stuff_spine_kernel(const ui
     if (threadIdx.x == 0) {
         meta->unstuffed = N;
         meta->scan_len = N + tot + 2u * nseg; // RSTn between segments + EOI
+        if (host_hdr)
+            meta->hdr_len = host_hdr;
     }
 }
 
@@ -405,12 +620,13 @@ struct DevOut {
 
 __global__ void __launch_bounds__(STUFF_THREADS) enc_stuff_write_kernel(const uint64_t *__restrict__ seg_byte, uint64_t nseg,
                                                                        const uint32_t *__restrict__ words, const uint64_t *__restrict__ tile_ff,
-                                                                       uint8_t *__restrict__ out, uint64_t cap)
+                                                                       const EncMeta *__restrict__ meta, uint8_t *__restrict__ out, uint64_t cap)
 {
     __shared__ unsigned long long smem[32];
     const uint64_t N = seg_byte[nseg], ntiles = (N + STUFF_TILE - 1) / STUFF_TILE;
     const SumOp op;
-    DevOut o{out, cap};
+    const uint64_t hdr = meta->hdr_len; // the scan starts after the header
+    DevOut o{out + hdr, cap > hdr ? cap - hdr : 0};
     for (uint64_t t = blockIdx.x; t < ntiles; t += gridDim.x) {
         const uint64_t i0 = min(N, t * STUFF_TILE + (uint64_t)threadIdx.x * STUFF_BYTES_PER_THREAD);
         const uint64_t i1 = min(N, i0 + STUFF_BYTES_PER_THREAD);
@@ -420,7 +636,7 @@ __global__ void __launch_bounds__(STUFF_THREADS) enc_stuff_write_kernel(const ui
     }
 }
 
-uint64_t unstuffed_bound(const EncGeom &g) { return (g.nblk * MAX_BLOCK_BITS + 7u) / 8u + g.nseg; }
+uint64_t unstuffed_bound(const EncGeom &g) { return (g.nblk * max_block_bits(g.flags) + 7u) / 8u + g.nseg; }
 
 } // namespace
 
@@ -458,22 +674,36 @@ cudaError_t launch_encode(const EncGeom &g, const EncBufs &b, cudaStream_t s, ui
         dc = b.dc;
         mark(user, KPEG_T_DC_SCAN);
     }
-    // E3
     const unsigned bgrid = (unsigned)((g.nblk + THREADS - 1) / THREADS);
-    enc_bits_kernel<<<bgrid, THREADS, 0, s>>>(g, b.tables, b.coef, dc, b.bits);
+    // EH, EB: this image's tables, and the header after the host's prefix
+    const EncTables *codes = b.tables;
+    const bool opt = (g.flags & KPEG_FLAG_OPTIMIZE_HUFFMAN) != 0;
+    if (opt) {
+        cudaError_t e = cudaMemsetAsync(b.hist, 0, 4u * huff::NSYM * sizeof(uint64_t), s);
+        if (e != cudaSuccess)
+            return e;
+        enc_hist_kernel<<<std::min(bgrid, HIST_GRID), THREADS, 0, s>>>(g, b.coef, dc, (unsigned long long *)b.hist);
+        enc_huff_build_kernel<<<1, 32 * (g.ncomp == 3 ? 4 : 2), 0, s>>>(g, (const unsigned long long *)b.hist, b.tables, b.opt_tables,
+                                                                          b.out, b.out_cap, b.hdr_len, b.meta);
+        *launches += 2;
+        codes = b.opt_tables;
+        mark(user, KPEG_T_ENTROPY_SCAN);
+    }
+    // E3
+    enc_bits_kernel<<<bgrid, THREADS, 0, s>>>(g, codes, b.coef, dc, b.bits);
     ++*launches;
     run_scan(BitsOp{b.bits, b.off, g.nblk}, g.nblk, 1, (unsigned long long *)b.agg, s, launches);
     run_scan(SegOp{b.off, b.seg_byte, g.nseg, g.seg_mcus * g.ncomp, g.nblk}, g.nseg, 1, (unsigned long long *)b.agg, s, launches);
     // E4
     const unsigned sgrid = (unsigned)std::min<uint64_t>(STREAM_GRID, unstuffed_bound(g) / STUFF_TILE + 1u);
     enc_zero_words_kernel<<<sgrid, THREADS, 0, s>>>(b.seg_byte + g.nseg, b.words);
-    enc_emit_kernel<<<bgrid, THREADS, 0, s>>>(g, b.tables, b.coef, dc, b.off, b.seg_byte, b.words);
+    enc_emit_kernel<<<bgrid, THREADS, 0, s>>>(g, codes, b.coef, dc, b.off, b.seg_byte, b.words);
     *launches += 2;
     mark(user, KPEG_T_ENTROPY_WRITE);
     // E5
     enc_stuff_count_kernel<<<sgrid, STUFF_THREADS, 0, s>>>(b.seg_byte, g.nseg, b.words, b.tile_ff);
-    enc_stuff_spine_kernel<<<1, STUFF_THREADS, 0, s>>>(b.seg_byte, g.nseg, b.tile_ff, b.meta);
-    enc_stuff_write_kernel<<<sgrid, STUFF_THREADS, 0, s>>>(b.seg_byte, g.nseg, b.words, b.tile_ff, b.out, b.out_cap);
+    enc_stuff_spine_kernel<<<1, STUFF_THREADS, 0, s>>>(b.seg_byte, g.nseg, b.tile_ff, opt ? 0u : b.hdr_len, b.meta);
+    enc_stuff_write_kernel<<<sgrid, STUFF_THREADS, 0, s>>>(b.seg_byte, g.nseg, b.words, b.tile_ff, b.meta, b.out, b.out_cap);
     *launches += 3;
     mark(user, KPEG_T_UNSTUFF);
     return cudaGetLastError();

@@ -14,12 +14,15 @@ namespace enc {
 struct EncMeta {
     uint64_t unstuffed; // bytes of the unstuffed stream (segments padded to bytes)
     uint64_t scan_len;  // bytes written after the header: stuffed scan + RSTn markers + EOI
+    uint64_t hdr_len;   // bytes of the header, where the scan starts (written by EB in optimised mode, else by E5)
 };
 
 // Device buffers of one encode (sizes: scratch_sizes).
 struct EncBufs {
     const uint8_t *pixels;  // [height][width][ncomp]
-    const EncTables *tables;
+    const EncTables *tables; // the cached per-quality tables (Annex K codes); never written
+    EncTables *opt_tables;   // KPEG_FLAG_OPTIMIZE_HUFFMAN: this encode's copy with the optimised codes (EB)
+    uint64_t *hist;          // KPEG_FLAG_OPTIMIZE_HUFFMAN: [4][257] symbol counts (EH), table order as in huff_opt.h
     int16_t *coef;          // [nblk][64] zig-zag
     int16_t *raw;           // [nblk] DC before the nudge
     int16_t *dc;            // [nblk] final DC (== raw without KPEG_FLAG_REF_PARITY)
@@ -31,8 +34,9 @@ struct EncBufs {
     void *agg;              // tile aggregates of the scans
     uint64_t *tile_ff;      // FF bytes per stuffing tile, then their exclusive scan
     EncMeta *meta;
-    uint8_t *out;           // where the stuffed scan goes (right after the header)
+    uint8_t *out;           // the file: the header (or, optimised, its prefix up to SOF0) is already there
     uint64_t out_cap;       // bytes writable at out
+    uint64_t hdr_len;       // bytes already at out: the whole header, or the prefix in optimised mode
 };
 
 enum { BUF_COEF, BUF_RAW, BUF_DC, BUF_HAS_AC, BUF_BITS, BUF_OFF, BUF_SEG, BUF_WORDS, BUF_AGG, BUF_TILE_FF, BUF_COUNT };
@@ -42,7 +46,7 @@ void scratch_sizes(const EncGeom &g, size_t sizes[BUF_COUNT]);
 // Stage hooks for the caller's profiling events: called after each stage with a KPEG_T_* index.
 typedef void (*StageMark)(void *user, int stage);
 
-// Enqueues E1..E5 on `s`.  Returns cudaSuccess or the first launch error.
+// Enqueues E1..E5 on `s` (with EH and EB between E2 and E3 in optimised mode).  Returns cudaSuccess or the first launch error.
 cudaError_t launch_encode(const EncGeom &g, const EncBufs &b, cudaStream_t s, uint32_t *launches, StageMark mark, void *user);
 
 } // namespace enc

@@ -1,5 +1,6 @@
 // encode_core.h -- per-block logic of the GPU baseline-JPEG encoder (csrc/encode.cu), written as KPEG_HD
-// functions so tests/emu/emu_encode.cpp replays exactly what the kernels run.
+// functions so tests/emu/emu_encode.cpp (and, with optimised tables, emu_encode_opt.cpp) replays exactly what the
+// kernels run.
 //
 // Exactness contract: the encoder writes byte for byte what kpeg_synth_encode_pixels (host/synth_encoder.cpp)
 // writes for the same pixels and parameters.  So the double arithmetic below is one correctly rounded multiply
@@ -14,22 +15,27 @@
 #include <stdint.h>
 
 #include "kpeg_common.h"
+#include "kpeg_cuda.h"
 
 namespace kpeg {
 namespace enc {
 
-// Largest coded block: 22 DC bits (category <= 11, code <= 11 bits) + 63 AC positions of <= 26 bits each
-// (code <= 16 bits + category <= 10).  Derivation in include/kpeg_cuda.h, kpeg_encode_bound.
+// Largest coded block: 22 DC bits (category <= 11, Annex K code <= 11 bits) + 63 AC positions of <= 26 bits each
+// (code <= 16 bits + category <= 10).  With optimised tables (KPEG_FLAG_OPTIMIZE_HUFFMAN) every code may be 16 bits
+// long: 27 DC bits + 63 x 26.  Derivation in include/kpeg_cuda.h, kpeg_encode_bound.
 constexpr uint32_t MAX_BLOCK_BITS = 22u + 63u * 26u;
+constexpr uint32_t MAX_BLOCK_BITS_OPT = 27u + 63u * 26u;
+
+KPEG_HD uint32_t max_block_bits(uint32_t flags) { return (flags & KPEG_FLAG_OPTIMIZE_HUFFMAN) ? MAX_BLOCK_BITS_OPT : MAX_BLOCK_BITS; }
 
 // Everything the kernels read; built on the host (encode_host.h) per quality and uploaded.
 struct EncTables {
     double cs[8][8];         // cs[x][u] = C(u)/2 * cos((2x+1) u pi / 16), host libm
     uint16_t qzz[2][64];     // quantiser of zig-zag position i: [0] luma, [1] chroma
     uint8_t nat[64];         // zig-zag index -> natural index
-    uint16_t dc_code[2][16]; // Annex K DC tables by category, [0] luma, [1] chroma
+    uint16_t dc_code[2][16]; // DC codes by category, [0] luma, [1] chroma (Annex K, or optimised per encode)
     uint8_t dc_len[2][16];
-    uint16_t ac_code[2][256]; // Annex K AC tables by run/size symbol
+    uint16_t ac_code[2][256]; // AC codes by run/size symbol
     uint8_t ac_len[2][256];
 };
 
@@ -154,31 +160,51 @@ KPEG_HD int category(int v)
 
 KPEG_HD uint32_t value_bits(int v, int cat) { return (uint32_t)(v < 0 ? v + (1 << cat) - 1 : v) & ((1u << cat) - 1u); }
 
-// Walks one block's codes in stream order: sink.put(bits, n) with n <= 27 (code and value bits together).
-// zz: the block's 64 zig-zag coefficients (zz[0] unused); diff: its DC difference; t: 0 luma, 1 chroma.
-template <class Sink>
-KPEG_HD void code_block(const EncTables &T, int t, int diff, const int16_t *zz, Sink &sink)
+// The one walk over a block's symbols, in stream order: v.dc(cat, diff), then per non-zero AC coefficient v.zrl() for
+// every 16 zeros before it beyond 15 and v.ac(run/size symbol, cat, value), and v.eob() when the block ends in zeros.
+// Code emission (E3, E4) and the symbol histogram (EH) are visitors of it, so they cannot disagree on the symbols.
+// zz: the block's 64 zig-zag coefficients (zz[0] unused); diff: its DC difference.
+template <class V>
+KPEG_HD void walk_block(int diff, const int16_t *zz, V &v)
 {
-    int cat = category(diff);
-    sink.put(((uint32_t)T.dc_code[t][cat] << cat) | value_bits(diff, cat), T.dc_len[t][cat] + cat);
+    v.dc(category(diff), diff);
     int run = 0;
     for (int i = 1; i < 64; ++i) {
-        const int v = zz[i];
-        if (v == 0) {
+        const int x = zz[i];
+        if (x == 0) {
             ++run;
             continue;
         }
         while (run > 15) {
-            sink.put(T.ac_code[t][0xF0], T.ac_len[t][0xF0]);
+            v.zrl();
             run -= 16;
         }
-        cat = category(v);
-        const int sym = (run << 4) | cat;
-        sink.put(((uint32_t)T.ac_code[t][sym] << cat) | value_bits(v, cat), T.ac_len[t][sym] + cat);
+        const int cat = category(x);
+        v.ac((run << 4) | cat, cat, x);
         run = 0;
     }
     if (run)
-        sink.put(T.ac_code[t][0x00], T.ac_len[t][0x00]);
+        v.eob();
+}
+
+// The walk's visitor that codes with table pair t (0 luma, 1 chroma): sink.put(bits, n) with n <= 27 -- code and value
+// bits together; a code is at most 16 bits with Annex K and with optimised tables alike, a DC value at most 11.
+template <class Sink>
+struct Coder {
+    const EncTables &T;
+    int t;
+    Sink &sink;
+    KPEG_HD void dc(int cat, int diff) { sink.put(((uint32_t)T.dc_code[t][cat] << cat) | value_bits(diff, cat), T.dc_len[t][cat] + cat); }
+    KPEG_HD void ac(int sym, int cat, int x) { sink.put(((uint32_t)T.ac_code[t][sym] << cat) | value_bits(x, cat), T.ac_len[t][sym] + cat); }
+    KPEG_HD void zrl() { sink.put(T.ac_code[t][0xF0], T.ac_len[t][0xF0]); }
+    KPEG_HD void eob() { sink.put(T.ac_code[t][0x00], T.ac_len[t][0x00]); }
+};
+
+template <class Sink>
+KPEG_HD void code_block(const EncTables &T, int t, int diff, const int16_t *zz, Sink &sink)
+{
+    Coder<Sink> c{T, t, sink};
+    walk_block(diff, zz, c);
 }
 
 struct BitCounter {

@@ -39,15 +39,24 @@ inline void build_tables(int quality, EncTables *T)
     }
 }
 
-// SOI .. SOS of the one interleaved scan (DRI when ri > 0)
-inline std::vector<uint8_t> file_header(int width, int height, int ncomp, int quality, int ri)
+// SOI .. SOF0: what comes before the Huffman tables (the host writes it in both modes)
+inline std::vector<uint8_t> file_prefix(int width, int height, int ncomp, int quality)
 {
     uint8_t qnat[2][64];
     jfif::scaled_qt(jfif::kLumaQ, quality, qnat[0]);
     jfif::scaled_qt(jfif::kChromaQ, quality, qnat[1]);
     std::vector<uint8_t> o;
-    jfif::write_frame_header(o, width, height, ncomp, qnat, ri);
-    jfif::write_sos(o, 0, ncomp);
+    jfif::write_frame_prefix(o, width, height, ncomp, qnat);
+    return o;
+}
+
+// SOI .. SOS of the one interleaved scan with the Annex K tables (DRI when ri > 0): the prefix and the tail the
+// optimised mode writes on the device (huff::put_header_tail) with its own tables
+inline std::vector<uint8_t> file_header(int width, int height, int ncomp, int quality, int ri)
+{
+    std::vector<uint8_t> o = file_prefix(width, height, ncomp, quality);
+    jfif::VecOut v{o};
+    huff::put_header_tail(v, ncomp, jfif::kAnnexKBits, jfif::kAnnexKVals, ri);
     return o;
 }
 
@@ -68,13 +77,13 @@ inline EncGeom geometry(int width, int height, int ncomp, int ri, uint32_t flags
     return g;
 }
 
-// Header + every block at MAX_BLOCK_BITS + one padding byte per segment, all doubled by stuffing (every byte
-// could be FF), + an RSTn marker between segments and EOI.
-inline uint64_t encode_bound(int width, int height, int ncomp, int quality, int ri)
+// Header + every block at max_block_bits + one padding byte per segment, all doubled by stuffing (every byte
+// could be FF), + an RSTn marker between segments and EOI.  The Annex K header is the longest either mode writes.
+inline uint64_t encode_bound(int width, int height, int ncomp, int quality, int ri, uint32_t flags = 0)
 {
-    const EncGeom g = geometry(width, height, ncomp, ri, 0);
+    const EncGeom g = geometry(width, height, ncomp, ri, flags);
     const uint64_t hdr = file_header(width, height, ncomp, quality, ri).size();
-    const uint64_t unstuffed = (g.nblk * MAX_BLOCK_BITS + 7u) / 8u + g.nseg;
+    const uint64_t unstuffed = (g.nblk * max_block_bits(flags) + 7u) / 8u + g.nseg;
     return hdr + 2u * unstuffed + 2u * (g.nseg - 1u) + 2u;
 }
 

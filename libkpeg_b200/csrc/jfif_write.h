@@ -15,6 +15,8 @@
 #include <cstring>
 #include <vector>
 
+#include "huff_opt.h"
+
 namespace kpeg {
 namespace jfif {
 
@@ -76,20 +78,7 @@ inline const ZigZag kZZ;
 struct HuffEnc {
     uint16_t code[256];
     uint8_t len[256];
-    HuffEnc(const uint8_t bits[16], const uint8_t *vals)
-    {
-        std::memset(len, 0, sizeof len);
-        std::memset(code, 0, sizeof code);
-        int c = 0, k = 0;
-        for (int L = 1; L <= 16; ++L) {
-            for (int i = 0; i < bits[L - 1]; ++i) {
-                code[vals[k]] = (uint16_t)c++;
-                len[vals[k]] = (uint8_t)L;
-                ++k;
-            }
-            c <<= 1;
-        }
-    }
+    HuffEnc(const uint8_t bits[16], const uint8_t *vals) { huff::canonical_codes(bits, vals, code, len); }
 };
 
 // The four Annex K tables in the order [0 = DC luma, 1 = AC luma, 2 = DC chroma, 3 = AC chroma].
@@ -127,22 +116,31 @@ inline void put16(std::vector<uint8_t> &o, int v)
     o.push_back((uint8_t)v);
 }
 
+// appends to a byte vector (the Out of the huff_opt.h writers)
+struct VecOut {
+    std::vector<uint8_t> &o;
+    void put(uint32_t b) { o.push_back((uint8_t)b); }
+};
+
 inline void put_dht(std::vector<uint8_t> &o, int tc_th, const uint8_t bits[16], const uint8_t *vals)
 {
-    int n = 0;
-    for (int i = 0; i < 16; ++i)
-        n += bits[i];
-    o.push_back(0xFF);
-    o.push_back(0xC4);
-    put16(o, 2 + 1 + 16 + n);
-    o.push_back((uint8_t)tc_th);
-    o.insert(o.end(), bits, bits + 16);
-    o.insert(o.end(), vals, vals + n);
+    VecOut v{o};
+    huff::put_dht(v, tc_th, bits, vals);
 }
 
-// SOI, APP0 (JFIF 1.1), DQT id0 [, DQT id1], SOF0, DHT 0x00, 0x10 [, 0x01, 0x11] [, DRI when dri > 0]:
-// everything up to the first SOS.  qnat: the scaled tables in natural order, [0] luma, [1] chroma.
-inline void write_frame_header(std::vector<uint8_t> &o, int W, int H, int nc, const uint8_t qnat[2][64], int dri)
+inline void put_dri(std::vector<uint8_t> &o, int dri)
+{
+    VecOut v{o};
+    huff::put_dri(v, dri);
+}
+
+// The four Annex K tables as BITS / HUFFVAL, [0 = DC luma, 1 = AC luma, 2 = DC chroma, 3 = AC chroma]
+inline const uint8_t *const kAnnexKBits[4] = {kDcLumaBits, kAcLumaBits, kDcChromaBits, kAcChromaBits};
+inline const uint8_t *const kAnnexKVals[4] = {kDcVals, kAcLumaVals, kDcVals, kAcChromaVals};
+
+// SOI, APP0 (JFIF 1.1), DQT id0 [, DQT id1], SOF0: the part of the header that does not depend on the Huffman
+// tables.  qnat: the scaled tables in natural order, [0] luma, [1] chroma.
+inline void write_frame_prefix(std::vector<uint8_t> &o, int W, int H, int nc, const uint8_t qnat[2][64])
 {
     const uint8_t soi_app0[] = {0xFF, 0xD8, 0xFF, 0xE0, 0x00, 0x10, 'J',  'F',  'I',  'F',
                                 0x00, 0x01, 0x01, 0x01, 0x00, 0x48, 0x00, 0x48, 0x00, 0x00};
@@ -167,34 +165,25 @@ inline void write_frame_header(std::vector<uint8_t> &o, int W, int H, int nc, co
         o.push_back(0x11);
         o.push_back((uint8_t)(c ? 1 : 0));
     }
-    put_dht(o, 0x00, kDcLumaBits, kDcVals);
-    put_dht(o, 0x10, kAcLumaBits, kAcLumaVals);
-    if (nc == 3) {
-        put_dht(o, 0x01, kDcChromaBits, kDcVals);
-        put_dht(o, 0x11, kAcChromaBits, kAcChromaVals);
-    }
-    if (dri > 0) {
-        o.push_back(0xFF);
-        o.push_back(0xDD);
-        put16(o, 4);
-        put16(o, dri);
-    }
+}
+
+// The prefix, then DHT 0x00, 0x10 [, 0x01, 0x11] with the given tables (Annex K by default) [, DRI when dri > 0]:
+// everything up to the first SOS.
+inline void write_frame_header(std::vector<uint8_t> &o, int W, int H, int nc, const uint8_t qnat[2][64], int dri,
+                               const uint8_t *const bits[4] = kAnnexKBits, const uint8_t *const vals[4] = kAnnexKVals)
+{
+    write_frame_prefix(o, W, H, nc, qnat);
+    for (int t = 0; t < (nc == 3 ? 4 : 2); ++t)
+        put_dht(o, ((t & 1) << 4) | (t >> 1), bits[t], vals[t]);
+    if (dri > 0)
+        put_dri(o, dri);
 }
 
 // SOS of a scan of components c0..c1-1 (luma tables for component 0, chroma tables for the others)
 inline void write_sos(std::vector<uint8_t> &o, int c0, int c1)
 {
-    o.push_back(0xFF);
-    o.push_back(0xDA);
-    put16(o, 6 + 2 * (c1 - c0));
-    o.push_back((uint8_t)(c1 - c0));
-    for (int c = c0; c < c1; ++c) {
-        o.push_back((uint8_t)(c + 1));
-        o.push_back((uint8_t)(c ? 0x11 : 0x00));
-    }
-    o.push_back(0x00);
-    o.push_back(0x3F);
-    o.push_back(0x00);
+    VecOut v{o};
+    huff::put_sos(v, c0, c1);
 }
 
 } // namespace jfif

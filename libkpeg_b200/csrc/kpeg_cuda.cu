@@ -89,9 +89,10 @@ struct Lane {
 };
 
 // Grow-only device scratch of the encoder (on lane 0's stream), and its tables, rebuilt when the quality changes.
+// opt_tables / hist: the optimised mode's per-encode tables and symbol counts (the cached tables stay Annex K).
 struct EncScratch {
     DevBuf buf[enc::BUF_COUNT];
-    DevBuf tables, meta, pixels, out;
+    DevBuf tables, meta, pixels, out, opt_tables, hist;
     PinBuf h_tables, h_meta;
     int quality = -1;
 };
@@ -597,7 +598,7 @@ int check_guards(kpeg_ctx *ctx, Lane &L)
                        {"enc.seg_byte", &ctx->enc.buf[enc::BUF_SEG]}, {"enc.words", &ctx->enc.buf[enc::BUF_WORDS]},
                        {"enc.agg", &ctx->enc.buf[enc::BUF_AGG]}, {"enc.tile_ff", &ctx->enc.buf[enc::BUF_TILE_FF]},
                        {"enc.tables", &ctx->enc.tables}, {"enc.meta", &ctx->enc.meta}, {"enc.pixels", &ctx->enc.pixels},
-                       {"enc.out", &ctx->enc.out}};
+                       {"enc.out", &ctx->enc.out}, {"enc.opt_tables", &ctx->enc.opt_tables}, {"enc.hist", &ctx->enc.hist}};
     uint8_t host[2 * GUARD_BYTES];
     for (const NamedBuf &nb : bufs) {
         const DevBuf &b = *nb.buf;
@@ -1804,7 +1805,7 @@ namespace {
 bool encode_params_ok(const kpeg_encode_params *p)
 {
     return p && p->width >= 1 && p->height >= 1 && (p->ncomp == 1 || p->ncomp == 3) && p->quality >= 1 && p->quality <= 100 &&
-           (p->flags & ~KPEG_FLAG_REF_PARITY) == 0u;
+           (p->flags & ~(KPEG_FLAG_REF_PARITY | KPEG_FLAG_OPTIMIZE_HUFFMAN)) == 0u;
 }
 
 void enc_mark(void *user, int stage)
@@ -1813,10 +1814,20 @@ void enc_mark(void *user, int stage)
     mark(ctx, ctx->lane[0], stage);
 }
 
-// Tables (per quality) and scratch, then E1..E5 on lane 0 and the read-back of the length word into h_meta.
-// d_out / out_cap: where the stuffed scan goes and how many bytes may be written there.
+bool encode_optimized(const kpeg_encode_params *p) { return (p->flags & KPEG_FLAG_OPTIMIZE_HUFFMAN) != 0u; }
+
+// What the host writes before the kernels: the whole header with the Annex K tables, or only SOI..SOF0 when the
+// optimised tables are built (and the rest of the header written) on the device.
+std::vector<uint8_t> encode_host_header(const kpeg_encode_params *p)
+{
+    return encode_optimized(p) ? enc::file_prefix(p->width, p->height, p->ncomp, p->quality)
+                               : enc::file_header(p->width, p->height, p->ncomp, p->quality, p->restart_interval);
+}
+
+// Tables (per quality) and scratch, then E1..E5 on lane 0 and the read-back of the length words into h_meta.
+// d_out / out_cap: the file and how many bytes may be written there; hdr_len: bytes of it the host has written.
 int encode_enqueue(kpeg_ctx *ctx, const kpeg_encode_params *p, const uint8_t *d_pixels, uint8_t *d_out, uint64_t out_cap,
-                   uint32_t *launches)
+                   uint64_t hdr_len, uint32_t *launches)
 {
     EncScratch &E = ctx->enc;
     cudaStream_t s = ctx->lane[0].stream;
@@ -1835,9 +1846,15 @@ int encode_enqueue(kpeg_ctx *ctx, const kpeg_encode_params *p, const uint8_t *d_
         TRY(ensure(ctx, s, E.buf[i], sz[i] + 16));
     TRY(ensure(ctx, s, E.meta, sizeof(enc::EncMeta)));
     TRY(ensure_pinned(ctx, s, E.h_meta, sizeof(enc::EncMeta)));
+    if (encode_optimized(p)) {
+        TRY(ensure(ctx, s, E.opt_tables, sizeof(enc::EncTables)));
+        TRY(ensure(ctx, s, E.hist, 4u * huff::NSYM * sizeof(uint64_t)));
+    }
     enc::EncBufs b;
     b.pixels = d_pixels;
     b.tables = (const enc::EncTables *)E.tables.p;
+    b.opt_tables = (enc::EncTables *)E.opt_tables.p;
+    b.hist = (uint64_t *)E.hist.p;
     b.coef = (int16_t *)E.buf[enc::BUF_COEF].p;
     b.raw = (int16_t *)E.buf[enc::BUF_RAW].p;
     b.dc = (int16_t *)E.buf[enc::BUF_DC].p;
@@ -1851,6 +1868,7 @@ int encode_enqueue(kpeg_ctx *ctx, const kpeg_encode_params *p, const uint8_t *d_
     b.meta = (enc::EncMeta *)E.meta.p;
     b.out = d_out;
     b.out_cap = out_cap;
+    b.hdr_len = hdr_len;
     CK(enc::launch_encode(g, b, s, launches, enc_mark, ctx));
     CK(cudaMemcpyAsync(E.h_meta.p, E.meta.p, sizeof(enc::EncMeta), cudaMemcpyDeviceToHost, s));
     return KPEG_OK;
@@ -1886,7 +1904,7 @@ extern "C" size_t kpeg_encode_bound(const kpeg_encode_params *p)
 {
     if (!encode_params_ok(p))
         return 0;
-    return (size_t)enc::encode_bound(p->width, p->height, p->ncomp, p->quality, p->restart_interval);
+    return (size_t)enc::encode_bound(p->width, p->height, p->ncomp, p->quality, p->restart_interval, p->flags);
 }
 
 extern "C" int kpeg_cuda_encode(kpeg_ctx *ctx, const kpeg_encode_params *p, const uint8_t *pixels, uint8_t *jpeg_out, size_t cap,
@@ -1900,26 +1918,29 @@ extern "C" int kpeg_cuda_encode(kpeg_ctx *ctx, const kpeg_encode_params *p, cons
     Lane &L = ctx->lane[0];
     EncScratch &E = ctx->enc;
     const size_t npix = (size_t)p->width * p->height * p->ncomp;
-    const std::vector<uint8_t> hdr = enc::file_header(p->width, p->height, p->ncomp, p->quality, p->restart_interval);
-    const size_t bound = (size_t)enc::encode_bound(p->width, p->height, p->ncomp, p->quality, p->restart_interval);
-    const size_t scan_cap = std::min(cap, bound) > hdr.size() ? std::min(cap, bound) - hdr.size() : 0;
+    const std::vector<uint8_t> hdr = encode_host_header(p);
+    const size_t bound = (size_t)enc::encode_bound(p->width, p->height, p->ncomp, p->quality, p->restart_interval, p->flags);
+    const size_t out_cap = std::min(cap, bound);
     TRY(ensure(ctx, L.stream, E.pixels, npix + 64));
-    TRY(ensure(ctx, L.stream, E.out, scan_cap + 64));
+    TRY(ensure(ctx, L.stream, E.out, out_cap + 64));
     mark(ctx, L, -1);
     CK(cudaMemcpyAsync(E.pixels.p, pixels, npix, cudaMemcpyHostToDevice, L.stream));
     mark(ctx, L, KPEG_T_H2D);
     uint32_t launches = 0;
-    TRY(encode_enqueue(ctx, p, (const uint8_t *)E.pixels.p, (uint8_t *)E.out.p, scan_cap, &launches));
+    TRY(encode_enqueue(ctx, p, (const uint8_t *)E.pixels.p, (uint8_t *)E.out.p, out_cap, hdr.size(), &launches));
     CK(cudaStreamSynchronize(L.stream));
     CK(cudaGetLastError());
     const enc::EncMeta *m = (const enc::EncMeta *)E.h_meta.p;
-    *jpeg_len = hdr.size() + m->scan_len;
+    *jpeg_len = m->hdr_len + m->scan_len;
     if (*jpeg_len > cap) {
         encode_stats(ctx, p, launches, stats);
         return fail(ctx, KPEG_ERR_NOMEM, "output buffer smaller than the encoded file (*jpeg_len = the size needed)");
     }
+    // what the host wrote (the whole Annex K header, or the prefix up to SOF0) is copied here; the rest comes from the
+    // device (optimised mode: the header's tail and the scan)
     memcpy(jpeg_out, hdr.data(), hdr.size());
-    CK(cudaMemcpyAsync(jpeg_out + hdr.size(), E.out.p, m->scan_len, cudaMemcpyDeviceToHost, L.stream));
+    CK(cudaMemcpyAsync(jpeg_out + hdr.size(), (const uint8_t *)E.out.p + hdr.size(), *jpeg_len - hdr.size(), cudaMemcpyDeviceToHost,
+                       L.stream));
     mark(ctx, L, KPEG_T_D2H);
     CK(cudaStreamSynchronize(L.stream));
     if (ctx->guard)
@@ -1937,19 +1958,19 @@ extern "C" int kpeg_cuda_encode_device(kpeg_ctx *ctx, const kpeg_encode_params *
     zero_stats(stats);
     finish_all_deferred(ctx);
     Lane &L = ctx->lane[0];
-    const std::vector<uint8_t> hdr = enc::file_header(p->width, p->height, p->ncomp, p->quality, p->restart_interval);
+    const std::vector<uint8_t> hdr = encode_host_header(p);
     mark(ctx, L, -1);
     if (cap)
         CK(cudaMemcpyAsync(d_out, hdr.data(), std::min(cap, hdr.size()), cudaMemcpyHostToDevice, L.stream));
-    const size_t scan_cap = cap > hdr.size() ? cap - hdr.size() : 0;
     uint32_t launches = 0;
-    TRY(encode_enqueue(ctx, p, d_pixels, d_out + hdr.size(), scan_cap, &launches));
+    TRY(encode_enqueue(ctx, p, d_pixels, d_out, cap, hdr.size(), &launches));
     CK(cudaStreamSynchronize(L.stream));
     CK(cudaGetLastError());
     if (ctx->guard)
         TRY(check_guards(ctx, L));
     encode_stats(ctx, p, launches, stats);
-    *jpeg_len = hdr.size() + ((const enc::EncMeta *)ctx->enc.h_meta.p)->scan_len;
+    const enc::EncMeta *m = (const enc::EncMeta *)ctx->enc.h_meta.p;
+    *jpeg_len = m->hdr_len + m->scan_len;
     if (*jpeg_len > cap)
         return fail(ctx, KPEG_ERR_NOMEM, "output buffer smaller than the encoded file (*jpeg_len = the size needed)");
     return KPEG_OK;

@@ -3,7 +3,7 @@
 //   kpeg -h              help text
 //   kpeg <file.jpg>      decode on the GPU, write <file>.ppm next to the input, log to kpeg.log + stdout
 //   kpeg <in.ppm> <out.jpg>   encode on the GPU (kpeg_cuda_encode): binary PPM (P6, maxval 255) as R,G,B or PGM (P5)
-//                        as one gray component -> baseline JPEG, Annex K tables, 4:4:4.  The reference's own
+//                        as one gray component -> baseline JPEG, Annex K (or, --optimize, per-image) tables, 4:4:4.  The reference's own
 //                        encoder is non-functional (reference README.md:23); this one writes byte for byte what
 //                        the synthetic reference encoder (host/synth_encoder.cpp) writes for the same pixels.
 // Exit status follows the reference: EXIT_SUCCESS for any 2- or 3-argument run, EXIT_FAILURE for
@@ -12,6 +12,7 @@
 //   --device N   CUDA device index
 //   --quality N  encoder: IJG quality 1..100 (default 90)
 //   --restart N  encoder: restart interval in MCUs (default 0: none)
+//   --optimize   encoder: Huffman tables optimised for the image (KPEG_FLAG_OPTIMIZE_HUFFMAN): smaller files
 //   --devices L  several devices, e.g. 0-7 or 0,2,3: the restart-interval tiles of the image are spread over them
 //   --quiet      log only to kpeg.log
 #include <cctype>
@@ -39,6 +40,7 @@ namespace
         std::cout << "<filename.ppm> <filename.jpg>   : Encode a PPM (P6) or PGM (P5) image to JPEG on the GPU" << std::endl;
         std::cout << "--quality N                     : Encoder quality 1..100 (default 90)" << std::endl;
         std::cout << "--restart N                     : Encoder restart interval in MCUs (default 0: none)" << std::endl;
+        std::cout << "--optimize                      : Encoder Huffman tables optimised for the image (smaller file)" << std::endl;
         std::cout << "-h                              : Print this help message and exit" << std::endl;
     }
 
@@ -56,6 +58,7 @@ namespace
         std::vector<int> devices;
         int quality = 90;
         int restart = 0;
+        bool optimize = false;
     };
 
     // "0-3", "0,2,5", "1": device list of --devices
@@ -144,7 +147,7 @@ namespace
         p.ncomp = (uint8_t)ncomp;
         p.quality = (uint8_t)opt.quality;
         p.restart_interval = (uint16_t)opt.restart;
-        p.flags = opt.parity ? KPEG_FLAG_REF_PARITY : 0u;
+        p.flags = ( opt.parity ? KPEG_FLAG_REF_PARITY : 0u ) | ( opt.optimize ? KPEG_FLAG_OPTIMIZE_HUFFMAN : 0u );
         kpeg_ctx* ctx = nullptr;
         if ( kpeg_cuda_acquire( opt.device, &ctx ) != KPEG_OK )
         {
@@ -210,6 +213,7 @@ int main( int argc, char** argv )
             else if ( a == "--devices" && i + 1 < argc ) opt.devices = parseDevices( argv[++i] );
             else if ( a == "--quality" && i + 1 < argc ) opt.quality = std::atoi( argv[++i] );
             else if ( a == "--restart" && i + 1 < argc ) opt.restart = std::atoi( argv[++i] );
+            else if ( a == "--optimize" ) opt.optimize = true;
             else args.push_back( a );
         }
 

@@ -5,7 +5,7 @@
 //
 // Pipeline: integer pseudo-random pixel field -> JFIF RGB->YCbCr -> 8x8 FDCT (double) ->
 // quantise (Annex K tables, IJG quality scaling) -> optional quirk-free DC nudge -> Huffman
-// entropy coding (Annex K tables) with byte stuffing and optional DRI/RSTn.  Everything after the
+// entropy coding (Annex K tables, or tables optimised for the image) with byte stuffing and optional DRI/RSTn.  Everything after the
 // pixel field is kpeg_synth_encode_pixels, which takes any pixels: it is the byte-exact reference
 // the GPU encoder (csrc/encode.cu) is tested against, so its arithmetic order is part of the
 // contract (built with -ffp-contract=off; the tables come from csrc/jfif_write.h).
@@ -240,9 +240,46 @@ int encode_pixels(const kpeg_synth_params *p, const uint8_t *px, uint8_t **out, 
     std::vector<uint8_t> o;
     o.reserve((size_t)g.nmcu * nc * 24 + 1024);
     const bool emit_rst = ri > 0 && (p->flags & KPEG_SYNTH_EMIT_RESTART);
-    write_frame_header(o, g.W, g.H, nc, qnat, emit_rst ? ri : 0);
-    const HuffEnc dcL(kDcLumaBits, kDcVals), dcC(kDcChromaBits, kDcVals);
-    const HuffEnc acL(kAcLumaBits, kAcLumaVals), acC(kAcChromaBits, kAcChromaVals);
+    // the Huffman tables: Annex K, or -- KPEG_SYNTH_OPTIMIZE_HUFFMAN -- optimal for this image's symbol counts, counted
+    // below exactly as the coding loop further down codes the symbols
+    const uint8_t *bits[4] = {kDcLumaBits, kAcLumaBits, kDcChromaBits, kAcChromaBits};
+    const uint8_t *vals[4] = {kDcVals, kAcLumaVals, kDcVals, kAcChromaVals};
+    uint8_t opt_bits[4][16], opt_vals[4][256];
+    if (p->flags & KPEG_SYNTH_OPTIMIZE_HUFFMAN) {
+        uint64_t freq[4][256] = {};
+        int pred[3] = {0, 0, 0};
+        for (long m = 0; m < g.nmcu; ++m) {
+            if (emit_rst && m && (m % ri) == 0)
+                pred[0] = pred[1] = pred[2] = 0;
+            for (int c = 0; c < nc; ++c) {
+                const int16_t *zz = &coef[((size_t)m * nc + c) * 64];
+                uint64_t *fd = freq[c ? 2 : 0], *fa = freq[c ? 3 : 1];
+                ++fd[category(zz[0] - pred[c])];
+                pred[c] = zz[0];
+                int run = 0;
+                for (int i = 1; i < 64; ++i) {
+                    if (zz[i] == 0) {
+                        ++run;
+                        continue;
+                    }
+                    for (; run > 15; run -= 16)
+                        ++fa[0xF0];
+                    ++fa[(run << 4) | category(zz[i])];
+                    run = 0;
+                }
+                if (run)
+                    ++fa[0x00];
+            }
+        }
+        for (int t = 0; t < (nc == 3 ? 4 : 2); ++t) {
+            kpeg::huff::optimal_table(freq[t], opt_bits[t], opt_vals[t]);
+            bits[t] = opt_bits[t];
+            vals[t] = opt_vals[t];
+        }
+    }
+    write_frame_header(o, g.W, g.H, nc, qnat, emit_rst ? ri : 0, bits, vals);
+    const HuffEnc dcL(bits[0], vals[0]), dcC(bits[2], vals[2]);
+    const HuffEnc acL(bits[1], vals[1]), acC(bits[3], vals[3]);
     BitWriter bw(o);
     // one interleaved scan of all components, or -- KPEG_SYNTH_NON_INTERLEAVED -- one scan per component (T.81 A.2.3:
     // the MCU of a non-interleaved scan is one block, blocks in raster order; the restart interval counts those)

@@ -15,6 +15,7 @@ EMIT_RESTART = 1
 GRAY_CONTENT = 2
 QUIRK_FREE = 4
 NON_INTERLEAVED = 8  # three-component files: one scan per component
+OPTIMIZE_HUFFMAN = 16  # Huffman tables optimised for the image (the GPU encoder's KPEG_FLAG_OPTIMIZE_HUFFMAN)
 
 
 class _Params(C.Structure):
