@@ -360,6 +360,63 @@ int kpeg_cuda_encode(kpeg_ctx *ctx, const kpeg_encode_params *p, const uint8_t *
 int kpeg_cuda_encode_device(kpeg_ctx *ctx, const kpeg_encode_params *p, const uint8_t *d_pixels, uint8_t *d_out, size_t cap,
                             size_t *jpeg_len, kpeg_stats *stats);
 
+/* ---- lossless transcode: baseline JPEG -> baseline JPEG on the GPU (csrc/transcode.cu) ---------------------------
+ * Re-codes the quantised coefficients of a whole baseline file (anything kpeg_parse_jfif_scans accepts: one or three
+ * components, 4:4:4, any DQT / DHT ids and contents, any restart interval, APPn / COM segments, three-component frames
+ * coded one scan per component) with other Huffman tables, another restart interval or one of the eight lossless
+ * transforms below, without going through pixels (what jpegtran does).  The output holds the SAME quantised coefficients
+ * in the T.81 sense (no SURVEY F1 rule), moved by the transform, in the encoder's layout, so that a file
+ * kpeg_cuda_encode wrote comes back byte for byte unchanged:
+ *   SOI, APP0 (JFIF 1.1); one DQT per quantiser id the components use, ascending, with the input's values (transposed,
+ *   Q'[u][v] = Q[v][u], by the transposing transforms); SOF0 with the output size, component ids 1..nc, sampling 0x11 and
+ *   the input's Tq per component; DHT (Annex K, or with KPEG_FLAG_OPTIMIZE_HUFFMAN the tables of kpeg_cuda_encode's
+ *   rule; the luma pair for component 0, the chroma pair for 1 and 2); [DRI]; one interleaved SOS and the scan; EOI.
+ * APPn and COM segments are not copied.  The output is always JFIF (the decoder reads every three-component file as
+ * YCbCr).  It is byte for byte what kpeg_synth_encode_coefficients (include/kpeg_synth.h) writes for the input's T.81
+ * coefficients after the transform.
+ *
+ * Transforms (numbered as libjpeg's JXFORM_CODE; u is the vertical frequency, v the horizontal one).  A transform whose
+ * flip would move a partial edge block gives KPEG_ERR_UNSUPPORTED (jpegtran -perfect):
+ *   NONE        W x H                                    FLIP_H    W x H, needs W % 8 == 0, negates odd v
+ *   FLIP_V      W x H, needs H % 8 == 0, negates odd u   TRANSPOSE H x W, F'[u][v] = F[v][u]
+ *   TRANSVERSE  H x W, needs W, H % 8 == 0               ROT90     H x W (clockwise: transpose, then flip-h), needs H % 8 == 0
+ *   ROT180      W x H, needs W, H % 8 == 0               ROT270    H x W (transpose, then flip-v), needs W % 8 == 0
+ * Range rules: every DC difference in the output's block order and segmentation must have category <= 11, and every AC
+ * coefficient must be within +-1023; else KPEG_ERR_UNSUPPORTED.  Files of 8-bit encoders satisfy both; a crafted file
+ * whose absolute DC drifts past 2047 may not once it is re-segmented or transformed.  Under these rules a block costs
+ * at most kpeg_encode_bound's 1660 bits (1665 optimised).
+ *
+ * Note on SURVEY F1: the coefficient identity is a T.81 statement.  With the restart interval and the orientation
+ * unchanged the DC differences are unchanged too, and the output then also decodes to the input's pixels under
+ * KPEG_FLAG_REF_PARITY; otherwise it may not, because the reference's F1 rule depends on the DC differences. */
+#define KPEG_XFORM_NONE 0u
+#define KPEG_XFORM_FLIP_H 1u
+#define KPEG_XFORM_FLIP_V 2u
+#define KPEG_XFORM_TRANSPOSE 3u
+#define KPEG_XFORM_TRANSVERSE 4u
+#define KPEG_XFORM_ROT90 5u
+#define KPEG_XFORM_ROT180 6u
+#define KPEG_XFORM_ROT270 7u
+#define KPEG_TRANSCODE_KEEP_RESTART (-1)
+typedef struct kpeg_transcode_params {
+    int32_t restart_interval; /* output MCUs per interval: -1 = the input's (its first scan's DRI), 0 = none, 1..65535 */
+    uint32_t transform;       /* KPEG_XFORM_* */
+    uint32_t flags;           /* 0 or KPEG_FLAG_OPTIMIZE_HUFFMAN; anything else is KPEG_ERR_ARG */
+} kpeg_transcode_params;
+/* Host only: the largest file kpeg_cuda_transcode can write for this input and these parameters (kpeg_encode_bound's
+ * derivation with up to three DQT segments in the header); 0 for a file the parser rejects, bad parameters or a
+ * transform whose precondition fails. */
+size_t kpeg_transcode_bound(const uint8_t *file, size_t len, const kpeg_transcode_params *p);
+/* Host buffers in and out, synchronous.  When the file is larger than cap: KPEG_ERR_NOMEM, *out_len = the size it needs,
+ * nothing written to out.  Errors: KPEG_ERR_FORMAT / KPEG_ERR_UNSUPPORTED for what the parser or the decoder rejects,
+ * KPEG_ERR_STREAM for corrupt entropy data, KPEG_ERR_UNSUPPORTED for the transform preconditions and the range rules,
+ * KPEG_ERR_ARG for bad parameters.  stats: the decode's stage slots as a decode fills them, and the whole re-encode
+ * (gather, table build, bit lengths, emission, stuffing) in ms[KPEG_T_IDCT], the slot of a decode's reconstruction;
+ * width / height / ncomp, scan_bytes, unstuffed_bytes and segments describe the output, subsequences and sync_rounds the
+ * input's decode, kernel_launches both. */
+int kpeg_cuda_transcode(kpeg_ctx *ctx, const uint8_t *file, size_t len, const kpeg_transcode_params *p, uint8_t *out,
+                        size_t cap, size_t *out_len, kpeg_stats *stats);
+
 #ifdef __cplusplus
 }
 #endif

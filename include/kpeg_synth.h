@@ -60,6 +60,23 @@ void kpeg_synth_free(uint8_t *buf);
  * KPEG_SYNTH_OPTIMIZE_HUFFMAN gives the file it writes with KPEG_FLAG_OPTIMIZE_HUFFMAN added. */
 int kpeg_synth_encode_pixels(const kpeg_synth_params *p, const uint8_t *pixels, uint8_t **out, size_t *out_len);
 
+/* The encoder's coding path over given quantised coefficients (what encode_pixels runs after the DC nudge):
+ * coef is [nblk][64] int16, blocks MCU-interleaved (one block per component per MCU), zig-zag order, DC absolute.
+ * Writes SOI, APP0, one DQT per quantiser id the components use (ascending, qt[id] in zig-zag order), SOF0 (ids 1..ncomp,
+ * sampling 0x11, tq[c]), DHT (Annex K or, KPEG_SYNTH_OPTIMIZE_HUFFMAN, optimised), [DRI when restart_interval > 0], one
+ * interleaved SOS, the scan with RSTn, EOI.  Returns -1 on bad parameters or when a DC difference has category > 11 or an
+ * AC coefficient is outside +-1023 (no baseline table codes them), -2 on allocation failure.  The reference of the GPU
+ * transcoder (kpeg_cuda_transcode). */
+typedef struct kpeg_synth_coef_frame {
+    int32_t width, height;    /* 1..65535 */
+    int32_t ncomp;            /* 1 or 3 */
+    uint8_t tq[3];            /* quantiser id (0..3) per component */
+    uint8_t qt[4][64];        /* quantisers by id, zig-zag order (only the ids in tq are written) */
+    int32_t restart_interval; /* MCUs, 0 = none */
+    uint32_t flags;           /* 0 or KPEG_SYNTH_OPTIMIZE_HUFFMAN */
+} kpeg_synth_coef_frame;
+int kpeg_synth_encode_coefficients(const kpeg_synth_coef_frame *f, const int16_t *coef, uint8_t **out, size_t *out_len);
+
 /* The source pixels the encoder compressed (before the lossy steps), for PSNR reporting.
  * dst is [height][width][file_components==1 or GRAY_CONTENT ? 1 : 3]. */
 int kpeg_synth_pixels(const kpeg_synth_params *p, uint8_t *dst);

@@ -9,6 +9,15 @@ raises when that library or a GPU is missing.
 from .api import (  # noqa: F401
     KPEG_FLAG_OPTIMIZE_HUFFMAN,
     KPEG_FLAG_REF_PARITY,
+    KPEG_TRANSCODE_KEEP_RESTART,
+    KPEG_XFORM_FLIP_H,
+    KPEG_XFORM_FLIP_V,
+    KPEG_XFORM_NONE,
+    KPEG_XFORM_ROT90,
+    KPEG_XFORM_ROT180,
+    KPEG_XFORM_ROT270,
+    KPEG_XFORM_TRANSPOSE,
+    KPEG_XFORM_TRANSVERSE,
     Decoder,
     EncodeParams,
     KpegError,
@@ -18,5 +27,7 @@ from .api import (  # noqa: F401
     encode_bound,
     parse_jfif,
     ppm_header,
+    TranscodeParams,
+    transcode_bound,
 )
 from .synth import SynthParams, synth_encode, synth_pixels  # noqa: F401

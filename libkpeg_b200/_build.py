@@ -68,6 +68,18 @@ def build_emu_encode_opt() -> None:
           "-Wno-unknown-pragmas", f"-I{ROOT / 'include'}", f"-I{PKG / 'csrc'}", "-o", str(out), str(src)], cwd=emu)
 
 
+def build_emu_transcode() -> None:
+    """tests/emu/emu_transcode.cpp: CPU replay of the lossless transcoder's gather and coded stages (test infrastructure)."""
+    emu = ROOT / "tests" / "emu"
+    out = emu / "libkpeg_emu_transcode.so"
+    src = emu / "emu_transcode.cpp"
+    deps = [src, *sorted((PKG / "csrc").glob("*.h")), ROOT / "include" / "kpeg_cuda.h"]
+    if out.exists() and all(out.stat().st_mtime >= d.stat().st_mtime for d in deps):
+        return
+    _run(["g++", "-std=c++17", "-O2", "-fPIC", "-shared", "-ffp-contract=off", "-fno-fast-math",
+          "-Wno-unknown-pragmas", f"-I{ROOT / 'include'}", f"-I{PKG / 'csrc'}", "-o", str(out), str(src)], cwd=emu)
+
+
 def have_nvcc() -> bool:
     from shutil import which
     return which(os.environ.get("NVCC", "nvcc")) is not None

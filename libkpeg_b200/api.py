@@ -19,6 +19,11 @@ KPEG_ERR_FORMAT, KPEG_ERR_UNSUPPORTED, KPEG_ERR_STREAM = -1, -2, -3
 KPEG_ERR_NOMEM, KPEG_ERR_CUDA, KPEG_ERR_ARG, KPEG_ERR_NOT_CONVERGED = -4, -5, -6, -7
 KPEG_FLAG_REF_PARITY = 1
 KPEG_FLAG_OPTIMIZE_HUFFMAN = 2  # encode only: Huffman tables optimised for the image (T.81 K.2) instead of Annex K
+# lossless transforms of kpeg_cuda_transcode (numbered as libjpeg's JXFORM_CODE)
+KPEG_XFORM_NONE, KPEG_XFORM_FLIP_H, KPEG_XFORM_FLIP_V, KPEG_XFORM_TRANSPOSE = 0, 1, 2, 3
+KPEG_XFORM_TRANSVERSE, KPEG_XFORM_ROT90, KPEG_XFORM_ROT180, KPEG_XFORM_ROT270 = 4, 5, 6, 7
+KPEG_TRANSCODE_KEEP_RESTART = -1
+XFORM_NAMES = ("none", "flip-h", "flip-v", "transpose", "transverse", "rot90", "rot180", "rot270")
 
 _ERR_NAMES = {
     -1: "KPEG_ERR_FORMAT", -2: "KPEG_ERR_UNSUPPORTED", -3: "KPEG_ERR_STREAM", -4: "KPEG_ERR_NOMEM",
@@ -82,6 +87,11 @@ class EncodeParams(C.Structure):
     """struct kpeg_encode_params"""
     _fields_ = [("width", C.c_uint16), ("height", C.c_uint16), ("ncomp", C.c_uint8), ("quality", C.c_uint8),
                 ("restart_interval", C.c_uint16), ("flags", C.c_uint32)]
+
+
+class TranscodeParams(C.Structure):
+    """struct kpeg_transcode_params"""
+    _fields_ = [("restart_interval", C.c_int32), ("transform", C.c_uint32), ("flags", C.c_uint32)]
 
 
 # every symbol include/kpeg_cuda.h declares: (restype, argtypes)
@@ -149,6 +159,9 @@ SYMBOLS = {
     "kpeg_cuda_encode": (C.c_int, [_vp, C.POINTER(EncodeParams), _vp, _vp, C.c_size_t, C.POINTER(C.c_size_t), C.POINTER(Stats)]),
     "kpeg_cuda_encode_device": (C.c_int, [_vp, C.POINTER(EncodeParams), _vp, _vp, C.c_size_t, C.POINTER(C.c_size_t),
                                          C.POINTER(Stats)]),
+    "kpeg_transcode_bound": (C.c_size_t, [_vp, C.c_size_t, C.POINTER(TranscodeParams)]),
+    "kpeg_cuda_transcode": (C.c_int, [_vp, _vp, C.c_size_t, C.POINTER(TranscodeParams), _vp, C.c_size_t, C.POINTER(C.c_size_t),
+                                     C.POINTER(Stats)]),
 }
 
 _lib = None
@@ -223,6 +236,23 @@ def encode_bound(width: int, height: int, ncomp: int, quality: int = 90, restart
     """kpeg_encode_bound: the largest file the GPU encoder can write for these parameters (host only)."""
     p = encode_params(width, height, ncomp, quality, restart_interval, flags)
     return int(load_cuda_library().kpeg_encode_bound(C.byref(p)))
+
+
+def transcode_params(restart_interval: int = KPEG_TRANSCODE_KEEP_RESTART, transform: int = KPEG_XFORM_NONE,
+                     optimize: bool = False) -> TranscodeParams:
+    """kpeg_transcode_params, range-checked (ValueError) before the fields are narrowed to their C types."""
+    if not (-1 <= restart_interval <= 65535 and 0 <= transform <= 7):
+        raise ValueError(f"transcode parameters out of range: restart {restart_interval}, transform {transform}")
+    return TranscodeParams(restart_interval, transform, KPEG_FLAG_OPTIMIZE_HUFFMAN if optimize else 0)
+
+
+def transcode_bound(data, restart_interval: int = KPEG_TRANSCODE_KEEP_RESTART, transform: int = KPEG_XFORM_NONE,
+                    optimize: bool = False) -> int:
+    """kpeg_transcode_bound: the largest file kpeg_cuda_transcode can write for this input (host only; 0 when the file,
+    the parameters or the transform's precondition are rejected)."""
+    buf = np.ascontiguousarray(np.frombuffer(data, dtype=np.uint8) if not isinstance(data, np.ndarray) else data)
+    p = transcode_params(restart_interval, transform, optimize)
+    return int(load_cuda_library().kpeg_transcode_bound(_ptr(buf), buf.size, C.byref(p)))
 
 
 def _image_shape(pixels: np.ndarray):
@@ -486,6 +516,38 @@ class Decoder:
             err.needed = n.value
             raise err
         self._check(rc, "kpeg_cuda_encode_device")
+        return n.value
+
+    # -- transcode ---------------------------------------------------------------------------------
+    def transcode(self, data, restart_interval: int = KPEG_TRANSCODE_KEEP_RESTART, transform: int = KPEG_XFORM_NONE,
+                  optimize: bool = False) -> bytes:
+        """Lossless transcode on the GPU (kpeg_cuda_transcode): the same quantised coefficients, moved by `transform`
+        (KPEG_XFORM_*), re-coded with another restart interval (-1 keeps the input's) and Annex K or, optimize, per-image
+        Huffman tables."""
+        buf = np.ascontiguousarray(np.frombuffer(data, dtype=np.uint8) if not isinstance(data, np.ndarray) else data)
+        p = transcode_params(restart_interval, transform, optimize)
+        cap = self._lib.kpeg_transcode_bound(_ptr(buf), buf.size, C.byref(p))
+        out = np.empty(max(int(cap), 1), dtype=np.uint8)
+        n = C.c_size_t(0)
+        rc = self._lib.kpeg_cuda_transcode(self._h, _ptr(buf), buf.size, C.byref(p), _ptr(out), cap, C.byref(n),
+                                           C.byref(self.last_stats))
+        self._check(rc, "kpeg_cuda_transcode")
+        return out[:n.value].tobytes()
+
+    def transcode_into(self, data, out: np.ndarray, restart_interval: int = KPEG_TRANSCODE_KEEP_RESTART,
+                       transform: int = KPEG_XFORM_NONE, optimize: bool = False) -> int:
+        """kpeg_cuda_transcode into a caller's buffer (pinned for speed); returns the length.  A buffer below it raises
+        KpegError(KPEG_ERR_NOMEM) with the size needed in `.needed`."""
+        buf = np.ascontiguousarray(np.frombuffer(data, dtype=np.uint8) if not isinstance(data, np.ndarray) else data)
+        p = transcode_params(restart_interval, transform, optimize)
+        n = C.c_size_t(0)
+        rc = self._lib.kpeg_cuda_transcode(self._h, _ptr(buf), buf.size, C.byref(p), _ptr(out), out.nbytes, C.byref(n),
+                                           C.byref(self.last_stats))
+        if rc == KPEG_ERR_NOMEM:
+            err = KpegError(rc, f"kpeg_cuda_transcode: {n.value} bytes needed, {out.nbytes} given")
+            err.needed = n.value
+            raise err
+        self._check(rc, "kpeg_cuda_transcode")
         return n.value
 
     def decode_batch_packed_device(self, plan: Plan, n: int, d_packed: int, packed_len: int, d_out: int):

@@ -674,6 +674,12 @@ cudaError_t launch_encode(const EncGeom &g, const EncBufs &b, cudaStream_t s, ui
         dc = b.dc;
         mark(user, KPEG_T_DC_SCAN);
     }
+    return launch_coded_stages(g, b, dc, s, launches, mark, user);
+}
+
+cudaError_t launch_coded_stages(const EncGeom &g, const EncBufs &b, const int16_t *dc, cudaStream_t s, uint32_t *launches, StageMark mark,
+                                void *user)
+{
     const unsigned bgrid = (unsigned)((g.nblk + THREADS - 1) / THREADS);
     // EH, EB: this image's tables, and the header after the host's prefix
     const EncTables *codes = b.tables;

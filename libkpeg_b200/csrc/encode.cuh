@@ -7,6 +7,7 @@
 #include <stdint.h>
 
 #include "encode_core.h"
+#include "transcode_core.h"
 
 namespace kpeg {
 namespace enc {
@@ -15,6 +16,8 @@ struct EncMeta {
     uint64_t unstuffed; // bytes of the unstuffed stream (segments padded to bytes)
     uint64_t scan_len;  // bytes written after the header: stuffed scan + RSTn markers + EOI
     uint64_t hdr_len;   // bytes of the header, where the scan starts (written by EB in optimised mode, else by E5)
+    uint32_t range_fail; // transcode only: TG found a coefficient no baseline table codes (transcode_core.h)
+    uint32_t pad;
 };
 
 // Device buffers of one encode (sizes: scratch_sizes).
@@ -48,7 +51,17 @@ typedef void (*StageMark)(void *user, int stage);
 
 // Enqueues E1..E5 on `s` (with EH and EB between E2 and E3 in optimised mode).  Returns cudaSuccess or the first launch error.
 cudaError_t launch_encode(const EncGeom &g, const EncBufs &b, cudaStream_t s, uint32_t *launches, StageMark mark, void *user);
+// The stages after E2 (EH and EB in optimised mode, then E3..E5) on b.coef and the final DC values dc: what
+// launch_encode runs after E1 / E2, and what the transcoder runs after TG.
+cudaError_t launch_coded_stages(const EncGeom &g, const EncBufs &b, const int16_t *dc, cudaStream_t s, uint32_t *launches,
+                                StageMark mark, void *user);
 
 } // namespace enc
+
+namespace tc {
+// TG (transcode.cu): the decoder's coefficient tiles -> coef [nblk][64] and dc [nblk] of the output, moved by g.xform;
+// *fail |= 1 when a value breaks the baseline range rules (zero it before).
+void launch_gather(const TcGeom &g, const void *tiles, int16_t *coef, int16_t *dc, uint32_t *fail, cudaStream_t s, uint32_t *launches);
+} // namespace tc
 } // namespace kpeg
 #endif

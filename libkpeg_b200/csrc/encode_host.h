@@ -42,11 +42,10 @@ inline void build_tables(int quality, EncTables *T)
 // SOI .. SOF0: what comes before the Huffman tables (the host writes it in both modes)
 inline std::vector<uint8_t> file_prefix(int width, int height, int ncomp, int quality)
 {
-    uint8_t qnat[2][64];
-    jfif::scaled_qt(jfif::kLumaQ, quality, qnat[0]);
-    jfif::scaled_qt(jfif::kChromaQ, quality, qnat[1]);
+    uint8_t qzz[4][64];
+    jfif::encoder_qzz(quality, qzz);
     std::vector<uint8_t> o;
-    jfif::write_frame_prefix(o, width, height, ncomp, qnat);
+    jfif::write_frame_prefix(o, width, height, ncomp, jfif::kEncoderTq, qzz);
     return o;
 }
 

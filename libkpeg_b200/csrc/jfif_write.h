@@ -138,20 +138,39 @@ inline void put_dri(std::vector<uint8_t> &o, int dri)
 inline const uint8_t *const kAnnexKBits[4] = {kDcLumaBits, kAcLumaBits, kDcChromaBits, kAcChromaBits};
 inline const uint8_t *const kAnnexKVals[4] = {kDcVals, kAcLumaVals, kDcVals, kAcChromaVals};
 
-// SOI, APP0 (JFIF 1.1), DQT id0 [, DQT id1], SOF0: the part of the header that does not depend on the Huffman
-// tables.  qnat: the scaled tables in natural order, [0] luma, [1] chroma.
-inline void write_frame_prefix(std::vector<uint8_t> &o, int W, int H, int nc, const uint8_t qnat[2][64])
+// The encoder's quantiser ids: luma table 0 for component 0, chroma table 1 for components 1 and 2.
+inline constexpr uint8_t kEncoderTq[3] = {0, 1, 1};
+
+// The encoder's quantisers for `quality` in zig-zag order, by id ([0] luma, [1] chroma; [2], [3] unused, zeroed).
+inline void encoder_qzz(int quality, uint8_t qzz[4][64])
+{
+    uint8_t qnat[2][64];
+    scaled_qt(kLumaQ, quality, qnat[0]);
+    scaled_qt(kChromaQ, quality, qnat[1]);
+    std::memset(qzz, 0, 4 * 64);
+    for (int t = 0; t < 2; ++t)
+        for (int i = 0; i < 64; ++i)
+            qzz[t][i] = qnat[t][kZZ.nat[i]];
+}
+
+// SOI, APP0 (JFIF 1.1), one DQT per quantiser id the components use (ascending), SOF0: the part of the header that does
+// not depend on the Huffman tables.  tq: each component's quantiser id; qzz: the tables by id, zig-zag order.
+inline void write_frame_prefix(std::vector<uint8_t> &o, int W, int H, int nc, const uint8_t tq[3], const uint8_t qzz[4][64])
 {
     const uint8_t soi_app0[] = {0xFF, 0xD8, 0xFF, 0xE0, 0x00, 0x10, 'J',  'F',  'I',  'F',
                                 0x00, 0x01, 0x01, 0x01, 0x00, 0x48, 0x00, 0x48, 0x00, 0x00};
     o.insert(o.end(), soi_app0, soi_app0 + sizeof soi_app0);
-    for (int t = 0; t < (nc == 3 ? 2 : 1); ++t) {
+    for (int t = 0; t < 4; ++t) {
+        bool used = false;
+        for (int c = 0; c < nc; ++c)
+            used |= tq[c] == t;
+        if (!used)
+            continue;
         o.push_back(0xFF);
         o.push_back(0xDB);
         put16(o, 67);
         o.push_back((uint8_t)t);
-        for (int i = 0; i < 64; ++i)
-            o.push_back(qnat[t][kZZ.nat[i]]);
+        o.insert(o.end(), qzz[t], qzz[t] + 64);
     }
     o.push_back(0xFF);
     o.push_back(0xC0);
@@ -163,16 +182,16 @@ inline void write_frame_prefix(std::vector<uint8_t> &o, int W, int H, int nc, co
     for (int c = 0; c < nc; ++c) {
         o.push_back((uint8_t)(c + 1));
         o.push_back(0x11);
-        o.push_back((uint8_t)(c ? 1 : 0));
+        o.push_back(tq[c]);
     }
 }
 
 // The prefix, then DHT 0x00, 0x10 [, 0x01, 0x11] with the given tables (Annex K by default) [, DRI when dri > 0]:
 // everything up to the first SOS.
-inline void write_frame_header(std::vector<uint8_t> &o, int W, int H, int nc, const uint8_t qnat[2][64], int dri,
+inline void write_frame_header(std::vector<uint8_t> &o, int W, int H, int nc, const uint8_t tq[3], const uint8_t qzz[4][64], int dri,
                                const uint8_t *const bits[4] = kAnnexKBits, const uint8_t *const vals[4] = kAnnexKVals)
 {
-    write_frame_prefix(o, W, H, nc, qnat);
+    write_frame_prefix(o, W, H, nc, tq, qzz);
     for (int t = 0; t < (nc == 3 ? 4 : 2); ++t)
         put_dht(o, ((t & 1) << 4) | (t >> 1), bits[t], vals[t]);
     if (dri > 0)

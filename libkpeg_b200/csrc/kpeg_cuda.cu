@@ -26,6 +26,7 @@
 #include "kernels.cuh"
 #include "kpeg_common.h"
 #include "kpeg_cuda.h"
+#include "transcode_host.h"
 
 using namespace kpeg;
 
@@ -706,6 +707,41 @@ void zero_stats(kpeg_stats *stats)
 {
     if (stats)
         memset(stats, 0, sizeof *stats);
+}
+
+// The three scans of a frame coded one scan per component, entropy-decoded one after another on lane 0 into the
+// components' tiles ctx->scan_tiles[c] (nmcu_padded blocks each); their figures are added to *stats.
+int entropy_decode_component_scans(kpeg_ctx *ctx, const kpeg_scan *scans, const uint8_t *file, uint32_t flags, uint32_t nmcu_padded,
+                                   kpeg_stats *stats)
+{
+    Lane &L = ctx->lane[0];
+    cudaStream_t s = L.stream;
+    for (int c = 0; c < 3; ++c)
+        TRY(ensure(ctx, s, ctx->scan_tiles[c], (size_t)nmcu_padded * 128u + 256u));
+    kpeg_stats part;
+    for (int k = 0; k < 3; ++k) {
+        kpeg_plan pl = scans[k].plan;
+        pl.flags = flags;
+        TRY(ensure(ctx, s, L.scan, scans[k].len + 64));
+        mark(ctx, L, -1);
+        CK(cudaMemcpyAsync(L.scan.p, file + scans[k].off, scans[k].len, cudaMemcpyHostToDevice, s));
+        mark(ctx, L, KPEG_T_H2D);
+        TRY(job_enqueue(ctx, 0, &pl, (const uint8_t *)L.scan.p, scans[k].len, 1, nullptr, {}, ctx->scan_tiles[scans[k].comp[0]].p));
+        memset(&part, 0, sizeof part);
+        TRY(job_finish(ctx, 0, stats ? &part : nullptr));
+        if (stats) {
+            stats->scan_bytes += part.scan_bytes;
+            stats->unstuffed_bytes += part.unstuffed_bytes;
+            stats->segments += part.segments;
+            stats->subsequences += part.subsequences;
+            stats->sync_rounds = std::max(stats->sync_rounds, part.sync_rounds);
+            stats->kernel_launches += part.kernel_launches;
+            for (int t = 0; t < KPEG_T_COUNT; ++t)
+                stats->ms[t] += part.ms[t];
+            stats->ms_total += part.ms_total;
+        }
+    }
+    return KPEG_OK;
 }
 
 // One large restart-marked image from host memory: bands of whole MCU rows, each a complete image of the same width
@@ -1530,32 +1566,8 @@ extern "C" int kpeg_cuda_decode_scans(kpeg_ctx *ctx, const kpeg_plan *frame, con
         return fail(ctx, grc, why);
     const uint32_t nstrips = (g3.mcus_per_image + IDCT_MCUS_PER_CTA - 1) / IDCT_MCUS_PER_CTA;
     const uint32_t nmcu_padded = nstrips * IDCT_MCUS_PER_CTA;
-    for (int c = 0; c < 3; ++c)
-        TRY(ensure(ctx, s, ctx->scan_tiles[c], (size_t)nmcu_padded * 128u + 256u));
-    kpeg_stats part;
+    TRY(entropy_decode_component_scans(ctx, scans, file, frame->flags, nmcu_padded, stats));
     uint32_t launches = 0;
-    for (int k = 0; k < 3; ++k) {
-        kpeg_plan pl = scans[k].plan;
-        pl.flags = frame->flags;
-        TRY(ensure(ctx, s, L.scan, scans[k].len + 64));
-        mark(ctx, L, -1);
-        CK(cudaMemcpyAsync(L.scan.p, file + scans[k].off, scans[k].len, cudaMemcpyHostToDevice, s));
-        mark(ctx, L, KPEG_T_H2D);
-        TRY(job_enqueue(ctx, 0, &pl, (const uint8_t *)L.scan.p, scans[k].len, 1, nullptr, {}, ctx->scan_tiles[scans[k].comp[0]].p));
-        memset(&part, 0, sizeof part);
-        TRY(job_finish(ctx, 0, stats ? &part : nullptr));
-        if (stats) {
-            stats->scan_bytes += part.scan_bytes;
-            stats->unstuffed_bytes += part.unstuffed_bytes;
-            stats->segments += part.segments;
-            stats->subsequences += part.subsequences;
-            stats->sync_rounds = std::max(stats->sync_rounds, part.sync_rounds);
-            stats->kernel_launches += part.kernel_launches;
-            for (int t = 0; t < KPEG_T_COUNT; ++t)
-                stats->ms[t] += part.ms[t];
-            stats->ms_total += part.ms_total;
-        }
-    }
     // the frame's tables (quantisers of the three components) for K3
     kpeg_plan fp = *frame;
     for (int c = 0; c < 3; ++c) { // K3 needs no Huffman tables, but the device tables are built from a whole plan
@@ -1824,34 +1836,39 @@ std::vector<uint8_t> encode_host_header(const kpeg_encode_params *p)
                                : enc::file_header(p->width, p->height, p->ncomp, p->quality, p->restart_interval);
 }
 
-// Tables (per quality) and scratch, then E1..E5 on lane 0 and the read-back of the length words into h_meta.
-// d_out / out_cap: the file and how many bytes may be written there; hdr_len: bytes of it the host has written.
-int encode_enqueue(kpeg_ctx *ctx, const kpeg_encode_params *p, const uint8_t *d_pixels, uint8_t *d_out, uint64_t out_cap,
-                   uint64_t hdr_len, uint32_t *launches)
+// The cached encoder tables (Annex K codes, the quantisers and cosines of `quality`), rebuilt when the quality changes.
+int encode_tables(kpeg_ctx *ctx, int quality)
 {
     EncScratch &E = ctx->enc;
     cudaStream_t s = ctx->lane[0].stream;
-    if (E.quality != p->quality) {
-        CK(cudaStreamSynchronize(s)); // nothing may still read the old tables or their staging copy
-        TRY(ensure_pinned(ctx, s, E.h_tables, sizeof(enc::EncTables)));
-        TRY(ensure(ctx, s, E.tables, sizeof(enc::EncTables)));
-        enc::build_tables(p->quality, (enc::EncTables *)E.h_tables.p);
-        CK(cudaMemcpyAsync(E.tables.p, E.h_tables.p, sizeof(enc::EncTables), cudaMemcpyHostToDevice, s));
-        E.quality = p->quality;
-    }
-    const enc::EncGeom g = enc::geometry(p->width, p->height, p->ncomp, p->restart_interval, p->flags);
+    if (E.quality == quality)
+        return KPEG_OK;
+    CK(cudaStreamSynchronize(s)); // nothing may still read the old tables or their staging copy
+    TRY(ensure_pinned(ctx, s, E.h_tables, sizeof(enc::EncTables)));
+    TRY(ensure(ctx, s, E.tables, sizeof(enc::EncTables)));
+    enc::build_tables(quality, (enc::EncTables *)E.h_tables.p);
+    CK(cudaMemcpyAsync(E.tables.p, E.h_tables.p, sizeof(enc::EncTables), cudaMemcpyHostToDevice, s));
+    E.quality = quality;
+    return KPEG_OK;
+}
+
+// The encoder's scratch for geometry g, and b's pointers into it (all but pixels and the output).
+int encode_scratch(kpeg_ctx *ctx, const enc::EncGeom &g, enc::EncBufs *bp)
+{
+    EncScratch &E = ctx->enc;
+    cudaStream_t s = ctx->lane[0].stream;
     size_t sz[enc::BUF_COUNT];
     enc::scratch_sizes(g, sz);
     for (int i = 0; i < enc::BUF_COUNT; ++i)
         TRY(ensure(ctx, s, E.buf[i], sz[i] + 16));
     TRY(ensure(ctx, s, E.meta, sizeof(enc::EncMeta)));
     TRY(ensure_pinned(ctx, s, E.h_meta, sizeof(enc::EncMeta)));
-    if (encode_optimized(p)) {
+    if (g.flags & KPEG_FLAG_OPTIMIZE_HUFFMAN) {
         TRY(ensure(ctx, s, E.opt_tables, sizeof(enc::EncTables)));
         TRY(ensure(ctx, s, E.hist, 4u * huff::NSYM * sizeof(uint64_t)));
     }
-    enc::EncBufs b;
-    b.pixels = d_pixels;
+    enc::EncBufs &b = *bp;
+    b = enc::EncBufs();
     b.tables = (const enc::EncTables *)E.tables.p;
     b.opt_tables = (enc::EncTables *)E.opt_tables.p;
     b.hist = (uint64_t *)E.hist.p;
@@ -1866,6 +1883,21 @@ int encode_enqueue(kpeg_ctx *ctx, const kpeg_encode_params *p, const uint8_t *d_
     b.agg = E.buf[enc::BUF_AGG].p;
     b.tile_ff = (uint64_t *)E.buf[enc::BUF_TILE_FF].p;
     b.meta = (enc::EncMeta *)E.meta.p;
+    return KPEG_OK;
+}
+
+// Tables (per quality) and scratch, then E1..E5 on lane 0 and the read-back of the length words into h_meta.
+// d_out / out_cap: the file and how many bytes may be written there; hdr_len: bytes of it the host has written.
+int encode_enqueue(kpeg_ctx *ctx, const kpeg_encode_params *p, const uint8_t *d_pixels, uint8_t *d_out, uint64_t out_cap,
+                   uint64_t hdr_len, uint32_t *launches)
+{
+    EncScratch &E = ctx->enc;
+    cudaStream_t s = ctx->lane[0].stream;
+    TRY(encode_tables(ctx, p->quality));
+    const enc::EncGeom g = enc::geometry(p->width, p->height, p->ncomp, p->restart_interval, p->flags);
+    enc::EncBufs b;
+    TRY(encode_scratch(ctx, g, &b));
+    b.pixels = d_pixels;
     b.out = d_out;
     b.out_cap = out_cap;
     b.hdr_len = hdr_len;
@@ -1973,5 +2005,172 @@ extern "C" int kpeg_cuda_encode_device(kpeg_ctx *ctx, const kpeg_encode_params *
     *jpeg_len = m->hdr_len + m->scan_len;
     if (*jpeg_len > cap)
         return fail(ctx, KPEG_ERR_NOMEM, "output buffer smaller than the encoded file (*jpeg_len = the size needed)");
+    return KPEG_OK;
+}
+
+// ==================================================================================================
+// Lossless transcode (csrc/transcode.cu, then the encoder's coded stages)
+// ==================================================================================================
+
+namespace {
+
+// What the output takes from the input: size, components, each component's quantiser id and the table in force when its
+// scan began, and the first scan's restart interval.  Two components that name one id with different tables (a DQT
+// redefined between the scans of a frame coded one scan per component) cannot share one DQT: KPEG_ERR_UNSUPPORTED.
+int transcode_input(const kpeg_plan &frame, const kpeg_scan *scans, int nscans, tc::TcInput &in, const char **why)
+{
+    memset(&in, 0, sizeof in);
+    in.width = frame.width;
+    in.height = frame.height;
+    in.ncomp = frame.ncomp;
+    in.restart = scans[0].plan.restart_interval;
+    bool have[4] = {false, false, false, false};
+    for (int k = 0; k < nscans; ++k)
+        for (int j = 0; j < scans[k].plan.ncomp; ++j) {
+            const int id = scans[k].plan.comp_tq[j];
+            uint8_t q[64];
+            for (int i = 0; i < 64; ++i)
+                q[i] = (uint8_t)scans[k].plan.qt[id][i]; // 8-bit tables: the parser rejects Pq != 0
+            if (have[id] && memcmp(in.qzz[id], q, 64) != 0) {
+                *why = "two components use one quantiser id with different tables";
+                return KPEG_ERR_UNSUPPORTED;
+            }
+            memcpy(in.qzz[id], q, 64);
+            have[id] = true;
+            in.tq[scans[k].comp[j]] = (uint8_t)id;
+        }
+    return KPEG_OK;
+}
+
+// parse + transcode_input + tc::plan
+int transcode_plan(const uint8_t *file, size_t len, const kpeg_transcode_params *p, kpeg_plan *frame, kpeg_scan *scans, int *nscans,
+                   tc::TcPlan *pl, const char **why)
+{
+    const int prc = kpeg_parse_jfif_scans(file, len, frame, scans, KPEG_MAX_SCANS, nscans);
+    if (prc != KPEG_OK) {
+        *why = prc == KPEG_ERR_UNSUPPORTED ? "unsupported JPEG coding" : "malformed JFIF container";
+        return prc;
+    }
+    tc::TcInput in;
+    TRY(transcode_input(*frame, scans, *nscans, in, why));
+    return tc::plan(in, *p, *pl, why);
+}
+
+// every stage of the re-encode is reported in the slot of a decode's reconstruction
+void tc_mark(void *user, int)
+{
+    kpeg_ctx *ctx = (kpeg_ctx *)user;
+    mark(ctx, ctx->lane[0], KPEG_T_IDCT);
+}
+
+} // namespace
+
+extern "C" size_t kpeg_transcode_bound(const uint8_t *file, size_t len, const kpeg_transcode_params *p)
+{
+    if (!file || !p)
+        return 0;
+    kpeg_plan frame;
+    kpeg_scan scans[KPEG_MAX_SCANS];
+    int nscans = 0;
+    tc::TcPlan pl;
+    const char *why = nullptr;
+    if (transcode_plan(file, len, p, &frame, scans, &nscans, &pl, &why) != KPEG_OK)
+        return 0;
+    return (size_t)tc::bound(pl);
+}
+
+// K0..K2 in T.81 mode into lane 0's tiles (one scan per component: into the components' tiles, then interleaved), TG
+// into the encoder's coefficient buffers, the range flag read back, then the encoder's coded stages and the copy-out.
+extern "C" int kpeg_cuda_transcode(kpeg_ctx *ctx, const uint8_t *file, size_t len, const kpeg_transcode_params *p, uint8_t *out,
+                                   size_t cap, size_t *out_len, kpeg_stats *stats)
+{
+    if (!ctx || !file || !p || !out || !out_len)
+        return KPEG_ERR_ARG;
+    kpeg_plan frame;
+    kpeg_scan scans[KPEG_MAX_SCANS];
+    int nscans = 0;
+    tc::TcPlan pl;
+    const char *why = nullptr;
+    const int prc = transcode_plan(file, len, p, &frame, scans, &nscans, &pl, &why);
+    if (prc != KPEG_OK)
+        return fail(ctx, prc, why);
+    CK(cudaSetDevice(ctx->device));
+    zero_stats(stats);
+    finish_all_deferred(ctx);
+    Lane &L = ctx->lane[0];
+    cudaStream_t s = L.stream;
+    const enc::EncGeom &g = pl.g.out;
+    // decode to coefficient tiles, T.81 (no F1 rule)
+    const uint32_t nmcu = (uint32_t)((frame.width + 7u) / 8u) * ((frame.height + 7u) / 8u);
+    const uint32_t nmcu_padded = (nmcu + IDCT_MCUS_PER_CTA - 1) / IDCT_MCUS_PER_CTA * IDCT_MCUS_PER_CTA;
+    TRY(ensure(ctx, s, L.tiles, (size_t)nmcu_padded * frame.ncomp * 128u + 256u)); // job_enqueue's size: no regrowth there
+    uint32_t launches = 0;
+    if (nscans == 1) {
+        kpeg_plan dp = scans[0].plan;
+        dp.flags = 0;
+        TRY(ensure(ctx, s, L.scan, scans[0].len + 64));
+        mark(ctx, L, -1);
+        CK(cudaMemcpyAsync(L.scan.p, file + scans[0].off, scans[0].len, cudaMemcpyHostToDevice, s));
+        mark(ctx, L, KPEG_T_H2D);
+        TRY(job_enqueue(ctx, 0, &dp, (const uint8_t *)L.scan.p, scans[0].len, 1, nullptr, {}, L.tiles.p));
+        TRY(job_finish(ctx, 0, stats));
+    } else {
+        TRY(entropy_decode_component_scans(ctx, scans, file, 0u, nmcu_padded, stats));
+        mark(ctx, L, -1);
+        launch_interleave_tiles(ctx->scan_tiles[0].p, ctx->scan_tiles[1].p, ctx->scan_tiles[2].p, L.tiles.p, nmcu_padded, s, &launches);
+        mark(ctx, L, KPEG_T_ENTROPY_WRITE);
+        add_times(ctx, L, stats);
+    }
+    // TG, and the range rules checked before anything is coded
+    EncScratch &E = ctx->enc;
+    if (E.quality < 0)
+        TRY(encode_tables(ctx, 90)); // only the Annex K codes are read, and they do not depend on the quality
+    enc::EncBufs b;
+    TRY(encode_scratch(ctx, g, &b));
+    const bool opt = (p->flags & KPEG_FLAG_OPTIMIZE_HUFFMAN) != 0u;
+    const std::vector<uint8_t> hdr = tc::header(pl, opt);
+    const size_t out_cap = std::min<size_t>(cap, (size_t)tc::bound(pl));
+    TRY(ensure(ctx, s, E.out, out_cap + 64));
+    enc::EncMeta *d_meta = (enc::EncMeta *)E.meta.p, *h_meta = (enc::EncMeta *)E.h_meta.p;
+    mark(ctx, L, -1);
+    CK(cudaMemsetAsync(d_meta, 0, sizeof(enc::EncMeta), s));
+    tc::launch_gather(pl.g, L.tiles.p, b.coef, b.dc, &d_meta->range_fail, s, &launches);
+    mark(ctx, L, KPEG_T_IDCT);
+    CK(cudaMemcpyAsync(&h_meta->range_fail, &d_meta->range_fail, sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    CK(cudaGetLastError());
+    add_times(ctx, L, stats);
+    if (h_meta->range_fail)
+        return fail(ctx, KPEG_ERR_UNSUPPORTED, "a DC difference or an AC coefficient of the output is beyond what baseline tables code");
+    b.out = (uint8_t *)E.out.p;
+    b.out_cap = out_cap;
+    b.hdr_len = hdr.size();
+    mark(ctx, L, -1);
+    CK(enc::launch_coded_stages(g, b, b.dc, s, &launches, tc_mark, ctx));
+    CK(cudaMemcpyAsync(h_meta, d_meta, sizeof(enc::EncMeta), cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    CK(cudaGetLastError());
+    *out_len = h_meta->hdr_len + h_meta->scan_len;
+    const bool fits = *out_len <= cap;
+    if (fits) {
+        memcpy(out, hdr.data(), hdr.size());
+        CK(cudaMemcpyAsync(out + hdr.size(), (const uint8_t *)E.out.p + hdr.size(), *out_len - hdr.size(), cudaMemcpyDeviceToHost, s));
+        mark(ctx, L, KPEG_T_D2H);
+        CK(cudaStreamSynchronize(s));
+    }
+    if (ctx->guard)
+        TRY(check_guards(ctx, L));
+    if (stats) {
+        stats->width = g.width;
+        stats->height = g.height;
+        stats->ncomp = g.ncomp;
+        stats->scan_bytes = h_meta->scan_len;
+        stats->unstuffed_bytes = h_meta->unstuffed;
+        stats->segments = (uint32_t)g.nseg;
+        stats->kernel_launches += launches;
+        add_times(ctx, L, stats);
+    }
+    if (!fits)
+        return fail(ctx, KPEG_ERR_NOMEM, "output buffer smaller than the transcoded file (*out_len = the size needed)");
     return KPEG_OK;
 }

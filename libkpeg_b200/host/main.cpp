@@ -13,8 +13,12 @@
 //   --quality N  encoder: IJG quality 1..100 (default 90)
 //   --restart N  encoder: restart interval in MCUs (default 0: none)
 //   --optimize   encoder: Huffman tables optimised for the image (KPEG_FLAG_OPTIMIZE_HUFFMAN): smaller files
+//   kpeg <in.jpg> <out.jpg>   (the first file starts with FF D8) lossless transcode on the GPU (kpeg_cuda_transcode):
+//                        the same quantised coefficients, re-coded; --restart N (default: the input's interval),
+//                        --optimize, --transform none|flip-h|flip-v|transpose|transverse|rot90|rot180|rot270
 //   --devices L  several devices, e.g. 0-7 or 0,2,3: the restart-interval tiles of the image are spread over them
 //   --quiet      log only to kpeg.log
+#include <algorithm>
 #include <cctype>
 #include <cstdio>
 #include <cstdlib>
@@ -41,6 +45,8 @@ namespace
         std::cout << "--quality N                     : Encoder quality 1..100 (default 90)" << std::endl;
         std::cout << "--restart N                     : Encoder restart interval in MCUs (default 0: none)" << std::endl;
         std::cout << "--optimize                      : Encoder Huffman tables optimised for the image (smaller file)" << std::endl;
+        std::cout << "<in.jpg> <out.jpg>              : Transcode a baseline JPEG losslessly on the GPU" << std::endl;
+        std::cout << "--transform T                   : Transcode: none, flip-h, flip-v, transpose, transverse, rot90, rot180, rot270" << std::endl;
         std::cout << "-h                              : Print this help message and exit" << std::endl;
     }
 
@@ -58,7 +64,9 @@ namespace
         std::vector<int> devices;
         int quality = 90;
         int restart = 0;
+        bool restart_given = false;
         bool optimize = false;
+        std::string transform = "none";
     };
 
     // "0-3", "0,2,5", "1": device list of --devices
@@ -177,6 +185,77 @@ namespace
                                        << ( ncomp == 3 ? " components" : " component" ) << ") to " << out << ": " << len << " bytes";
     }
 
+    bool readFile( const std::string& filename, std::vector<uint8_t>& data )
+    {
+        std::ifstream in( filename, std::ios::binary );
+        if ( !in ) return false;
+        data.assign( std::istreambuf_iterator<char>( in ), std::istreambuf_iterator<char>() );
+        return true;
+    }
+
+    bool startsWithSOI( const std::string& filename )
+    {
+        std::ifstream in( filename, std::ios::binary );
+        unsigned char b[2] = { 0, 0 };
+        return in.read( (char*)b, 2 ) && b[0] == 0xFF && b[1] == 0xD8;
+    }
+
+    void transcodeJPEG( const std::string& in, const std::string& out, const Options& opt )
+    {
+        static const char* const names[] = { "none", "flip-h", "flip-v", "transpose", "transverse", "rot90", "rot180", "rot270" };
+        int xform = -1;
+        for ( int t = 0; t < 8; ++t )
+            if ( opt.transform == names[t] ) xform = t;
+        if ( !isValidFilename( out ) )
+        {
+            LOG(kpeg::Logger::Level::ERROR) << "Invalid output file name passed.";
+            return;
+        }
+        if ( xform < 0 || ( opt.restart_given && ( opt.restart < 0 || opt.restart > 65535 ) ) )
+        {
+            LOG(kpeg::Logger::Level::ERROR) << "An error ocurred while transcoding: --transform must be one of none, flip-h, flip-v, "
+                                               "transpose, transverse, rot90, rot180, rot270 and --restart 0..65535";
+            return;
+        }
+        std::vector<uint8_t> data;
+        if ( !readFile( in, data ) )
+        {
+            LOG(kpeg::Logger::Level::ERROR) << "An error ocurred while transcoding: cannot open " << in;
+            return;
+        }
+        kpeg_transcode_params p = {};
+        p.restart_interval = opt.restart_given ? opt.restart : KPEG_TRANSCODE_KEEP_RESTART;
+        p.transform = (uint32_t)xform;
+        p.flags = opt.optimize ? KPEG_FLAG_OPTIMIZE_HUFFMAN : 0u;
+        kpeg_ctx* ctx = nullptr;
+        if ( kpeg_cuda_acquire( opt.device, &ctx ) != KPEG_OK )
+        {
+            LOG(kpeg::Logger::Level::ERROR) << "An error ocurred while transcoding: no usable CUDA device (there is no CPU transcode path)";
+            return;
+        }
+        std::vector<uint8_t> jpeg( std::max<std::size_t>( kpeg_transcode_bound( data.data(), data.size(), &p ), 1 ) );
+        std::size_t len = 0;
+        const int rc = kpeg_cuda_transcode( ctx, data.data(), data.size(), &p, jpeg.data(), jpeg.size(), &len, nullptr );
+        const std::string err = rc == KPEG_OK ? "" : kpeg_cuda_last_error( ctx );
+        kpeg_cuda_release( opt.device, ctx );
+        if ( rc != KPEG_OK )
+        {
+            LOG(kpeg::Logger::Level::ERROR) << "An error ocurred while transcoding: " << in << ": " << err;
+            return;
+        }
+        std::ofstream o( out, std::ios::binary );
+        o.write( (const char*)jpeg.data(), (std::streamsize)len );
+        o.close();
+        if ( !o )
+        {
+            std::remove( out.c_str() );
+            LOG(kpeg::Logger::Level::ERROR) << "An error ocurred while transcoding: cannot write " << out;
+            return;
+        }
+        LOG(kpeg::Logger::Level::INFO) << "Transcoded " << in << " (" << data.size() << " bytes) to " << out << " (" << opt.transform
+                                       << "): " << len << " bytes";
+    }
+
     void decodeJPEG( const std::string& filename, const Options& opt )
     {
         if ( !isValidFilename( filename ) )
@@ -212,7 +291,8 @@ int main( int argc, char** argv )
             else if ( a == "--device" && i + 1 < argc ) opt.device = std::atoi( argv[++i] );
             else if ( a == "--devices" && i + 1 < argc ) opt.devices = parseDevices( argv[++i] );
             else if ( a == "--quality" && i + 1 < argc ) opt.quality = std::atoi( argv[++i] );
-            else if ( a == "--restart" && i + 1 < argc ) opt.restart = std::atoi( argv[++i] );
+            else if ( a == "--restart" && i + 1 < argc ) { opt.restart = std::atoi( argv[++i] ); opt.restart_given = true; }
+            else if ( a == "--transform" && i + 1 < argc ) opt.transform = argv[++i];
             else if ( a == "--optimize" ) opt.optimize = true;
             else args.push_back( a );
         }
@@ -232,6 +312,11 @@ int main( int argc, char** argv )
         if ( args.size() == 1 )
         {
             decodeJPEG( args[0], opt );
+            return EXIT_SUCCESS;
+        }
+        if ( args.size() == 2 && startsWithSOI( args[0] ) )
+        {
+            transcodeJPEG( args[0], args[1], opt );
             return EXIT_SUCCESS;
         }
         if ( args.size() == 2 )

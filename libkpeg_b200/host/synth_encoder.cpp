@@ -134,18 +134,18 @@ Geometry geometry(const kpeg_synth_params *p)
     return g;
 }
 
+int encode_coefficients(const kpeg_synth_coef_frame &f, const int16_t *coef, bool split, uint8_t **out, size_t *out_len);
+
 // The coding path over a pixel buffer [H][W][nc_content].
 int encode_pixels(const kpeg_synth_params *p, const uint8_t *px, uint8_t **out, size_t *out_len)
 {
     const Geometry g = geometry(p);
     const int nc = g.nc_file;
 
-    uint8_t qnat[2][64];
-    scaled_qt(kLumaQ, p->quality, qnat[0]);
-    scaled_qt(kChromaQ, p->quality, qnat[1]);
-
     double cs[8][8]; // cs[x][u] = C(u)/2 * cos((2x+1) u pi / 16)
     fdct_cosines(cs);
+    uint8_t qzz[4][64]; // the quantisers by id, zig-zag order
+    encoder_qzz(p->quality, qzz);
 
     // quantised coefficients, [mcu][comp][zig-zag]
     std::vector<int16_t> coef;
@@ -185,13 +185,13 @@ int encode_pixels(const kpeg_synth_params *p, const uint8_t *px, uint8_t **out, 
                             tmp[r * 8 + v] = s;
                         }
                     int16_t *zz = &coef[(m * nc + c) * 64];
-                    const uint8_t *qt = qnat[c ? 1 : 0];
+                    const uint8_t *qt = qzz[c ? 1 : 0];
                     for (int i = 0; i < 64; ++i) {
                         int u = kZZ.nat[i] >> 3, v = kZZ.nat[i] & 7;
                         double s = 0;
                         for (int r = 0; r < 8; ++r)
                             s += tmp[r * 8 + v] * cs[r][u];
-                        long qv = std::lround(s / qt[kZZ.nat[i]]);
+                        long qv = std::lround(s / qt[i]);
                         long lim = i == 0 ? 2047 : 1023;
                         zz[i] = (int16_t)std::max(-lim, std::min(lim, qv));
                     }
@@ -210,6 +210,7 @@ int encode_pixels(const kpeg_synth_params *p, const uint8_t *px, uint8_t **out, 
     }
 
     const int ri = p->restart_interval;
+    const bool emit_rst = ri > 0 && (p->flags & KPEG_SYNTH_EMIT_RESTART);
     if (p->flags & KPEG_SYNTH_QUIRK_FREE) {
         int prev[3] = {0, 0, 0};
         for (long m = 0; m < g.nmcu; ++m) {
@@ -237,18 +238,59 @@ int encode_pixels(const kpeg_synth_params *p, const uint8_t *px, uint8_t **out, 
         }
     }
 
+    kpeg_synth_coef_frame f = {};
+    f.width = g.W;
+    f.height = g.H;
+    f.ncomp = nc;
+    std::memcpy(f.tq, kEncoderTq, sizeof f.tq);
+    std::memcpy(f.qt, qzz, sizeof f.qt);
+    f.restart_interval = emit_rst ? ri : 0;
+    f.flags = p->flags & KPEG_SYNTH_OPTIMIZE_HUFFMAN;
+    return encode_coefficients(f, coef.data(), nc == 3 && (p->flags & KPEG_SYNTH_NON_INTERLEAVED), out, out_len);
+}
+
+// The baseline range rules: every DC difference (prediction per component, reset at every segment's first MCU) has
+// category <= 11, every AC coefficient is within +-1023.  Beyond them no baseline Huffman table has a symbol.
+bool codable(const kpeg_synth_coef_frame &f, const int16_t *coef, long nmcu)
+{
+    const int nc = f.ncomp, ri = f.restart_interval;
+    int pred[3] = {0, 0, 0};
+    for (long m = 0; m < nmcu; ++m) {
+        if (ri > 0 && m % ri == 0)
+            pred[0] = pred[1] = pred[2] = 0;
+        for (int c = 0; c < nc; ++c) {
+            const int16_t *zz = &coef[((size_t)m * nc + c) * 64];
+            if (category(zz[0] - pred[c]) > 11)
+                return false;
+            pred[c] = zz[0];
+            for (int i = 1; i < 64; ++i)
+                if (zz[i] < -1023 || zz[i] > 1023)
+                    return false;
+        }
+    }
+    return true;
+}
+
+// The coding path from quantised coefficients [mcu][comp][zig-zag] (DC absolute): header, the scan (or, split, one scan
+// per component), EOI.
+int encode_coefficients(const kpeg_synth_coef_frame &f, const int16_t *coef, bool split, uint8_t **out, size_t *out_len)
+{
+    const int nc = f.ncomp, ri = f.restart_interval;
+    const long nmcu = (long)((f.width + 7) / 8) * ((f.height + 7) / 8);
+    if (!codable(f, coef, nmcu))
+        return -1;
     std::vector<uint8_t> o;
-    o.reserve((size_t)g.nmcu * nc * 24 + 1024);
-    const bool emit_rst = ri > 0 && (p->flags & KPEG_SYNTH_EMIT_RESTART);
+    o.reserve((size_t)nmcu * nc * 24 + 1024);
+    const bool emit_rst = ri > 0;
     // the Huffman tables: Annex K, or -- KPEG_SYNTH_OPTIMIZE_HUFFMAN -- optimal for this image's symbol counts, counted
     // below exactly as the coding loop further down codes the symbols
     const uint8_t *bits[4] = {kDcLumaBits, kAcLumaBits, kDcChromaBits, kAcChromaBits};
     const uint8_t *vals[4] = {kDcVals, kAcLumaVals, kDcVals, kAcChromaVals};
     uint8_t opt_bits[4][16], opt_vals[4][256];
-    if (p->flags & KPEG_SYNTH_OPTIMIZE_HUFFMAN) {
+    if (f.flags & KPEG_SYNTH_OPTIMIZE_HUFFMAN) {
         uint64_t freq[4][256] = {};
         int pred[3] = {0, 0, 0};
-        for (long m = 0; m < g.nmcu; ++m) {
+        for (long m = 0; m < nmcu; ++m) {
             if (emit_rst && m && (m % ri) == 0)
                 pred[0] = pred[1] = pred[2] = 0;
             for (int c = 0; c < nc; ++c) {
@@ -277,18 +319,17 @@ int encode_pixels(const kpeg_synth_params *p, const uint8_t *px, uint8_t **out, 
             vals[t] = opt_vals[t];
         }
     }
-    write_frame_header(o, g.W, g.H, nc, qnat, emit_rst ? ri : 0, bits, vals);
+    write_frame_header(o, f.width, f.height, nc, f.tq, f.qt, ri, bits, vals);
     const HuffEnc dcL(bits[0], vals[0]), dcC(bits[2], vals[2]);
     const HuffEnc acL(bits[1], vals[1]), acC(bits[3], vals[3]);
     BitWriter bw(o);
     // one interleaved scan of all components, or -- KPEG_SYNTH_NON_INTERLEAVED -- one scan per component (T.81 A.2.3:
     // the MCU of a non-interleaved scan is one block, blocks in raster order; the restart interval counts those)
-    const bool split = nc == 3 && (p->flags & KPEG_SYNTH_NON_INTERLEAVED);
     for (int scan = 0; scan < (split ? nc : 1); ++scan) {
         const int c0 = split ? scan : 0, c1 = split ? scan + 1 : nc;
         write_sos(o, c0, c1);
         int pred[3] = {0, 0, 0};
-        for (long m = 0; m < g.nmcu; ++m) {
+        for (long m = 0; m < nmcu; ++m) {
             if (emit_rst && m && (m % ri) == 0) {
                 bw.flush_ones();
                 o.push_back(0xFF);
@@ -388,6 +429,18 @@ extern "C" int kpeg_synth_encode(const kpeg_synth_params *p, uint8_t **out, size
     for (auto &t : th)
         t.join();
     return encode_pixels(p, px.data(), out, out_len);
+}
+
+extern "C" int kpeg_synth_encode_coefficients(const kpeg_synth_coef_frame *f, const int16_t *coef, uint8_t **out, size_t *out_len)
+{
+    if (!f || !coef || !out || !out_len || f->width < 1 || f->height < 1 || f->width > 65535 || f->height > 65535 ||
+        (f->ncomp != 1 && f->ncomp != 3) || f->restart_interval < 0 || f->restart_interval > 65535 ||
+        (f->flags & ~KPEG_SYNTH_OPTIMIZE_HUFFMAN) != 0u)
+        return -1;
+    for (int c = 0; c < f->ncomp; ++c)
+        if (f->tq[c] > 3)
+            return -1;
+    return encode_coefficients(*f, coef, false, out, out_len);
 }
 
 extern "C" void kpeg_synth_free(uint8_t *buf) { std::free(buf); }

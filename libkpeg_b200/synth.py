@@ -41,6 +41,12 @@ class SynthParams:
                        self.seed, self.noise_amp, self.threads)
 
 
+class CoefFrame(C.Structure):
+    """struct kpeg_synth_coef_frame"""
+    _fields_ = [("width", C.c_int32), ("height", C.c_int32), ("ncomp", C.c_int32), ("tq", C.c_uint8 * 3),
+                ("qt", (C.c_uint8 * 64) * 4), ("restart_interval", C.c_int32), ("flags", C.c_uint32)]
+
+
 _lib = None
 
 
@@ -59,6 +65,9 @@ def _load():
         lib.kpeg_synth_encode_pixels.restype = C.c_int
         lib.kpeg_synth_encode_pixels.argtypes = [C.POINTER(_Params), C.c_void_p, C.POINTER(C.POINTER(C.c_uint8)),
                                                  C.POINTER(C.c_size_t)]
+        lib.kpeg_synth_encode_coefficients.restype = C.c_int
+        lib.kpeg_synth_encode_coefficients.argtypes = [C.POINTER(CoefFrame), C.c_void_p, C.POINTER(C.POINTER(C.c_uint8)),
+                                                       C.POINTER(C.c_size_t)]
         lib.kpeg_synth_pixels.restype = C.c_int
         lib.kpeg_synth_pixels.argtypes = [C.POINTER(_Params), C.c_void_p]
         _lib = lib
@@ -108,3 +117,35 @@ def synth_pixels(p: SynthParams) -> np.ndarray:
     if rc != 0:
         raise RuntimeError(f"kpeg_synth_pixels failed: {rc}")
     return out
+
+
+def synth_encode_coefficients(width: int, height: int, coef: np.ndarray, tq, qt, restart_interval: int = 0,
+                              optimize: bool = False) -> np.ndarray | None:
+    """The synth's coding path over quantised coefficients (kpeg_synth_encode_coefficients): coef [nblk, 64] int16,
+    MCU-interleaved, zig-zag, DC absolute; tq: each component's quantiser id; qt: {id: 64 values in zig-zag order}.
+    The reference of the GPU transcoder.  None when a value breaks the baseline range rules."""
+    lib = _load()
+    nc = len(tq)
+    f = CoefFrame()
+    f.width, f.height, f.ncomp = width, height, nc
+    for c, t in enumerate(tq):
+        f.tq[c] = t
+    for t, table in qt.items():
+        for i, v in enumerate(table):
+            f.qt[t][i] = int(v)
+    f.restart_interval = restart_interval
+    f.flags = OPTIMIZE_HUFFMAN if optimize else 0
+    cf = np.ascontiguousarray(coef, dtype=np.int16)
+    if cf.shape != (((width + 7) // 8) * ((height + 7) // 8) * nc, 64):
+        raise ValueError(f"expected {((width + 7) // 8) * ((height + 7) // 8) * nc} blocks of 64, got {cf.shape}")
+    out = C.POINTER(C.c_uint8)()
+    n = C.c_size_t(0)
+    rc = lib.kpeg_synth_encode_coefficients(C.byref(f), cf.ctypes.data, C.byref(out), C.byref(n))
+    if rc == -1:
+        return None
+    if rc != 0:
+        raise RuntimeError(f"kpeg_synth_encode_coefficients failed: {rc}")
+    try:
+        return np.ctypeslib.as_array(out, shape=(n.value,)).copy()
+    finally:
+        lib.kpeg_synth_free(out)
