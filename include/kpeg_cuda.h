@@ -38,6 +38,19 @@ extern "C" {
 /* Encode only (kpeg_encode_params.flags): code with Huffman tables optimised for the image (T.81 K.2) instead of the
  * Annex K ones.  The decode entry points ignore it. */
 #define KPEG_FLAG_OPTIMIZE_HUFFMAN 2u
+/* Decode only (kpeg_plan.flags and the `flags` argument of the file entry points): reduced-size output, what libjpeg's
+ * scale_num / scale_denom = 1/2, 1/4, 1/8 (djpeg -scale 1/N) give.  The image comes out ceil(W/N) x ceil(H/N) (libjpeg's
+ * jdiv_round_up), in the usual layouts.  The quantised coefficients are decoded exactly as at full size
+ * (KPEG_FLAG_REF_PARITY still selects the DC-difference rule); only the reconstruction differs: per 8x8 block the
+ * dequantised coefficients go through libjpeg-turbo's reduced IDCTs (jidctred.c: jpeg_idct_4x4, _2x2, _1x1; CONST_BITS 13,
+ * PASS1_BITS 2, 64-bit products, the post-IDCT range-limit table indexed with & 1023, which wraps) and three components
+ * through libjpeg's integer ycc_rgb_convert (SCALEBITS 16).  So at a reduced scale the colours are libjpeg's, not the
+ * reference's float path; at full size (no scale bits) nothing changes.  kpeg_output_size gives the output size.
+ * Encode and transcode reject these bits (KPEG_ERR_ARG). */
+#define KPEG_FLAG_SCALE_1_2 4u
+#define KPEG_FLAG_SCALE_1_4 8u
+#define KPEG_FLAG_SCALE_1_8 12u
+#define KPEG_FLAG_SCALE_MASK 12u
 
 /* One Huffman table as it appears in a DHT segment (Types.hpp:116, Decoder.cpp:366-459). */
 typedef struct kpeg_huff_spec {
@@ -74,7 +87,8 @@ enum {
     KPEG_T_ENTROPY_SCAN,   /* K1: segmented scan of slot counts and DC sums over the subsequences          */
     KPEG_T_ENTROPY_WRITE,  /* K2: record expansion + DC prediction -> coefficient tiles (or the Huffman final pass) */
     KPEG_T_DC_SCAN,        /* fallback only: DC prediction + tile conversion behind the Huffman final pass  */
-    KPEG_T_IDCT,           /* K3: fused dequant + IDCT + colour + store, and the exact re-evaluation pass  */
+    KPEG_T_IDCT,           /* K3: fused dequant + IDCT + colour + store, and the exact re-evaluation pass;
+                              reduced-size decodes (KPEG_FLAG_SCALE_*): the reduced-size reconstruction kernel */
     KPEG_T_D2H,            /* device -> host copy of the pixels (host-pointer entry points only)          */
     KPEG_T_RELAY_SPARSE,   /* K1: later relay rounds (work list only) up to the fixed point               */
     KPEG_T_IDCT_PATCH,     /* (not used: the exact pass is timed with KPEG_T_IDCT)                         */
@@ -84,7 +98,7 @@ enum {
 /* Per-decode statistics.  Stage times are filled only while profiling is enabled
  * (kpeg_cuda_set_profiling); they are CUDA-event times on the decode stream, in milliseconds. */
 typedef struct kpeg_stats {
-    uint32_t width, height, ncomp;
+    uint32_t width, height, ncomp; /* of the output image (the reduced size with KPEG_FLAG_SCALE_*) */
     uint64_t scan_bytes;        /* stuffed entropy-coded bytes handed in                  */
     uint64_t unstuffed_bytes;   /* after FF00 / RSTn removal                              */
     uint32_t segments;          /* restart intervals found (1 when there is no DRI)       */
@@ -97,6 +111,11 @@ typedef struct kpeg_stats {
 } kpeg_stats;
 
 typedef struct kpeg_ctx kpeg_ctx;
+
+/* Host-only: bytes of the decoded image of `plan` (its dimensions, components and KPEG_FLAG_SCALE_* bits); *w / *h (either
+ * may be NULL) receive the output width and height.  0 for a NULL plan or one with a zero dimension or 2 components.  Every
+ * "width*height*ncomp" below means this size when scale bits are set; a batch holds its images back to back at it. */
+size_t kpeg_output_size(const kpeg_plan *plan, uint32_t *w, uint32_t *h);
 
 /* ---- host-side container parse (no CUDA) --------------------------------------------------
  * Replaces JPEGDecoder::decodeImageFile's marker loop + parseSegmentInfo + the parse* members
@@ -165,7 +184,7 @@ int kpeg_cuda_memcpy_d2h(kpeg_ctx *ctx, void *dst, const void *src, size_t bytes
  * convertYCbCrToRGB (MCU.cpp:64-279) and Image::createImageFromMCUs (Image.cpp:20-86).
  *
  *  scan, scan_len : HOST pointer to the stuffed entropy-coded bytes (may contain RSTn markers).
- *  pixels_out     : HOST buffer of width*height*ncomp bytes; interleaved R,G,B rows top-down for
+ *  pixels_out     : HOST buffer of width*height*ncomp bytes (kpeg_output_size); interleaved R,G,B rows top-down for
  *                   ncomp==3 (the payload Image::dumpRawData writes, Image.cpp:129-135), one gray
  *                   byte per pixel for ncomp==1.
  * Synchronous: returns after the pixels are in pixels_out.  An image of 64 MB of pixels or more whose restart interval is
@@ -276,7 +295,7 @@ int kpeg_cuda_decode_tiled(const int *devices, int ndev, const kpeg_plan *plan, 
                            uint8_t *pixels_out, kpeg_stats *stats);
 int kpeg_cuda_decode_file_tiled(const int *devices, int ndev, const uint8_t *file, size_t len, uint32_t flags,
                                 uint8_t *pixels_out, size_t cap, kpeg_plan *plan_out, kpeg_stats *stats);
-/* Same, the frame assembled in DEVICE memory of dst_device (d_frame: height*width*ncomp bytes there): every band
+/* Same, the frame assembled in DEVICE memory of dst_device (d_frame: kpeg_output_size bytes there): every band
  * travels by one peer copy over NVLink (staged by the driver where there is no peer access), so a consumer on
  * dst_device never pays PCIe. */
 int kpeg_cuda_decode_tiled_device(const int *devices, int ndev, const kpeg_plan *plan, const uint8_t *scan, size_t scan_len,
@@ -290,7 +309,8 @@ int kpeg_cuda_decode_to_peer(kpeg_ctx *ctx, const kpeg_plan *plan, const uint8_t
 /* ---- output formats written on the GPU ------------------------------------------------------------------------
  * The file Image::dumpRawData writes (Image.cpp:108-140: P6 header, then R,G,B rows) assembled in device memory:
  * d_out[*ppm_off, *ppm_off + *ppm_len) holds it (ppm_off < 16 keeps the payload aligned for the kernels' vector
- * stores; d_out must be 16-byte aligned, cap >= 176 + 3*width*height).  One-component images come out as R = G = B. */
+ * stores; d_out must be 16-byte aligned, cap >= 176 + 3*width*height of the output size: with KPEG_FLAG_SCALE_* the header
+ * carries the reduced dimensions).  One-component images come out as R = G = B. */
 int kpeg_cuda_decode_ppm_device(kpeg_ctx *ctx, const kpeg_plan *plan, const uint8_t *d_scan, size_t scan_len, uint8_t *d_out,
                                 size_t cap, size_t *ppm_off, size_t *ppm_len, kpeg_stats *stats);
 /* Interleaved R,G,B (the decode output) -> three planes [3][npixels], both in device memory. */

@@ -9,6 +9,10 @@ raises when that library or a GPU is missing.
 from .api import (  # noqa: F401
     KPEG_FLAG_OPTIMIZE_HUFFMAN,
     KPEG_FLAG_REF_PARITY,
+    KPEG_FLAG_SCALE_1_2,
+    KPEG_FLAG_SCALE_1_4,
+    KPEG_FLAG_SCALE_1_8,
+    KPEG_FLAG_SCALE_MASK,
     KPEG_TRANSCODE_KEEP_RESTART,
     KPEG_XFORM_FLIP_H,
     KPEG_XFORM_FLIP_V,
@@ -24,6 +28,7 @@ from .api import (  # noqa: F401
     Plan,
     Stats,
     load_cuda_library,
+    output_shape,
     encode_bound,
     parse_jfif,
     ppm_header,

@@ -80,6 +80,23 @@ def build_emu_transcode() -> None:
           "-Wno-unknown-pragmas", f"-I{ROOT / 'include'}", f"-I{PKG / 'csrc'}", "-o", str(out), str(src)], cwd=emu)
 
 
+def build_emu_scaled() -> None:
+    """tests/emu: CPU replay of the reduced-size reconstruction (emu_scaled.cpp, over csrc/idct_reduced.h) and its C
+    reference restated from libjpeg (ref_scaled.c) -- test infrastructure."""
+    emu = ROOT / "tests" / "emu"
+    hdrs = [*sorted((PKG / "csrc").glob("*.h")), ROOT / "include" / "kpeg_cuda.h"]
+    for out, src, cmd in (
+        (emu / "libkpeg_emu_scaled.so", emu / "emu_scaled.cpp",
+         ["g++", "-std=c++17", "-O2", "-fPIC", "-shared", "-Wall", "-Wno-unknown-pragmas", f"-I{ROOT / 'include'}",
+          f"-I{PKG / 'csrc'}"]),
+        (emu / "libkpeg_ref_scaled.so", emu / "ref_scaled.c", ["gcc", "-std=c11", "-O2", "-fPIC", "-shared", "-Wall"]),
+    ):
+        deps = [src, *hdrs]
+        if out.exists() and all(out.stat().st_mtime >= d.stat().st_mtime for d in deps):
+            continue
+        _run([*cmd, "-o", str(out), str(src)], cwd=emu)
+
+
 def have_nvcc() -> bool:
     from shutil import which
     return which(os.environ.get("NVCC", "nvcc")) is not None

@@ -19,6 +19,9 @@ KPEG_ERR_FORMAT, KPEG_ERR_UNSUPPORTED, KPEG_ERR_STREAM = -1, -2, -3
 KPEG_ERR_NOMEM, KPEG_ERR_CUDA, KPEG_ERR_ARG, KPEG_ERR_NOT_CONVERGED = -4, -5, -6, -7
 KPEG_FLAG_REF_PARITY = 1
 KPEG_FLAG_OPTIMIZE_HUFFMAN = 2  # encode only: Huffman tables optimised for the image (T.81 K.2) instead of Annex K
+# decode only: reduced-size output (libjpeg's scale 1/2, 1/4, 1/8 with its reduced IDCTs and integer colour)
+KPEG_FLAG_SCALE_1_2, KPEG_FLAG_SCALE_1_4, KPEG_FLAG_SCALE_1_8, KPEG_FLAG_SCALE_MASK = 4, 8, 12, 12
+_SCALE_FLAGS = {1: 0, 2: KPEG_FLAG_SCALE_1_2, 4: KPEG_FLAG_SCALE_1_4, 8: KPEG_FLAG_SCALE_1_8}
 # lossless transforms of kpeg_cuda_transcode (numbered as libjpeg's JXFORM_CODE)
 KPEG_XFORM_NONE, KPEG_XFORM_FLIP_H, KPEG_XFORM_FLIP_V, KPEG_XFORM_TRANSPOSE = 0, 1, 2, 3
 KPEG_XFORM_TRANSVERSE, KPEG_XFORM_ROT90, KPEG_XFORM_ROT180, KPEG_XFORM_ROT270 = 4, 5, 6, 7
@@ -103,6 +106,7 @@ SYMBOLS = {
     "kpeg_cuda_decode_scans": (C.c_int, [_vp, C.POINTER(Plan), C.POINTER(Scan), C.c_int, _vp, C.c_size_t, _vp, C.POINTER(Stats)]),
     "kpeg_cuda_decode_files": (C.c_int, [_vp, C.c_int, C.POINTER(_vp), C.POINTER(C.c_size_t), C.c_uint32, C.POINTER(_vp), C.POINTER(C.c_size_t),
                                          C.POINTER(Plan), C.POINTER(C.c_int), C.POINTER(Stats)]),
+    "kpeg_output_size": (C.c_size_t, [C.POINTER(Plan), C.POINTER(C.c_uint32), C.POINTER(C.c_uint32)]),
     "kpeg_cuda_create": (C.c_int, [C.c_int, C.POINTER(_vp)]),
     "kpeg_cuda_destroy": (None, [_vp]),
     "kpeg_cuda_last_error": (C.c_char_p, [_vp]),
@@ -213,6 +217,35 @@ def parse_jfif_scans(data: bytes | np.ndarray):
     if rc != KPEG_OK:
         raise KpegError(rc, "kpeg_parse_jfif_scans")
     return frame, [scans[i] for i in range(n.value)]
+
+
+def scale_flags(flags: int, scale: int) -> int:
+    """`flags` with its KPEG_FLAG_SCALE_* bits set for an output of 1/scale the size (scale 1, 2, 4 or 8)."""
+    if scale not in _SCALE_FLAGS:
+        raise ValueError(f"scale must be 1, 2, 4 or 8, not {scale!r}")
+    return (flags & ~KPEG_FLAG_SCALE_MASK) | _SCALE_FLAGS[scale]
+
+
+def _scaled_flags(flags: int, scale: int | None) -> int:
+    """flags itself (scale None: its own KPEG_FLAG_SCALE_* bits decide), or flags asking for 1/scale the size"""
+    return flags if scale is None else scale_flags(flags, scale)
+
+
+def _scaled_plan(plan: Plan, scale: int | None) -> Plan:
+    """plan itself (scale None: its own flags decide), or a copy whose flags ask for 1/scale the size"""
+    if scale is None:
+        return plan
+    p = Plan.from_buffer_copy(plan)
+    p.flags = scale_flags(p.flags, scale)
+    return p
+
+
+def output_shape(plan: Plan) -> tuple:
+    """Shape of the decoded image of `plan` at the size its flags ask for (kpeg_output_size): (H, W, 3) or (H, W)."""
+    w, h = C.c_uint32(0), C.c_uint32(0)
+    if load_cuda_library().kpeg_output_size(C.byref(plan), C.byref(w), C.byref(h)) == 0:
+        raise KpegError(KPEG_ERR_ARG, "kpeg_output_size: bad plan geometry")
+    return (h.value, w.value, 3) if plan.ncomp == 3 else (h.value, w.value)
 
 
 def ppm_header(width: int, height: int) -> bytes:
@@ -337,7 +370,11 @@ class Decoder:
         return self._lib.kpeg_cuda_stream(self._h) or 0
 
     # -- decode -------------------------------------------------------------------------------
-    def decode_file(self, data, flags: int = KPEG_FLAG_REF_PARITY, out: np.ndarray | None = None) -> np.ndarray:
+    def decode_file(self, data, flags: int = KPEG_FLAG_REF_PARITY, out: np.ndarray | None = None,
+                    scale: int | None = None) -> np.ndarray:
+        """scale 1, 2, 4, 8: the image at 1/scale the size (sets the KPEG_FLAG_SCALE_* bits of flags; None: as flags has
+        them)."""
+        flags = _scaled_flags(flags, scale)
         buf = np.frombuffer(data, dtype=np.uint8) if not isinstance(data, np.ndarray) else data
         frame, scans = parse_jfif_scans(buf)
         if len(scans) == 1:
@@ -347,27 +384,29 @@ class Decoder:
         # one scan per component: kpeg_cuda_decode_scans
         frame.flags = flags
         buf = np.ascontiguousarray(buf)
-        shape = (frame.height, frame.width, frame.ncomp)
+        shape = output_shape(frame)
         if out is None:
             out = np.empty(shape, dtype=np.uint8)
-        assert out.nbytes == frame.height * frame.width * frame.ncomp and out.flags.c_contiguous
+        assert out.nbytes == int(np.prod(shape)) and out.flags.c_contiguous
         arr = (Scan * len(scans))(*scans)
         rc = self._lib.kpeg_cuda_decode_scans(self._h, C.byref(frame), arr, len(scans), _ptr(buf), buf.size, _ptr(out),
                                               C.byref(self.last_stats))
         self._check(rc, "kpeg_cuda_decode_scans")
         return out.reshape(shape)
 
-    def decode_files(self, files: list, flags: int = KPEG_FLAG_REF_PARITY):
+    def decode_files(self, files: list, flags: int = KPEG_FLAG_REF_PARITY, scale: int | None = None):
         """kpeg_cuda_decode_files: any mix of files in one call -> (list of images, or None where a file failed; list of
-        per-file return codes).  Files with identical plans are decoded as one batch."""
+        per-file return codes).  Files with identical plans are decoded as one batch.  scale: as in decode_file."""
+        flags = _scaled_flags(flags, scale)
         bufs = [np.ascontiguousarray(np.frombuffer(f, dtype=np.uint8) if not isinstance(f, np.ndarray) else f) for f in files]
         n = len(bufs)
         outs, shapes = [], []
         for b in bufs:
             try:
                 frame, _ = parse_jfif_scans(b)
-                shapes.append((frame.height, frame.width, 3) if frame.ncomp == 3 else (frame.height, frame.width))
-                outs.append(np.empty(int(frame.height) * frame.width * frame.ncomp, dtype=np.uint8))
+                frame.flags = flags
+                shapes.append(output_shape(frame))
+                outs.append(np.empty(int(np.prod(shapes[-1])), dtype=np.uint8))
             except KpegError:
                 shapes.append(None)
                 outs.append(np.empty(1, dtype=np.uint8))
@@ -380,21 +419,24 @@ class Decoder:
         codes = [int(r) for r in res]
         return [o.reshape(sh) if (c == KPEG_OK and sh is not None) else None for o, sh, c in zip(outs, shapes, codes)], codes
 
-    def decode_scan(self, plan: Plan, scan: np.ndarray, out: np.ndarray | None = None) -> np.ndarray:
+    def decode_scan(self, plan: Plan, scan: np.ndarray, out: np.ndarray | None = None, scale: int | None = None) -> np.ndarray:
+        """scale 1, 2, 4, 8 sets the plan's KPEG_FLAG_SCALE_* bits (None: as the plan has them)."""
+        plan = _scaled_plan(plan, scale)
         scan = np.ascontiguousarray(scan, dtype=np.uint8)
-        shape = (plan.height, plan.width, plan.ncomp) if plan.ncomp == 3 else (plan.height, plan.width)
+        shape = output_shape(plan)
         if out is None:
             out = np.empty(shape, dtype=np.uint8)
-        assert out.nbytes == plan.height * plan.width * plan.ncomp and out.flags.c_contiguous
+        assert out.nbytes == int(np.prod(shape)) and out.flags.c_contiguous
         rc = self._lib.kpeg_cuda_decode(self._h, C.byref(plan), _ptr(scan), scan.size, _ptr(out),
                                         C.byref(self.last_stats))
         self._check(rc, "kpeg_cuda_decode")
         return out.reshape(shape)
 
-    def decode_batch(self, plan: Plan, scans: list[np.ndarray], outs: list[np.ndarray] | None = None):
+    def decode_batch(self, plan: Plan, scans: list[np.ndarray], outs: list[np.ndarray] | None = None, scale: int | None = None):
+        plan = _scaled_plan(plan, scale)
         n = len(scans)
         scans = [np.ascontiguousarray(s, dtype=np.uint8) for s in scans]
-        shape = (plan.height, plan.width, plan.ncomp) if plan.ncomp == 3 else (plan.height, plan.width)
+        shape = output_shape(plan)
         if outs is None:
             outs = [np.empty(shape, dtype=np.uint8) for _ in range(n)]
         sp = (_vp * n)(*[_ptr(s) for s in scans])
@@ -425,7 +467,9 @@ class Decoder:
     def d2h(self, dst: np.ndarray, dptr: int):
         self._check(self._lib.kpeg_cuda_memcpy_d2h(self._h, _ptr(dst), dptr, dst.nbytes), "memcpy_d2h")
 
-    def decode_device(self, plan: Plan, d_scan: int, scan_len: int, d_out: int):
+    def decode_device(self, plan: Plan, d_scan: int, scan_len: int, d_out: int, scale: int | None = None):
+        """d_out receives output_shape(plan) bytes (with scale: of the plan at that scale)."""
+        plan = _scaled_plan(plan, scale)
         rc = self._lib.kpeg_cuda_decode_device(self._h, C.byref(plan), d_scan, scan_len, d_out,
                                                C.byref(self.last_stats))
         self._check(rc, "kpeg_cuda_decode_device")
@@ -477,8 +521,9 @@ class Decoder:
         self._pending.clear()
         self._check(rc, "kpeg_cuda_wait")
 
-    def decode_ppm_device(self, plan: Plan, d_scan: int, scan_len: int, d_out: int, cap: int):
+    def decode_ppm_device(self, plan: Plan, d_scan: int, scan_len: int, d_out: int, cap: int, scale: int | None = None):
         """GPU-side PPM writer (kpeg_cuda_decode_ppm_device) -> (offset, length) of the file inside d_out."""
+        plan = _scaled_plan(plan, scale)
         off, ln = C.c_size_t(0), C.c_size_t(0)
         rc = self._lib.kpeg_cuda_decode_ppm_device(self._h, C.byref(plan), d_scan, scan_len, d_out, cap, C.byref(off),
                                                    C.byref(ln), C.byref(self.last_stats))
@@ -556,13 +601,16 @@ class Decoder:
         self._check(rc, "kpeg_cuda_decode_batch_packed_device")
 
 
-def decode_file_tiled(devices: list[int], data, flags: int = KPEG_FLAG_REF_PARITY, out: np.ndarray | None = None):
+def decode_file_tiled(devices: list[int], data, flags: int = KPEG_FLAG_REF_PARITY, out: np.ndarray | None = None,
+                      scale: int | None = None):
     """One image over several GPUs (kpeg_cuda_decode_file_tiled): restart-interval bands, one per listed device, each
-    decoded into its rows of ONE host frame.  Returns (pixels, Stats)."""
+    decoded into its rows of ONE host frame (scale: as in Decoder.decode_file).  Returns (pixels, Stats)."""
     lib = load_cuda_library()
+    flags = _scaled_flags(flags, scale)
     buf = np.frombuffer(data, dtype=np.uint8) if not isinstance(data, np.ndarray) else data
     plan, _, _ = parse_jfif(buf)
-    shape = (plan.height, plan.width, plan.ncomp) if plan.ncomp == 3 else (plan.height, plan.width)
+    plan.flags = flags
+    shape = output_shape(plan)
     if out is None:
         out = np.empty(shape, dtype=np.uint8)
     dv = (C.c_int * len(devices))(*devices)
@@ -577,7 +625,7 @@ def decode_tiled(devices: list[int], plan: Plan, scan: np.ndarray, out: np.ndarr
     """kpeg_cuda_decode_tiled on an already parsed image: restart-interval bands of `scan`, one per listed device (a
     device may be listed several times: its bands then overlap their copies and kernels), into the rows of `out`."""
     lib = load_cuda_library()
-    assert out.nbytes == plan.height * plan.width * plan.ncomp and out.flags.c_contiguous and scan.flags.c_contiguous
+    assert out.nbytes == int(np.prod(output_shape(plan))) and out.flags.c_contiguous and scan.flags.c_contiguous
     dv = (C.c_int * len(devices))(*devices)
     st = Stats()
     rc = lib.kpeg_cuda_decode_tiled(dv, len(devices), C.byref(plan), _ptr(scan), scan.size, _ptr(out), C.byref(st))

@@ -10,6 +10,7 @@
 //
 //   stage 0  by the copy engine: the tile (12 KB for RGB) and the quantiser table arrive with bulk copies
 //            (cp.async.bulk + mbarrier, SASS UBLKCP); the tile that will run in this CTA's slot next is pulled into L2
+//            (k3_tile.cuh, shared with the reduced-size kernel of k3_scaled.cu)
 //   stage 1  one thread = one 8x8 block, all 64 values in registers, two fp32 lanes per instruction (FADD2 / FMUL2 /
 //            FFMA2): biased 16-bit -> fp32 by byte permute + one packed subtract (no I2F), dequantise (AAN prescale
 //            folded into the quantiser), de-zigzag by register renaming, separable fp32 IDCT, rounding, tie-band test;
@@ -32,6 +33,7 @@
 
 #include "entropy_core.h"
 #include "idct_core.h"
+#include "k3_tile.cuh"
 #include "kernels.cuh"
 #include "kpeg_common.h"
 
@@ -76,11 +78,6 @@ __device__ __forceinline__ int tie_sample(int w, int b)
     const int k = 15 - (b & 15);
     return (4 * w + (k >> 2)) * 8 + ((b & 16) ? 0 : 4) + (k & 3);
 }
-
-#ifndef KPEG_IDCT_PREFETCH_AHEAD
-#define KPEG_IDCT_PREFETCH_AHEAD 1184
-#endif
-constexpr uint32_t IDCT_PREFETCH_AHEAD = KPEG_IDCT_PREFETCH_AHEAD; // strips: 148 SMs x 8 CTAs, the strip that runs in this CTA's slot next
 
 constexpr int TIE_LIST_CAP = IDCT_TIE_LIST_CAP; // (block, sample) entries per strip; a strip with more walks its blocks' masks instead
 constexpr uint32_t TIE_EMPTY = 0xFFFFFFFFu;     // tie record without a pixel
@@ -284,35 +281,6 @@ __device__ __forceinline__ uint32_t colour_px(int y, int cb, int cr)
     return (uint32_t)clamp_u8(R) | ((uint32_t)clamp_u8(G) << 8) | ((uint32_t)clamp_u8(B) << 16);
 }
 
-// ---- bulk copies by the copy engine ------------------------------------------------------------------
-__device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count)
-{
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes)
-{
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity)
-{
-    asm volatile("{\n"
-                 ".reg .pred p;\n"
-                 "KPEG_MBAR_WAIT:\n"
-                 "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-                 "@p bra KPEG_MBAR_DONE;\n"
-                 "bra KPEG_MBAR_WAIT;\n"
-                 "KPEG_MBAR_DONE:\n"
-                 "}" ::"r"(bar), "r"(parity) : "memory");
-}
-__device__ __forceinline__ void bulk_load(uint32_t dst, const void *src, uint32_t bytes, uint32_t bar)
-{
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
-}
-
 // ---- colour of one pixel row of an MCU ---------------------------------------------------------------
 // Colour of the eight pixels of one row of an MCU -> 24 channel values, three variants chosen per MCU:
 //   COLOUR_PLAIN    ycc_to_rgb_fast's arithmetic on pixel pairs (FFMA2 / FADD2); its range precondition holds for
@@ -492,15 +460,7 @@ __global__ void __launch_bounds__(NC * IDCT_MCUS_PER_CTA, NC == 3 ? KPEG_IDCT_MI
     // ---- stage 0: tile and quantisers by the copy engine, strip origin ------------------------------------------
     const uint32_t bar = smem_u32(&sm.mbar);
     if (t == 0) {
-        constexpr uint32_t table_bytes = NC * 64u * 4u, tile_bytes = NB * 128u;
-        const char *tile = reinterpret_cast<const char *>(a.tiles) + (size_t)strip * tile_bytes;
-        mbar_init(bar, 1);
-        mbar_expect_tx(bar, table_bytes + tile_bytes);
-        bulk_load(smem_u32(sm.coef), tile, tile_bytes, bar);
-        bulk_load(smem_u32(sm.qpair), a.tables->qpair, table_bytes, bar);
-        // the tile of the strip that will run in this CTA's slot next: DRAM -> L2 now
-        if (strip + IDCT_PREFETCH_AHEAD < a.nstrips)
-            asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(tile + (size_t)IDCT_PREFETCH_AHEAD * tile_bytes), "r"(tile_bytes) : "memory");
+        k3_load_strip<NC>(a.tiles, strip, a.nstrips, sm.coef, a.tables->qpair, NC * 64u * 4u, sm.qpair, bar);
         sm.ntie = 0;
         sm.any_huge = 0;
         const uint32_t img = mcu0 / a.g.mcus_per_image, mi = mcu0 - img * a.g.mcus_per_image;
@@ -935,6 +895,8 @@ uint32_t k3_strip_slots(uint32_t ncomp) { return (uint32_t)IDCT_MCUS_PER_CTA * n
 
 cudaError_t launch_idct(const IdctArgs &a_in, cudaStream_t s, uint32_t *launches)
 {
+    if (scale_denom(a_in.g.flags) != 1u)
+        return launch_idct_scaled(a_in, s, launches);
     IdctArgs a = a_in;
     const uint32_t total_mcus = a.g.nimages * a.g.mcus_per_image;
     const uint32_t grid = (total_mcus + IDCT_MCUS_PER_CTA - 1) / IDCT_MCUS_PER_CTA;

@@ -143,7 +143,9 @@ void launch_matrix_from_tiles(const void *tiles, int16_t *coef, uint32_t total_b
 // three one-component tile sets (one scan per component) -> the MCU-interleaved tiles K3 consumes
 void launch_interleave_tiles(const void *t0, const void *t1, const void *t2, void *out, uint32_t nmcu_padded, cudaStream_t s,
                              uint32_t *launches);
+// K3, or -- when a.g.flags has KPEG_FLAG_SCALE_* bits -- the reduced-size reconstruction (k3_scaled.cu) in its place
 cudaError_t launch_idct(const IdctArgs &a, cudaStream_t s, uint32_t *launches);
+cudaError_t launch_idct_scaled(const IdctArgs &a, cudaStream_t s, uint32_t *launches);
 void k3_configure();                      // function attributes of the K3 kernels (called by kernels_configure)
 uint32_t k3_strip_slots(uint32_t ncomp);  // coefficient slots one K3 strip covers
 

@@ -109,6 +109,27 @@ struct JobGeom {
     uint32_t sub_bits;        // bits per speculative subsequence (multiple of 32)
 };
 
+// ---- output geometry ------------------------------------------------------------------------------------------
+// The decoded image of a plan: full size, or 1/2, 1/4, 1/8 of it (KPEG_FLAG_SCALE_* of kpeg_cuda.h: scale code in bits 2..3)
+// rounded up as libjpeg's jdiv_round_up does.  Every buffer size, row placement and copy of the decode path goes
+// through this one description.
+constexpr uint32_t SCALE_FLAG_SHIFT = 2u, SCALE_FLAG_MASK = 12u;
+KPEG_HD uint32_t scale_denom(uint32_t flags) { return 1u << ((flags & SCALE_FLAG_MASK) >> SCALE_FLAG_SHIFT); }
+
+struct OutGeom {
+    uint32_t width, height, ncomp; // of one output image
+    uint32_t scale;                // 1, 2, 4 or 8
+    KPEG_HD uint64_t row_bytes() const { return (uint64_t)width * ncomp; }
+    KPEG_HD uint64_t bytes() const { return row_bytes() * height; } // one image; a batch holds its images back to back
+    KPEG_HD uint32_t mcu_row(uint32_t r) const { return r * 8u / scale; } // output row where MCU row r begins
+};
+
+KPEG_HD OutGeom out_geom(uint32_t width, uint32_t height, uint32_t ncomp, uint32_t flags)
+{
+    const uint32_t s = scale_denom(flags);
+    return OutGeom{(width + s - 1u) / s, (height + s - 1u) / s, ncomp, s};
+}
+
 // First absolute coefficient slot (block*64 + zig-zag index) of restart segment `seg`.
 KPEG_HD uint32_t seg_slot_base(const JobGeom &g, uint32_t seg)
 {
@@ -118,6 +139,8 @@ KPEG_HD uint32_t seg_slot_base(const JobGeom &g, uint32_t seg)
     uint32_t r = seg - img * g.segs_per_image;
     return (img * g.mcus_per_image + r * g.restart_interval) * g.ncomp * 64u;
 }
+
+KPEG_HD OutGeom out_geom(const JobGeom &g) { return out_geom(g.width, g.height, g.ncomp, g.flags); }
 
 // ---- status word bits (device -> host) -----------------------------------------------------------
 constexpr uint32_t ST_BAD_CODE = 1u;       // a bit pattern that is no Huffman code was consumed by the final decode

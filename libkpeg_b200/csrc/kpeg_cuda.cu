@@ -157,6 +157,13 @@ struct kpeg_ctx {
 
 namespace {
 
+static_assert(SCALE_FLAG_MASK == KPEG_FLAG_SCALE_MASK && (KPEG_FLAG_SCALE_1_2 >> SCALE_FLAG_SHIFT) == 1u &&
+                  (KPEG_FLAG_SCALE_1_4 >> SCALE_FLAG_SHIFT) == 2u && (KPEG_FLAG_SCALE_1_8 >> SCALE_FLAG_SHIFT) == 3u,
+              "kpeg_common.h's scale codes (scale_denom) are kpeg_cuda.h's KPEG_FLAG_SCALE_*");
+
+// the decoded image of a plan (full size or reduced: KPEG_FLAG_SCALE_*)
+OutGeom out_of(const kpeg_plan *pl) { return out_geom(pl->width, pl->height, pl->ncomp, pl->flags); }
+
 int fail(kpeg_ctx *c, int code, const char *what, cudaError_t e = cudaSuccess)
 {
     char buf[512];
@@ -681,8 +688,9 @@ int job_finish(kpeg_ctx *ctx, int li, kpeg_stats *stats)
     ctx->last_lane = li;
     ctx->last_g = J.g;
     if (stats) {
-        stats->width = J.g.width;
-        stats->height = J.g.height;
+        const OutGeom o = out_geom(J.g);
+        stats->width = o.width;
+        stats->height = o.height;
         stats->ncomp = J.g.ncomp;
         stats->scan_bytes += J.scan_len;
         stats->unstuffed_bytes += h_meta->total_kept;
@@ -803,7 +811,6 @@ int decode_banded(kpeg_ctx *ctx, const kpeg_plan *plan, const uint8_t *scan, siz
         }
         mark(ctx, L, KPEG_T_H2D);
     }
-    const size_t row_bytes = (size_t)plan->width * plan->ncomp;
     int rc = KPEG_OK, used[NLANES], nused = 0;
     uint32_t row0 = 0; // first MCU row of the band
     for (uint32_t k = 0; k < parts && rc == KPEG_OK; ++k) {
@@ -821,12 +828,13 @@ int decode_banded(kpeg_ctx *ctx, const kpeg_plan *plan, const uint8_t *scan, siz
         const uint32_t y0 = row0 * 8u, y1 = std::min<uint32_t>((row0 + rows) * 8u, plan->height);
         kpeg_plan bp = *plan;
         bp.height = (uint16_t)(y1 - y0);
-        const size_t bpix = row_bytes * (y1 - y0);
+        const OutGeom bo = out_of(&bp); // the band's output: its rows begin where its first MCU row's do
+        const size_t bpix = bo.bytes();
         rc = ensure(ctx, L.stream, L.pixels, bpix + 64);
         if (rc != KPEG_OK)
             break;
         rc = job_enqueue(ctx, (int)k, &bp, (const uint8_t *)L.scan.p, end[k] - begin[k], 1, (uint8_t *)L.pixels.p,
-                         {Copy{pixels_out + (size_t)y0 * row_bytes, L.pixels.p, bpix}});
+                         {Copy{pixels_out + (size_t)bo.mcu_row(row0) * bo.row_bytes(), L.pixels.p, bpix}});
         if (rc == KPEG_OK)
             used[nused++] = (int)k;
         row0 += rows;
@@ -842,8 +850,9 @@ int decode_banded(kpeg_ctx *ctx, const kpeg_plan *plan, const uint8_t *scan, siz
     for (uint32_t k = 0; k < parts; ++k) // lanes whose copies were issued but whose band was never enqueued
         cudaStreamSynchronize(ctx->lane[k].stream);
     if (stats) {
-        stats->width = plan->width;
-        stats->height = plan->height;
+        const OutGeom o = out_of(plan);
+        stats->width = o.width;
+        stats->height = o.height;
     }
     return rc;
 }
@@ -853,6 +862,18 @@ int decode_banded(kpeg_ctx *ctx, const kpeg_plan *plan, const uint8_t *scan, siz
 // ==================================================================================================
 // C ABI
 // ==================================================================================================
+
+extern "C" size_t kpeg_output_size(const kpeg_plan *plan, uint32_t *w, uint32_t *h)
+{
+    if (!plan || plan->width == 0 || plan->height == 0 || (plan->ncomp != 1 && plan->ncomp != 3))
+        return 0;
+    const OutGeom o = out_of(plan);
+    if (w)
+        *w = o.width;
+    if (h)
+        *h = o.height;
+    return (size_t)o.bytes();
+}
 
 extern "C" int kpeg_cuda_device_count(void)
 {
@@ -1123,8 +1144,10 @@ extern "C" int kpeg_cuda_decode(kpeg_ctx *ctx, const kpeg_plan *plan, const uint
     Lane &L = ctx->lane[0];
     if (L.job.active) // a deferred job still reads this lane's scan / pixel buffers: complete it before they can move
         finish_deferred(ctx, 0);
-    const size_t npix = (size_t)plan->width * plan->height * plan->ncomp;
-    if (ctx->band_parts > 1 && plan->restart_interval != 0 && npix >= ((size_t)64 << 20)) {
+    // bands pay off for a large image whatever its output size: the decision is taken on the full-size pixels
+    const size_t full_pix = (size_t)plan->width * plan->height * plan->ncomp;
+    const size_t npix = out_of(plan).bytes();
+    if (ctx->band_parts > 1 && plan->restart_interval != 0 && full_pix >= ((size_t)64 << 20)) {
         const int brc = decode_banded(ctx, plan, scan, scan_len, pixels_out, stats);
         if (brc != KPEG_ERR_UNSUPPORTED) // UNSUPPORTED: the restart interval does not line up with MCU rows -- whole image below
             return brc;
@@ -1189,7 +1212,7 @@ extern "C" int kpeg_cuda_decode_batch_packed_device_split(kpeg_ctx *ctx, const k
                                                     d_pixels_out, stats);
     CK(cudaSetDevice(ctx->device));
     zero_stats(stats);
-    const size_t npix = (size_t)plan->width * plan->height * plan->ncomp;
+    const size_t npix = out_of(plan).bytes();
     const int parts = std::max(1, std::min({n, NLANES, ctx->split_parts}));
     for (int li = 0; li < parts; ++li) {
         const int lo = (int)((long long)n * li / parts), hi = (int)((long long)n * (li + 1) / parts);
@@ -1224,7 +1247,7 @@ extern "C" int kpeg_cuda_submit_batch_packed_device(kpeg_ctx *ctx, const kpeg_pl
     if (!ctx || !plan || n <= 0 || !d_packed || !packed_offsets || !d_pixels_out)
         return KPEG_ERR_ARG;
     CK(cudaSetDevice(ctx->device));
-    const size_t npix = (size_t)plan->width * plan->height * plan->ncomp;
+    const size_t npix = out_of(plan).bytes();
     // consecutive submissions already overlap; cutting one further only shortens its kernels (measured)
     const int parts = ctx->profiling ? 1 : std::max(1, std::min({n, NLANES, ctx->submit_parts}));
     for (int k = 0; k < parts; ++k) {
@@ -1302,7 +1325,7 @@ extern "C" int kpeg_cuda_submit_batch(kpeg_ctx *ctx, const kpeg_plan *plan, int 
     if (!ctx || !plan || n <= 0 || !scans || !scan_lens || !pixels_out)
         return KPEG_ERR_ARG;
     CK(cudaSetDevice(ctx->device));
-    const size_t npix = (size_t)plan->width * plan->height * plan->ncomp;
+    const size_t npix = out_of(plan).bytes(); // per output image
     // chunking: pipeline only when the pixel traffic is worth it (>= 32 MB); chunks of about 8 MB of pixels
     // or more each, at most host_chunks of them
     int per_chunk = n;
@@ -1442,7 +1465,7 @@ extern "C" int kpeg_cuda_decode_to_peer(kpeg_ctx *ctx, const kpeg_plan *plan, co
     Lane &L = ctx->lane[0];
     if (L.job.active)
         finish_deferred(ctx, 0);
-    const size_t npix = (size_t)plan->width * plan->height * plan->ncomp;
+    const size_t npix = out_of(plan).bytes();
     const bool local = dst_device == ctx->device && (reinterpret_cast<uintptr_t>(d_dst) & 7u) == 0;
     TRY(ensure(ctx, L.stream, L.scan, scan_len + 64));
     if (!local) {
@@ -1488,9 +1511,10 @@ extern "C" int kpeg_cuda_decode_ppm_device(kpeg_ctx *ctx, const kpeg_plan *plan,
     if (L.job.active)
         finish_deferred(ctx, 0);
     char header[160];
-    const int hl = kpeg_ppm_header(plan->width, plan->height, header, sizeof header);
+    const OutGeom o = out_of(plan);
+    const int hl = kpeg_ppm_header((int)o.width, (int)o.height, header, sizeof header);
     const size_t pad = (16u - (size_t)hl % 16u) % 16u;
-    const size_t npx = (size_t)plan->width * plan->height;
+    const size_t npx = (size_t)o.width * o.height;
     if (pad + (size_t)hl + npx * 3u > cap)
         return fail(ctx, KPEG_ERR_ARG, "PPM buffer too small");
     TRY(ensure_pinned(ctx, L.stream, L.h_stage, 256));
@@ -1577,7 +1601,8 @@ extern "C" int kpeg_cuda_decode_scans(kpeg_ctx *ctx, const kpeg_plan *frame, con
     memcpy(fp.ht, scans[0].plan.ht, sizeof fp.ht);
     memcpy(fp.ht_present, scans[0].plan.ht_present, sizeof fp.ht_present);
     TRY(upload_plan(ctx, &fp));
-    const size_t npix = (size_t)frame->width * frame->height * 3u;
+    const OutGeom o = out_of(frame);
+    const size_t npix = o.bytes();
     TRY(ensure(ctx, s, L.tiles, (size_t)nmcu_padded * 3u * 128u + 256u));
     TRY(ensure(ctx, s, L.pixels, npix + 64));
     TRY(ensure(ctx, s, L.tie_rec, (size_t)nstrips * IDCT_TIE_LIST_CAP * sizeof(uint4)));
@@ -1607,8 +1632,8 @@ extern "C" int kpeg_cuda_decode_scans(kpeg_ctx *ctx, const kpeg_plan *frame, con
     ctx->last_lane = 0;
     ctx->last_g = g3; // kpeg_cuda_read_coefficients: the interleaved tiles
     if (stats) {
-        stats->width = frame->width;
-        stats->height = frame->height;
+        stats->width = o.width;
+        stats->height = o.height;
         stats->ncomp = 3;
         stats->exact_samples += h_meta->exact_samples;
         stats->kernel_launches += launches;
@@ -1631,7 +1656,7 @@ extern "C" int kpeg_cuda_decode_file(kpeg_ctx *ctx, const uint8_t *file, size_t 
     frame.flags = flags;
     if (plan_out)
         *plan_out = frame;
-    if ((size_t)frame.width * frame.height * frame.ncomp > cap)
+    if (out_of(&frame).bytes() > cap)
         return fail(ctx, KPEG_ERR_ARG, "pixel buffer too small");
     return kpeg_cuda_decode_scans(ctx, &frame, scans, nscans, file, len, pixels_out, stats);
 }
@@ -1684,7 +1709,7 @@ extern "C" int kpeg_cuda_decode_files(kpeg_ctx *ctx, int n, const uint8_t *const
         f.frame.flags = flags;
         if (plans_out)
             plans_out[i] = f.frame;
-        if ((size_t)f.frame.width * f.frame.height * f.frame.ncomp > caps[i]) {
+        if (out_of(&f.frame).bytes() > caps[i]) {
             note(i, KPEG_ERR_ARG, "pixel buffer too small");
             continue;
         }

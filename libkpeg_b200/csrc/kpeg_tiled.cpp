@@ -14,6 +14,7 @@
 #include <thread>
 #include <vector>
 
+#include "kpeg_common.h"
 #include "kpeg_cuda.h"
 
 namespace {
@@ -73,7 +74,8 @@ struct BandJob {
     kpeg_plan plan;
     const uint8_t *scan = nullptr;
     size_t len = 0;
-    uint32_t row0 = 0, rows = 0; // pixel rows
+    uint32_t row0 = 0, rows = 0; // pixel rows of the full-size image
+    size_t out_off = 0;         // where the band's output rows begin in the frame (reduced-size decodes: the reduced rows)
     int rc = KPEG_OK;
     std::string err;
     kpeg_stats stats;
@@ -182,6 +184,8 @@ int make_bands(const int *devices, int ndev, const kpeg_plan *plan, const uint8_
         j.len = (size_t)(b1[(size_t)k] - b0[(size_t)k]);
         j.row0 = r0;
         j.rows = r1 - r0;
+        const kpeg::OutGeom o = kpeg::out_geom(plan->width, plan->height, plan->ncomp, plan->flags);
+        j.out_off = (size_t)o.mcu_row(row[(size_t)k]) * o.row_bytes();
         memset(&j.stats, 0, sizeof j.stats);
         jobs.push_back(j);
     }
@@ -211,8 +215,9 @@ void sum_stats(const std::vector<BandJob> &jobs, const kpeg_plan *plan, kpeg_sta
     if (!stats)
         return;
     memset(stats, 0, sizeof *stats);
-    stats->width = plan->width;
-    stats->height = plan->height;
+    const kpeg::OutGeom o = kpeg::out_geom(plan->width, plan->height, plan->ncomp, plan->flags);
+    stats->width = o.width;
+    stats->height = o.height;
     stats->ncomp = plan->ncomp;
     for (const BandJob &j : jobs) {
         stats->scan_bytes += j.stats.scan_bytes;
@@ -239,7 +244,6 @@ extern "C" int kpeg_cuda_decode_tiled(const int *devices, int ndev, const kpeg_p
         t_tiled_err = "restart markers do not match the restart interval";
         return src;
     }
-    const size_t row_bytes = (size_t)plan->width * plan->ncomp;
     const int rc = run_bands(jobs, [&](BandJob &j) {
         kpeg_ctx *ctx = nullptr;
         j.rc = kpeg_cuda_acquire(j.device, &ctx);
@@ -247,7 +251,7 @@ extern "C" int kpeg_cuda_decode_tiled(const int *devices, int ndev, const kpeg_p
             j.err = "no usable CUDA device";
             return;
         }
-        j.rc = kpeg_cuda_decode(ctx, &j.plan, j.scan, j.len, pixels_out + (size_t)j.row0 * row_bytes, &j.stats);
+        j.rc = kpeg_cuda_decode(ctx, &j.plan, j.scan, j.len, pixels_out + j.out_off, &j.stats);
         if (j.rc != KPEG_OK)
             j.err = kpeg_cuda_last_error(ctx);
         kpeg_cuda_release(j.device, ctx);
@@ -256,7 +260,7 @@ extern "C" int kpeg_cuda_decode_tiled(const int *devices, int ndev, const kpeg_p
     return rc;
 }
 
-// Same, the frame assembled in DEVICE memory of `dst_device` (d_frame: height * width * ncomp bytes, allocated by the
+// Same, the frame assembled in DEVICE memory of `dst_device` (d_frame: kpeg_output_size bytes, allocated by the
 // caller on that device): every band is decoded on its own GPU and its rows travel by one peer copy (NVLink; staged
 // through the host by the driver where peer access is unavailable).  A consumer on dst_device never pays PCIe.
 extern "C" int kpeg_cuda_decode_tiled_device(const int *devices, int ndev, const kpeg_plan *plan, const uint8_t *scan,
@@ -271,7 +275,6 @@ extern "C" int kpeg_cuda_decode_tiled_device(const int *devices, int ndev, const
         t_tiled_err = "restart markers do not match the restart interval";
         return src;
     }
-    const size_t row_bytes = (size_t)plan->width * plan->ncomp;
     const int rc = run_bands(jobs, [&](BandJob &j) {
         kpeg_ctx *ctx = nullptr;
         j.rc = kpeg_cuda_acquire(j.device, &ctx);
@@ -279,7 +282,7 @@ extern "C" int kpeg_cuda_decode_tiled_device(const int *devices, int ndev, const
             j.err = "no usable CUDA device";
             return;
         }
-        j.rc = kpeg_cuda_decode_to_peer(ctx, &j.plan, j.scan, j.len, dst_device, d_frame + (size_t)j.row0 * row_bytes, &j.stats);
+        j.rc = kpeg_cuda_decode_to_peer(ctx, &j.plan, j.scan, j.len, dst_device, d_frame + j.out_off, &j.stats);
         if (j.rc != KPEG_OK)
             j.err = kpeg_cuda_last_error(ctx);
         kpeg_cuda_release(j.device, ctx);
@@ -303,7 +306,7 @@ extern "C" int kpeg_cuda_decode_file_tiled(const int *devices, int ndev, const u
     plan.flags = flags;
     if (plan_out)
         *plan_out = plan;
-    if ((size_t)plan.width * plan.height * plan.ncomp > cap) {
+    if (kpeg_output_size(&plan, nullptr, nullptr) > cap) {
         t_tiled_err = "pixel buffer too small";
         return KPEG_ERR_ARG;
     }

@@ -17,6 +17,8 @@
 //                        the same quantised coefficients, re-coded; --restart N (default: the input's interval),
 //                        --optimize, --transform none|flip-h|flip-v|transpose|transverse|rot90|rot180|rot270
 //   --devices L  several devices, e.g. 0-7 or 0,2,3: the restart-interval tiles of the image are spread over them
+//   --scale 1/N  decode: N = 2, 4 or 8 writes <file>.ppm at 1/N the size (KPEG_FLAG_SCALE_*: libjpeg's reduced IDCTs and
+//                integer colour, as djpeg -scale 1/N); 1/1 or no --scale is the full-size decode of the drop-in JPEGDecoder
 //   --quiet      log only to kpeg.log
 #include <algorithm>
 #include <cctype>
@@ -47,6 +49,7 @@ namespace
         std::cout << "--optimize                      : Encoder Huffman tables optimised for the image (smaller file)" << std::endl;
         std::cout << "<in.jpg> <out.jpg>              : Transcode a baseline JPEG losslessly on the GPU" << std::endl;
         std::cout << "--transform T                   : Transcode: none, flip-h, flip-v, transpose, transverse, rot90, rot180, rot270" << std::endl;
+        std::cout << "--scale 1/N                     : Decode at 1/2, 1/4 or 1/8 the size (libjpeg's reduced IDCTs)" << std::endl;
         std::cout << "-h                              : Print this help message and exit" << std::endl;
     }
 
@@ -67,6 +70,7 @@ namespace
         bool restart_given = false;
         bool optimize = false;
         std::string transform = "none";
+        std::string scale = "1/1";
     };
 
     // "0-3", "0,2,5", "1": device list of --devices
@@ -256,11 +260,97 @@ namespace
                                        << "): " << len << " bytes";
     }
 
+    // --scale 2, 4, 8: the reduced-size decode through the C ABI (the drop-in JPEGDecoder has the reference's interface,
+    // which has no scale), written as dumpRawData writes the full-size image: <name up to ".jpg">.ppm, P6, gray as R = G = B
+    void decodeScaled( const std::string& filename, const Options& opt, uint32_t scaleFlag )
+    {
+        std::vector<uint8_t> data;
+        if ( !readFile( filename, data ) )
+        {
+            LOG(kpeg::Logger::Level::ERROR) << "Unable to open file: " << filename;
+            return;
+        }
+        kpeg_plan frame;
+        kpeg_scan scans[KPEG_MAX_SCANS];
+        int nscans = 0;
+        if ( kpeg_parse_jfif_scans( data.data(), data.size(), &frame, scans, KPEG_MAX_SCANS, &nscans ) != KPEG_OK )
+        {
+            LOG(kpeg::Logger::Level::ERROR) << "An error ocurred while decoding: " << filename << ": not a supported baseline JPEG";
+            return;
+        }
+        const uint32_t flags = ( opt.parity ? KPEG_FLAG_REF_PARITY : 0u ) | scaleFlag;
+        frame.flags = flags;
+        uint32_t w = 0, h = 0;
+        std::vector<uint8_t> pixels( kpeg_output_size( &frame, &w, &h ) );
+        int rc;
+        std::string err;
+        if ( !opt.devices.empty() )
+        {
+            rc = kpeg_cuda_decode_file_tiled( opt.devices.data(), (int)opt.devices.size(), data.data(), data.size(), flags, pixels.data(),
+                                              pixels.size(), nullptr, nullptr );
+            err = kpeg_tiled_last_error();
+        }
+        else
+        {
+            kpeg_ctx* ctx = nullptr;
+            rc = kpeg_cuda_acquire( opt.device, &ctx );
+            if ( rc == KPEG_OK )
+            {
+                rc = kpeg_cuda_decode_file( ctx, data.data(), data.size(), flags, pixels.data(), pixels.size(), nullptr, nullptr );
+                err = kpeg_cuda_last_error( ctx );
+                kpeg_cuda_release( opt.device, ctx );
+            }
+            else
+                err = "no usable CUDA device (there is no CPU decode path)";
+        }
+        if ( rc != KPEG_OK )
+        {
+            LOG(kpeg::Logger::Level::ERROR) << "An error ocurred while decoding: " << filename << ": " << err;
+            return;
+        }
+        const std::string target = filename.substr( 0, filename.find( ".jpg" ) ) + ".ppm";
+        std::ofstream out( target, std::ios::out | std::ios::binary );
+        char header[160];
+        const int hl = kpeg_ppm_header( (int)w, (int)h, header, sizeof header );
+        out.write( header, hl );
+        if ( frame.ncomp == 3 )
+            out.write( (const char*)pixels.data(), (std::streamsize)pixels.size() );
+        else
+            for ( uint8_t v : pixels )
+            {
+                const char rgb[3] = { (char)v, (char)v, (char)v };
+                out.write( rgb, 3 );
+            }
+        out.close();
+        if ( !out )
+        {
+            std::remove( target.c_str() );
+            LOG(kpeg::Logger::Level::ERROR) << "Unable to create dump file \'" << target << "\'.";
+            return;
+        }
+        LOG(kpeg::Logger::Level::INFO) << "Decoded " << filename << " at " << opt.scale << " (" << w << "x" << h
+                                       << "): raw image data dumped to file: \'" << target << "\'.";
+    }
+
     void decodeJPEG( const std::string& filename, const Options& opt )
     {
         if ( !isValidFilename( filename ) )
         {
             LOG(kpeg::Logger::Level::ERROR) << "Invalid input file name passed.";
+            return;
+        }
+        static const char* const scales[] = { "1/1", "1/2", "1/4", "1/8" };
+        int code = -1;
+        for ( int k = 0; k < 4; ++k )
+            if ( opt.scale == scales[k] ) code = k;
+        if ( code < 0 )
+        {
+            LOG(kpeg::Logger::Level::ERROR) << "Unknown scale '" << opt.scale << "' (1/1, 1/2, 1/4 or 1/8).";
+            return;
+        }
+        if ( code > 0 )
+        {
+            decodeScaled( filename, opt, (uint32_t)code * KPEG_FLAG_SCALE_1_2 );
             return;
         }
         kpeg::JPEGDecoder decoder;
@@ -294,6 +384,7 @@ int main( int argc, char** argv )
             else if ( a == "--restart" && i + 1 < argc ) { opt.restart = std::atoi( argv[++i] ); opt.restart_given = true; }
             else if ( a == "--transform" && i + 1 < argc ) opt.transform = argv[++i];
             else if ( a == "--optimize" ) opt.optimize = true;
+            else if ( a == "--scale" && i + 1 < argc ) opt.scale = argv[++i];
             else args.push_back( a );
         }
 
