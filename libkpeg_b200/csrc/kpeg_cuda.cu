@@ -32,10 +32,24 @@ using namespace kpeg;
 
 namespace {
 
+// Grow-only device scratch (ensure), freed with its owner.  Not movable: guard mode keeps pointers to the buffers.
 struct DevBuf {
+    const char *name;    // in guard-mode messages
     void *p = nullptr;   // what the kernels get
     size_t cap = 0;
     void *raw = nullptr; // the allocation (== p, or p - GUARD_BYTES in guard mode)
+
+    DevBuf(const char *n) : name(n) {}
+    DevBuf(const DevBuf &) = delete;
+    DevBuf &operator=(const DevBuf &) = delete;
+    ~DevBuf() { release(); }
+    void release()
+    {
+        if (raw)
+            cudaFree(raw);
+        raw = p = nullptr;
+        cap = 0;
+    }
 };
 
 // KPEG_GUARD=1 (debugging aid; the pool this was developed on has no compute-sanitizer): every device buffer is
@@ -43,9 +57,22 @@ struct DevBuf {
 constexpr size_t GUARD_BYTES = 256;
 constexpr int GUARD_PATTERN = 0xA5;
 
+// Grow-only pinned host memory (ensure_pinned), freed with its owner.
 struct PinBuf {
     void *p = nullptr;
     size_t cap = 0;
+
+    PinBuf() = default;
+    PinBuf(const PinBuf &) = delete;
+    PinBuf &operator=(const PinBuf &) = delete;
+    ~PinBuf() { release(); }
+    cudaError_t release()
+    {
+        const cudaError_t e = p ? cudaFreeHost(p) : cudaSuccess;
+        p = nullptr;
+        cap = 0;
+        return e;
+    }
 };
 
 constexpr int MAX_EVENTS = 192;
@@ -77,23 +104,37 @@ struct Job {
 
 struct Lane {
     cudaStream_t stream = nullptr;
-    DevBuf scan, words, seg_bit, tile_kept, tile_rst, cls, state, work, seg_hint, start_slot, scan_tiles;
-    DevBuf coef, dcdiff, dc, tiles, tie_rec, tie_cnt, pixels, meta, rec, nrec, rec_alt, strip_sub, dcs, dcpre, scan_tiles_dcs;
+    DevBuf scan{"scan"}, words{"words"}, seg_bit{"seg_bit"}, tile_kept{"tile_kept"}, tile_rst{"tile_rst"}, cls{"cls"},
+        state{"state"}, work{"work"}, seg_hint{"seg_hint"}, start_slot{"start_slot"}, scan_tiles{"scan_tiles"};
+    DevBuf coef{"coef"}, dcdiff{"dcdiff"}, dc{"dc"}, tiles{"tiles"}, tie_rec{"tie_rec"}, tie_cnt{"tie_cnt"}, pixels{"pixels"},
+        meta{"meta"}, rec{"rec"}, nrec{"nrec"}, rec_alt{"rec_alt"}, strip_sub{"strip_sub"}, dcs{"dcs"}, dcpre{"dcpre"},
+        scan_tiles_dcs{"scan_tiles_dcs"};
     PinBuf h_meta;
     // host-buffer batches: pinned staging of the small scans + the separator positions, and their device copy
     PinBuf h_stage, h_ends;
-    DevBuf d_ends, d_stage;
+    DevBuf d_ends{"d_ends"}, d_stage{"d_stage"};
     cudaEvent_t ev[MAX_EVENTS] = {};
     int ev_stage[MAX_EVENTS] = {};
     int nev = 0;
     Job job;
+
+    ~Lane()
+    {
+        for (cudaEvent_t e : ev)
+            if (e)
+                cudaEventDestroy(e);
+        if (stream)
+            cudaStreamDestroy(stream);
+    }
 };
 
 // Grow-only device scratch of the encoder (on lane 0's stream), and its tables, rebuilt when the quality changes.
 // opt_tables / hist: the optimised mode's per-encode tables and symbol counts (the cached tables stay Annex K).
 struct EncScratch {
-    DevBuf buf[enc::BUF_COUNT];
-    DevBuf tables, meta, pixels, out, opt_tables, hist;
+    DevBuf buf[enc::BUF_COUNT] = {{"enc.coef"}, {"enc.raw"},      {"enc.dc"},    {"enc.has_ac"}, {"enc.bits"},
+                                  {"enc.off"},  {"enc.seg_byte"}, {"enc.words"}, {"enc.agg"},    {"enc.tile_ff"}}; // BUF_* order
+    DevBuf tables{"enc.tables"}, meta{"enc.meta"}, pixels{"enc.pixels"}, out{"enc.out"}, opt_tables{"enc.opt_tables"},
+        hist{"enc.hist"};
     PinBuf h_tables, h_meta;
     int quality = -1;
 };
@@ -118,7 +159,7 @@ struct kpeg_ctx {
     int submit_parts = 1;    // jobs one deferred submission is cut into (KPEG_SUBMIT_SPLIT)
     // bands a large restart-marked image from host memory is cut into, one per lane (KPEG_BANDS; 1 = off)
     int band_parts = 4;
-    DevBuf band_counts;     // RSTn markers counted per band (decode_banded)
+    DevBuf band_counts{"band_counts"}; // RSTn markers counted per band (decode_banded)
     PinBuf h_band_counts;
     // result copies of the lanes leave one after another (each waits for the one enqueued before it): copies to the
     // host that run at the same time share the link AND slow each other down (measured: four concurrent 200 MB copies
@@ -132,8 +173,9 @@ struct kpeg_ctx {
     cudaEvent_t d2h_done = nullptr;
     Lane lane[NLANES];
 
-    DevBuf tables, merged;
-    DevBuf scan_tiles[3]; // frames coded one scan per component: the components' tiles before they are interleaved
+    DevBuf tables{"tables"}, merged{"merged"};
+    // frames coded one scan per component: the components' tiles before they are interleaved
+    DevBuf scan_tiles[3] = {{"scan_tiles[0]"}, {"scan_tiles[1]"}, {"scan_tiles[2]"}};
     PinBuf h_tables, h_sep;
     cudaEvent_t tables_ready = nullptr;
     kpeg_plan plan_cached;
@@ -146,6 +188,7 @@ struct kpeg_ctx {
     // lane's previous job is finished only when the lane comes up again, so several batches are in flight
     bool counted = false; // registered with kernels_context_created
     bool guard = false;   // KPEG_GUARD=1
+    std::vector<const DevBuf *> guarded; // guard mode: every buffer allocated so far (check_guards)
     bool plan_fits_records = true;
     int next_lane = 0;
     int deferred_rc = KPEG_OK;
@@ -153,6 +196,15 @@ struct kpeg_ctx {
     kpeg_stats deferred_stats = {};
 
     EncScratch enc; // kpeg_cuda_encode*
+
+    // the buffers free themselves after this; kpeg_cuda_destroy has synchronised every lane
+    ~kpeg_ctx()
+    {
+        if (tables_ready)
+            cudaEventDestroy(tables_ready);
+        if (d2h_done)
+            cudaEventDestroy(d2h_done);
+    }
 };
 
 namespace {
@@ -190,21 +242,13 @@ int fail(kpeg_ctx *c, int code, const char *what, cudaError_t e = cudaSuccess)
             return rc_;                                                                                                \
     } while (0)
 
-void dev_free(DevBuf &b)
-{
-    if (b.raw)
-        cudaFree(b.raw);
-    b.raw = b.p = nullptr;
-    b.cap = 0;
-}
-
 int ensure(kpeg_ctx *ctx, cudaStream_t stream, DevBuf &b, size_t bytes)
 {
     if (bytes <= b.cap)
         return KPEG_OK;
     if (b.raw) {
         CK(cudaStreamSynchronize(stream));
-        dev_free(b);
+        b.release();
     }
     const bool guard = ctx->guard;
     const size_t want = guard ? ((bytes + 15u) & ~(size_t)15u) : bytes + bytes / 8 + 256;
@@ -216,6 +260,8 @@ int ensure(kpeg_ctx *ctx, cudaStream_t stream, DevBuf &b, size_t bytes)
     b.p = b.raw;
     if (guard) {
         b.p = (uint8_t *)b.raw + GUARD_BYTES;
+        if (std::find(ctx->guarded.begin(), ctx->guarded.end(), &b) == ctx->guarded.end())
+            ctx->guarded.push_back(&b);
         CK(cudaMemsetAsync(b.raw, GUARD_PATTERN, GUARD_BYTES, stream));
         CK(cudaMemsetAsync((uint8_t *)b.p + want, GUARD_PATTERN, GUARD_BYTES, stream));
     }
@@ -229,9 +275,7 @@ int ensure_pinned(kpeg_ctx *ctx, cudaStream_t stream, PinBuf &b, size_t bytes)
         return KPEG_OK;
     if (b.p) {
         CK(cudaStreamSynchronize(stream));
-        CK(cudaFreeHost(b.p));
-        b.p = nullptr;
-        b.cap = 0;
+        CK(b.release());
     }
     const size_t want = bytes + bytes / 8 + 256;
     cudaError_t e = cudaMallocHost(&b.p, want);
@@ -412,6 +456,66 @@ void finish_deferred(kpeg_ctx *ctx, int li)
     }
 }
 
+// every pending deferred submission is completed first (its outcome is reported by kpeg_cuda_wait)
+void finish_all_deferred(kpeg_ctx *ctx)
+{
+    for (int i = 0; i < NLANES; ++i)
+        if (ctx->lane[i].job.active)
+            finish_deferred(ctx, i);
+}
+
+// Lane 0 with no deferred job on it: such a job still reads the lane's scan / pixel buffers, which the caller is about to
+// reuse.  Only lane 0: a deferred batch on the other lanes keeps overlapping the caller's synchronous work.
+Lane &idle_lane0(kpeg_ctx *ctx)
+{
+    if (ctx->lane[0].job.active)
+        finish_deferred(ctx, 0);
+    return ctx->lane[0];
+}
+
+void reset_deferred(kpeg_ctx *ctx)
+{
+    ctx->deferred_rc = KPEG_OK;
+    ctx->deferred_err.clear();
+    memset(&ctx->deferred_stats, 0, sizeof ctx->deferred_stats);
+}
+
+// A synchronous call that runs its work as deferred submissions: the outcome of the caller's earlier submissions (for
+// the caller's kpeg_cuda_wait) is set aside while it runs and restored when it returns.  Those submissions must be
+// finished first (finish_all_deferred).
+struct DeferredOutcomeSaved {
+    kpeg_ctx *ctx;
+    const int rc;
+    const std::string err;
+    const kpeg_stats stats;
+
+    explicit DeferredOutcomeSaved(kpeg_ctx *c) : ctx(c), rc(c->deferred_rc), err(c->deferred_err), stats(c->deferred_stats)
+    {
+        reset_deferred(c);
+    }
+    ~DeferredOutcomeSaved()
+    {
+        ctx->deferred_rc = rc;
+        ctx->deferred_err = err;
+        ctx->deferred_stats = stats;
+    }
+};
+
+// K3's arguments for geometry g on lane L: its tie lists and meta, and the context's tables
+IdctArgs idct_args(kpeg_ctx *ctx, Lane &L, const JobGeom &g, uint32_t nstrips, const void *tiles, uint8_t *pixels)
+{
+    IdctArgs ia = {};
+    ia.tiles = tiles;
+    ia.nstrips = nstrips;
+    ia.tables = (const DeviceTables *)ctx->tables.p;
+    ia.pixels = pixels;
+    ia.tie_rec = (uint4 *)L.tie_rec.p;
+    ia.tie_cnt = (uint32_t *)L.tie_cnt.p;
+    ia.meta = (DevMeta *)L.meta.p;
+    ia.g = g;
+    return ia;
+}
+
 // Enqueue the whole device pipeline for one job whose stuffed bytes are (or will be, in stream
 // order) at d_scan.  Optimistic: the stages downstream of the relay are issued before it is known
 // whether the pre-issued relay rounds reached the fixed point; job_finish repairs that if not.
@@ -424,9 +528,7 @@ int job_enqueue(kpeg_ctx *ctx, int li, const kpeg_plan *pl, const uint8_t *d_sca
     if (J.active) // a deferred job still owns this lane's scratch: complete it first
         finish_deferred(ctx, li);
     if (ctx->have_plan && !same_tables(&ctx->plan_cached, pl))
-        for (int i = 0; i < NLANES; ++i) // the tables are shared: nothing deferred may outlive them
-            if (ctx->lane[i].job.active)
-                finish_deferred(ctx, i);
+        finish_all_deferred(ctx); // the tables are shared: nothing deferred may outlive them
     JobGeom g;
     const char *why = nullptr;
     uint32_t sub_bits = ctx->sub_bits;
@@ -550,15 +652,7 @@ int job_enqueue(kpeg_ctx *ctx, int li, const kpeg_plan *pl, const uint8_t *d_sca
     xa.meta = d_meta;
     xa.g = g;
 
-    IdctArgs &ia = J.ia;
-    ia.tiles = tiles;
-    ia.nstrips = nstrips;
-    ia.tables = (const DeviceTables *)ctx->tables.p;
-    ia.pixels = d_pixels;
-    ia.tie_rec = (uint4 *)L.tie_rec.p;
-    ia.tie_cnt = (uint32_t *)L.tie_cnt.p;
-    ia.meta = d_meta;
-    ia.g = g;
+    J.ia = idct_args(ctx, L, g, nstrips, tiles, d_pixels);
 
     launch_entropy_cold(ea, s, &J.launches);
     mark(ctx, L, KPEG_T_ENTROPY_COLD);
@@ -584,33 +678,16 @@ int job_enqueue(kpeg_ctx *ctx, int li, const kpeg_plan *pl, const uint8_t *d_sca
     return enqueue_downstream(ctx, L);
 }
 
-struct NamedBuf {
-    const char *name;
-    DevBuf *buf;
-};
-
-// guard mode: the bytes on either side of every device buffer of the lane must still hold the pattern
-int check_guards(kpeg_ctx *ctx, Lane &L)
+// guard mode: the bytes on either side of every device buffer of the context must still hold the pattern.  The lanes
+// are synchronised first: a buffer of another lane may have its guard areas still to be written on that lane's stream.
+int check_guards(kpeg_ctx *ctx)
 {
-    NamedBuf bufs[] = {{"cls", &L.cls},           {"scan", &L.scan},         {"words", &L.words},       {"seg_bit", &L.seg_bit},
-                       {"tile_kept", &L.tile_kept}, {"tile_rst", &L.tile_rst}, {"state", &L.state},       {"work", &L.work},
-                       {"seg_hint", &L.seg_hint}, {"start_slot", &L.start_slot}, {"scan_tiles", &L.scan_tiles},
-                       {"coef", &L.coef},         {"dcdiff", &L.dcdiff},     {"tiles", &L.tiles},       {"tie_rec", &L.tie_rec},   {"tie_cnt", &L.tie_cnt},     {"strip_sub", &L.strip_sub}, {"dc", &L.dc}, {"dcs", &L.dcs}, {"dcpre", &L.dcpre}, {"scan_tiles_dcs", &L.scan_tiles_dcs}, {"d_ends", &L.d_ends},
-                       {"pixels", &L.pixels},     {"meta", &L.meta},
-                       {"rec", &L.rec},           {"nrec", &L.nrec},         {"rec_alt", &L.rec_alt},   {"tables", &ctx->tables},
-                       {"d_stage", &L.d_stage},   {"scan_tiles[0]", &ctx->scan_tiles[0]}, {"scan_tiles[1]", &ctx->scan_tiles[1]},
-                       {"scan_tiles[2]", &ctx->scan_tiles[2]}, {"band_counts", &ctx->band_counts}, {"merged", &ctx->merged},
-                       {"enc.coef", &ctx->enc.buf[enc::BUF_COEF]}, {"enc.raw", &ctx->enc.buf[enc::BUF_RAW]},
-                       {"enc.dc", &ctx->enc.buf[enc::BUF_DC]}, {"enc.has_ac", &ctx->enc.buf[enc::BUF_HAS_AC]},
-                       {"enc.bits", &ctx->enc.buf[enc::BUF_BITS]}, {"enc.off", &ctx->enc.buf[enc::BUF_OFF]},
-                       {"enc.seg_byte", &ctx->enc.buf[enc::BUF_SEG]}, {"enc.words", &ctx->enc.buf[enc::BUF_WORDS]},
-                       {"enc.agg", &ctx->enc.buf[enc::BUF_AGG]}, {"enc.tile_ff", &ctx->enc.buf[enc::BUF_TILE_FF]},
-                       {"enc.tables", &ctx->enc.tables}, {"enc.meta", &ctx->enc.meta}, {"enc.pixels", &ctx->enc.pixels},
-                       {"enc.out", &ctx->enc.out}, {"enc.opt_tables", &ctx->enc.opt_tables}, {"enc.hist", &ctx->enc.hist}};
+    for (Lane &L : ctx->lane)
+        CK(cudaStreamSynchronize(L.stream));
     uint8_t host[2 * GUARD_BYTES];
-    for (const NamedBuf &nb : bufs) {
-        const DevBuf &b = *nb.buf;
-        if (!b.raw || b.raw == b.p)
+    for (const DevBuf *bp : ctx->guarded) {
+        const DevBuf &b = *bp;
+        if (!b.raw)
             continue;
         CK(cudaMemcpy(host, b.raw, GUARD_BYTES, cudaMemcpyDeviceToHost));
         CK(cudaMemcpy(host + GUARD_BYTES, (const uint8_t *)b.p + b.cap, GUARD_BYTES, cudaMemcpyDeviceToHost));
@@ -618,7 +695,7 @@ int check_guards(kpeg_ctx *ctx, Lane &L)
             if (host[i] != (uint8_t)GUARD_PATTERN) {
                 char msg[160];
                 snprintf(msg, sizeof msg, "guard bytes %s device buffer '%s' (%zu bytes) were overwritten at offset %zu",
-                         i < GUARD_BYTES ? "before" : "after", nb.name, b.cap, i % GUARD_BYTES);
+                         i < GUARD_BYTES ? "before" : "after", b.name, b.cap, i % GUARD_BYTES);
                 return fail(ctx, KPEG_ERR_CUDA, msg);
             }
     }
@@ -684,7 +761,7 @@ int job_finish(kpeg_ctx *ctx, int li, kpeg_stats *stats)
         TRY(enqueue_downstream(ctx, L));
     }
     if (ctx->guard)
-        TRY(check_guards(ctx, L));
+        TRY(check_guards(ctx));
     ctx->last_lane = li;
     ctx->last_g = J.g;
     if (stats) {
@@ -717,37 +794,50 @@ void zero_stats(kpeg_stats *stats)
         memset(stats, 0, sizeof *stats);
 }
 
+// the figures of one part of a call added to the call's, as job_finish adds a job's (the output size is the caller's)
+void add_stats(kpeg_stats &to, const kpeg_stats &part)
+{
+    to.scan_bytes += part.scan_bytes;
+    to.unstuffed_bytes += part.unstuffed_bytes;
+    to.segments += part.segments;
+    to.subsequences += part.subsequences;
+    to.sync_rounds = std::max(to.sync_rounds, part.sync_rounds);
+    to.exact_samples += part.exact_samples;
+    to.kernel_launches += part.kernel_launches;
+    for (int t = 0; t < KPEG_T_COUNT; ++t)
+        to.ms[t] += part.ms[t];
+    to.ms_total += part.ms_total;
+}
+
+// A scan in host memory decoded on lane 0 (which the caller has made idle), complete on return: copied into the lane's
+// scan buffer, then job_enqueue's pixels / d2h / tiles_only and job_finish's stats.
+int decode_host_scan(kpeg_ctx *ctx, const kpeg_plan *pl, const uint8_t *scan, size_t scan_len, uint8_t *d_pixels,
+                     std::vector<Copy> d2h, void *tiles_only, kpeg_stats *stats)
+{
+    Lane &L = ctx->lane[0];
+    TRY(ensure(ctx, L.stream, L.scan, scan_len + 64));
+    mark(ctx, L, -1);
+    CK(cudaMemcpyAsync(L.scan.p, scan, scan_len, cudaMemcpyHostToDevice, L.stream));
+    mark(ctx, L, KPEG_T_H2D);
+    TRY(job_enqueue(ctx, 0, pl, (const uint8_t *)L.scan.p, scan_len, 1, d_pixels, std::move(d2h), tiles_only));
+    return job_finish(ctx, 0, stats);
+}
+
 // The three scans of a frame coded one scan per component, entropy-decoded one after another on lane 0 into the
 // components' tiles ctx->scan_tiles[c] (nmcu_padded blocks each); their figures are added to *stats.
 int entropy_decode_component_scans(kpeg_ctx *ctx, const kpeg_scan *scans, const uint8_t *file, uint32_t flags, uint32_t nmcu_padded,
                                    kpeg_stats *stats)
 {
-    Lane &L = ctx->lane[0];
-    cudaStream_t s = L.stream;
     for (int c = 0; c < 3; ++c)
-        TRY(ensure(ctx, s, ctx->scan_tiles[c], (size_t)nmcu_padded * 128u + 256u));
-    kpeg_stats part;
+        TRY(ensure(ctx, ctx->lane[0].stream, ctx->scan_tiles[c], (size_t)nmcu_padded * 128u + 256u));
     for (int k = 0; k < 3; ++k) {
         kpeg_plan pl = scans[k].plan;
         pl.flags = flags;
-        TRY(ensure(ctx, s, L.scan, scans[k].len + 64));
-        mark(ctx, L, -1);
-        CK(cudaMemcpyAsync(L.scan.p, file + scans[k].off, scans[k].len, cudaMemcpyHostToDevice, s));
-        mark(ctx, L, KPEG_T_H2D);
-        TRY(job_enqueue(ctx, 0, &pl, (const uint8_t *)L.scan.p, scans[k].len, 1, nullptr, {}, ctx->scan_tiles[scans[k].comp[0]].p));
-        memset(&part, 0, sizeof part);
-        TRY(job_finish(ctx, 0, stats ? &part : nullptr));
-        if (stats) {
-            stats->scan_bytes += part.scan_bytes;
-            stats->unstuffed_bytes += part.unstuffed_bytes;
-            stats->segments += part.segments;
-            stats->subsequences += part.subsequences;
-            stats->sync_rounds = std::max(stats->sync_rounds, part.sync_rounds);
-            stats->kernel_launches += part.kernel_launches;
-            for (int t = 0; t < KPEG_T_COUNT; ++t)
-                stats->ms[t] += part.ms[t];
-            stats->ms_total += part.ms_total;
-        }
+        kpeg_stats part = {};
+        TRY(decode_host_scan(ctx, &pl, file + scans[k].off, scans[k].len, nullptr, {}, ctx->scan_tiles[scans[k].comp[0]].p,
+                             stats ? &part : nullptr));
+        if (stats)
+            add_stats(*stats, part);
     }
     return KPEG_OK;
 }
@@ -791,9 +881,7 @@ int decode_banded(kpeg_ctx *ctx, const kpeg_plan *plan, const uint8_t *scan, siz
         begin[k] = end[k - 1] + 2u;
     }
     end[parts - 1] = scan_len;
-    for (int i = 0; i < NLANES; ++i)
-        if (ctx->lane[i].job.active)
-            finish_deferred(ctx, i);
+    finish_all_deferred(ctx);
     // copies in + marker counts, every band on its own lane
     TRY(ensure(ctx, ctx->lane[0].stream, ctx->band_counts, NLANES * sizeof(uint32_t)));
     TRY(ensure_pinned(ctx, ctx->lane[0].stream, ctx->h_band_counts, NLANES * sizeof(uint32_t)));
@@ -966,51 +1054,9 @@ extern "C" void kpeg_cuda_destroy(kpeg_ctx *ctx)
     cudaSetDevice(ctx->device);
     if (ctx->counted)
         kernels_context_destroyed();
-    for (Lane &L : ctx->lane) {
+    for (Lane &L : ctx->lane) // the members free the buffers: nothing may still use one
         if (L.stream)
             cudaStreamSynchronize(L.stream);
-        DevBuf *bufs[] = {&L.cls,  &L.scan, &L.words,    &L.seg_bit,    &L.tile_kept,  &L.tile_rst, &L.state,
-                          &L.work, &L.seg_hint, &L.start_slot, &L.scan_tiles, &L.coef,     &L.dcdiff, &L.tiles, &L.tie_rec, &L.tie_cnt,
-                          &L.strip_sub, &L.dc, &L.dcs, &L.dcpre, &L.scan_tiles_dcs, &L.pixels, &L.meta,
-                          &L.rec,  &L.nrec,       &L.rec_alt};
-        for (DevBuf *b : bufs)
-            dev_free(*b);
-        if (L.h_meta.p)
-            cudaFreeHost(L.h_meta.p);
-        if (L.h_stage.p)
-            cudaFreeHost(L.h_stage.p);
-        if (L.h_ends.p)
-            cudaFreeHost(L.h_ends.p);
-        dev_free(L.d_ends);
-        dev_free(L.d_stage);
-        for (int i = 0; i < MAX_EVENTS; ++i)
-            if (L.ev[i])
-                cudaEventDestroy(L.ev[i]);
-        if (L.stream)
-            cudaStreamDestroy(L.stream);
-    }
-    dev_free(ctx->tables);
-    dev_free(ctx->merged);
-    if (ctx->h_tables.p)
-        cudaFreeHost(ctx->h_tables.p);
-    if (ctx->h_sep.p)
-        cudaFreeHost(ctx->h_sep.p);
-    if (ctx->tables_ready)
-        cudaEventDestroy(ctx->tables_ready);
-    if (ctx->d2h_done)
-        cudaEventDestroy(ctx->d2h_done);
-    for (DevBuf &b : ctx->scan_tiles)
-        dev_free(b);
-    dev_free(ctx->band_counts);
-    if (ctx->h_band_counts.p)
-        cudaFreeHost(ctx->h_band_counts.p);
-    for (DevBuf &b : ctx->enc.buf)
-        dev_free(b);
-    for (DevBuf *b : {&ctx->enc.tables, &ctx->enc.meta, &ctx->enc.pixels, &ctx->enc.out})
-        dev_free(*b);
-    for (PinBuf *b : {&ctx->enc.h_tables, &ctx->enc.h_meta})
-        if (b->p)
-            cudaFreeHost(b->p);
     delete ctx;
 }
 
@@ -1141,9 +1187,7 @@ extern "C" int kpeg_cuda_decode(kpeg_ctx *ctx, const kpeg_plan *plan, const uint
         return KPEG_ERR_ARG;
     CK(cudaSetDevice(ctx->device));
     zero_stats(stats);
-    Lane &L = ctx->lane[0];
-    if (L.job.active) // a deferred job still reads this lane's scan / pixel buffers: complete it before they can move
-        finish_deferred(ctx, 0);
+    Lane &L = idle_lane0(ctx);
     // bands pay off for a large image whatever its output size: the decision is taken on the full-size pixels
     const size_t full_pix = (size_t)plan->width * plan->height * plan->ncomp;
     const size_t npix = out_of(plan).bytes();
@@ -1152,14 +1196,8 @@ extern "C" int kpeg_cuda_decode(kpeg_ctx *ctx, const kpeg_plan *plan, const uint
         if (brc != KPEG_ERR_UNSUPPORTED) // UNSUPPORTED: the restart interval does not line up with MCU rows -- whole image below
             return brc;
     }
-    TRY(ensure(ctx, L.stream, L.scan, scan_len + 64));
     TRY(ensure(ctx, L.stream, L.pixels, npix + 64));
-    mark(ctx, L, -1);
-    CK(cudaMemcpyAsync(L.scan.p, scan, scan_len, cudaMemcpyHostToDevice, L.stream));
-    mark(ctx, L, KPEG_T_H2D);
-    TRY(job_enqueue(ctx, 0, plan, (const uint8_t *)L.scan.p, scan_len, 1, (uint8_t *)L.pixels.p,
-                    {Copy{pixels_out, L.pixels.p, npix}}));
-    return job_finish(ctx, 0, stats);
+    return decode_host_scan(ctx, plan, scan, scan_len, (uint8_t *)L.pixels.p, {Copy{pixels_out, L.pixels.p, npix}}, nullptr, stats);
 }
 
 // Batch stream format: the n stuffed scans back to back, each followed by one 2-byte RSTn marker
@@ -1280,9 +1318,7 @@ extern "C" int kpeg_cuda_wait(kpeg_ctx *ctx, kpeg_stats *stats)
     const int rc = ctx->deferred_rc;
     if (rc != KPEG_OK)
         ctx->err = ctx->deferred_err;
-    ctx->deferred_rc = KPEG_OK;
-    ctx->deferred_err.clear();
-    memset(&ctx->deferred_stats, 0, sizeof ctx->deferred_stats);
+    reset_deferred(ctx);
     return rc;
 }
 
@@ -1294,9 +1330,7 @@ extern "C" int kpeg_cuda_decode_batch_device(kpeg_ctx *ctx, const kpeg_plan *pla
         return KPEG_ERR_ARG;
     CK(cudaSetDevice(ctx->device));
     zero_stats(stats);
-    Lane &L = ctx->lane[0];
-    if (L.job.active) // as in kpeg_cuda_decode
-        finish_deferred(ctx, 0);
+    Lane &L = idle_lane0(ctx);
     const size_t total = (size_t)(scan_offsets[n] - scan_offsets[0]) + 2u * (size_t)n;
     TRY(ensure(ctx, L.stream, L.scan, total + 64));
     const uint8_t *sep = (const uint8_t *)ctx->h_sep.p;
@@ -1430,26 +1464,11 @@ extern "C" int kpeg_cuda_decode_batch(kpeg_ctx *ctx, const kpeg_plan *plan, int 
     if (!ctx || !plan || n <= 0 || !scans || !scan_lens || !pixels_out)
         return KPEG_ERR_ARG;
     zero_stats(stats);
-    // earlier deferred submissions keep their own outcome for the caller's kpeg_cuda_wait
-    for (int i = 0; i < NLANES; ++i)
-        if (ctx->lane[i].job.active)
-            finish_deferred(ctx, i);
-    const int saved_rc = ctx->deferred_rc;
-    const std::string saved_err = ctx->deferred_err;
-    const kpeg_stats saved_stats = ctx->deferred_stats;
-    ctx->deferred_rc = KPEG_OK;
-    ctx->deferred_err.clear();
-    memset(&ctx->deferred_stats, 0, sizeof ctx->deferred_stats);
-    int rc = kpeg_cuda_submit_batch(ctx, plan, n, scans, scan_lens, pixels_out);
+    finish_all_deferred(ctx);
+    const DeferredOutcomeSaved saved(ctx);
+    const int rc = kpeg_cuda_submit_batch(ctx, plan, n, scans, scan_lens, pixels_out);
     const int wrc = kpeg_cuda_wait(ctx, stats);
-    if (rc == KPEG_OK)
-        rc = wrc;
-    const std::string my_err = ctx->err;
-    ctx->deferred_rc = saved_rc;
-    ctx->deferred_err = saved_err;
-    ctx->deferred_stats = saved_stats;
-    ctx->err = my_err;
-    return rc;
+    return rc != KPEG_OK ? rc : wrc;
 }
 
 // One band of a tiled decode whose frame lives on another GPU: decode here, then one peer copy of the band's rows
@@ -1462,12 +1481,9 @@ extern "C" int kpeg_cuda_decode_to_peer(kpeg_ctx *ctx, const kpeg_plan *plan, co
         return KPEG_ERR_ARG;
     CK(cudaSetDevice(ctx->device));
     zero_stats(stats);
-    Lane &L = ctx->lane[0];
-    if (L.job.active)
-        finish_deferred(ctx, 0);
+    Lane &L = idle_lane0(ctx);
     const size_t npix = out_of(plan).bytes();
     const bool local = dst_device == ctx->device && (reinterpret_cast<uintptr_t>(d_dst) & 7u) == 0;
-    TRY(ensure(ctx, L.stream, L.scan, scan_len + 64));
     if (!local) {
         TRY(ensure(ctx, L.stream, L.pixels, npix + 64));
         int can = 0;
@@ -1479,17 +1495,13 @@ extern "C" int kpeg_cuda_decode_to_peer(kpeg_ctx *ctx, const kpeg_plan *plan, co
             cudaGetLastError();
         }
     }
-    mark(ctx, L, -1);
-    CK(cudaMemcpyAsync(L.scan.p, scan, scan_len, cudaMemcpyHostToDevice, L.stream));
-    mark(ctx, L, KPEG_T_H2D);
     std::vector<Copy> out;
     if (!local) {
         Copy c{d_dst, L.pixels.p, npix};
         c.peer = dst_device;
         out.push_back(c);
     }
-    TRY(job_enqueue(ctx, 0, plan, (const uint8_t *)L.scan.p, scan_len, 1, local ? d_dst : (uint8_t *)L.pixels.p, std::move(out)));
-    return job_finish(ctx, 0, stats);
+    return decode_host_scan(ctx, plan, scan, scan_len, local ? d_dst : (uint8_t *)L.pixels.p, std::move(out), nullptr, stats);
 }
 
 // GPU-side PPM writer: the bytes Image::dumpRawData puts into <name>.ppm (reference src/Image.cpp:108-140: the P6
@@ -1507,9 +1519,7 @@ extern "C" int kpeg_cuda_decode_ppm_device(kpeg_ctx *ctx, const kpeg_plan *plan,
         return fail(ctx, KPEG_ERR_ARG, "PPM buffer must be 16-byte aligned");
     CK(cudaSetDevice(ctx->device));
     zero_stats(stats);
-    Lane &L = ctx->lane[0];
-    if (L.job.active)
-        finish_deferred(ctx, 0);
+    Lane &L = idle_lane0(ctx);
     char header[160];
     const OutGeom o = out_of(plan);
     const int hl = kpeg_ppm_header((int)o.width, (int)o.height, header, sizeof header);
@@ -1541,9 +1551,7 @@ extern "C" int kpeg_cuda_interleaved_to_planar(kpeg_ctx *ctx, const uint8_t *d_r
     if (!ctx || !d_rgb || !d_planes)
         return KPEG_ERR_ARG;
     CK(cudaSetDevice(ctx->device));
-    Lane &L = ctx->lane[0];
-    if (L.job.active)
-        finish_deferred(ctx, 0);
+    Lane &L = idle_lane0(ctx);
     launch_rgb_to_planar(d_rgb, d_planes, npixels, L.stream);
     CK(cudaStreamSynchronize(L.stream));
     CK(cudaGetLastError());
@@ -1578,9 +1586,7 @@ extern "C" int kpeg_cuda_decode_scans(kpeg_ctx *ctx, const kpeg_plan *frame, con
     }
     CK(cudaSetDevice(ctx->device));
     zero_stats(stats);
-    for (int i = 0; i < NLANES; ++i)
-        if (ctx->lane[i].job.active)
-            finish_deferred(ctx, i);
+    finish_all_deferred(ctx);
     Lane &L = ctx->lane[0];
     cudaStream_t s = L.stream;
     JobGeom g3;
@@ -1611,16 +1617,7 @@ extern "C" int kpeg_cuda_decode_scans(kpeg_ctx *ctx, const kpeg_plan *frame, con
     CK(cudaMemsetAsync(d_meta, 0, sizeof(DevMeta), s));
     mark(ctx, L, -1);
     launch_interleave_tiles(ctx->scan_tiles[0].p, ctx->scan_tiles[1].p, ctx->scan_tiles[2].p, L.tiles.p, nmcu_padded, s, &launches);
-    IdctArgs ia;
-    ia.tiles = L.tiles.p;
-    ia.nstrips = nstrips;
-    ia.tables = (const DeviceTables *)ctx->tables.p;
-    ia.pixels = (uint8_t *)L.pixels.p;
-    ia.tie_rec = (uint4 *)L.tie_rec.p;
-    ia.tie_cnt = (uint32_t *)L.tie_cnt.p;
-    ia.meta = d_meta;
-    ia.g = g3;
-    CK(launch_idct(ia, s, &launches));
+    CK(launch_idct(idct_args(ctx, L, g3, nstrips, L.tiles.p, (uint8_t *)L.pixels.p), s, &launches));
     mark(ctx, L, KPEG_T_IDCT);
     CK(cudaMemcpyAsync(pixels_out, L.pixels.p, npix, cudaMemcpyDeviceToHost, s));
     mark(ctx, L, KPEG_T_D2H);
@@ -1628,7 +1625,7 @@ extern "C" int kpeg_cuda_decode_scans(kpeg_ctx *ctx, const kpeg_plan *frame, con
     CK(cudaStreamSynchronize(s));
     CK(cudaGetLastError());
     if (ctx->guard)
-        TRY(check_guards(ctx, L));
+        TRY(check_guards(ctx));
     ctx->last_lane = 0;
     ctx->last_g = g3; // kpeg_cuda_read_coefficients: the interleaved tiles
     if (stats) {
@@ -1730,31 +1727,9 @@ extern "C" int kpeg_cuda_decode_files(kpeg_ctx *ctx, int n, const uint8_t *const
         groups[g].lens.push_back(f.scans[0].len);
         groups[g].outs.push_back(pixels_out[i]);
     }
-    // earlier deferred submissions keep their own outcome for the caller's kpeg_cuda_wait
-    for (int i = 0; i < NLANES; ++i)
-        if (ctx->lane[i].job.active)
-            finish_deferred(ctx, i);
-    const int saved_rc = ctx->deferred_rc;
-    const std::string saved_err = ctx->deferred_err;
-    const kpeg_stats saved_stats = ctx->deferred_stats;
-    auto reset_deferred = [&]() {
-        ctx->deferred_rc = KPEG_OK;
-        ctx->deferred_err.clear();
-        memset(&ctx->deferred_stats, 0, sizeof ctx->deferred_stats);
-    };
-    auto add_stats = [&](const kpeg_stats &p) {
-        if (!stats)
-            return;
-        stats->scan_bytes += p.scan_bytes;
-        stats->unstuffed_bytes += p.unstuffed_bytes;
-        stats->segments += p.segments;
-        stats->subsequences += p.subsequences;
-        stats->sync_rounds = std::max(stats->sync_rounds, p.sync_rounds);
-        stats->exact_samples += p.exact_samples;
-        stats->kernel_launches += p.kernel_launches;
-    };
+    finish_all_deferred(ctx);
+    const DeferredOutcomeSaved saved(ctx);
     // every group is submitted, then ONE wait: the groups overlap on the lanes like consecutive batches do
-    reset_deferred();
     int all_rc = KPEG_OK;
     for (Group &g : groups) {
         const int rc = kpeg_cuda_submit_batch(ctx, &g.plan, (int)g.members.size(), g.scans.data(), g.lens.data(), g.outs.data());
@@ -1762,16 +1737,17 @@ extern "C" int kpeg_cuda_decode_files(kpeg_ctx *ctx, int n, const uint8_t *const
             all_rc = rc;
     }
     {
-        kpeg_stats part;
+        kpeg_stats part = {};
         const int wrc = kpeg_cuda_wait(ctx, &part);
         if (all_rc == KPEG_OK)
             all_rc = wrc;
-        add_stats(part);
+        if (stats)
+            add_stats(*stats, part);
     }
     if (all_rc != KPEG_OK) {
         // something failed, and a deferred failure does not say where: group by group, then file by file
         for (Group &g : groups) {
-            reset_deferred();
+            reset_deferred(ctx);
             int rc = kpeg_cuda_submit_batch(ctx, &g.plan, (int)g.members.size(), g.scans.data(), g.lens.data(), g.outs.data());
             kpeg_stats part;
             const int wrc = kpeg_cuda_wait(ctx, &part);
@@ -1794,15 +1770,17 @@ extern "C" int kpeg_cuda_decode_files(kpeg_ctx *ctx, int n, const uint8_t *const
         File &f = fl[(size_t)i];
         if (f.rc != KPEG_OK || f.nscans == 1)
             continue;
-        kpeg_stats part;
+        kpeg_stats part = {};
         const int rc = kpeg_cuda_decode_scans(ctx, &f.frame, f.scans, f.nscans, files[i], lens[i], pixels_out[i], &part);
-        add_stats(part);
+        if (stats)
+            add_stats(*stats, part);
         if (rc != KPEG_OK)
             note(i, rc, ctx->err.c_str());
     }
-    ctx->deferred_rc = saved_rc;
-    ctx->deferred_err = saved_err;
-    ctx->deferred_stats = saved_stats;
+    if (stats) { // no stage times: the groups' jobs overlap on the lanes, so their sum is no time of this call
+        memset(stats->ms, 0, sizeof stats->ms);
+        stats->ms_total = 0.0f;
+    }
     if (results)
         for (int i = 0; i < n; ++i)
             results[i] = fl[(size_t)i].rc;
@@ -1913,13 +1891,12 @@ int encode_scratch(kpeg_ctx *ctx, const enc::EncGeom &g, enc::EncBufs *bp)
 
 // Tables (per quality) and scratch, then E1..E5 on lane 0 and the read-back of the length words into h_meta.
 // d_out / out_cap: the file and how many bytes may be written there; hdr_len: bytes of it the host has written.
-int encode_enqueue(kpeg_ctx *ctx, const kpeg_encode_params *p, const uint8_t *d_pixels, uint8_t *d_out, uint64_t out_cap,
+int encode_enqueue(kpeg_ctx *ctx, int quality, const enc::EncGeom &g, const uint8_t *d_pixels, uint8_t *d_out, uint64_t out_cap,
                    uint64_t hdr_len, uint32_t *launches)
 {
     EncScratch &E = ctx->enc;
     cudaStream_t s = ctx->lane[0].stream;
-    TRY(encode_tables(ctx, p->quality));
-    const enc::EncGeom g = enc::geometry(p->width, p->height, p->ncomp, p->restart_interval, p->flags);
+    TRY(encode_tables(ctx, quality));
     enc::EncBufs b;
     TRY(encode_scratch(ctx, g, &b));
     b.pixels = d_pixels;
@@ -1931,28 +1908,46 @@ int encode_enqueue(kpeg_ctx *ctx, const kpeg_encode_params *p, const uint8_t *d_
     return KPEG_OK;
 }
 
-void encode_stats(kpeg_ctx *ctx, const kpeg_encode_params *p, uint32_t launches, kpeg_stats *stats)
+// the encoder's figures for the file of geometry g that lane 0 has coded (h_meta read back)
+void encode_stats(kpeg_ctx *ctx, const enc::EncGeom &g, uint32_t launches, kpeg_stats *stats)
 {
     if (!stats)
         return;
     const enc::EncMeta *m = (const enc::EncMeta *)ctx->enc.h_meta.p;
-    const enc::EncGeom g = enc::geometry(p->width, p->height, p->ncomp, p->restart_interval, p->flags);
-    stats->width = p->width;
-    stats->height = p->height;
-    stats->ncomp = p->ncomp;
+    stats->width = g.width;
+    stats->height = g.height;
+    stats->ncomp = g.ncomp;
     stats->scan_bytes = m->scan_len;
     stats->unstuffed_bytes = m->unstuffed;
     stats->segments = (uint32_t)g.nseg;
-    stats->kernel_launches = launches;
+    stats->kernel_launches += launches;
     add_times(ctx, ctx->lane[0], stats);
 }
 
-// every pending deferred submission is completed first (its outcome is reported by kpeg_cuda_wait)
-void finish_all_deferred(kpeg_ctx *ctx)
+// The end of an encode into host memory, once the coded stages are enqueued on lane 0 (h_meta's read-back included):
+// *len = the file's size; when it fits in cap, the part of the header the host wrote (the whole Annex K header, or the
+// prefix up to SOF0) and the rest from the device (optimised mode: the header's tail, then the scan) go to out.  Then the
+// guard check and the figures; KPEG_ERR_NOMEM with too_small when the file does not fit.
+int finish_encoded_file(kpeg_ctx *ctx, const std::vector<uint8_t> &hdr, const enc::EncGeom &g, uint32_t launches, uint8_t *out,
+                        size_t cap, size_t *len, kpeg_stats *stats, const char *too_small)
 {
-    for (int i = 0; i < NLANES; ++i)
-        if (ctx->lane[i].job.active)
-            finish_deferred(ctx, i);
+    Lane &L = ctx->lane[0];
+    CK(cudaStreamSynchronize(L.stream));
+    CK(cudaGetLastError());
+    const enc::EncMeta *m = (const enc::EncMeta *)ctx->enc.h_meta.p;
+    *len = m->hdr_len + m->scan_len;
+    const bool fits = *len <= cap;
+    if (fits) {
+        memcpy(out, hdr.data(), hdr.size());
+        CK(cudaMemcpyAsync(out + hdr.size(), (const uint8_t *)ctx->enc.out.p + hdr.size(), *len - hdr.size(), cudaMemcpyDeviceToHost,
+                           L.stream));
+        mark(ctx, L, KPEG_T_D2H);
+        CK(cudaStreamSynchronize(L.stream));
+    }
+    if (ctx->guard)
+        TRY(check_guards(ctx));
+    encode_stats(ctx, g, launches, stats);
+    return fits ? KPEG_OK : fail(ctx, KPEG_ERR_NOMEM, too_small);
 }
 
 } // namespace
@@ -1978,32 +1973,16 @@ extern "C" int kpeg_cuda_encode(kpeg_ctx *ctx, const kpeg_encode_params *p, cons
     const std::vector<uint8_t> hdr = encode_host_header(p);
     const size_t bound = (size_t)enc::encode_bound(p->width, p->height, p->ncomp, p->quality, p->restart_interval, p->flags);
     const size_t out_cap = std::min(cap, bound);
+    const enc::EncGeom g = enc::geometry(p->width, p->height, p->ncomp, p->restart_interval, p->flags);
     TRY(ensure(ctx, L.stream, E.pixels, npix + 64));
     TRY(ensure(ctx, L.stream, E.out, out_cap + 64));
     mark(ctx, L, -1);
     CK(cudaMemcpyAsync(E.pixels.p, pixels, npix, cudaMemcpyHostToDevice, L.stream));
     mark(ctx, L, KPEG_T_H2D);
     uint32_t launches = 0;
-    TRY(encode_enqueue(ctx, p, (const uint8_t *)E.pixels.p, (uint8_t *)E.out.p, out_cap, hdr.size(), &launches));
-    CK(cudaStreamSynchronize(L.stream));
-    CK(cudaGetLastError());
-    const enc::EncMeta *m = (const enc::EncMeta *)E.h_meta.p;
-    *jpeg_len = m->hdr_len + m->scan_len;
-    if (*jpeg_len > cap) {
-        encode_stats(ctx, p, launches, stats);
-        return fail(ctx, KPEG_ERR_NOMEM, "output buffer smaller than the encoded file (*jpeg_len = the size needed)");
-    }
-    // what the host wrote (the whole Annex K header, or the prefix up to SOF0) is copied here; the rest comes from the
-    // device (optimised mode: the header's tail and the scan)
-    memcpy(jpeg_out, hdr.data(), hdr.size());
-    CK(cudaMemcpyAsync(jpeg_out + hdr.size(), (const uint8_t *)E.out.p + hdr.size(), *jpeg_len - hdr.size(), cudaMemcpyDeviceToHost,
-                       L.stream));
-    mark(ctx, L, KPEG_T_D2H);
-    CK(cudaStreamSynchronize(L.stream));
-    if (ctx->guard)
-        TRY(check_guards(ctx, L));
-    encode_stats(ctx, p, launches, stats);
-    return KPEG_OK;
+    TRY(encode_enqueue(ctx, p->quality, g, (const uint8_t *)E.pixels.p, (uint8_t *)E.out.p, out_cap, hdr.size(), &launches));
+    return finish_encoded_file(ctx, hdr, g, launches, jpeg_out, cap, jpeg_len, stats,
+                               "output buffer smaller than the encoded file (*jpeg_len = the size needed)");
 }
 
 extern "C" int kpeg_cuda_encode_device(kpeg_ctx *ctx, const kpeg_encode_params *p, const uint8_t *d_pixels, uint8_t *d_out, size_t cap,
@@ -2016,16 +1995,17 @@ extern "C" int kpeg_cuda_encode_device(kpeg_ctx *ctx, const kpeg_encode_params *
     finish_all_deferred(ctx);
     Lane &L = ctx->lane[0];
     const std::vector<uint8_t> hdr = encode_host_header(p);
+    const enc::EncGeom g = enc::geometry(p->width, p->height, p->ncomp, p->restart_interval, p->flags);
     mark(ctx, L, -1);
     if (cap)
         CK(cudaMemcpyAsync(d_out, hdr.data(), std::min(cap, hdr.size()), cudaMemcpyHostToDevice, L.stream));
     uint32_t launches = 0;
-    TRY(encode_enqueue(ctx, p, d_pixels, d_out, cap, hdr.size(), &launches));
+    TRY(encode_enqueue(ctx, p->quality, g, d_pixels, d_out, cap, hdr.size(), &launches));
     CK(cudaStreamSynchronize(L.stream));
     CK(cudaGetLastError());
     if (ctx->guard)
-        TRY(check_guards(ctx, L));
-    encode_stats(ctx, p, launches, stats);
+        TRY(check_guards(ctx));
+    encode_stats(ctx, g, launches, stats);
     const enc::EncMeta *m = (const enc::EncMeta *)ctx->enc.h_meta.p;
     *jpeg_len = m->hdr_len + m->scan_len;
     if (*jpeg_len > cap)
@@ -2133,12 +2113,7 @@ extern "C" int kpeg_cuda_transcode(kpeg_ctx *ctx, const uint8_t *file, size_t le
     if (nscans == 1) {
         kpeg_plan dp = scans[0].plan;
         dp.flags = 0;
-        TRY(ensure(ctx, s, L.scan, scans[0].len + 64));
-        mark(ctx, L, -1);
-        CK(cudaMemcpyAsync(L.scan.p, file + scans[0].off, scans[0].len, cudaMemcpyHostToDevice, s));
-        mark(ctx, L, KPEG_T_H2D);
-        TRY(job_enqueue(ctx, 0, &dp, (const uint8_t *)L.scan.p, scans[0].len, 1, nullptr, {}, L.tiles.p));
-        TRY(job_finish(ctx, 0, stats));
+        TRY(decode_host_scan(ctx, &dp, file + scans[0].off, scans[0].len, nullptr, {}, L.tiles.p, stats));
     } else {
         TRY(entropy_decode_component_scans(ctx, scans, file, 0u, nmcu_padded, stats));
         mark(ctx, L, -1);
@@ -2173,29 +2148,6 @@ extern "C" int kpeg_cuda_transcode(kpeg_ctx *ctx, const uint8_t *file, size_t le
     mark(ctx, L, -1);
     CK(enc::launch_coded_stages(g, b, b.dc, s, &launches, tc_mark, ctx));
     CK(cudaMemcpyAsync(h_meta, d_meta, sizeof(enc::EncMeta), cudaMemcpyDeviceToHost, s));
-    CK(cudaStreamSynchronize(s));
-    CK(cudaGetLastError());
-    *out_len = h_meta->hdr_len + h_meta->scan_len;
-    const bool fits = *out_len <= cap;
-    if (fits) {
-        memcpy(out, hdr.data(), hdr.size());
-        CK(cudaMemcpyAsync(out + hdr.size(), (const uint8_t *)E.out.p + hdr.size(), *out_len - hdr.size(), cudaMemcpyDeviceToHost, s));
-        mark(ctx, L, KPEG_T_D2H);
-        CK(cudaStreamSynchronize(s));
-    }
-    if (ctx->guard)
-        TRY(check_guards(ctx, L));
-    if (stats) {
-        stats->width = g.width;
-        stats->height = g.height;
-        stats->ncomp = g.ncomp;
-        stats->scan_bytes = h_meta->scan_len;
-        stats->unstuffed_bytes = h_meta->unstuffed;
-        stats->segments = (uint32_t)g.nseg;
-        stats->kernel_launches += launches;
-        add_times(ctx, L, stats);
-    }
-    if (!fits)
-        return fail(ctx, KPEG_ERR_NOMEM, "output buffer smaller than the transcoded file (*out_len = the size needed)");
-    return KPEG_OK;
+    return finish_encoded_file(ctx, hdr, g, launches, out, cap, out_len, stats,
+                               "output buffer smaller than the transcoded file (*out_len = the size needed)");
 }
