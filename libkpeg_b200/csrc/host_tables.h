@@ -55,6 +55,35 @@ inline int build_device_tables(const kpeg_plan *pl, DeviceTables *T, const char 
     return KPEG_OK;
 }
 
+// Records per subsequence the relay passes keep room for: 3/8 of its bits covers every table whose value-carrying
+// symbols take at least 3 bits (code >= 2 bits + value >= 1 bit: all of Annex K); a stream that needs more sets
+// ST_REC_OVERFLOW and is redone with the Huffman final pass.
+inline uint32_t rec_kmax_of(uint32_t sub_bits) { return (sub_bits * 3u / 8u + 7u) & ~7u; }
+
+// Whether the 1-bits that pad an interval before its RSTn marker (at most 7, T.81 F.1.2.3) can hold a whole DC symbol of
+// the first component: its table has an all-ones code (it fills the code space, which T.81 C and libjpeg do not allow)
+// whose length plus category is at most 7.  The decoder takes a symbol that fits before a boundary for data
+// (entropy_core.h relay_run), so such padding would count as one more block.  That is harmless after the last MCU of
+// a job, which is where a single image without restart markers has its only padding.
+inline bool restart_padding_decodes(const kpeg_plan *pl)
+{
+    const unsigned td = pl->comp_td[0];
+    if (td > 3 || !pl->ht_present[0][td])
+        return false;
+    const kpeg_huff_spec &h = pl->ht[0][td];
+    uint32_t space = 0, nsym = 0; // code space in units of 2^-16
+    int last_len = 0;
+    for (int L = 1; L <= 16; ++L) {
+        space += (uint32_t)h.counts[L - 1] << (16 - L);
+        nsym += h.counts[L - 1];
+        if (h.counts[L - 1])
+            last_len = L;
+    }
+    if (space != (1u << 16) || nsym == 0 || nsym > 256)
+        return false; // the last code is all ones only in a table that fills the code space
+    return last_len + (h.symbols[nsym - 1] & 15) <= 7;
+}
+
 inline int make_job_geom(const kpeg_plan *pl, uint32_t nimages, uint32_t sub_bits, JobGeom *g, const char **why)
 {
     if (pl->width == 0 || pl->height == 0 || (pl->ncomp != 1 && pl->ncomp != 3) || nimages == 0) {

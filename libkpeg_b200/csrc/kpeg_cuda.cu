@@ -544,6 +544,9 @@ int job_enqueue(kpeg_ctx *ctx, int li, const kpeg_plan *pl, const uint8_t *d_sca
     int rc = make_job_geom(pl, nimages, sub_bits, &g, &why);
     if (rc != KPEG_OK)
         return fail(ctx, rc, why);
+    if ((pl->restart_interval != 0 || nimages > 1) && restart_padding_decodes(pl))
+        return fail(ctx, KPEG_ERR_UNSUPPORTED, "the DC table fills the code space: the padding before a restart or image "
+                                               "boundary would decode as a symbol (one image without restart markers decodes)");
     if (scan_len == 0 || scan_len >= (1ull << 29))
         return fail(ctx, KPEG_ERR_ARG, "entropy-coded segment must be 1 byte .. 512 MiB");
     TRY(upload_plan(ctx, pl));
@@ -574,10 +577,8 @@ int job_enqueue(kpeg_ctx *ctx, int li, const kpeg_plan *pl, const uint8_t *d_sca
     TRY(ensure(ctx, s, L.tie_cnt, (size_t)nstrips * sizeof(uint32_t)));
     TRY(ensure(ctx, s, L.meta, sizeof(DevMeta)));
     TRY(ensure_pinned(ctx, s, L.h_meta, sizeof(DevMeta)));
-    // records: one per value-carrying symbol.  3/8 of the subsequence's bits covers every table whose value-carrying
-    // symbols take at least 3 bits (code >= 2 bits + value >= 1 bit: all of Annex K); a stream that needs more sets
-    // ST_REC_OVERFLOW and is redone with the Huffman final pass
-    const uint32_t rec_kmax = (g.sub_bits * 3u / 8u + 7u) & ~7u;
+    // records: one per value-carrying symbol (host_tables.h rec_kmax_of)
+    const uint32_t rec_kmax = rec_kmax_of(g.sub_bits);
     const uint32_t rec_alt_cap = nsub_max / 4u + 1024u; // beyond it a redone subsequence rewrites its interleaved column
     if (ctx->use_records) {
         TRY(ensure(ctx, s, L.rec, (size_t)rec_kmax * ((size_t)nsub_max / 32u + 1u) * 32u * sizeof(uint32_t)));
@@ -1714,7 +1715,9 @@ extern "C" int kpeg_cuda_decode_files(kpeg_ctx *ctx, int n, const uint8_t *const
             continue; // one scan per component: decoded on its own below
         kpeg_plan pl = f.scans[0].plan;
         pl.flags = flags;
-        size_t g = 0;
+        // a plan whose padding can decode as a symbol has no batches (job_enqueue): such files are one job each
+        const bool alone = restart_padding_decodes(&pl);
+        size_t g = alone ? groups.size() : 0;
         while (g < groups.size() && memcmp(&groups[g].plan, &pl, sizeof pl) != 0)
             ++g;
         if (g == groups.size()) {

@@ -73,7 +73,8 @@ extern "C" {
 
 // info[0]=status, [1]=nsub, [2]=relay rounds until the fixed point, [3]=exact IDCT samples,
 // [4]=exact colour pixels, [5]=total_bits, [6]=final_slot, [7]=record final pass == Huffman final pass,
-// [8]=most records in one subsequence
+// [8]=most records in one subsequence, [9]=subsequences with more records than the product keeps room for (rec_kmax_of:
+// the device would redo the job with the Huffman final pass)
 int emu_decode(const uint8_t *scan, size_t scan_len, const kpeg_plan *plan, uint32_t nimages, uint32_t sub_bits,
                int16_t *coef_out, uint8_t *pixels_out, uint32_t *info)
 {
@@ -185,7 +186,7 @@ int emu_decode(const uint8_t *scan, size_t scan_len, const kpeg_plan *plan, uint
         };
         std::vector<int16_t> coef2((size_t)g.total_blocks * 64, 0);
         const uint32_t total_slots = g.total_blocks * 64u;
-        uint32_t st2 = 0, max_rec = 0;
+        uint32_t st2 = 0, max_rec = 0, over_kmax = 0;
         std::vector<long long> dcs(nsub, 0), dcpre(nsub, 0); // K2 as a scan: per-subsequence DC sums and their segmented prefix
         std::vector<std::vector<uint32_t>> all_recs(nsub);
         for (uint32_t sub = 0; sub < nsub; ++sub) {
@@ -209,6 +210,7 @@ int emu_decode(const uint8_t *scan, size_t scan_len, const kpeg_plan *plan, uint
             if (out.p != X[sub].p || ((out.cz ^ X[sub].cz) & CZ_STATE_MASK) || out.n != X[sub].n || out.seg != X[sub].seg)
                 records_ok = 0;
             max_rec = std::max<uint32_t>(max_rec, d.nrec);
+            over_kmax += d.nrec > rec_kmax_of(sub_bits) ? 1u : 0u;
             // entropy_scan_apply_kernel
             const uint32_t begin = start[sub], fin = sub + 1 < nsub ? start[sub + 1] : final_slot;
             st2 |= (out.cz & CZ_BAD_CODE) ? ST_BAD_CODE : 0u;
@@ -284,8 +286,10 @@ int emu_decode(const uint8_t *scan, size_t scan_len, const kpeg_plan *plan, uint
             records_ok = 0;
         if ((status != 0) != (st2 != 0)) // a stream one flavour rejects, the other must reject too
             records_ok = 0;
-        if (info)
+        if (info) {
             info[8] = max_rec;
+            info[9] = over_kmax;
+        }
     }
     // K2
     {
@@ -482,6 +486,60 @@ uint32_t emu_huff_lookup(const uint8_t counts[16], const uint8_t *symbols, int i
     delete L;
     return e;
 }
+
+// The same lookup over n windows at once: out[i] = emu_huff_lookup(.., wins[i], mode).
+void emu_huff_lookup_many(const uint8_t counts[16], const uint8_t *symbols, int is_ac, const uint32_t *wins, uint32_t n, int mode,
+                          uint32_t *out)
+{
+    LutSet *L = new LutSet;
+    HuffCanon canon;
+    const bool ok = build_huff_lut(counts, symbols, is_ac != 0, L, 0, &canon) == 0;
+    const PlainLuts PL{L, &canon};
+    for (uint32_t i = 0; i < n; ++i) {
+        const uint32_t win = wins[i];
+        uint32_t e = 0xFFFFFFFFu;
+        if (ok && mode == 1) {
+            e = ENTRY_INVALID;
+            const uint32_t w16 = win >> 16;
+            for (int len = 1; len <= 16; ++len)
+                if (w16 < canon.bound[len]) {
+                    const uint32_t k = canon.first_idx[len] + ((w16 >> (16 - len)) - canon.first_code[len]);
+                    e = pack_entry((uint32_t)len, canon.symbols[k & 255u], is_ac != 0);
+                    break;
+                }
+        } else if (ok) {
+            e = PL.fast(0, win >> (32 - LUT_BITS));
+            if ((e & 31u) == 0u)
+                e = PL.slow(0, win, e);
+        }
+        out[i] = e;
+    }
+    delete L;
+}
+
+// How the kernels' tables hold one Huffman table: *long_n = second-level entries in use, canonical[prefix] = 1 for
+// every LUT_BITS-bit prefix that starts a longer code but got no sub-table (those codes take huff_slow_lookup).
+// Returns the number of such prefixes, or -1 if the table does not build.
+int emu_huff_layout(const uint8_t counts[16], const uint8_t *symbols, int is_ac, uint32_t *long_n, uint8_t *canonical)
+{
+    LutSet *L = new LutSet;
+    HuffCanon canon;
+    int n = -1;
+    if (build_huff_lut(counts, symbols, is_ac != 0, L, 0, &canon) == 0) {
+        n = 0;
+        *long_n = L->long_n[0];
+        for (uint32_t prefix = 0; prefix < (uint32_t)LUT_SIZE; ++prefix) {
+            const bool longer = (prefix << (16 - LUT_BITS)) >= canon.bound[LUT_BITS] && (prefix << (16 - LUT_BITS)) < canon.bound[16];
+            canonical[prefix] = longer && L->fast[0][prefix] == 0 ? 1u : 0u;
+            n += canonical[prefix];
+        }
+    }
+    delete L;
+    return n;
+}
+
+// host_tables.h restart_padding_decodes: 1 if the job refuses restart intervals and batches for this plan
+int emu_restart_padding_decodes(const kpeg_plan *plan) { return restart_padding_decodes(plan) ? 1 : 0; }
 
 int emu_zigzag(int i) { return zigzag_to_natural(i); }
 

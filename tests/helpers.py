@@ -133,6 +133,12 @@ def emu():
         lib.emu_classify_compare.argtypes = [C.c_void_p, C.c_uint32, C.POINTER(C.c_int)]
         lib.emu_huff_lookup.restype = C.c_uint32
         lib.emu_huff_lookup.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_uint32, C.c_int]
+        lib.emu_huff_lookup_many.restype = None
+        lib.emu_huff_lookup_many.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_uint32, C.c_int, C.c_void_p]
+        lib.emu_huff_layout.restype = C.c_int
+        lib.emu_huff_layout.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.POINTER(C.c_uint32), C.c_void_p]
+        lib.emu_restart_padding_decodes.restype = C.c_int
+        lib.emu_restart_padding_decodes.argtypes = [C.c_void_p]
         lib.emu_zigzag.restype = C.c_int
         lib.emu_zigzag.argtypes = [C.c_int]
         lib.emu_pair_tables.restype = C.c_int
@@ -170,4 +176,4 @@ def emu_decode(data, flags: int = 1, sub_bits: int = 512, want_pixels: bool = Tr
             pixels = pixels[..., 0]
     return dict(coef=coef, pixels=pixels, status=int(info[0]), nsub=int(info[1]), rounds=int(info[2]),
                 exact=int(info[3]), colour_exact=int(info[4]), total_bits=int(info[5]), final_slot=int(info[6]),
-                records_ok=bool(info[7]), max_records=int(info[8]), plan=plan)
+                records_ok=bool(info[7]), max_records=int(info[8]), subs_over_kmax=int(info[9]), plan=plan)

@@ -34,14 +34,19 @@ def permuted_table(counts, symbols, seed):
 
 
 class BitWriter:
+    """bits: bits written so far, padding included -- the bit position in the scan once stuffed bytes and markers are
+    taken out."""
+
     def __init__(self):
         self.out = bytearray()
         self.acc = 0
         self.n = 0
+        self.bits = 0
 
     def put(self, code, length):
         self.acc = (self.acc << length) | (code & ((1 << length) - 1))
         self.n += length
+        self.bits += length
         while self.n >= 8:
             b = (self.acc >> (self.n - 8)) & 0xFF
             self.out.append(b)
@@ -54,6 +59,11 @@ class BitWriter:
         if self.n:
             self.put((1 << (8 - self.n)) - 1, 8 - self.n)
 
+    def marker(self, m):
+        """Pad to a byte with 1-bits (T.81 F.1.2.3) and write marker 0xFF m (RSTn)."""
+        self.flush()
+        self.out += bytes([0xFF, m])
+
 
 def _category(v):
     return int(abs(int(v))).bit_length()
@@ -64,13 +74,20 @@ def _magnitude_bits(v, cat):
     return v if v >= 0 else v + (1 << cat) - 1
 
 
-def encode_blocks(bw, blocks, dc_codes, ac_codes, pred):
-    """blocks: iterable of (component, int16[64]); pred: running DC predictors (list, updated in place)."""
+def encode_blocks(bw, blocks, dc_codes, ac_codes, pred, marks=None):
+    """blocks: iterable of (component, int16[64]); pred: running DC predictors (list, updated in place).
+    marks: a list that gets (bw.bits, component, is_ac, symbol, code length, category) of every symbol written."""
+    def put(c, is_ac, sym, size):
+        code = (ac_codes if is_ac else dc_codes)[c][sym]
+        if marks is not None:
+            marks.append((bw.bits, c, is_ac, sym, code[1], size))
+        bw.put(*code)
+
     for c, blk in blocks:
         diff = int(blk[0]) - pred[c]
         pred[c] = int(blk[0])
         cat = _category(diff)
-        bw.put(*dc_codes[c][cat])
+        put(c, False, cat, cat)
         if cat:
             bw.put(_magnitude_bits(diff, cat), cat)
         run = 0
@@ -83,14 +100,14 @@ def encode_blocks(bw, blocks, dc_codes, ac_codes, pred):
                 run += 1
                 continue
             while run > 15:
-                bw.put(*ac_codes[c][0xF0])
+                put(c, True, 0xF0, 0)
                 run -= 16
             cat = _category(v)
-            bw.put(*ac_codes[c][(run << 4) | cat])
+            put(c, True, (run << 4) | cat, cat)
             bw.put(_magnitude_bits(v, cat), cat)
             run = 0
         if last < 63:
-            bw.put(*ac_codes[c][0x00])
+            put(c, True, 0x00, 0)
 
 
 def _seg(marker, payload):
@@ -98,9 +115,11 @@ def _seg(marker, payload):
 
 
 def write_jpeg(coef, width, height, ncomp, qts, tq, dc_tables, ac_tables, td, ta, comp_ids=(1, 2, 3),
-               interleaved=True, extra_segments=b"", scan_order=None, redefine=None):
+               interleaved=True, extra_segments=b"", scan_order=None, redefine=None, restart_interval=0, marks=None):
     """coef [blocks][64] (MCU-interleaved, zig-zag, DC integrated).  qts: {id: 64 values (zig-zag)};
     dc_tables / ac_tables: {id: (counts[16], symbols)}; tq / td / ta: table id per component.
+    restart_interval: MCUs per interval (a DRI segment, RSTn markers after every interval, predictors reset, T.81
+    F.1.2.3 / F.2.1.3.1); marks: see encode_blocks (bit positions count from the start of the scan they are in).
     Non-interleaved files only: scan_order = the components in the order their scans are written (default 0, 1, 2);
     redefine = {component: (dc_tables, ac_tables, td, ta)}: DHT segments written right before that component's scan
     (they REPLACE tables of the same id, T.81 B.2.4.2) and the selectors that scan uses."""
@@ -116,6 +135,8 @@ def write_jpeg(coef, width, height, ncomp, qts, tq, dc_tables, ac_tables, td, ta
     for c in range(ncomp):
         sof += bytes([comp_ids[c], 0x11, tq[c]])
     out += _seg(0xC0, sof)
+    if restart_interval:
+        out += _seg(0xDD, int(restart_interval).to_bytes(2, "big"))
     for cls, tabs in ((0, dc_tables), (1, ac_tables)):
         for tid, (counts, symbols) in tabs.items():
             n = int(sum(counts))
@@ -141,7 +162,14 @@ def write_jpeg(coef, width, height, ncomp, qts, tq, dc_tables, ac_tables, td, ta
         out += _seg(0xDA, sos)
         bw = BitWriter()
         pred = [0] * ncomp
-        encode_blocks(bw, ((c, coef[m * ncomp + c]) for m in range(mx * my) for c in comps), dc_codes, ac_codes, pred)
+        nmcu = mx * my
+        step = restart_interval or nmcu
+        for i, m0 in enumerate(range(0, nmcu, step)):
+            if m0:
+                bw.marker(0xD0 + (i - 1) % 8)
+                pred = [0] * ncomp
+            encode_blocks(bw, ((c, coef[m * ncomp + c]) for m in range(m0, min(m0 + step, nmcu)) for c in comps), dc_codes,
+                          ac_codes, pred, marks)
         bw.flush()
         out += bw.out
     out += b"\xff\xd9"
