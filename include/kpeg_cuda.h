@@ -98,7 +98,7 @@ enum {
 /* Per-decode statistics.  Stage times are filled only while profiling is enabled
  * (kpeg_cuda_set_profiling); they are CUDA-event times on the decode stream, in milliseconds. */
 typedef struct kpeg_stats {
-    uint32_t width, height, ncomp; /* of the output image (the reduced size with KPEG_FLAG_SCALE_*) */
+    uint32_t width, height, ncomp; /* of the output image (the reduced size with KPEG_FLAG_SCALE_*; a crop's rectangle) */
     uint64_t scan_bytes;        /* stuffed entropy-coded bytes handed in                  */
     uint64_t unstuffed_bytes;   /* after FF00 / RSTn removal                              */
     uint32_t segments;          /* restart intervals found (1 when there is no DRI)       */
@@ -259,6 +259,37 @@ int kpeg_cuda_decode_file(kpeg_ctx *ctx, const uint8_t *file, size_t len, uint32
  * (text: kpeg_cuda_last_error).  Host buffers (ideally pinned) in and out; synchronous. */
 int kpeg_cuda_decode_files(kpeg_ctx *ctx, int n, const uint8_t *const *files, const size_t *lens, uint32_t flags,
                            uint8_t *const *pixels_out, const size_t *caps, kpeg_plan *plans_out, int *results, kpeg_stats *stats);
+
+/* ---- crop decode ------------------------------------------------------------------------------------------------------
+ * A rectangle of the output image: x, y, width, height in pixels of the image the same call without a crop would produce
+ * (the full image, or the reduced one with KPEG_FLAG_SCALE_* bits, as libjpeg crops its scaled output).  The result is
+ * byte for byte that output's rows y .. y+height-1, columns x .. x+width-1, written tightly packed (rows of
+ * width*ncomp bytes); in both parity modes, at every scale.  The rectangle is exact: it is not widened to MCU boundaries
+ * (djpeg -crop is).  An empty rectangle, or one that reaches past the output image, returns KPEG_ERR_ARG before any work
+ * is enqueued.  The whole stream is still entropy-decoded (where each block begins depends on every symbol before it),
+ * so corruption anywhere in it is KPEG_ERR_STREAM; only the strips of 32 MCUs that hold pixels of the rectangle are
+ * expanded and reconstructed, and only the rectangle's bytes are written and copied.  kpeg_stats.width / height report
+ * the rectangle (a batch: the first image's).  After a crop decode kpeg_cuda_read_coefficients returns
+ * KPEG_ERR_UNSUPPORTED until the next decode without a crop on the context.  There are no tiled, deferred or
+ * multi-file crop forms. */
+typedef struct kpeg_crop {
+    uint32_t x, y, width, height;
+} kpeg_crop;
+
+/* kpeg_cuda_decode, cropped: pixels_out is a HOST buffer of crop->width*crop->height*ncomp bytes.  One job on the
+ * context's first lane (never cut into bands). */
+int kpeg_cuda_decode_crop(kpeg_ctx *ctx, const kpeg_plan *plan, const uint8_t *scan, size_t scan_len, const kpeg_crop *crop,
+                          uint8_t *pixels_out, kpeg_stats *stats);
+/* kpeg_cuda_decode_device, cropped: DEVICE pointers in and out. */
+int kpeg_cuda_decode_crop_device(kpeg_ctx *ctx, const kpeg_plan *plan, const uint8_t *d_scan, size_t scan_len,
+                                 const kpeg_crop *crop, uint8_t *d_pixels_out, kpeg_stats *stats);
+/* kpeg_cuda_decode_batch, cropped: image i's rectangle is crops[i], pixels_out[i] holds
+ * crops[i].width*crops[i].height*ncomp bytes.  One kernel sequence per chunk, as kpeg_cuda_decode_batch. */
+int kpeg_cuda_decode_batch_crop(kpeg_ctx *ctx, const kpeg_plan *plan, int n, const uint8_t *const *scans,
+                                const size_t *scan_lens, const kpeg_crop *crops, uint8_t *const *pixels_out, kpeg_stats *stats);
+/* kpeg_cuda_decode_file, cropped (frames coded one scan per component too): cap is checked against the crop's bytes. */
+int kpeg_cuda_decode_file_crop(kpeg_ctx *ctx, const uint8_t *file, size_t len, uint32_t flags, const kpeg_crop *crop,
+                               uint8_t *pixels_out, size_t cap, kpeg_plan *plan_out, kpeg_stats *stats);
 
 /* Parity hook: the quantised coefficients of the LAST decode on this context, as the reference
  * holds them transiently inside MCU::constructMCU (MCU.cpp:93-108): [block][64] int16, blocks

@@ -22,11 +22,14 @@ from .api import (  # noqa: F401
     KPEG_XFORM_ROT270,
     KPEG_XFORM_TRANSPOSE,
     KPEG_XFORM_TRANSVERSE,
+    Crop,
     Decoder,
     EncodeParams,
     KpegError,
     Plan,
     Stats,
+    crop_shape,
+    crop_struct,
     load_cuda_library,
     output_shape,
     encode_bound,

@@ -97,6 +97,18 @@ def build_emu_scaled() -> None:
         _run([*cmd, "-o", str(out), str(src)], cwd=emu)
 
 
+def build_emu_crop() -> None:
+    """tests/emu/emu_crop.cpp: the crop decode's geometry (csrc/crop_geom.h) compiled for the host (test infrastructure)."""
+    emu = ROOT / "tests" / "emu"
+    out = emu / "libkpeg_emu_crop.so"
+    src = emu / "emu_crop.cpp"
+    deps = [src, *sorted((PKG / "csrc").glob("*.h"))]
+    if out.exists() and all(out.stat().st_mtime >= d.stat().st_mtime for d in deps):
+        return
+    _run(["g++", "-std=c++17", "-O2", "-fPIC", "-shared", "-Wall", "-Wno-unknown-pragmas", f"-I{ROOT / 'include'}",
+          f"-I{PKG / 'csrc'}", "-o", str(out), str(src)], cwd=emu)
+
+
 def have_nvcc() -> bool:
     from shutil import which
     return which(os.environ.get("NVCC", "nvcc")) is not None

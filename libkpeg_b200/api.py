@@ -97,6 +97,11 @@ class TranscodeParams(C.Structure):
     _fields_ = [("restart_interval", C.c_int32), ("transform", C.c_uint32), ("flags", C.c_uint32)]
 
 
+class Crop(C.Structure):
+    """struct kpeg_crop: a rectangle of the output image (x, y, width, height in its pixels)"""
+    _fields_ = [("x", C.c_uint32), ("y", C.c_uint32), ("width", C.c_uint32), ("height", C.c_uint32)]
+
+
 # every symbol include/kpeg_cuda.h declares: (restype, argtypes)
 _u8p = C.POINTER(C.c_uint8)
 _vp = C.c_void_p
@@ -122,6 +127,12 @@ SYMBOLS = {
     "kpeg_cuda_memcpy_d2h": (C.c_int, [_vp, _vp, _vp, C.c_size_t]),
     "kpeg_cuda_decode": (C.c_int, [_vp, C.POINTER(Plan), _vp, C.c_size_t, _vp, C.POINTER(Stats)]),
     "kpeg_cuda_decode_device": (C.c_int, [_vp, C.POINTER(Plan), _vp, C.c_size_t, _vp, C.POINTER(Stats)]),
+    "kpeg_cuda_decode_crop": (C.c_int, [_vp, C.POINTER(Plan), _vp, C.c_size_t, C.POINTER(Crop), _vp, C.POINTER(Stats)]),
+    "kpeg_cuda_decode_crop_device": (C.c_int, [_vp, C.POINTER(Plan), _vp, C.c_size_t, C.POINTER(Crop), _vp, C.POINTER(Stats)]),
+    "kpeg_cuda_decode_batch_crop": (C.c_int, [_vp, C.POINTER(Plan), C.c_int, C.POINTER(_vp), C.POINTER(C.c_size_t),
+                                              C.POINTER(Crop), C.POINTER(_vp), C.POINTER(Stats)]),
+    "kpeg_cuda_decode_file_crop": (C.c_int, [_vp, _vp, C.c_size_t, C.c_uint32, C.POINTER(Crop), _vp, C.c_size_t,
+                                             C.POINTER(Plan), C.POINTER(Stats)]),
     "kpeg_cuda_decode_batch": (C.c_int, [_vp, C.POINTER(Plan), C.c_int, C.POINTER(_vp), C.POINTER(C.c_size_t),
                                         C.POINTER(_vp), C.POINTER(Stats)]),
     "kpeg_cuda_decode_batch_device": (C.c_int, [_vp, C.POINTER(Plan), C.c_int, _vp, C.POINTER(C.c_uint64), _vp,
@@ -248,6 +259,27 @@ def output_shape(plan: Plan) -> tuple:
     return (h.value, w.value, 3) if plan.ncomp == 3 else (h.value, w.value)
 
 
+def crop_struct(crop) -> Crop:
+    """(x, y, w, h) -> kpeg_crop.  ValueError for anything but four non-negative integers with w, h >= 1 (whether the
+    rectangle lies inside the image is the decoder's check: KPEG_ERR_ARG)."""
+    try:
+        vals = tuple(crop)
+    except TypeError:
+        raise ValueError(f"crop must be (x, y, w, h), not {crop!r}") from None
+    if len(vals) != 4 or not all(isinstance(v, (int, np.integer)) and not isinstance(v, bool) for v in vals):
+        raise ValueError(f"crop must be four integers (x, y, w, h), not {crop!r}")
+    x, y, w, h = (int(v) for v in vals)
+    if x < 0 or y < 0 or w < 1 or h < 1 or max(x, y, w, h) >= 1 << 32:
+        raise ValueError(f"crop (x, y, w, h) needs x, y >= 0 and w, h >= 1, not {crop!r}")
+    return Crop(x, y, w, h)
+
+
+def crop_shape(plan: Plan, crop) -> tuple:
+    """Shape of the crop (x, y, w, h) of plan's decoded image: (h, w, 3) or (h, w), as output_shape."""
+    c = crop_struct(crop)
+    return (c.height, c.width, 3) if plan.ncomp == 3 else (c.height, c.width)
+
+
 def ppm_header(width: int, height: int) -> bytes:
     lib = load_cuda_library()
     buf = C.create_string_buffer(256)
@@ -371,11 +403,23 @@ class Decoder:
 
     # -- decode -------------------------------------------------------------------------------
     def decode_file(self, data, flags: int = KPEG_FLAG_REF_PARITY, out: np.ndarray | None = None,
-                    scale: int | None = None) -> np.ndarray:
+                    scale: int | None = None, crop=None) -> np.ndarray:
         """scale 1, 2, 4, 8: the image at 1/scale the size (sets the KPEG_FLAG_SCALE_* bits of flags; None: as flags has
-        them)."""
+        them).  crop (x, y, w, h): only that rectangle of the output image (kpeg_cuda_decode_file_crop)."""
         flags = _scaled_flags(flags, scale)
+        c = None if crop is None else crop_struct(crop)
         buf = np.frombuffer(data, dtype=np.uint8) if not isinstance(data, np.ndarray) else data
+        if c is not None:
+            buf = np.ascontiguousarray(buf)
+            frame, _ = parse_jfif_scans(buf)
+            shape = crop_shape(frame, crop)
+            if out is None:
+                out = np.empty(shape, dtype=np.uint8)
+            assert out.nbytes == int(np.prod(shape)) and out.flags.c_contiguous
+            rc = self._lib.kpeg_cuda_decode_file_crop(self._h, _ptr(buf), buf.size, flags, C.byref(c), _ptr(out), out.nbytes,
+                                                      None, C.byref(self.last_stats))
+            self._check(rc, "kpeg_cuda_decode_file_crop")
+            return out.reshape(shape)
         frame, scans = parse_jfif_scans(buf)
         if len(scans) == 1:
             plan = scans[0].plan
@@ -419,10 +463,22 @@ class Decoder:
         codes = [int(r) for r in res]
         return [o.reshape(sh) if (c == KPEG_OK and sh is not None) else None for o, sh, c in zip(outs, shapes, codes)], codes
 
-    def decode_scan(self, plan: Plan, scan: np.ndarray, out: np.ndarray | None = None, scale: int | None = None) -> np.ndarray:
-        """scale 1, 2, 4, 8 sets the plan's KPEG_FLAG_SCALE_* bits (None: as the plan has them)."""
+    def decode_scan(self, plan: Plan, scan: np.ndarray, out: np.ndarray | None = None, scale: int | None = None,
+                    crop=None) -> np.ndarray:
+        """scale 1, 2, 4, 8 sets the plan's KPEG_FLAG_SCALE_* bits (None: as the plan has them).  crop (x, y, w, h): only
+        that rectangle of the output image (kpeg_cuda_decode_crop)."""
         plan = _scaled_plan(plan, scale)
+        c = None if crop is None else crop_struct(crop)
         scan = np.ascontiguousarray(scan, dtype=np.uint8)
+        if c is not None:
+            shape = crop_shape(plan, crop)
+            if out is None:
+                out = np.empty(shape, dtype=np.uint8)
+            assert out.nbytes == int(np.prod(shape)) and out.flags.c_contiguous
+            rc = self._lib.kpeg_cuda_decode_crop(self._h, C.byref(plan), _ptr(scan), scan.size, C.byref(c), _ptr(out),
+                                                 C.byref(self.last_stats))
+            self._check(rc, "kpeg_cuda_decode_crop")
+            return out.reshape(shape)
         shape = output_shape(plan)
         if out is None:
             out = np.empty(shape, dtype=np.uint8)
@@ -432,10 +488,27 @@ class Decoder:
         self._check(rc, "kpeg_cuda_decode")
         return out.reshape(shape)
 
-    def decode_batch(self, plan: Plan, scans: list[np.ndarray], outs: list[np.ndarray] | None = None, scale: int | None = None):
+    def decode_batch(self, plan: Plan, scans: list[np.ndarray], outs: list[np.ndarray] | None = None, scale: int | None = None,
+                     crops: list | None = None):
+        """crops: one rectangle (x, y, w, h) per image; image i's output is then that rectangle of it
+        (kpeg_cuda_decode_batch_crop)."""
         plan = _scaled_plan(plan, scale)
         n = len(scans)
+        if crops is not None:
+            if len(crops) != n:
+                raise ValueError(f"decode_batch: {n} scans but {len(crops)} crops")
+            cs = [crop_struct(c) for c in crops]
         scans = [np.ascontiguousarray(s, dtype=np.uint8) for s in scans]
+        if crops is not None:
+            if outs is None:
+                outs = [np.empty(crop_shape(plan, c), dtype=np.uint8) for c in crops]
+            sp = (_vp * n)(*[_ptr(s) for s in scans])
+            sl = (C.c_size_t * n)(*[s.size for s in scans])
+            op = (_vp * n)(*[_ptr(o) for o in outs])
+            rc = self._lib.kpeg_cuda_decode_batch_crop(self._h, C.byref(plan), n, sp, sl, (Crop * n)(*cs), op,
+                                                       C.byref(self.last_stats))
+            self._check(rc, "kpeg_cuda_decode_batch_crop")
+            return outs
         shape = output_shape(plan)
         if outs is None:
             outs = [np.empty(shape, dtype=np.uint8) for _ in range(n)]
@@ -467,9 +540,16 @@ class Decoder:
     def d2h(self, dst: np.ndarray, dptr: int):
         self._check(self._lib.kpeg_cuda_memcpy_d2h(self._h, _ptr(dst), dptr, dst.nbytes), "memcpy_d2h")
 
-    def decode_device(self, plan: Plan, d_scan: int, scan_len: int, d_out: int, scale: int | None = None):
-        """d_out receives output_shape(plan) bytes (with scale: of the plan at that scale)."""
+    def decode_device(self, plan: Plan, d_scan: int, scan_len: int, d_out: int, scale: int | None = None, crop=None):
+        """d_out receives output_shape(plan) bytes (with scale: of the plan at that scale); with crop (x, y, w, h), the
+        crop_shape(plan, crop) bytes of that rectangle (kpeg_cuda_decode_crop_device)."""
         plan = _scaled_plan(plan, scale)
+        if crop is not None:
+            c = crop_struct(crop)
+            rc = self._lib.kpeg_cuda_decode_crop_device(self._h, C.byref(plan), d_scan, scan_len, C.byref(c), d_out,
+                                                        C.byref(self.last_stats))
+            self._check(rc, "kpeg_cuda_decode_crop_device")
+            return
         rc = self._lib.kpeg_cuda_decode_device(self._h, C.byref(plan), d_scan, scan_len, d_out,
                                                C.byref(self.last_stats))
         self._check(rc, "kpeg_cuda_decode_device")

@@ -11,6 +11,7 @@
 
 #include <stdint.h>
 
+#include "crop_geom.h"
 #include "kpeg_common.h"
 
 #ifdef __CUDA_ARCH__
@@ -169,6 +170,16 @@ KPEG_HD uint64_t scaled_pixel_offset(const JobGeom &g, const OutGeom &o, uint32_
     if (ox >= o.width || oy >= o.height)
         return ~(uint64_t)0;
     return (uint64_t)img * o.bytes() + (uint64_t)oy * o.row_bytes() + (uint64_t)ox * o.ncomp;
+}
+
+// The same pixel in a crop decode's output (crop_geom.h): its byte offset in the crop of its image, or CROP_SKIP outside
+// the rectangle (which lies inside the output image: the ragged edge needs no test of its own).
+KPEG_HD uint64_t scaled_crop_offset(const JobGeom &g, const OutGeom &o, const CropWin *crop, uint32_t m, uint32_t r, uint32_t c)
+{
+    const uint32_t K = 8u / o.scale;
+    const uint32_t img = m / g.mcus_per_image, mi = m - img * g.mcus_per_image;
+    const uint32_t by = mi / g.mcus_x, bx = mi - by * g.mcus_x;
+    return crop_pixel_offset(crop[img], o.ncomp, bx * K + c, by * K + r);
 }
 
 } // namespace red

@@ -66,7 +66,8 @@ struct ExpandSmem {
     uint32_t mi0;        // MCU-in-image of the strip's first MCU
 };
 
-template <int NC>
+// LISTED (crop decode): CTA i expands strip a.strip_list[i]; the other strips' tiles are not written
+template <int NC, bool LISTED>
 __global__ void __launch_bounds__(EXPAND_THREADS, KPEG_EXPAND_MIN_CTAS) expand_kernel(ExpandArgs a)
 {
     constexpr int NM = IDCT_MCUS_PER_CTA;
@@ -77,7 +78,7 @@ __global__ void __launch_bounds__(EXPAND_THREADS, KPEG_EXPAND_MIN_CTAS) expand_k
 
     const int t = threadIdx.x;
     const uint32_t warp = (uint32_t)t >> 5, lane = (uint32_t)t & 31u;
-    const uint32_t strip = blockIdx.x;
+    const uint32_t strip = LISTED ? __ldg(a.strip_list + blockIdx.x) : blockIdx.x;
     const uint32_t mcu0 = strip * NM, blk0 = mcu0 * NC;
     const uint32_t total_mcus = a.g.nimages * a.g.mcus_per_image;
     const uint32_t s0 = blk0 * 64u; // first slot of the strip; slots are < 2^32 (host_tables.h)
@@ -85,10 +86,12 @@ __global__ void __launch_bounds__(EXPAND_THREADS, KPEG_EXPAND_MIN_CTAS) expand_k
     // ---- stage A ---------------------------------------------------------------------------------------
     const uint32_t nsub = a.meta->nsub;
     const uint32_t first0 = min(__ldg(a.strip_sub + strip), nsub - 1u);
-    if (EXPAND_PREFETCH_AHEAD != 0u && strip + EXPAND_PREFETCH_AHEAD < a.nstrips) {
+    const bool prefetch = LISTED ? blockIdx.x + EXPAND_PREFETCH_AHEAD < a.nlisted : strip + EXPAND_PREFETCH_AHEAD < a.nstrips;
+    if (EXPAND_PREFETCH_AHEAD != 0u && prefetch) {
         // the record lines a strip that starts about one CTA lifetime from now will read: DRAM -> L2 now, so that its
         // batches wait for L2, not for DRAM.  (Which strip that is need not be exact.)
-        const uint32_t fs = min(__ldg(a.strip_sub + strip + EXPAND_PREFETCH_AHEAD), nsub - 1u);
+        const uint32_t ahead = LISTED ? __ldg(a.strip_list + blockIdx.x + EXPAND_PREFETCH_AHEAD) : strip + EXPAND_PREFETCH_AHEAD;
+        const uint32_t fs = min(__ldg(a.strip_sub + ahead), nsub - 1u);
         const char *g0 = reinterpret_cast<const char *>(a.rec + ((size_t)(fs >> 5) * a.rec_kmax) * 32u);
         const uint32_t lines = min(a.rec_kmax, EXPAND_PREFETCH_LINES);
         for (uint32_t k = (uint32_t)t; k < 2u * lines; k += EXPAND_THREADS) {
@@ -318,10 +321,16 @@ void launch_expand(const ExpandArgs &a, cudaStream_t s, uint32_t *launches)
 {
     const uint32_t total_mcus = a.g.nimages * a.g.mcus_per_image;
     const uint32_t grid = (total_mcus + IDCT_MCUS_PER_CTA - 1) / IDCT_MCUS_PER_CTA;
-    if (a.g.ncomp == 3)
-        expand_kernel<3><<<grid, EXPAND_THREADS, 0, s>>>(a);
-    else
-        expand_kernel<1><<<grid, EXPAND_THREADS, 0, s>>>(a);
+    if (a.strip_list) {
+        if (a.g.ncomp == 3)
+            expand_kernel<3, true><<<a.nlisted, EXPAND_THREADS, 0, s>>>(a);
+        else
+            expand_kernel<1, true><<<a.nlisted, EXPAND_THREADS, 0, s>>>(a);
+    } else if (a.g.ncomp == 3) {
+        expand_kernel<3, false><<<grid, EXPAND_THREADS, 0, s>>>(a);
+    } else {
+        expand_kernel<1, false><<<grid, EXPAND_THREADS, 0, s>>>(a);
+    }
     ++*launches;
 }
 

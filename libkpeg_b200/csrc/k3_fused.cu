@@ -439,8 +439,10 @@ __device__ __forceinline__ void st_shared_u16(uint32_t addr, uint32_t v)
     asm volatile("st.shared.u16 [%0], %1;" ::"r"(addr), "h"((uint16_t)v) : "memory");
 }
 
-template <int NC>
-__global__ void __launch_bounds__(NC * IDCT_MCUS_PER_CTA, NC == 3 ? KPEG_IDCT_MIN_CTAS : 16) idct_kernel(IdctArgs a)
+// CROP (crop decode, crop_geom.h): CTA i reconstructs strip a.strip_list[i], and every store -- the rows of stage 2, the
+// colour-exact rewrites, the tie records and the pixels stage 3 repaints -- keeps to a.crop[image]
+template <int NC, bool CROP>
+__global__ void __launch_bounds__(NC * IDCT_MCUS_PER_CTA, NC == 3 ? KPEG_IDCT_MIN_CTAS : 16) idct_kernel(K3Args<CROP> a)
 {
     constexpr int NM = IDCT_MCUS_PER_CTA;
     constexpr int NB = NM * NC;
@@ -452,7 +454,7 @@ __global__ void __launch_bounds__(NC * IDCT_MCUS_PER_CTA, NC == 3 ? KPEG_IDCT_MI
     const int ml = t % NM;   // == lane
     const int bl = ml * NC + comp; // block index inside the CTA's strip (MCU-interleaved)
     const uint32_t total_mcus = a.g.nimages * a.g.mcus_per_image;
-    const uint32_t strip = blockIdx.x;
+    const uint32_t strip = k3_strip(a);
     const uint32_t mcu0 = strip * NM;
     const uint32_t m = mcu0 + ml;
     const bool active = m < total_mcus;
@@ -460,7 +462,7 @@ __global__ void __launch_bounds__(NC * IDCT_MCUS_PER_CTA, NC == 3 ? KPEG_IDCT_MI
     // ---- stage 0: tile and quantisers by the copy engine, strip origin ------------------------------------------
     const uint32_t bar = smem_u32(&sm.mbar);
     if (t == 0) {
-        k3_load_strip<NC>(a.tiles, strip, a.nstrips, sm.coef, a.tables->qpair, NC * 64u * 4u, sm.qpair, bar);
+        k3_load_strip<NC, CROP>(a.tiles, strip, k3_nstrips(a), sm.coef, a.tables->qpair, NC * 64u * 4u, sm.qpair, bar, k3_list(a));
         sm.ntie = 0;
         sm.any_huge = 0;
         const uint32_t img = mcu0 / a.g.mcus_per_image, mi = mcu0 - img * a.g.mcus_per_image;
@@ -596,7 +598,19 @@ __global__ void __launch_bounds__(NC * IDCT_MCUS_PER_CTA, NC == 3 ? KPEG_IDCT_MI
         mcu_origin((uint32_t)ml, img, by, bx);
         uint8_t *img_base = a.pixels + (size_t)img * W * H * NC;
         const bool full_w = bx * 8u + 8u <= W;
-        const bool vec_ok = full_w && (W % 8u == 0u) && ((reinterpret_cast<uintptr_t>(a.pixels) & 7u) == 0);
+        // crop: the block's columns [c_lo, c_hi) lie inside the rectangle; 8-byte stores when all eight do and the
+        // rectangle keeps them aligned
+        CropWin win = {};
+        uint32_t c_lo = 0, c_hi = 0;
+        if constexpr (CROP) {
+            win = a.crop[img];
+            const uint32_t x = bx * 8u;
+            c_lo = win.x0 > x ? min(win.x0 - x, 8u) : 0u;
+            c_hi = win.x0 + win.w > x ? min(win.x0 + win.w - x, 8u) : 0u;
+        }
+        const bool vec_ok = CROP ? c_lo == 0u && c_hi == 8u && ((win.x0 | win.w) & 7u) == 0u &&
+                                       (((reinterpret_cast<uintptr_t>(a.pixels) | win.out_off) & 7u) == 0u)
+                                 : full_w && (W % 8u == 0u) && ((reinterpret_cast<uintptr_t>(a.pixels) & 7u) == 0);
         int mode = COLOUR_PLAIN;
         if constexpr (NC == 3) {
             const uint32_t f0 = sm.flag[ml * NC], f1 = sm.flag[ml * NC + 1], f2 = sm.flag[ml * NC + 2];
@@ -606,6 +620,9 @@ __global__ void __launch_bounds__(NC * IDCT_MCUS_PER_CTA, NC == 3 ? KPEG_IDCT_MI
             const uint32_t y = by * 8u + row;
             if (y >= H)
                 continue;
+            if constexpr (CROP)
+                if (y - win.y0 >= win.h || c_lo >= c_hi)
+                    continue;
             const float4 y0 = sm.samp[((0 * 8 + row) * 2 + 0) * NM + ml], y1 = sm.samp[((0 * 8 + row) * 2 + 1) * NM + ml];
             uint32_t out[2 * NC];
             uint32_t redo = 0;
@@ -635,10 +652,17 @@ __global__ void __launch_bounds__(NC * IDCT_MCUS_PER_CTA, NC == 3 ? KPEG_IDCT_MI
                 out[1] = pack4_sat(v[4], v[5], v[6], v[7]);
             }
             uint8_t *dst = img_base + ((size_t)y * W + bx * 8u) * NC;
+            if constexpr (CROP) // where column bx * 8 of row y would be in the crop (the bytes before c_lo are not stored)
+                dst = a.pixels + (long long)(win.out_off + ((uint64_t)(y - win.y0) * win.w + bx * 8u) * NC) - (long long)win.x0 * NC;
             if (vec_ok) {
 #pragma unroll
                 for (int k = 0; k < NC; ++k)
                     reinterpret_cast<uint2 *>(dst)[k] = make_uint2(out[2 * k], out[2 * k + 1]);
+            } else if constexpr (CROP) {
+#pragma unroll
+                for (int j = 0; j < 8 * NC; ++j)
+                    if ((uint32_t)j >= c_lo * NC && (uint32_t)j < c_hi * NC)
+                        dst[j] = (uint8_t)(out[j >> 2] >> (8 * (j & 3)));
             } else {
                 const uint32_t nbytes = (full_w ? 8u : W - bx * 8u) * NC;
 #pragma unroll
@@ -651,6 +675,9 @@ __global__ void __launch_bounds__(NC * IDCT_MCUS_PER_CTA, NC == 3 ? KPEG_IDCT_MI
                 redo &= redo - 1u;
                 if (bx * 8u + (uint32_t)j >= W)
                     continue;
+                if constexpr (CROP)
+                    if ((uint32_t)j < c_lo || (uint32_t)j >= c_hi)
+                        continue;
                 const float *sp = reinterpret_cast<const float *>(sm.samp);
                 const int sy = (int)sp[(((0 * 8 + row) * 2 + (j >> 2)) * NM + ml) * 4 + (j & 3)];
                 const int sb = (int)sp[(((1 * 8 + row) * 2 + (j >> 2)) * NM + ml) * 4 + (j & 3)];
@@ -694,6 +721,12 @@ __global__ void __launch_bounds__(NC * IDCT_MCUS_PER_CTA, NC == 3 ? KPEG_IDCT_MI
         const uint32_t px = bx * 8u + (uint32_t)(s & 7), py = by * 8u + (uint32_t)(s >> 3);
         if (px >= W || py >= H)
             return;
+        uint64_t coff = 0;
+        if constexpr (CROP) {
+            coff = crop_pixel_offset(a.crop[img], NC, px, py);
+            if (coff == CROP_SKIP)
+                return;
+        }
         const int y = (int)spf[samp_index(0, mm_l, s)];
         int cb = 0, cr = 0;
         if (NC == 3) {
@@ -701,7 +734,7 @@ __global__ void __launch_bounds__(NC * IDCT_MCUS_PER_CTA, NC == 3 ? KPEG_IDCT_MI
             cr = (int)spf[samp_index(NC - 1, mm_l, s)];
         }
         const uint32_t v = colour_px<NC>(y, cb, cr);
-        uint8_t *dst = a.pixels + ((size_t)img * W * H + (size_t)py * W + px) * NC;
+        uint8_t *dst = CROP ? a.pixels + coff : a.pixels + ((size_t)img * W * H + (size_t)py * W + px) * NC;
         dst[0] = (uint8_t)v;
         if (NC == 3) {
             dst[1] = (uint8_t)(v >> 8);
@@ -728,8 +761,16 @@ __global__ void __launch_bounds__(NC * IDCT_MCUS_PER_CTA, NC == 3 ? KPEG_IDCT_MI
             uint32_t img, by, bx;
             mcu_origin(mm_l, img, by, bx);
             const uint32_t px = bx * 8u + (uint32_t)(sidx & 7), py = by * 8u + (uint32_t)(sidx >> 3);
-            if ((flags & (0u - flags)) == (1u << c) && !(huge & BLK_HUGE) && mcu0 + mm_l < total_mcus && px < W && py < H) {
+            bool listed = (flags & (0u - flags)) == (1u << c) && !(huge & BLK_HUGE) && mcu0 + mm_l < total_mcus && px < W && py < H;
+            uint64_t coff = 0;
+            if constexpr (CROP) { // a pixel outside the rectangle is not listed
+                coff = listed ? crop_pixel_offset(a.crop[img], NC, px, py) : CROP_SKIP;
+                listed = coff != CROP_SKIP;
+            }
+            if (listed) {
                 r.x = img * W * H + py * W + px; // pixels of a job are < 2^32 (host_tables.h)
+                if constexpr (CROP)
+                    r.x = (uint32_t)(coff / NC); // the pixel's index in the crop output
                 r.y = mcu0 + mm_l;
                 auto biased = [&](uint32_t c) { return ((uint32_t)(int)spf[samp_index(c, mm_l, sidx)] + COEF_BIAS) & 0xFFFFu; };
                 r.z = (uint32_t)sidx | (flags << 8) | (biased(0) << 16);
@@ -782,11 +823,17 @@ __global__ void __launch_bounds__(NC * IDCT_MCUS_PER_CTA, NC == 3 ? KPEG_IDCT_MI
             const uint32_t px = bx * 8u + (uint32_t)(s & 7), py = by * 8u + (uint32_t)(s >> 3);
             if (px >= W || py >= H)
                 continue;
+            uint64_t coff = 0;
+            if constexpr (CROP) {
+                coff = crop_pixel_offset(a.crop[img], NC, px, py);
+                if (coff == CROP_SKIP)
+                    continue;
+            }
             int e[3] = {0, 0, 0};
             for (int c = 0; c < NC; ++c)
                 e[c] = exact_sample_global<NC>(gtiles, a.tables, blk0 + mm_l * NC + (uint32_t)c, (uint32_t)c, s);
             const uint32_t v = NC == 3 ? colour_exact_int(e[0], e[1], e[2]) : (uint32_t)clamp_u8(e[0] + 128);
-            uint8_t *dst = a.pixels + ((size_t)img * W * H + (size_t)py * W + px) * NC;
+            uint8_t *dst = CROP ? a.pixels + coff : a.pixels + ((size_t)img * W * H + (size_t)py * W + px) * NC;
             dst[0] = (uint8_t)v;
             if (NC == 3) {
                 dst[1] = (uint8_t)(v >> 8);
@@ -827,16 +874,21 @@ __device__ __noinline__ int exact_sample_global(const uint4 *tiles, const Device
 
 constexpr int PATCH_WARPS = 8;
 
-template <int NC>
-__global__ void __launch_bounds__(PATCH_WARPS * 32) idct_patch_kernel(IdctArgs a)
+// CROP: the strips are those of a.strip_list (the tie counts of the others are stale from earlier jobs); the records hold
+// pixel indices in the crop output already
+template <int NC, bool CROP>
+__global__ void __launch_bounds__(PATCH_WARPS * 32) idct_patch_kernel(K3Args<CROP> a)
 {
     // one CTA per 32 strips; its warps share the passes over the group's records (a pass = 32 records, one per lane):
     // every pass is a long serial chain, so it is the number of warps in flight that hides it
     const uint32_t lane = threadIdx.x & 31u, wl = threadIdx.x >> 5;
     const uint4 *tiles = reinterpret_cast<const uint4 *>(a.tiles);
-    for (uint32_t s0 = blockIdx.x * 32u; s0 < a.nstrips; s0 += gridDim.x * 32u) {
-        const uint32_t strip = s0 + lane;
-        const uint32_t cnt = strip < a.nstrips ? min(__ldg(a.tie_cnt + strip), (uint32_t)TIE_LIST_CAP) : 0u;
+    const uint32_t nstrips = k3_nstrips(a);
+    for (uint32_t s0 = blockIdx.x * 32u; s0 < nstrips; s0 += gridDim.x * 32u) {
+        uint32_t strip = s0 + lane;
+        if constexpr (CROP)
+            strip = s0 + lane < nstrips ? __ldg(a.strip_list + s0 + lane) : 0u;
+        const uint32_t cnt = (CROP ? s0 + lane : strip) < nstrips ? min(__ldg(a.tie_cnt + strip), (uint32_t)TIE_LIST_CAP) : 0u;
         uint32_t incl = cnt; // inclusive scan of the 32 strips' counts
 #pragma unroll
         for (int d = 1; d < 32; d <<= 1) {
@@ -856,9 +908,12 @@ __global__ void __launch_bounds__(PATCH_WARPS * 32) idct_patch_kernel(IdctArgs a
                     lo += (uint32_t)step;
             }
             const uint32_t before = __shfl_sync(0xffffffffu, incl - cnt, (int)min(lo, 31u));
+            uint32_t rstrip = s0 + lo;
+            if constexpr (CROP)
+                rstrip = __shfl_sync(0xffffffffu, strip, (int)min(lo, 31u));
             if (e >= total)
                 continue;
-            const uint4 r = __ldg(a.tie_rec + (size_t)(s0 + lo) * TIE_LIST_CAP + (e - before));
+            const uint4 r = __ldg(a.tie_rec + (size_t)rstrip * TIE_LIST_CAP + (e - before));
             if (r.x == TIE_EMPTY)
                 continue;
             const int s = (int)(r.z & 63u);
@@ -887,30 +942,36 @@ __global__ void __launch_bounds__(PATCH_WARPS * 32) idct_patch_kernel(IdctArgs a
 
 void k3_configure()
 {
-    cudaFuncSetAttribute(idct_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(IdctSmem<3>));
-    cudaFuncSetAttribute(idct_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(IdctSmem<1>));
+    cudaFuncSetAttribute(idct_kernel<3, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(IdctSmem<3>));
+    cudaFuncSetAttribute(idct_kernel<1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(IdctSmem<1>));
+    cudaFuncSetAttribute(idct_kernel<3, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(IdctSmem<3>));
+    cudaFuncSetAttribute(idct_kernel<1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(IdctSmem<1>));
 }
 
 uint32_t k3_strip_slots(uint32_t ncomp) { return (uint32_t)IDCT_MCUS_PER_CTA * ncomp * 64u; }
 
-cudaError_t launch_idct(const IdctArgs &a_in, cudaStream_t s, uint32_t *launches)
+cudaError_t launch_idct(const IdctCropArgs &a_in, cudaStream_t s, uint32_t *launches)
 {
     if (scale_denom(a_in.g.flags) != 1u)
         return launch_idct_scaled(a_in, s, launches);
-    IdctArgs a = a_in;
+    const IdctCropArgs &a = a_in;
+    const IdctArgs &whole = a;
     const uint32_t total_mcus = a.g.nimages * a.g.mcus_per_image;
-    const uint32_t grid = (total_mcus + IDCT_MCUS_PER_CTA - 1) / IDCT_MCUS_PER_CTA;
+    const bool crop = a.crop != nullptr;
+    const uint32_t grid = crop ? a.nlisted : (total_mcus + IDCT_MCUS_PER_CTA - 1) / IDCT_MCUS_PER_CTA;
     if (a.g.ncomp == 3)
-        idct_kernel<3><<<grid, 3 * IDCT_MCUS_PER_CTA, sizeof(IdctSmem<3>), s>>>(a);
+        crop ? idct_kernel<3, true><<<grid, 3 * IDCT_MCUS_PER_CTA, sizeof(IdctSmem<3>), s>>>(a)
+             : idct_kernel<3, false><<<grid, 3 * IDCT_MCUS_PER_CTA, sizeof(IdctSmem<3>), s>>>(whole);
     else
-        idct_kernel<1><<<grid, IDCT_MCUS_PER_CTA, sizeof(IdctSmem<1>), s>>>(a);
+        crop ? idct_kernel<1, true><<<grid, IDCT_MCUS_PER_CTA, sizeof(IdctSmem<1>), s>>>(a)
+             : idct_kernel<1, false><<<grid, IDCT_MCUS_PER_CTA, sizeof(IdctSmem<1>), s>>>(whole);
     ++*launches;
     // the pixels inside the tie band: a small grid (a few records per strip), full warps
     const uint32_t pgrid = std::min<uint32_t>((grid + 31u) / 32u, 148u * 16u);
     if (a.g.ncomp == 3)
-        idct_patch_kernel<3><<<pgrid, PATCH_WARPS * 32, 0, s>>>(a);
+        crop ? idct_patch_kernel<3, true><<<pgrid, PATCH_WARPS * 32, 0, s>>>(a) : idct_patch_kernel<3, false><<<pgrid, PATCH_WARPS * 32, 0, s>>>(whole);
     else
-        idct_patch_kernel<1><<<pgrid, PATCH_WARPS * 32, 0, s>>>(a);
+        crop ? idct_patch_kernel<1, true><<<pgrid, PATCH_WARPS * 32, 0, s>>>(a) : idct_patch_kernel<1, false><<<pgrid, PATCH_WARPS * 32, 0, s>>>(whole);
     ++*launches;
     return cudaSuccess;
 }

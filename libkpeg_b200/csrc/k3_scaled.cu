@@ -14,6 +14,8 @@
 #include <stddef.h>
 #include <stdint.h>
 
+#include <type_traits>
+
 #include "entropy_core.h"
 #include "idct_reduced.h"
 #include "k3_tile.cuh"
@@ -24,8 +26,9 @@ namespace kpeg {
 
 static_assert(offsetof(DeviceTables, qint) % 16 == 0, "qint is staged by a bulk copy");
 
-template <int NC, int S>
-__global__ void __launch_bounds__(NC * IDCT_MCUS_PER_CTA) idct_scaled_kernel(IdctArgs a)
+// CROP: CTA i reconstructs strip a.strip_list[i], and stores only the pixels inside a.crop[image] (crop_geom.h)
+template <int NC, int S, bool CROP>
+__global__ void __launch_bounds__(NC * IDCT_MCUS_PER_CTA) idct_scaled_kernel(K3Args<CROP> a)
 {
     constexpr int NM = IDCT_MCUS_PER_CTA;
     constexpr int NB = NM * NC;
@@ -40,13 +43,13 @@ __global__ void __launch_bounds__(NC * IDCT_MCUS_PER_CTA) idct_scaled_kernel(Idc
     const int ml = t % NM;
     const int bl = ml * NC + comp;
     const uint32_t total_mcus = a.g.nimages * a.g.mcus_per_image;
-    const uint32_t strip = blockIdx.x;
+    const uint32_t strip = k3_strip(a);
     const uint32_t mcu0 = strip * NM;
 
     // ---- stage 0 ----------------------------------------------------------------------------------------------
     const uint32_t bar = smem_u32(&mbar);
     if (t == 0) {
-        k3_load_strip<NC>(a.tiles, strip, a.nstrips, coef, a.tables->qint, NC * 64u * 4u, q, bar);
+        k3_load_strip<NC, CROP>(a.tiles, strip, k3_nstrips(a), coef, a.tables->qint, NC * 64u * 4u, q, bar, k3_list(a));
         mbar_wait(bar, 0);
     }
     __syncthreads();
@@ -70,7 +73,11 @@ __global__ void __launch_bounds__(NC * IDCT_MCUS_PER_CTA) idct_scaled_kernel(Idc
         const uint32_t m = mcu0 + px.ml;
         if (m >= total_mcus)
             continue;
-        const uint64_t off = red::scaled_pixel_offset(a.g, o, m, px.r, px.c);
+        uint64_t off;
+        if constexpr (CROP)
+            off = red::scaled_crop_offset(a.g, o, a.crop, m, px.r, px.c);
+        else
+            off = red::scaled_pixel_offset(a.g, o, m, px.r, px.c);
         if (off == ~(uint64_t)0)
             continue;
         const int s = (int)(px.r * K + px.c);
@@ -86,21 +93,33 @@ __global__ void __launch_bounds__(NC * IDCT_MCUS_PER_CTA) idct_scaled_kernel(Idc
     }
 }
 
-cudaError_t launch_idct_scaled(const IdctArgs &a, cudaStream_t s, uint32_t *launches)
+cudaError_t launch_idct_scaled(const IdctCropArgs &a, cudaStream_t s, uint32_t *launches)
 {
     const uint32_t total_mcus = a.g.nimages * a.g.mcus_per_image;
-    const uint32_t grid = (total_mcus + IDCT_MCUS_PER_CTA - 1) / IDCT_MCUS_PER_CTA;
     const uint32_t S = scale_denom(a.g.flags);
-    const bool rgb = a.g.ncomp == 3;
+    const bool rgb = a.g.ncomp == 3, crop = a.crop != nullptr;
+    const uint32_t grid = crop ? a.nlisted : (total_mcus + IDCT_MCUS_PER_CTA - 1) / IDCT_MCUS_PER_CTA;
     const uint32_t threads = a.g.ncomp * IDCT_MCUS_PER_CTA;
-    if (S == 2)
-        rgb ? idct_scaled_kernel<3, 2><<<grid, threads, 0, s>>>(a) : idct_scaled_kernel<1, 2><<<grid, threads, 0, s>>>(a);
-    else if (S == 4)
-        rgb ? idct_scaled_kernel<3, 4><<<grid, threads, 0, s>>>(a) : idct_scaled_kernel<1, 4><<<grid, threads, 0, s>>>(a);
-    else if (S == 8)
-        rgb ? idct_scaled_kernel<3, 8><<<grid, threads, 0, s>>>(a) : idct_scaled_kernel<1, 8><<<grid, threads, 0, s>>>(a);
-    else
+    auto go = [&](auto NCC, auto SC, auto CC) {
+        constexpr bool CROP = decltype(CC)::value;
+        idct_scaled_kernel<decltype(NCC)::value, decltype(SC)::value, CROP><<<grid, threads, 0, s>>>(static_cast<const K3Args<CROP> &>(a));
+    };
+    using C1 = std::integral_constant<int, 1>;
+    using C3 = std::integral_constant<int, 3>;
+    auto by_scale = [&](auto NCC, auto CC) {
+        if (S == 2)
+            go(NCC, std::integral_constant<int, 2>{}, CC);
+        else if (S == 4)
+            go(NCC, std::integral_constant<int, 4>{}, CC);
+        else
+            go(NCC, std::integral_constant<int, 8>{}, CC);
+    };
+    if (S != 2 && S != 4 && S != 8)
         return cudaErrorInvalidValue;
+    if (crop)
+        rgb ? by_scale(C3{}, std::true_type{}) : by_scale(C1{}, std::true_type{});
+    else
+        rgb ? by_scale(C3{}, std::false_type{}) : by_scale(C1{}, std::false_type{});
     ++*launches;
     return cudaSuccess;
 }

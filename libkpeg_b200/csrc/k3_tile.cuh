@@ -6,6 +6,8 @@
 
 #include <stdint.h>
 
+#include <type_traits>
+
 #include "kernels.cuh"
 
 namespace kpeg {
@@ -45,10 +47,11 @@ __device__ __forceinline__ void bulk_load(uint32_t dst, const void *src, uint32_
 
 // Issued by one thread: the tile of `strip` (NC * IDCT_MCUS_PER_CTA blocks of 128 bytes) -> tile_smem and table_bytes of
 // `table` -> table_smem, both completing on the barrier `bar` (wait with mbar_wait(bar, 0)).  Addresses and sizes are
-// multiples of 16 bytes.
-template <int NC>
+// multiples of 16 bytes.  LISTED (crop decode): the CTAs run the strips of `list` (n entries; this is entry blockIdx.x), and
+// the prefetch looks ahead in the list; otherwise CTA i runs strip i of n.
+template <int NC, bool LISTED = false>
 __device__ __forceinline__ void k3_load_strip(const void *tiles, uint32_t strip, uint32_t nstrips, void *tile_smem, const void *table,
-                                              uint32_t table_bytes, void *table_smem, uint32_t bar)
+                                              uint32_t table_bytes, void *table_smem, uint32_t bar, const uint32_t *list = nullptr)
 {
     constexpr uint32_t tile_bytes = NC * IDCT_MCUS_PER_CTA * 128u;
     const char *tile = reinterpret_cast<const char *>(tiles) + (size_t)strip * tile_bytes;
@@ -57,9 +60,44 @@ __device__ __forceinline__ void k3_load_strip(const void *tiles, uint32_t strip,
     bulk_load(smem_u32(tile_smem), tile, tile_bytes, bar);
     bulk_load(smem_u32(table_smem), table, table_bytes, bar);
     // the tile of the strip that will run in this CTA's slot next: DRAM -> L2 now
-    if (strip + IDCT_PREFETCH_AHEAD < nstrips)
+    if constexpr (LISTED) {
+        if (blockIdx.x + IDCT_PREFETCH_AHEAD < nstrips)
+            asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(reinterpret_cast<const char *>(tiles) +
+                                                                               (size_t)__ldg(list + blockIdx.x + IDCT_PREFETCH_AHEAD) * tile_bytes),
+                         "r"(tile_bytes) : "memory");
+    } else if (strip + IDCT_PREFETCH_AHEAD < nstrips) {
         asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(tile + (size_t)IDCT_PREFETCH_AHEAD * tile_bytes), "r"(tile_bytes) : "memory");
+    }
 }
+
+// The strip CTA blockIdx.x reconstructs, the strips of the launch and their list (nullptr: CTA i runs strip i): crop
+// decodes run the listed strips only (IdctCropArgs), whole-image decodes every strip (IdctArgs).
+template <class A>
+__device__ __forceinline__ uint32_t k3_strip(const A &a)
+{
+    if constexpr (std::is_same_v<A, IdctCropArgs>)
+        return __ldg(a.strip_list + blockIdx.x);
+    else
+        return blockIdx.x;
+}
+template <class A>
+__device__ __forceinline__ uint32_t k3_nstrips(const A &a)
+{
+    if constexpr (std::is_same_v<A, IdctCropArgs>)
+        return a.nlisted;
+    else
+        return a.nstrips;
+}
+template <class A>
+__device__ __forceinline__ const uint32_t *k3_list(const A &a)
+{
+    if constexpr (std::is_same_v<A, IdctCropArgs>)
+        return a.strip_list;
+    else
+        return nullptr;
+}
+template <bool CROP>
+using K3Args = std::conditional_t<CROP, IdctCropArgs, IdctArgs>;
 
 } // namespace kpeg
 #endif

@@ -4,6 +4,7 @@
 
 #include <cuda_runtime.h>
 
+#include "crop_geom.h"
 #include "kpeg_common.h"
 
 namespace kpeg {
@@ -101,6 +102,8 @@ struct ExpandArgs {
     uint32_t nstrips;
     DevMeta *meta;
     JobGeom g;
+    const uint32_t *strip_list; // crop decode: the strips to expand, sorted (nlisted of them); nullptr: every strip
+    uint32_t nlisted;
 };
 
 // K3 (k3_fused.cu): dequantise + de-zigzag + IDCT + level shift + colour + store, from the coefficient tiles
@@ -115,6 +118,14 @@ struct IdctArgs {
     JobGeom g;
 };
 constexpr int IDCT_TIE_LIST_CAP = 96; // a strip with more ties than this resolves them inside K3
+
+// K3 of a crop decode (crop_geom.h): only the listed strips are reconstructed, and every store goes through crop[image].
+// The kernels of a whole-image decode take the plain IdctArgs, so their code is the same as without crop decodes.
+struct IdctCropArgs : IdctArgs {
+    const uint32_t *strip_list = nullptr; // [nlisted], sorted
+    uint32_t nlisted = 0;
+    const CropWin *crop = nullptr;        // [nimages]; nullptr: no crop, every strip
+};
 
 
 void kernels_context_created();   // contexts of this process share the device: the cooperative relay loops of
@@ -144,8 +155,8 @@ void launch_matrix_from_tiles(const void *tiles, int16_t *coef, uint32_t total_b
 void launch_interleave_tiles(const void *t0, const void *t1, const void *t2, void *out, uint32_t nmcu_padded, cudaStream_t s,
                              uint32_t *launches);
 // K3, or -- when a.g.flags has KPEG_FLAG_SCALE_* bits -- the reduced-size reconstruction (k3_scaled.cu) in its place
-cudaError_t launch_idct(const IdctArgs &a, cudaStream_t s, uint32_t *launches);
-cudaError_t launch_idct_scaled(const IdctArgs &a, cudaStream_t s, uint32_t *launches);
+cudaError_t launch_idct(const IdctCropArgs &a, cudaStream_t s, uint32_t *launches);
+cudaError_t launch_idct_scaled(const IdctCropArgs &a, cudaStream_t s, uint32_t *launches);
 void k3_configure();                      // function attributes of the K3 kernels (called by kernels_configure)
 uint32_t k3_strip_slots(uint32_t ncomp);  // coefficient slots one K3 strip covers
 

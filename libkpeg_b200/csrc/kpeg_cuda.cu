@@ -91,7 +91,9 @@ struct Job {
     JobGeom g = {};
     EntropyArgs ea = {};
     ExpandArgs xa = {};
-    IdctArgs ia = {};
+    IdctCropArgs ia = {};
+    bool crop = false;              // a crop decode: tiles exist for the listed strips only
+    uint32_t crop_w = 0, crop_h = 0; // its first image's rectangle (kpeg_stats)
     int rounds = 0;
     uint32_t launches = 0;
     uint32_t extra_iterations = 0;
@@ -113,6 +115,9 @@ struct Lane {
     // host-buffer batches: pinned staging of the small scans + the separator positions, and their device copy
     PinBuf h_stage, h_ends;
     DevBuf d_ends{"d_ends"}, d_stage{"d_stage"};
+    // crop decodes: the images' windows (CropWin) followed by the strip list, staged in pinned memory, one copy
+    PinBuf h_crop;
+    DevBuf crop{"crop"};
     cudaEvent_t ev[MAX_EVENTS] = {};
     int ev_stage[MAX_EVENTS] = {};
     int nev = 0;
@@ -183,6 +188,7 @@ struct kpeg_ctx {
 
     int last_lane = -1; // lane of the last finished job (kpeg_cuda_read_coefficients)
     JobGeom last_g = {};
+    bool last_crop = false; // the last decode was a crop: its tiles are incomplete
 
     // deferred submissions (kpeg_cuda_submit_* / kpeg_cuda_wait): lanes are handed out round-robin and a
     // lane's previous job is finished only when the lane comes up again, so several batches are in flight
@@ -502,9 +508,9 @@ struct DeferredOutcomeSaved {
 };
 
 // K3's arguments for geometry g on lane L: its tie lists and meta, and the context's tables
-IdctArgs idct_args(kpeg_ctx *ctx, Lane &L, const JobGeom &g, uint32_t nstrips, const void *tiles, uint8_t *pixels)
+IdctCropArgs idct_args(kpeg_ctx *ctx, Lane &L, const JobGeom &g, uint32_t nstrips, const void *tiles, uint8_t *pixels)
 {
-    IdctArgs ia = {};
+    IdctCropArgs ia = {};
     ia.tiles = tiles;
     ia.nstrips = nstrips;
     ia.tables = (const DeviceTables *)ctx->tables.p;
@@ -516,11 +522,29 @@ IdctArgs idct_args(kpeg_ctx *ctx, Lane &L, const JobGeom &g, uint32_t nstrips, c
     return ia;
 }
 
+// A crop decode on lane L: the windows of the job's images (wins[nimages], crop_geom.h) and the list of the strips that
+// hold their pixels go to the device with one copy; ia then runs the listed strips and stores through the windows.
+int upload_crop(kpeg_ctx *ctx, Lane &L, const JobGeom &g, const CropWin *wins, IdctCropArgs &ia)
+{
+    const std::vector<uint32_t> list = crop_strip_list(g, wins, IDCT_MCUS_PER_CTA);
+    const size_t win_bytes = ((size_t)g.nimages * sizeof(CropWin) + 15u) & ~(size_t)15u;
+    const size_t bytes = win_bytes + list.size() * sizeof(uint32_t);
+    TRY(ensure_pinned(ctx, L.stream, L.h_crop, bytes));
+    TRY(ensure(ctx, L.stream, L.crop, bytes));
+    memcpy(L.h_crop.p, wins, (size_t)g.nimages * sizeof(CropWin));
+    memcpy((uint8_t *)L.h_crop.p + win_bytes, list.data(), list.size() * sizeof(uint32_t));
+    CK(cudaMemcpyAsync(L.crop.p, L.h_crop.p, bytes, cudaMemcpyHostToDevice, L.stream));
+    ia.crop = (const CropWin *)L.crop.p;
+    ia.strip_list = (const uint32_t *)((const uint8_t *)L.crop.p + win_bytes);
+    ia.nlisted = (uint32_t)list.size();
+    return KPEG_OK;
+}
+
 // Enqueue the whole device pipeline for one job whose stuffed bytes are (or will be, in stream
 // order) at d_scan.  Optimistic: the stages downstream of the relay are issued before it is known
 // whether the pre-issued relay rounds reached the fixed point; job_finish repairs that if not.
 int job_enqueue(kpeg_ctx *ctx, int li, const kpeg_plan *pl, const uint8_t *d_scan, size_t scan_len, uint32_t nimages,
-                uint8_t *d_pixels, std::vector<Copy> d2h, void *tiles_only = nullptr)
+                uint8_t *d_pixels, std::vector<Copy> d2h, void *tiles_only = nullptr, const CropWin *crop = nullptr)
 {
     Lane &L = ctx->lane[li];
     Job &J = L.job;
@@ -585,6 +609,10 @@ int job_enqueue(kpeg_ctx *ctx, int li, const kpeg_plan *pl, const uint8_t *d_sca
         TRY(ensure(ctx, s, L.nrec, (size_t)nsub_max * sizeof(uint32_t)));
         TRY(ensure(ctx, s, L.rec_alt, (size_t)rec_alt_cap * rec_kmax * sizeof(uint32_t)));
     }
+
+    IdctCropArgs crop_ia = {};
+    if (crop) // K2 and K3 will run the listed strips only
+        TRY(upload_crop(ctx, L, g, crop, crop_ia));
 
     J = Job();
     J.use_records = ctx->use_records && ctx->plan_fits_records;
@@ -654,6 +682,14 @@ int job_enqueue(kpeg_ctx *ctx, int li, const kpeg_plan *pl, const uint8_t *d_sca
     xa.g = g;
 
     J.ia = idct_args(ctx, L, g, nstrips, tiles, d_pixels);
+    if (crop) {
+        J.ia.strip_list = xa.strip_list = crop_ia.strip_list;
+        J.ia.nlisted = xa.nlisted = crop_ia.nlisted;
+        J.ia.crop = crop_ia.crop;
+        J.crop = true;
+        J.crop_w = crop[0].w;
+        J.crop_h = crop[0].h;
+    }
 
     launch_entropy_cold(ea, s, &J.launches);
     mark(ctx, L, KPEG_T_ENTROPY_COLD);
@@ -765,10 +801,11 @@ int job_finish(kpeg_ctx *ctx, int li, kpeg_stats *stats)
         TRY(check_guards(ctx));
     ctx->last_lane = li;
     ctx->last_g = J.g;
+    ctx->last_crop = J.crop;
     if (stats) {
         const OutGeom o = out_geom(J.g);
-        stats->width = o.width;
-        stats->height = o.height;
+        stats->width = J.crop ? J.crop_w : o.width;
+        stats->height = J.crop ? J.crop_h : o.height;
         stats->ncomp = J.g.ncomp;
         stats->scan_bytes += J.scan_len;
         stats->unstuffed_bytes += h_meta->total_kept;
@@ -813,16 +850,28 @@ void add_stats(kpeg_stats &to, const kpeg_stats &part)
 // A scan in host memory decoded on lane 0 (which the caller has made idle), complete on return: copied into the lane's
 // scan buffer, then job_enqueue's pixels / d2h / tiles_only and job_finish's stats.
 int decode_host_scan(kpeg_ctx *ctx, const kpeg_plan *pl, const uint8_t *scan, size_t scan_len, uint8_t *d_pixels,
-                     std::vector<Copy> d2h, void *tiles_only, kpeg_stats *stats)
+                     std::vector<Copy> d2h, void *tiles_only, kpeg_stats *stats, const CropWin *crop = nullptr)
 {
     Lane &L = ctx->lane[0];
     TRY(ensure(ctx, L.stream, L.scan, scan_len + 64));
     mark(ctx, L, -1);
     CK(cudaMemcpyAsync(L.scan.p, scan, scan_len, cudaMemcpyHostToDevice, L.stream));
     mark(ctx, L, KPEG_T_H2D);
-    TRY(job_enqueue(ctx, 0, pl, (const uint8_t *)L.scan.p, scan_len, 1, d_pixels, std::move(d2h), tiles_only));
+    TRY(job_enqueue(ctx, 0, pl, (const uint8_t *)L.scan.p, scan_len, 1, d_pixels, std::move(d2h), tiles_only, crop));
     return job_finish(ctx, 0, stats);
 }
+
+// A caller's rectangle, checked against the output image of plan (KPEG_ERR_ARG when empty or not inside it)
+int check_crop(kpeg_ctx *ctx, const kpeg_plan *pl, const kpeg_crop *c)
+{
+    if (!c || !crop_fits(out_of(pl), c->x, c->y, c->width, c->height))
+        return fail(ctx, KPEG_ERR_ARG, "crop rectangle is empty or reaches past the output image");
+    return KPEG_OK;
+}
+
+size_t crop_bytes(const kpeg_crop &c, uint32_t ncomp) { return (size_t)c.width * c.height * ncomp; }
+
+CropWin crop_win(const kpeg_crop &c, uint64_t out_off) { return CropWin{c.x, c.y, c.width, c.height, out_off}; }
 
 // The three scans of a frame coded one scan per component, entropy-decoded one after another on lane 0 into the
 // components' tiles ctx->scan_tiles[c] (nmcu_padded blocks each); their figures are added to *stats.
@@ -1201,6 +1250,35 @@ extern "C" int kpeg_cuda_decode(kpeg_ctx *ctx, const kpeg_plan *plan, const uint
     return decode_host_scan(ctx, plan, scan, scan_len, (uint8_t *)L.pixels.p, {Copy{pixels_out, L.pixels.p, npix}}, nullptr, stats);
 }
 
+extern "C" int kpeg_cuda_decode_crop(kpeg_ctx *ctx, const kpeg_plan *plan, const uint8_t *scan, size_t scan_len,
+                                     const kpeg_crop *crop, uint8_t *pixels_out, kpeg_stats *stats)
+{
+    if (!ctx || !plan || !scan || !pixels_out)
+        return KPEG_ERR_ARG;
+    TRY(check_crop(ctx, plan, crop));
+    CK(cudaSetDevice(ctx->device));
+    zero_stats(stats);
+    Lane &L = idle_lane0(ctx);
+    const size_t npix = crop_bytes(*crop, plan->ncomp);
+    const CropWin win = crop_win(*crop, 0);
+    TRY(ensure(ctx, L.stream, L.pixels, npix + 64));
+    return decode_host_scan(ctx, plan, scan, scan_len, (uint8_t *)L.pixels.p, {Copy{pixels_out, L.pixels.p, npix}}, nullptr, stats, &win);
+}
+
+extern "C" int kpeg_cuda_decode_crop_device(kpeg_ctx *ctx, const kpeg_plan *plan, const uint8_t *d_scan, size_t scan_len,
+                                            const kpeg_crop *crop, uint8_t *d_pixels_out, kpeg_stats *stats)
+{
+    if (!ctx || !plan || !d_scan || !d_pixels_out)
+        return KPEG_ERR_ARG;
+    TRY(check_crop(ctx, plan, crop));
+    CK(cudaSetDevice(ctx->device));
+    zero_stats(stats);
+    const CropWin win = crop_win(*crop, 0);
+    mark(ctx, ctx->lane[0], -1);
+    TRY(job_enqueue(ctx, 0, plan, d_scan, scan_len, 1, d_pixels_out, {}, nullptr, &win));
+    return job_finish(ctx, 0, stats);
+}
+
 // Batch stream format: the n stuffed scans back to back, each followed by one 2-byte RSTn marker
 // (FF D0+(i&7)); to K0 an image boundary is then just another restart boundary.
 extern "C" size_t kpeg_batch_packed_size(int n, const size_t *scan_lens)
@@ -1354,18 +1432,26 @@ extern "C" int kpeg_cuda_decode_batch_device(kpeg_ctx *ctx, const kpeg_plan *pla
 // rotate through the lanes, so copies in, kernels and copies out of different chunks -- and of consecutive
 // submissions -- overlap.  The end-to-end path is bound by the copy out (3 bytes per pixel over PCIe): the
 // point is to keep that copy engine busy from the first chunk to the last.
-extern "C" int kpeg_cuda_submit_batch(kpeg_ctx *ctx, const kpeg_plan *plan, int n, const uint8_t *const *scans,
-                                      const size_t *scan_lens, uint8_t *const *pixels_out)
+namespace {
+
+// crops == nullptr: whole images; otherwise image i's output is its rectangle crops[i] (checked by the caller)
+int submit_batch(kpeg_ctx *ctx, const kpeg_plan *plan, int n, const uint8_t *const *scans, const size_t *scan_lens,
+                 uint8_t *const *pixels_out, const kpeg_crop *crops)
 {
-    if (!ctx || !plan || n <= 0 || !scans || !scan_lens || !pixels_out)
-        return KPEG_ERR_ARG;
     CK(cudaSetDevice(ctx->device));
     const size_t npix = out_of(plan).bytes(); // per output image
+    auto out_bytes = [&](int i) { return crops ? crop_bytes(crops[i], plan->ncomp) : npix; };
+    size_t all_out = npix * (size_t)n;
+    if (crops) {
+        all_out = 0;
+        for (int i = 0; i < n; ++i)
+            all_out += out_bytes(i);
+    }
     // chunking: pipeline only when the pixel traffic is worth it (>= 32 MB); chunks of about 8 MB of pixels
     // or more each, at most host_chunks of them
     int per_chunk = n;
-    if (n >= 2 && npix * (size_t)n >= (32u << 20)) {
-        const int min_imgs = (int)std::max<size_t>(1, (8u << 20) / std::max<size_t>(npix, 1));
+    if (n >= 2 && all_out >= (32u << 20)) {
+        const int min_imgs = (int)std::max<size_t>(1, (8u << 20) / std::max<size_t>(all_out / (size_t)n, 1));
         per_chunk = std::max(min_imgs, (n + ctx->host_chunks - 1) / ctx->host_chunks);
     }
     const int nchunks = (n + per_chunk - 1) / per_chunk;
@@ -1379,8 +1465,12 @@ extern "C" int kpeg_cuda_submit_batch(kpeg_ctx *ctx, const kpeg_plan *plan, int 
         size_t total = 0;
         for (int i = i0; i < i1; ++i)
             total += scan_lens[i] + 2;
+        // where each image's output begins in the chunk's pixel buffer
+        std::vector<size_t> at((size_t)m + 1, 0);
+        for (int i = i0; i < i1; ++i)
+            at[(size_t)(i - i0) + 1] = at[(size_t)(i - i0)] + out_bytes(i);
         TRY(ensure(ctx, L.stream, L.scan, total + 64));
-        TRY(ensure(ctx, L.stream, L.pixels, npix * (size_t)m + 64));
+        TRY(ensure(ctx, L.stream, L.pixels, at[(size_t)m] + 64));
         // Copies in.  A cudaMemcpyAsync costs the host a couple of microseconds whatever its size, so (1) the 2-byte
         // separators are written by a kernel from a table of positions (one small copy per chunk), (2) runs of small
         // scans are gathered in pinned staging memory first and go over as one copy, (3) large scans go straight
@@ -1448,14 +1538,29 @@ extern "C" int kpeg_cuda_submit_batch(kpeg_ctx *ctx, const kpeg_plan *plan, int 
         std::vector<Copy> d2h;
         for (int i = i0; i < i1;) {
             int j = i + 1;
-            while (j < i1 && pixels_out[j] == pixels_out[j - 1] + npix)
+            while (j < i1 && pixels_out[j] == pixels_out[j - 1] + out_bytes(j - 1))
                 ++j;
-            d2h.push_back(Copy{pixels_out[i], (uint8_t *)L.pixels.p + npix * (size_t)(i - i0), npix * (size_t)(j - i)});
+            d2h.push_back(Copy{pixels_out[i], (uint8_t *)L.pixels.p + at[(size_t)(i - i0)], at[(size_t)(j - i0)] - at[(size_t)(i - i0)]});
             i = j;
         }
-        TRY(job_enqueue(ctx, li, plan, (const uint8_t *)L.scan.p, total, (uint32_t)m, (uint8_t *)L.pixels.p, std::move(d2h)));
+        std::vector<CropWin> wins;
+        if (crops)
+            for (int i = i0; i < i1; ++i)
+                wins.push_back(crop_win(crops[i], at[(size_t)(i - i0)]));
+        TRY(job_enqueue(ctx, li, plan, (const uint8_t *)L.scan.p, total, (uint32_t)m, (uint8_t *)L.pixels.p, std::move(d2h), nullptr,
+                        crops ? wins.data() : nullptr));
     }
     return KPEG_OK;
+}
+
+} // namespace
+
+extern "C" int kpeg_cuda_submit_batch(kpeg_ctx *ctx, const kpeg_plan *plan, int n, const uint8_t *const *scans,
+                                      const size_t *scan_lens, uint8_t *const *pixels_out)
+{
+    if (!ctx || !plan || n <= 0 || !scans || !scan_lens || !pixels_out)
+        return KPEG_ERR_ARG;
+    return submit_batch(ctx, plan, n, scans, scan_lens, pixels_out, nullptr);
 }
 
 // Host-pointer batch, complete on return: a submission followed by a wait of its own.
@@ -1469,6 +1574,28 @@ extern "C" int kpeg_cuda_decode_batch(kpeg_ctx *ctx, const kpeg_plan *plan, int 
     const DeferredOutcomeSaved saved(ctx);
     const int rc = kpeg_cuda_submit_batch(ctx, plan, n, scans, scan_lens, pixels_out);
     const int wrc = kpeg_cuda_wait(ctx, stats);
+    return rc != KPEG_OK ? rc : wrc;
+}
+
+// Host-pointer batch of crops, complete on return: kpeg_cuda_decode_batch with a rectangle per image.  Every rectangle is
+// checked before anything is enqueued.
+extern "C" int kpeg_cuda_decode_batch_crop(kpeg_ctx *ctx, const kpeg_plan *plan, int n, const uint8_t *const *scans,
+                                           const size_t *scan_lens, const kpeg_crop *crops, uint8_t *const *pixels_out,
+                                           kpeg_stats *stats)
+{
+    if (!ctx || !plan || n <= 0 || !scans || !scan_lens || !pixels_out || !crops)
+        return KPEG_ERR_ARG;
+    for (int i = 0; i < n; ++i)
+        TRY(check_crop(ctx, plan, &crops[i]));
+    zero_stats(stats);
+    finish_all_deferred(ctx);
+    const DeferredOutcomeSaved saved(ctx);
+    const int rc = submit_batch(ctx, plan, n, scans, scan_lens, pixels_out, crops);
+    const int wrc = kpeg_cuda_wait(ctx, stats);
+    if (stats) {
+        stats->width = crops[0].width;
+        stats->height = crops[0].height;
+    }
     return rc != KPEG_OK ? rc : wrc;
 }
 
@@ -1563,17 +1690,20 @@ extern "C" int kpeg_cuda_interleaved_to_planar(kpeg_ctx *ctx, const uint8_t *d_r
 // K1 and K2 run on it unchanged and leave the component's coefficient tiles (DC prediction and the reference's
 // DC-difference rule included: both are per component); one kernel interleaves the three tile sets into MCU order and
 // K3 runs as for an interleaved file.  Synchronous, on lane 0; not a throughput path.
-extern "C" int kpeg_cuda_decode_scans(kpeg_ctx *ctx, const kpeg_plan *frame, const kpeg_scan *scans, int nscans, const uint8_t *file,
-                                      size_t file_len, uint8_t *pixels_out, kpeg_stats *stats)
+namespace {
+
+// crop == nullptr: the whole output image; otherwise the rectangle *crop of it (checked by the caller)
+int decode_scans(kpeg_ctx *ctx, const kpeg_plan *frame, const kpeg_scan *scans, int nscans, const uint8_t *file, size_t file_len,
+                 uint8_t *pixels_out, const kpeg_crop *crop, kpeg_stats *stats)
 {
-    if (!ctx || !frame || !scans || nscans < 1 || !file || !pixels_out)
-        return KPEG_ERR_ARG;
     for (int k = 0; k < nscans; ++k)
         if (scans[k].off > file_len || scans[k].len > file_len - scans[k].off)
             return fail(ctx, KPEG_ERR_ARG, "scan outside the file");
     if (nscans == 1 && scans[0].plan.ncomp == frame->ncomp) {
         kpeg_plan pl = scans[0].plan;
         pl.flags = frame->flags;
+        if (crop)
+            return kpeg_cuda_decode_crop(ctx, &pl, file + scans[0].off, scans[0].len, crop, pixels_out, stats);
         return kpeg_cuda_decode(ctx, &pl, file + scans[0].off, scans[0].len, pixels_out, stats);
     }
     if (frame->ncomp != 3 || nscans != 3)
@@ -1609,7 +1739,7 @@ extern "C" int kpeg_cuda_decode_scans(kpeg_ctx *ctx, const kpeg_plan *frame, con
     memcpy(fp.ht_present, scans[0].plan.ht_present, sizeof fp.ht_present);
     TRY(upload_plan(ctx, &fp));
     const OutGeom o = out_of(frame);
-    const size_t npix = o.bytes();
+    const size_t npix = crop ? crop_bytes(*crop, 3) : o.bytes();
     TRY(ensure(ctx, s, L.tiles, (size_t)nmcu_padded * 3u * 128u + 256u));
     TRY(ensure(ctx, s, L.pixels, npix + 64));
     TRY(ensure(ctx, s, L.tie_rec, (size_t)nstrips * IDCT_TIE_LIST_CAP * sizeof(uint4)));
@@ -1617,8 +1747,12 @@ extern "C" int kpeg_cuda_decode_scans(kpeg_ctx *ctx, const kpeg_plan *frame, con
     DevMeta *d_meta = (DevMeta *)L.meta.p, *h_meta = (DevMeta *)L.h_meta.p;
     CK(cudaMemsetAsync(d_meta, 0, sizeof(DevMeta), s));
     mark(ctx, L, -1);
+    IdctCropArgs ia = idct_args(ctx, L, g3, nstrips, L.tiles.p, (uint8_t *)L.pixels.p);
+    const CropWin win = crop ? crop_win(*crop, 0) : CropWin{};
+    if (crop)
+        TRY(upload_crop(ctx, L, g3, &win, ia));
     launch_interleave_tiles(ctx->scan_tiles[0].p, ctx->scan_tiles[1].p, ctx->scan_tiles[2].p, L.tiles.p, nmcu_padded, s, &launches);
-    CK(launch_idct(idct_args(ctx, L, g3, nstrips, L.tiles.p, (uint8_t *)L.pixels.p), s, &launches));
+    CK(launch_idct(ia, s, &launches));
     mark(ctx, L, KPEG_T_IDCT);
     CK(cudaMemcpyAsync(pixels_out, L.pixels.p, npix, cudaMemcpyDeviceToHost, s));
     mark(ctx, L, KPEG_T_D2H);
@@ -1629,9 +1763,10 @@ extern "C" int kpeg_cuda_decode_scans(kpeg_ctx *ctx, const kpeg_plan *frame, con
         TRY(check_guards(ctx));
     ctx->last_lane = 0;
     ctx->last_g = g3; // kpeg_cuda_read_coefficients: the interleaved tiles
+    ctx->last_crop = crop != nullptr;
     if (stats) {
-        stats->width = o.width;
-        stats->height = o.height;
+        stats->width = crop ? crop->width : o.width;
+        stats->height = crop ? crop->height : o.height;
         stats->ncomp = 3;
         stats->exact_samples += h_meta->exact_samples;
         stats->kernel_launches += launches;
@@ -1640,11 +1775,10 @@ extern "C" int kpeg_cuda_decode_scans(kpeg_ctx *ctx, const kpeg_plan *frame, con
     return KPEG_OK;
 }
 
-extern "C" int kpeg_cuda_decode_file(kpeg_ctx *ctx, const uint8_t *file, size_t len, uint32_t flags, uint8_t *pixels_out,
-                                     size_t cap, kpeg_plan *plan_out, kpeg_stats *stats)
+// the rectangle *crop of a file's output (nullptr: all of it), through decode_scans
+int decode_file(kpeg_ctx *ctx, const uint8_t *file, size_t len, uint32_t flags, const kpeg_crop *crop, uint8_t *pixels_out,
+                size_t cap, kpeg_plan *plan_out, kpeg_stats *stats)
 {
-    if (!ctx || !file || !pixels_out)
-        return KPEG_ERR_ARG;
     kpeg_plan frame;
     kpeg_scan scans[KPEG_MAX_SCANS];
     int nscans = 0;
@@ -1654,9 +1788,37 @@ extern "C" int kpeg_cuda_decode_file(kpeg_ctx *ctx, const uint8_t *file, size_t 
     frame.flags = flags;
     if (plan_out)
         *plan_out = frame;
-    if (out_of(&frame).bytes() > cap)
+    if (crop)
+        TRY(check_crop(ctx, &frame, crop));
+    if ((crop ? crop_bytes(*crop, frame.ncomp) : out_of(&frame).bytes()) > cap)
         return fail(ctx, KPEG_ERR_ARG, "pixel buffer too small");
-    return kpeg_cuda_decode_scans(ctx, &frame, scans, nscans, file, len, pixels_out, stats);
+    return decode_scans(ctx, &frame, scans, nscans, file, len, pixels_out, crop, stats);
+}
+
+} // namespace
+
+extern "C" int kpeg_cuda_decode_scans(kpeg_ctx *ctx, const kpeg_plan *frame, const kpeg_scan *scans, int nscans, const uint8_t *file,
+                                      size_t file_len, uint8_t *pixels_out, kpeg_stats *stats)
+{
+    if (!ctx || !frame || !scans || nscans < 1 || !file || !pixels_out)
+        return KPEG_ERR_ARG;
+    return decode_scans(ctx, frame, scans, nscans, file, file_len, pixels_out, nullptr, stats);
+}
+
+extern "C" int kpeg_cuda_decode_file(kpeg_ctx *ctx, const uint8_t *file, size_t len, uint32_t flags, uint8_t *pixels_out,
+                                     size_t cap, kpeg_plan *plan_out, kpeg_stats *stats)
+{
+    if (!ctx || !file || !pixels_out)
+        return KPEG_ERR_ARG;
+    return decode_file(ctx, file, len, flags, nullptr, pixels_out, cap, plan_out, stats);
+}
+
+extern "C" int kpeg_cuda_decode_file_crop(kpeg_ctx *ctx, const uint8_t *file, size_t len, uint32_t flags, const kpeg_crop *crop,
+                                          uint8_t *pixels_out, size_t cap, kpeg_plan *plan_out, kpeg_stats *stats)
+{
+    if (!ctx || !file || !pixels_out || !crop)
+        return KPEG_ERR_ARG;
+    return decode_file(ctx, file, len, flags, crop, pixels_out, cap, plan_out, stats);
 }
 
 // Any mix of files.  Files with identical plans (dimensions, tables, restart interval) travel together as ONE batch --
@@ -1802,6 +1964,8 @@ extern "C" int kpeg_cuda_read_coefficients(kpeg_ctx *ctx, int16_t *out, size_t c
     Lane &L = ctx->lane[ctx->last_lane];
     if (L.job.active)
         return fail(ctx, KPEG_ERR_ARG, "the lane of the last decode is busy with a deferred submission");
+    if (ctx->last_crop)
+        return fail(ctx, KPEG_ERR_UNSUPPORTED, "the last decode was a crop: it left the coefficients of the listed strips only");
     const size_t n = (size_t)ctx->last_g.total_blocks * 64u;
     if (cap < n)
         return fail(ctx, KPEG_ERR_ARG, "coefficient buffer too small");

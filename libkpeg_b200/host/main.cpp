@@ -19,6 +19,8 @@
 //   --devices L  several devices, e.g. 0-7 or 0,2,3: the restart-interval tiles of the image are spread over them
 //   --scale 1/N  decode: N = 2, 4 or 8 writes <file>.ppm at 1/N the size (KPEG_FLAG_SCALE_*: libjpeg's reduced IDCTs and
 //                integer colour, as djpeg -scale 1/N); 1/1 or no --scale is the full-size decode of the drop-in JPEGDecoder
+//   --crop WxH+X+Y  decode: <file>.ppm holds only that rectangle of the output image (after --scale), exactly (djpeg -crop
+//                widens it to iMCU boundaries; this does not); kpeg_cuda_decode_file_crop
 //   --quiet      log only to kpeg.log
 #include <algorithm>
 #include <cctype>
@@ -50,6 +52,7 @@ namespace
         std::cout << "<in.jpg> <out.jpg>              : Transcode a baseline JPEG losslessly on the GPU" << std::endl;
         std::cout << "--transform T                   : Transcode: none, flip-h, flip-v, transpose, transverse, rot90, rot180, rot270" << std::endl;
         std::cout << "--scale 1/N                     : Decode at 1/2, 1/4 or 1/8 the size (libjpeg's reduced IDCTs)" << std::endl;
+        std::cout << "--crop WxH+X+Y                  : Decode only that rectangle of the (scaled) image" << std::endl;
         std::cout << "-h                              : Print this help message and exit" << std::endl;
     }
 
@@ -71,7 +74,29 @@ namespace
         bool optimize = false;
         std::string transform = "none";
         std::string scale = "1/1";
+        bool crop_given = false;
+        kpeg_crop crop = {};
     };
+
+    // "WxH+X+Y" (djpeg's -crop syntax; every part required, decimal) -> crop; false when malformed
+    bool parseCrop( const std::string& s, kpeg_crop& c )
+    {
+        unsigned long v[4];
+        const char seps[4] = { 'x', '+', '+', '\0' };
+        std::size_t i = 0;
+        for ( int k = 0; k < 4; ++k )
+        {
+            const std::size_t j = i;
+            while ( i < s.size() && std::isdigit( (unsigned char)s[i] ) ) ++i;
+            if ( i == j || i - j > 10 ) return false;
+            v[k] = std::stoul( s.substr( j, i - j ) );
+            if ( v[k] > 0xFFFFFFFFul ) return false;
+            if ( k < 3 ) { if ( i >= s.size() || s[i] != seps[k] ) return false; ++i; }
+        }
+        if ( i != s.size() || v[0] == 0 || v[1] == 0 ) return false;
+        c.width = (uint32_t)v[0]; c.height = (uint32_t)v[1]; c.x = (uint32_t)v[2]; c.y = (uint32_t)v[3];
+        return true;
+    }
 
     // "0-3", "0,2,5", "1": device list of --devices
     std::vector<int> parseDevices( const std::string& s )
@@ -260,8 +285,9 @@ namespace
                                        << "): " << len << " bytes";
     }
 
-    // --scale 2, 4, 8: the reduced-size decode through the C ABI (the drop-in JPEGDecoder has the reference's interface,
-    // which has no scale), written as dumpRawData writes the full-size image: <name up to ".jpg">.ppm, P6, gray as R = G = B
+    // --scale 2, 4, 8 and --crop: the reduced-size or cropped decode through the C ABI (the drop-in JPEGDecoder has the
+    // reference's interface, which has neither), written as dumpRawData writes the full-size image: <name up to ".jpg">.ppm,
+    // P6, gray as R = G = B
     void decodeScaled( const std::string& filename, const Options& opt, uint32_t scaleFlag )
     {
         std::vector<uint8_t> data;
@@ -281,7 +307,19 @@ namespace
         const uint32_t flags = ( opt.parity ? KPEG_FLAG_REF_PARITY : 0u ) | scaleFlag;
         frame.flags = flags;
         uint32_t w = 0, h = 0;
-        std::vector<uint8_t> pixels( kpeg_output_size( &frame, &w, &h ) );
+        size_t bytes = kpeg_output_size( &frame, &w, &h );
+        if ( opt.crop_given )
+        {
+            if ( !opt.devices.empty() )
+            {
+                LOG(kpeg::Logger::Level::ERROR) << "--crop decodes on one device (no --devices).";
+                return;
+            }
+            w = opt.crop.width;
+            h = opt.crop.height;
+            bytes = (size_t)w * h * frame.ncomp;
+        }
+        std::vector<uint8_t> pixels( bytes );
         int rc;
         std::string err;
         if ( !opt.devices.empty() )
@@ -296,7 +334,9 @@ namespace
             rc = kpeg_cuda_acquire( opt.device, &ctx );
             if ( rc == KPEG_OK )
             {
-                rc = kpeg_cuda_decode_file( ctx, data.data(), data.size(), flags, pixels.data(), pixels.size(), nullptr, nullptr );
+                rc = opt.crop_given ? kpeg_cuda_decode_file_crop( ctx, data.data(), data.size(), flags, &opt.crop, pixels.data(), pixels.size(),
+                                                                  nullptr, nullptr )
+                                    : kpeg_cuda_decode_file( ctx, data.data(), data.size(), flags, pixels.data(), pixels.size(), nullptr, nullptr );
                 err = kpeg_cuda_last_error( ctx );
                 kpeg_cuda_release( opt.device, ctx );
             }
@@ -328,7 +368,7 @@ namespace
             LOG(kpeg::Logger::Level::ERROR) << "Unable to create dump file \'" << target << "\'.";
             return;
         }
-        LOG(kpeg::Logger::Level::INFO) << "Decoded " << filename << " at " << opt.scale << " (" << w << "x" << h
+        LOG(kpeg::Logger::Level::INFO) << "Decoded " << filename << " at " << opt.scale << ( opt.crop_given ? ", cropped" : "" ) << " (" << w << "x" << h
                                        << "): raw image data dumped to file: \'" << target << "\'.";
     }
 
@@ -348,7 +388,7 @@ namespace
             LOG(kpeg::Logger::Level::ERROR) << "Unknown scale '" << opt.scale << "' (1/1, 1/2, 1/4 or 1/8).";
             return;
         }
-        if ( code > 0 )
+        if ( code > 0 || opt.crop_given )
         {
             decodeScaled( filename, opt, (uint32_t)code * KPEG_FLAG_SCALE_1_2 );
             return;
@@ -385,6 +425,17 @@ int main( int argc, char** argv )
             else if ( a == "--transform" && i + 1 < argc ) opt.transform = argv[++i];
             else if ( a == "--optimize" ) opt.optimize = true;
             else if ( a == "--scale" && i + 1 < argc ) opt.scale = argv[++i];
+            else if ( a == "--crop" )
+            {
+                if ( i + 1 >= argc || !parseCrop( argv[i + 1], opt.crop ) )
+                {
+                    std::cout << "Malformed --crop '" << ( i + 1 < argc ? argv[i + 1] : "" ) << "': expected WxH+X+Y, e.g. 224x224+16+8" << std::endl;
+                    printHelp();
+                    return EXIT_FAILURE;
+                }
+                opt.crop_given = true;
+                ++i;
+            }
             else args.push_back( a );
         }
 
